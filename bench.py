@@ -2,7 +2,7 @@
 """Benchmark of the per-gene-cluster k-mer streaming hot path (BASELINE.json).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
-                    [--config 2|3|4|5] [--extra 3,4,5 | --no-extra]
+                    [--config 2|3|4|5] [--extra 3,4,5 | --no-extra] [--dump-outputs DIR]
 
 Headline (default `--config 2`): a step = one pass of K1..K4 over the whole synthetic
 pangenome of BASELINE.json configs[1] (500 genomes x 4,000 gene clusters, 1.2 kb cut sequences,
@@ -18,6 +18,11 @@ sample a --targets strain), #4 10,000 genomes x 5,000 clusters sharded over the 
 (strong scaling), #5 50,000 genomes x 8,000 clusters with the cluster-absent encoding,
 1,000 clusters per rank (the full config at N = 8), each with ONE global pattern exchange at
 the end of the run, as a real run does.
+
+`--steps K` is the number of timed steps of the headline: K executions of the resident batch,
+or K passes over all batches when the headline config is streamed.  `--dump-outputs DIR` then
+writes what the last of them computed (rows, pattern bits, per-cluster sums) to DIR as .npy
+files (class OutputDump); the inputs are seeded, so two builds can be compared on them.
 
 `--impl reference` times the UNMODIFIED reference's own hot functions (cluster_cutter +
 pattern_hasher of oracle/_ref/panfeed/panfeed.py, installed from /root/reference by
@@ -85,7 +90,13 @@ def parse():
     p.add_argument("--no-e2e", action="store_true")
     p.add_argument("--no-selfcheck", action="store_true")
     p.add_argument("--cpu-seconds", type=float, default=15.0)
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="after the timed steps, write what the last step computed to DIR/<name>.npy "
+                        "(float64, at most 64 MB in all; see OutputDump)")
+    args = p.parse_args()
+    if args.steps < 1:
+        p.error("--steps must be at least 1")
+    return args
 
 
 def config_of(args, cid):
@@ -464,6 +475,137 @@ def workload_config(cfg, world):
 
 
 # --------------------------------------------------------------------------
+# --dump-outputs
+# --------------------------------------------------------------------------
+DUMP_BYTES = 64 * 10 ** 6
+DUMP_SEED = 0x5EED5EED
+
+
+def _mix64(x):
+    """splitmix64 finaliser of a uint64 array."""
+    with np.errstate(over="ignore"):
+        x = x + np.uint64(0x9E3779B97F4A7C15)
+        x = (x ^ (x >> np.uint64(30))) * np.uint64(0xBF58476D1CE4E5B9)
+        x = (x ^ (x >> np.uint64(27))) * np.uint64(0x94D049BB133111EB)
+        return x ^ (x >> np.uint64(31))
+
+
+def _halves(x):
+    """uint64 -> (high, low) 32-bit halves, each exact in float64."""
+    return x >> np.uint64(32), x & np.uint64(0xFFFFFFFF)
+
+
+class OutputDump:
+    """What the timed path computed in its last step, as pf_collect hands it to a caller, written
+    so that two builds can be compared array for array.  All arrays are float64 holding exact
+    integers.  Pattern ids are numbered in discovery order, so each row carries the bits of its
+    pattern instead, and rows are sorted by (cluster, k-mer).
+
+      row_cluster [m]         global cluster id of the row
+      row_kmer [m, 4]         the k-mer as 32-bit words (k <= 32: the first two are 0)
+      row_count [m]           samples that carry the k-mer
+      row_pattern_bits [m, W] its presence bitset, 32 samples a word
+      cluster_id, cluster_rows, cluster_count_sum, cluster_samples [clusters]
+                              every cluster: its rows, the sum of their counts, the popcount of
+                              its cluster pattern
+      totals [4]              rows, new k-mer patterns, new cluster patterns, positional records
+
+    m is every row when they fit DUMP_BYTES; otherwise a fixed sample: the rows with the smallest
+    seeded hash of (cluster, k-mer).  That sample depends on neither the row order nor on how the
+    step was split into batches."""
+
+    def __init__(self, n_samples, n_clusters):
+        self.W = (n_samples + 31) // 32
+        per_row = 8 * (1 + 4 + 1 + self.W)
+        self.m = max(1, (DUMP_BYTES - 8 * (4 * n_clusters + 4) - 4096) // per_row)
+        self.rows = None
+        self.clusters = []
+        self.totals = np.zeros(4, np.float64)
+
+    @staticmethod
+    def _bits(ctx, r, ns, ids, width):
+        """Bits of pattern ids: this batch's new patterns from the result, older ones exported
+        from the context's table."""
+        key = "new_cluster_patterns" if ns else "new_kmer_patterns"
+        base = r["cluster_pattern_base" if ns else "kmer_pattern_base"]
+        ids = ids.astype(np.int64)
+        out = np.zeros((len(ids), width), np.uint32)
+        new = ids >= base
+        out[new] = r[key][ids[new] - base][:, :width]
+        if not new.all():
+            old, inv = np.unique(ids[~new], return_inverse=True)
+            table = np.stack([ctx.export_patterns(ns, i, 1)[0, :width] for i in old.tolist()])
+            out[~new] = table[inv]
+        return out
+
+    def add(self, r, hb, ctx):
+        """One collected batch (the result views are read here, not kept)."""
+        narrow, wide = len(r["row_cluster"]), len(r["wide_row_cluster"])
+        cl = np.concatenate([r["row_cluster"], r["wide_row_cluster"]]).astype(np.uint64)    # cluster ids
+        k0 = np.concatenate([np.zeros(narrow, np.uint64), r["wide_row_kmer"][:, 0]])
+        k1 = np.concatenate([r["row_kmer"], r["wide_row_kmer"][:, 1]])
+        count = np.concatenate([r["row_count"], r["wide_row_count"]])
+        pid = np.concatenate([r["row_pattern"], r["wide_row_pattern"]])
+        cid = hb.clusters["id"].astype(np.uint64)      # cluster_pattern is in this (batch) order
+        nc = len(cid)
+        by_id = np.argsort(cid, kind="stable")
+        local = by_id[np.searchsorted(cid[by_id], cl)]
+
+        cbits = self._bits(ctx, r, 1, r["cluster_pattern"], self.W)
+        self.clusters.append(np.stack([
+            cid.astype(np.float64),
+            np.bincount(local, minlength=nc).astype(np.float64),
+            np.bincount(local, weights=count.astype(np.float64), minlength=nc),
+            np.unpackbits(cbits.view(np.uint8), axis=1).sum(axis=1).astype(np.float64)], axis=1))
+        self.totals += [narrow + wide, len(r["new_kmer_patterns"]), len(r["new_cluster_patterns"]), r["n_pos"]]
+
+        h = _mix64(_mix64(_mix64(cl ^ np.uint64(DUMP_SEED)) ^ k0) ^ k1)
+        if self.rows is not None and len(self.rows["h"]) >= self.m:
+            sel = np.flatnonzero(h <= self.rows["h"].max())
+        else:
+            sel = np.arange(len(h))
+        if len(sel) > self.m:
+            sel = sel[np.argpartition(h[sel], self.m - 1)[:self.m]]
+        batch = {"h": h[sel], "cl": cl[sel], "k0": k0[sel], "k1": k1[sel], "count": count[sel],
+                 "bits": self._bits(ctx, r, 0, pid[sel], self.W)}
+        if self.rows is not None:
+            batch = {n: np.concatenate([self.rows[n], batch[n]]) for n in batch}
+        if len(batch["h"]) > self.m:
+            keep = batch["h"] <= np.partition(batch["h"], self.m - 1)[self.m - 1]
+            batch = {n: a[keep] for n, a in batch.items()}
+        self.rows = batch
+
+    def write(self, out_dir):
+        """DIR/<name>.npy for every array; returns {name: shape} and the bytes written."""
+        rows = self.rows
+        if len(rows["h"]) > self.m:            # hash ties at the cut: keep the smallest keys
+            o = np.lexsort((rows["k1"], rows["k0"], rows["cl"], rows["h"]))[:self.m]
+            rows = {n: a[o] for n, a in rows.items()}
+        o = np.lexsort((rows["k1"], rows["k0"], rows["cl"]))
+        clusters = np.concatenate(self.clusters)
+        clusters = clusters[np.argsort(clusters[:, 0], kind="stable")]
+        arrays = {
+            "row_cluster": rows["cl"][o],
+            "row_kmer": np.stack(_halves(rows["k0"][o]) + _halves(rows["k1"][o]), axis=1),
+            "row_count": rows["count"][o],
+            "row_pattern_bits": rows["bits"][o],
+            "cluster_id": clusters[:, 0], "cluster_rows": clusters[:, 1],
+            "cluster_count_sum": clusters[:, 2], "cluster_samples": clusters[:, 3],
+            "totals": self.totals,
+        }
+        os.makedirs(out_dir, exist_ok=True)
+        shapes, nbytes = {}, 0
+        for name, a in arrays.items():
+            a = np.ascontiguousarray(a, dtype=np.float64)
+            np.save(os.path.join(out_dir, name + ".npy"), a)
+            shapes[name] = list(a.shape)
+            nbytes += a.nbytes
+        assert nbytes <= DUMP_BYTES, nbytes
+        return {"dir": out_dir, "arrays": shapes, "bytes": nbytes,
+                "rows_sampled": bool(len(o) < self.totals[0])}
+
+
+# --------------------------------------------------------------------------
 # B200 arm
 # --------------------------------------------------------------------------
 class Env:
@@ -572,7 +714,7 @@ def h2d_bytes(hb):
 STAGE_KEYS = ("ms_extract", "ms_hist", "ms_sort", "ms_mark", "ms_count", "ms_reduce", "ms_dedup", "ms_total")
 
 
-def run_streamed(cfg, env, args, passes=1, warm_passes=1):
+def run_streamed(cfg, env, args, passes=1, warm_passes=1, dump=None):
     """One BASELINE config at FULL size, batch after batch (the inputs of configs 4 / 5 do not
     fit the host comfortably and a run of the product streams batches anyway).  Per pass:
       resident  pf_upload (untimed) + pf_execute timed with the library's CUDA events on the
@@ -581,7 +723,8 @@ def run_streamed(cfg, env, args, passes=1, warm_passes=1):
                 clock, summed over the batches;
     both followed by ONE global pattern exchange (N > 1), as in a real run.  The batches come
     from pf_synth_fill (bases generated on the device, copied to reused pinned host buffers)
-    outside the timed regions."""
+    outside the timed regions.  `dump` (an OutputDump) is given the results of every batch of
+    the last resident pass."""
     from panfeed_b200 import capi
     torch = env.torch
     first, n_cl, total = rank_clusters(cfg, env)
@@ -639,6 +782,8 @@ def run_streamed(cfg, env, args, passes=1, warm_passes=1):
                     for k_ in STAGE_KEYS:
                         tot["stages"][k_] += st[k_]
                     r = ctx.collect(copy=False)
+                    if dump is not None and pass_i == warm_passes + passes - 1:
+                        dump.add(r, hb, ctx)
                 else:
                     t0 = time.perf_counter()
                     ctx.submit(hb)
@@ -774,10 +919,13 @@ def main():
             extra_ids = [3, 4, 5]
 
     if cfg["id"] != 2 or cfg["batch"] < cfg["clusters"]:
-        # a streamed config as the headline: K passes over all its batches
+        # a streamed config as the headline: K = --steps passes over all its batches
+        dump = None
+        if args.dump_outputs and rank == 0:
+            dump = OutputDump(cfg["samples"], rank_clusters(cfg, env)[1])
         sampler = ClockSampler(local, period=0.05)
         sampler.start()
-        r = run_streamed(cfg, env, args, passes=max(1, min(args.steps, 3)), warm_passes=max(1, min(args.warmup, 3)))
+        r = run_streamed(cfg, env, args, passes=args.steps, warm_passes=max(1, min(args.warmup, 3)), dump=dump)
         clocks = sampler.stop()
         if rank == 0:
             e2e = r.get("e2e")
@@ -791,6 +939,8 @@ def main():
                         "value": e2e["bases_per_s"], "unit": "bases/s", "ms_per_step": e2e["ms"],
                         "h2d_bytes_per_step": e2e["h2d_bytes"], "d2h_bytes_per_step": e2e["d2h_bytes"]},
                     "roofline": None, "exchange_selfcheck": selfcheck, "affinity": env.affinity}
+            if dump is not None:
+                line["dump_outputs"] = dump.write(args.dump_outputs)
             emit(line)
         if world > 1:
             dist.barrier()
@@ -853,7 +1003,12 @@ def main():
     total_bases = env.reduce(n_bases, "sum")
     value = total_bases / (ms_step * 1e-3)
     # sizes of one step: read from a collect of the last execution
-    ctx.collect(copy=False)
+    r = ctx.collect(copy=False)
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        dump = OutputDump(S, C)
+        dump.add(r, hb, ctx)
+        dumped = dump.write(args.dump_outputs)
     st = ctx.stats()
     M = st["instances"]             # exactly one collected batch so far
     U = st["unique_kmers"]
@@ -924,6 +1079,8 @@ def main():
         line["affinity"] = env.affinity
         if extra:
             line["extra_configs"] = extra
+        if dumped is not None:
+            line["dump_outputs"] = dumped
         if not args.no_cpu_baseline and world == 1:      # reported at N = 1 only
             line["cpu_baseline"] = cpu_baseline_c(hb, S, k, cfg["maf"], cfg["cm"], args.cpu_seconds)
         emit(line)

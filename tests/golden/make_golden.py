@@ -7,7 +7,8 @@ test-only pyfaidx stand-in on PYTHONPATH, once per argument combination of
 pangenome written by make_fixture.py, and stores the three output files
 gzip-compressed under tests/golden/expected/<mode>/.  Also writes
 hot_kats.json: known answers obtained by calling the reference's
-`cluster_cutter` / `pattern_hasher` directly (panfeed.py:23-235).
+`cluster_cutter` / `pattern_hasher` directly (panfeed.py:23-235), and
+cli_options.json: the reference's parsed command line with every default.
 
 This only works in the build container (needs /root/reference).  The outputs
 are committed; the GPU box and the tests read the committed files only.
@@ -197,6 +198,26 @@ def hot_kats():
     print("hot_kats ok")
 
 
+def cli_options():
+    """The reference's parsed command line (vars(get_options()), __main__.py:84-223) for the
+    two required options only: every destination with its default."""
+    argv = ["-g", "x", "-p", "y"]
+    code = ("import sys, json; sys.argv = ['panfeed'] + json.loads(sys.argv[1]); "
+            "from panfeed.__main__ import get_options; print(json.dumps(vars(get_options())))")
+    env = dict(os.environ, PYTHONPATH=STANDIN + os.pathsep + REF)
+    r = subprocess.run([sys.executable, "-c", code, json.dumps(argv)], env=env,
+                       capture_output=True, text=True, check=True)
+    options = json.loads(r.stdout.strip().splitlines()[-1])
+    doc = {"argv": argv,
+           "source": "vars(get_options()) of the unmodified reference's panfeed/__main__.py "
+                     "for `panfeed -g x -p y`",
+           "options": dict(sorted(options.items()))}
+    with open(os.path.join(HERE, "expected", "cli_options.json"), "w") as fh:
+        json.dump(doc, fh, indent=1)
+        fh.write("\n")
+    print("cli_options ok")
+
+
 if __name__ == "__main__":
     if not os.path.isdir(os.path.join(HERE, "fixture")):
         sys.path.insert(0, HERE)
@@ -204,3 +225,4 @@ if __name__ == "__main__":
         make_fixture.build(os.path.join(HERE, "fixture"))
     run_modes()
     hot_kats()
+    cli_options()

@@ -25,6 +25,12 @@ def hot_kats():
         return json.load(fh)
 
 
+def cli_options():
+    """The reference's parsed command line for a minimal argument list: {"argv", "options"}."""
+    with open(os.path.join(EXPECTED, "cli_options.json")) as fh:
+        return json.load(fh)
+
+
 def cli_kwargs(args):
     """Translate a reference-style argument list into keyword arguments
     (options of /root/reference/panfeed/__main__.py:84-223)."""

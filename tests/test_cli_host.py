@@ -127,22 +127,15 @@ def test_cli_stop_on_missing_raises(feeder, tmp_path, monkeypatch):
     assert os.path.getsize(os.path.join(str(tmp_path / "out2"), "kmers_to_hashes.tsv")) > 100
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/panfeed"), reason="needs the reference tree (build container)")
 def test_cli_options_and_defaults_are_the_references():
-    """Every option of the reference's command line (`/root/reference/panfeed/__main__.py:84-223`)
-    exists here with the same destination and default; only --device and the feeder switches
-    are new.  (Runs where the reference tree is; the GPU box has no /root/reference.)"""
-    import subprocess
-    import sys
-    code = ("import sys, json; sys.argv = ['panfeed', '-g', 'x', '-p', 'y']; "
-            "from panfeed.__main__ import get_options; print(json.dumps(vars(get_options())))")
-    env = dict(os.environ, PYTHONPATH=os.path.join(helpers.GOLDEN, "pyfaidx_standin") + os.pathsep + "/root/reference")
-    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, env=env)
-    assert r.returncode == 0, r.stderr[-2000:]
-    import json
-    ref = json.loads(r.stdout.strip().splitlines()[-1])
+    """Every option of the reference's command line (`panfeed/__main__.py:84-223`) exists here
+    with the same destination and default; only --device and the feeder switches are new.  The
+    reference's parsed options are stored in tests/golden/expected/cli_options.json
+    (tests/golden/make_golden.py)."""
+    gold = helpers.cli_options()
+    ref = gold["options"]
     from panfeed_b200.__main__ import get_options
-    ours = vars(get_options(["-g", "x", "-p", "y"]))
+    ours = vars(get_options(gold["argv"]))
     assert len(ref) >= 20
     for name, default in ref.items():
         assert name in ours, name
