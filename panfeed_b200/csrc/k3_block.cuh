@@ -5,7 +5,11 @@
 // a few hundred distinct k-mers between them (one per haplotype and position), however many
 // samples there are.
 //
-//   kA_block_aggregate  one CTA per (cluster, run of 16 window positions[, slice of 512 samples]).
+//   kA_block_aggregate  work item: (cluster, run of 16 window positions[, slice of 512 samples]).
+//                       A CTA walks a SEGMENT of consecutive runs of one (cluster, slice): it
+//                       keeps its sequences' descriptors and words in registers from run to
+//                       run (one new 64-bit word per sequence every second run) and undoes
+//                       only what a run touched in its tables.
 //                       Level 1: every sequence contributes the R = k + 15 bases its 16
 //                       windows cover as ONE 128-bit chunk; identical chunks (same haplotype)
 //                       meet in a shared-memory chunk table and only OR one sample bit there:
@@ -15,7 +19,8 @@
 //                       a shared-memory open-addressing table and takes the chunk's whole
 //                       W-word sample bitset.  The CTA ends by writing its distinct k-mers,
 //                       bitsets and popcounts ("partial rows") to a slab in HBM: ~1/30 of the
-//                       bytes the records would have taken, written once.
+//                       bytes the records would have taken, written once.  Every run keeps
+//                       its own slab, so the kernels after kA see per-run items.
 //   kB1/kB3             a k-mer can start in two runs (indels, clamped flanks, paralogs,
 //                       repeats), so the partial rows of one cluster are merged by FULL key in a
 //                       per-cluster open-addressing table in global memory: the first row of a
@@ -226,7 +231,7 @@ __global__ void plan_item_desc(const uint32_t* __restrict__ item_base, const uin
 // shared-memory table
 // ---------------------------------------------------------------------------
 struct BlkHead {           // 64 bytes at the start of kA's shared memory (see ARunView)
-  uint32_t n_unique, overflow, n_pass, row_base, ok, work, pad[10];
+  uint32_t n_unique, overflow, n_pass, row_base, ok, work, seg[2], pad[8];
 };
 __device__ __forceinline__ uint32_t ld_volatile_shared(const uint32_t* p) {
   return *reinterpret_cast<const volatile uint32_t*>(p);
@@ -253,11 +258,15 @@ struct BlkPlan {
   uint32_t slice_samples;        // multiple of 32
   const uint32_t* slice_seq;     // [n_clusters][n_slices + 1] first sequence (cluster-relative) of every slice
   const uint4* item_desc;        // [n_items * n_slices] {first seq, end seq (absolute), first window, cluster}
+  uint32_t n_run_items;          // (cluster, run) items of the batch
 };
 
-// Shared memory of kA.  Both tables hand out DENSE row ids on insertion and the inserting
-// thread clears its row before publishing the id, so nothing but the (small) key / state
-// arrays is initialised per block and the epilogue needs no compaction pass.
+// Shared memory of kA.  Both tables hand out DENSE row ids on insertion, so the epilogue needs
+// no compaction pass.  The tables are cleared once per CTA; after a run only what it touched is
+// undone: the key slot of every k-mer row (rslot) and the state slot of every chunk id (cslot)
+// are recorded on insertion, the pool rows are zeroed as they are copied out, and the chunk rows
+// 0..n_chunks-1 are cleared.  An overflowing run may have claimed slots without a row; after it
+// everything is cleared.
 //
 // chunk table: the R = k + 15 bases that the 16 windows of a run cover, as a 128-bit key
 //   (top-aligned).  Sequences of a cluster are copies of a few haplotypes, so the ~500
@@ -277,6 +286,8 @@ struct ARunView {
   uint32_t* crows;         // [ccap * WS]
   uint16_t* rowid;         // [slots]
   uint16_t* cmeta;         // [ccap]  low byte: bitset word of the chunk's first sample; bit 15: other words too
+  uint16_t* rslot;         // [cap + 1]  key slot of row id
+  uint16_t* cslot;         // [ccap]     state slot of chunk id
   uint32_t mask, shift, cmask, cshift, cap, ccap;
 };
 __host__ __device__ inline uint32_t blkA_ccap(uint32_t cslots) { return cslots * 3u / 4u; }
@@ -284,7 +295,7 @@ __host__ __device__ inline uint32_t blkA_ccap(uint32_t cslots) { return cslots *
 __host__ __device__ inline uint32_t blkA_smem_bytes(uint32_t slots, uint32_t cap, uint32_t cslots, uint32_t W) {
   const uint32_t ccap = blkA_ccap(cslots), WS = W | 1u;
   return (uint32_t)sizeof(BlkHead) + slots * 8u + (cap + 1u) * 8u + ccap * 16u + cslots * 4u +
-         (cap + 1u) * WS * 4u + ccap * WS * 4u + slots * 2u + ccap * 2u + 16u;
+         (cap + 1u) * WS * 4u + ccap * WS * 4u + slots * 2u + ccap * 2u + (cap + 1u) * 2u + ccap * 2u + 16u;
 }
 __device__ __forceinline__ ARunView arun_view(unsigned char* raw, uint32_t slots, uint32_t cap, uint32_t cslots, uint32_t W) {
   ARunView a;
@@ -301,6 +312,8 @@ __device__ __forceinline__ ARunView arun_view(unsigned char* raw, uint32_t slots
   a.crows = a.pool + (a.cap + 1u) * WS;
   a.rowid = reinterpret_cast<uint16_t*>(a.crows + a.ccap * WS);
   a.cmeta = a.rowid + slots;
+  a.rslot = a.cmeta + a.ccap;
+  a.cslot = a.rslot + (a.cap + 1u);
   a.mask = slots - 1u;
   a.shift = 32u - (uint32_t)__popc(a.mask);
   a.cmask = cslots - 1u;
@@ -332,6 +345,7 @@ __device__ __noinline__ uint32_t chunk_find_or_insert(const ARunView a, uint64_t
           return 0xffffffffu;
         }
         a.cmeta[id] = (uint16_t)wofs;
+        a.cslot[id] = (uint16_t)s;
         *reinterpret_cast<volatile uint64_t*>(&a.ckhi[id]) = hi;
         *reinterpret_cast<volatile uint64_t*>(&a.cklo[id]) = lo;
         __threadfence_block();
@@ -356,6 +370,7 @@ __device__ __noinline__ uint32_t kmer_row_slow(const ARunView a, uint64_t key, u
       if (cur == ~0ull) {                                     // this thread owns the new slot
         uint32_t id = atomicAdd(&a.h->n_unique, 1u);
         if (id >= a.cap) { a.h->overflow = 1u; id = a.cap; }
+        else a.rslot[id] = (uint16_t)h;
         a.rkey[id] = key;
         __threadfence_block();
         *reinterpret_cast<volatile uint16_t*>(&a.rowid[h]) = (uint16_t)id;
@@ -378,6 +393,12 @@ __device__ __noinline__ uint32_t kmer_row_slow(const ARunView a, uint64_t key, u
 #ifndef PF_KA_MIN_CTAS
 #define PF_KA_MIN_CTAS 4
 #endif
+// A CTA walks SEGMENTS: `seg_runs` consecutive (cluster, run) items of one slice (item =
+// run_item * n_slices + slice), taken from counters[LC_SEGMENT] after the first one; with an
+// item list (a rescue launch) a segment is one listed item.  Every run still gets its own slab.
+// Across the runs of a segment a thread keeps its first two sequences of the (cluster, slice) in
+// registers: descriptor and the 64-bit words wi, wi + 1 of the run plus wi + 2, requested a run
+// ahead of its use.  A run starts at a multiple of 16, so its R <= 47 bases lie in two words.
 template <bool CANON>
 __global__ void __launch_bounds__(kBlkThreads, PF_KA_MIN_CTAS)
 kA_block_aggregate(const uint64_t* __restrict__ bases, const uint32_t* __restrict__ ambbits,
@@ -386,37 +407,22 @@ kA_block_aggregate(const uint64_t* __restrict__ bases, const uint32_t* __restric
                    uint32_t* __restrict__ slab_base, uint32_t* __restrict__ slab_count,
                    uint32_t* __restrict__ slab_cnt /* popcount of every partial row */,
                    uint32_t partial_capacity, uint32_t* __restrict__ counters,
-                   const uint32_t* __restrict__ item_list /* null: item = blockIdx.x */,
+                   const uint32_t* __restrict__ item_list /* null: segments of seg_runs runs */,
+                   uint32_t n_segs, uint32_t seg_runs,
                    uint32_t* __restrict__ rescue_items /* out: items whose table overflowed */) {
   extern __shared__ __align__(16) unsigned char blk_raw[];
   const uint32_t W = plan.W, WS = W | 1u;
   const ARunView a = arun_view(blk_raw, plan.slots, plan.cap, plan.cslots, W);
   const uint32_t tid = threadIdx.x;
-  const uint32_t item = item_list ? item_list[blockIdx.x] : blockIdx.x;
 
-  const uint4 desc = __ldg(plan.item_desc + item);
-  const uint32_t seq_lo = desc.x, seq_hi = desc.y, s_rel = desc.z;    // sequences, first window of the run
-  if (seq_lo == seq_hi) {                            // no sample of this slice carries the cluster
-    if (tid == 0) { slab_count[item] = 0; slab_base[item] = 0; }
-    return;
-  }
-  const uint32_t sample0 = plan.n_slices > 1 ? (item % plan.n_slices) * plan.slice_samples : 0u;
-  // the thread's first sequence is requested before the tables are initialised
-  uint4 raw_first = make_uint4(0, 0, 0, 0);
-  if (seq_lo + tid < seq_hi) raw_first = __ldg(reinterpret_cast<const uint4*>(seqs + seq_lo + tid));
-
-  for (uint32_t i = tid; i < plan.slots; i += kBlkThreads) { a.keys[i] = ~0ull; a.rowid[i] = 0xffffu; }
-  for (uint32_t i = tid; i < plan.cslots; i += kBlkThreads) a.cstate[i] = kChunkEmpty;
-  // all bitset rows are cleared here by the whole CTA: a lone inserting lane clearing its own
-  // row costs a warp instruction per word
-  for (uint32_t i = tid; i < (a.cap + 1u) * WS; i += kBlkThreads) a.pool[i] = 0u;
-  for (uint32_t i = tid; i < a.ccap * WS; i += kBlkThreads) a.crows[i] = 0u;
+  auto clear_tables = [&]() {
+    for (uint32_t i = tid; i < plan.slots; i += kBlkThreads) { a.keys[i] = ~0ull; a.rowid[i] = 0xffffu; }
+    for (uint32_t i = tid; i < plan.cslots; i += kBlkThreads) a.cstate[i] = kChunkEmpty;
+    for (uint32_t i = tid; i < (a.cap + 1u) * WS; i += kBlkThreads) a.pool[i] = 0u;
+    for (uint32_t i = tid; i < a.ccap * WS; i += kBlkThreads) a.crows[i] = 0u;
+  };
+  clear_tables();
   if (tid == 0) { a.h->n_unique = 0; a.h->overflow = 0; a.h->work = 0; a.h->n_pass = 0; }
-  uint64_t wf0 = 0, wf1 = 0, wf2 = 0;
-  if (raw_first.y >= (uint32_t)k && s_rel < raw_first.y - (uint32_t)k + 1u) {
-    const uint64_t* w = bases + raw_first.x + (s_rel >> 5);
-    wf0 = __ldg(w); wf1 = __ldg(w + 1); wf2 = __ldg(w + 2);
-  }
   __syncthreads();
 
   const uint32_t sh64 = 64u - 2u * (uint32_t)k;
@@ -444,118 +450,201 @@ kA_block_aggregate(const uint64_t* __restrict__ bases, const uint32_t* __restric
     else { put_bits(fwd, src, first_word, nw); put_bits(rc, src, first_word, nw); }
   };
 
-  // ---- phase 1: every sequence's run -> chunk table (or, for ragged / ambiguous runs and a
-  //      full chunk table, straight into the k-mer table) ------------------------------------
-  for (uint32_t si = seq_lo + tid; si < seq_hi; si += kBlkThreads) {
-    const bool first = si == seq_lo + tid;
-    const uint4 raw = first ? raw_first : __ldg(reinterpret_cast<const uint4*>(seqs + si));
-    const uint32_t len = raw.y;
-    if (len < (uint32_t)k) continue;
-    const uint32_t nwin = len - (uint32_t)k + 1u;
-    if (s_rel >= nwin) continue;
-    const uint32_t nv = min((uint32_t)kBlkRun, nwin - s_rel);
-    const uint32_t sample = (raw.z & 0x7fffffffu) - sample0;      // rank inside the slice
-    const bool amb = (raw.z >> 31) != 0u;
-    const uint32_t wofs = sample >> 5, bit = 1u << (sample & 31u);
-    // three words cover the run: 16 + k - 1 <= 47 bases from an offset < 32
-    const uint64_t* w = bases + raw.x + (s_rel >> 5);
-    const uint64_t w0 = first ? wf0 : __ldg(w), w1 = first ? wf1 : __ldg(w + 1), w2 = first ? wf2 : __ldg(w + 2);
-    const uint32_t o0 = s_rel & 31u;
-    uint64_t hi = w0, lo = w1;
-    if (o0) {
-      hi = (w0 << (2u * o0)) | (w1 >> (64u - 2u * o0));
-      lo = (w1 << (2u * o0)) | (w2 >> (64u - 2u * o0));
+  // the thread's sequences j = 0, 1 of the (cluster, slice) whose first sequence is st_lo, at
+  // word index st_wi: window count (0: none), sample | ambiguity flag, first word, words
+  uint32_t st_lo = 0xffffffffu, st_wi = 0;
+  uint32_t nw0 = 0, nw1 = 0, sf0 = 0, sf1 = 0, wo0 = 0, wo1 = 0;
+  uint64_t c0 = 0, n0 = 0, p0 = 0, c1 = 0, n1 = 0, p1 = 0;
+
+  uint32_t seg = blockIdx.x;
+  for (uint32_t it = 0; seg < n_segs; ++it) {
+    uint32_t r0 = 0, r1 = 1, slice = 0;
+    if (!item_list) {
+      slice = seg % plan.n_slices;
+      r0 = seg / plan.n_slices * seg_runs;
+      r1 = min(r0 + seg_runs, plan.n_run_items);
     }
-    uint32_t cs = 0xffffffffu;
-    if (nv == (uint32_t)kBlkRun && !amb) cs = chunk_find_or_insert(a, hi & cm_hi, lo & cm_lo, wofs);
-    if (cs != 0xffffffffu) {
-      atomicOr(&a.crows[cs * WS + wofs], bit);
-      const uint16_t meta = a.cmeta[cs];            // most chunks are one sample's: remember if not
-      if ((meta & 0xffu) != wofs && !(meta & 0x8000u)) a.cmeta[cs] = meta | 0x8000u;
-    } else {
-      const uint32_t* ab = amb ? ambbits + raw.w : nullptr;
-      for (uint32_t q = 0; q < nv; ++q) {
-        bool dead = false;
-        if (amb) {
-          const uint32_t p = s_rel + q;
-          const uint32_t wi = p >> 5, bs = p & 31u;
-          const uint64_t two = ((uint64_t)ab[wi] << 32) | (uint64_t)ab[wi + 1];
-          dead = ((two << bs) >> (64 - k)) != 0ull;
+    for (uint32_t r = r0; r < r1; ++r) {
+      const uint32_t item = item_list ? item_list[seg] : r * plan.n_slices + slice;
+      const uint4 desc = __ldg(plan.item_desc + item);
+      const uint32_t seq_lo = desc.x, seq_hi = desc.y, s_rel = desc.z;   // sequences, first window of the run
+      if (seq_lo == seq_hi) {                          // no sample of this slice carries the cluster
+        if (tid == 0) { slab_count[item] = 0; slab_base[item] = 0; }
+        continue;
+      }
+      const uint32_t sample0 = plan.n_slices > 1 ? (item % plan.n_slices) * plan.slice_samples : 0u;
+      const uint32_t wi = s_rel >> 5;
+
+      // ---- the register-held sequences at this run: new (cluster, slice) or position -> load,
+      //      next word -> slide by one word and request the one after ---------------------------
+      auto fetch = [&](uint32_t nw, uint32_t wo, uint64_t& c, uint64_t& n, uint64_t& p) {
+        c = 0; n = 0; p = 0;
+        if (s_rel < nw) {
+          const uint64_t* w = bases + wo + wi;
+          c = __ldg(w); n = __ldg(w + 1);
+          if (32u * (wi + 1u) < nw) p = __ldg(w + 2);
         }
-        if (!dead) {
-          const uint64_t x = q ? ((hi << (2u * q)) | (lo >> (64u - 2u * q))) : hi;
-          put_kmer(x >> sh64, &bit, wofs, 1u);
+      };
+      auto slide = [&](uint32_t nw, uint32_t wo, uint64_t& c, uint64_t& n, uint64_t& p) {
+        c = n; n = p; p = 0;
+        if (32u * (wi + 1u) < nw) p = __ldg(bases + wo + wi + 2u);
+      };
+      if (seq_lo != st_lo) {
+        nw0 = 0; nw1 = 0;
+        if (seq_lo + tid < seq_hi) {
+          const uint4 raw = __ldg(reinterpret_cast<const uint4*>(seqs + seq_lo + tid));
+          nw0 = raw.y >= (uint32_t)k ? raw.y - (uint32_t)k + 1u : 0u; sf0 = raw.z; wo0 = raw.x;
+        }
+        if (seq_lo + tid + kBlkThreads < seq_hi) {
+          const uint4 raw = __ldg(reinterpret_cast<const uint4*>(seqs + seq_lo + tid + kBlkThreads));
+          nw1 = raw.y >= (uint32_t)k ? raw.y - (uint32_t)k + 1u : 0u; sf1 = raw.z; wo1 = raw.x;
         }
       }
-    }
-  }
-  __syncthreads();
+      if (seq_lo == st_lo && wi == st_wi + 1u) {
+        slide(nw0, wo0, c0, n0, p0);
+        slide(nw1, wo1, c1, n1, p1);
+      } else if (seq_lo != st_lo || wi != st_wi) {
+        fetch(nw0, wo0, c0, n0, p0);
+        fetch(nw1, wo1, c1, n1, p1);
+      }
+      st_lo = seq_lo;
+      st_wi = wi;
 
-  // ---- phase 2: distinct chunks x 16 windows -> k-mer table, whole sample bitsets at a time ----
-  const uint32_t n_chunks = min(a.h->work, a.ccap);
-  const uint32_t n_pairs = n_chunks * (uint32_t)kBlkRun;
-  // pairs cost very different amounts (a new k-mer is an insertion, a many-sample chunk ORs W
-  // words): the first round is static, after it the warps take 32 pairs at a time from a counter
-  for (uint32_t p0 = (tid & ~31u);;) {
-    const uint32_t p = p0 + (tid & 31u);
-    if (p < n_pairs) {
-      const uint32_t cs = p >> 4, q = p & 15u;
-      const uint64_t hi = a.ckhi[cs], lo = a.cklo[cs];
-      const uint64_t x = q ? ((hi << (2u * q)) | (lo >> (64u - 2u * q))) : hi;
-      const uint16_t meta = a.cmeta[cs];
-      if (meta & 0x8000u) put_kmer(x >> sh64, a.crows + cs * WS, 0u, W);
-      else put_kmer(x >> sh64, a.crows + cs * WS + (meta & 0xffu), meta & 0xffu, 1u);
-    }
-    __syncwarp();
-    uint32_t nx = 0;
-    if ((tid & 31u) == 0u) nx = atomicAdd(&a.h->n_pass, 32u);
-    p0 = (uint32_t)kBlkThreads + __shfl_sync(kFull, nx, 0);
-    if (p0 >= n_pairs) break;
-  }
-  __syncthreads();
+      // ---- phase 1: every sequence's run -> chunk table (or, for ragged / ambiguous runs and a
+      //      full chunk table, straight into the k-mer table) ----------------------------------
+      for (uint32_t j = 0, si = seq_lo + tid; si < seq_hi; ++j, si += kBlkThreads) {
+        uint32_t nwin, sf;
+        uint64_t w0, w1;
+        if (j < 2u) {
+          nwin = j ? nw1 : nw0; sf = j ? sf1 : sf0; w0 = j ? c1 : c0; w1 = j ? n1 : n0;
+        } else {                                      // beyond 2 x threads: from global memory
+          const uint4 raw = __ldg(reinterpret_cast<const uint4*>(seqs + si));
+          nwin = raw.y >= (uint32_t)k ? raw.y - (uint32_t)k + 1u : 0u;
+          sf = raw.z;
+          w0 = 0; w1 = 0;
+          if (s_rel < nwin) { const uint64_t* w = bases + raw.x + wi; w0 = __ldg(w); w1 = __ldg(w + 1); }
+        }
+        if (s_rel >= nwin) continue;
+        const uint32_t nv = min((uint32_t)kBlkRun, nwin - s_rel);
+        const uint32_t sample = (sf & 0x7fffffffu) - sample0;      // rank inside the slice
+        const bool amb = (sf >> 31) != 0u;
+        const uint32_t wofs = sample >> 5, bit = 1u << (sample & 31u);
+        const uint32_t o0 = s_rel & 31u;
+        uint64_t hi = w0, lo = w1;
+        if (o0) {
+          hi = (w0 << (2u * o0)) | (w1 >> (64u - 2u * o0));
+          lo = w1 << (2u * o0);
+        }
+        uint32_t cs = 0xffffffffu;
+        if (nv == (uint32_t)kBlkRun && !amb) cs = chunk_find_or_insert(a, hi & cm_hi, lo & cm_lo, wofs);
+        if (cs != 0xffffffffu) {
+          atomicOr(&a.crows[cs * WS + wofs], bit);
+          const uint16_t meta = a.cmeta[cs];            // most chunks are one sample's: remember if not
+          if ((meta & 0xffu) != wofs && !(meta & 0x8000u)) a.cmeta[cs] = meta | 0x8000u;
+        } else {
+          const uint32_t* ab = amb ? ambbits + seqs[si].amb_word_off : nullptr;
+          for (uint32_t q = 0; q < nv; ++q) {
+            bool dead = false;
+            if (amb) {
+              const uint32_t p = s_rel + q;
+              const uint32_t wj = p >> 5, bs = p & 31u;
+              const uint64_t two = ((uint64_t)ab[wj] << 32) | (uint64_t)ab[wj + 1];
+              dead = ((two << bs) >> (64 - k)) != 0ull;
+            }
+            if (!dead) {
+              const uint64_t x = q ? ((hi << (2u * q)) | (lo >> (64u - 2u * q))) : hi;
+              put_kmer(x >> sh64, &bit, wofs, 1u);
+            }
+          }
+        }
+      }
+      __syncthreads();
 
-  if (a.h->overflow) {
-    if (tid == 0) {
-      slab_count[item] = kBlkOverflow;
-      slab_base[item] = 0;
-      atomicExch(&counters[LC_TABLE_OVERFLOW], 1u);
-      rescue_items[atomicAdd(&counters[LC_RESCUE], 1u)] = item;
+      // ---- phase 2: distinct chunks x 16 windows -> k-mer table, whole sample bitsets at a time ----
+      const uint32_t n_chunks = min(a.h->work, a.ccap);
+      const uint32_t n_pairs = n_chunks * (uint32_t)kBlkRun;
+      // pairs cost very different amounts (a new k-mer is an insertion, a many-sample chunk ORs W
+      // words): the first round is static, after it the warps take 32 pairs at a time from a counter
+      for (uint32_t q0 = (tid & ~31u);;) {
+        const uint32_t p = q0 + (tid & 31u);
+        if (p < n_pairs) {
+          const uint32_t cs = p >> 4, q = p & 15u;
+          const uint64_t hi = a.ckhi[cs], lo = a.cklo[cs];
+          const uint64_t x = q ? ((hi << (2u * q)) | (lo >> (64u - 2u * q))) : hi;
+          const uint16_t meta = a.cmeta[cs];
+          if (meta & 0x8000u) put_kmer(x >> sh64, a.crows + cs * WS, 0u, W);
+          else put_kmer(x >> sh64, a.crows + cs * WS + (meta & 0xffu), meta & 0xffu, 1u);
+        }
+        __syncwarp();
+        uint32_t nx = 0;
+        if ((tid & 31u) == 0u) nx = atomicAdd(&a.h->n_pass, 32u);
+        q0 = (uint32_t)kBlkThreads + __shfl_sync(kFull, nx, 0);
+        if (q0 >= n_pairs) break;
+      }
+      __syncthreads();
+
+      // ---- epilogue: the slab of this run (n partial rows from a bump allocator), then the
+      //      tables are reset for the next run -----------------------------------------------
+      const bool overflow = a.h->overflow != 0u;
+      const uint32_t n = a.h->n_unique;
+      if (tid == 0) {
+        if (overflow) {
+          slab_count[item] = kBlkOverflow;
+          slab_base[item] = 0;
+          atomicExch(&counters[LC_TABLE_OVERFLOW], 1u);
+          rescue_items[atomicAdd(&counters[LC_RESCUE], 1u)] = item;
+        } else {
+          const uint32_t b = atomicAdd(&counters[LC_PARTIALS], n);
+          a.h->row_base = b;
+          a.h->ok = 1;
+          slab_base[item] = b;
+          slab_count[item] = n;
+          if ((uint64_t)b + n > partial_capacity) {
+            a.h->ok = 0;
+            slab_count[item] = 0;
+            atomicExch(&counters[LC_PARTIAL_OVERFLOW], 1u);
+          }
+        }
+      }
+      __syncthreads();
+      if (tid == 0) { a.h->n_unique = 0; a.h->overflow = 0; a.h->work = 0; a.h->n_pass = 0; }
+      if (!overflow && a.h->ok) {
+        const size_t base = a.h->row_base;
+        const uint32_t WP = plan.WP;
+        for (uint32_t r = tid; r < n; r += kBlkThreads) {
+          slab_keys[base + r] = a.rkey[r];
+          uint32_t* src = a.pool + r * WS;
+          uint4* dst = reinterpret_cast<uint4*>(slab_rows + (base + r) * WP);
+          uint32_t cnt = 0;
+          for (uint32_t q = 0; q < WP; q += 4) {
+            uint4 x;
+            x.x = src[q];
+            x.y = q + 1 < W ? src[q + 1] : 0u;
+            x.z = q + 2 < W ? src[q + 2] : 0u;
+            x.w = q + 3 < W ? src[q + 3] : 0u;
+            dst[q >> 2] = x;
+            cnt += __popc(x.x) + __popc(x.y) + __popc(x.z) + __popc(x.w);
+          }
+          slab_cnt[base + r] = cnt;
+          for (uint32_t q = 0; q < W; ++q) src[q] = 0u;
+          const uint32_t h = a.rslot[r];
+          a.keys[h] = ~0ull;
+          a.rowid[h] = 0xffffu;
+        }
+        for (uint32_t c = tid; c < n_chunks; c += kBlkThreads) a.cstate[a.cslot[c]] = kChunkEmpty;
+        for (uint32_t i = tid; i < n_chunks * WS; i += kBlkThreads) a.crows[i] = 0u;
+      } else {
+        clear_tables();
+      }
+      __syncthreads();
     }
-    return;
-  }
-  // the slab of this block: n partial rows from a bump allocator
-  const uint32_t n = a.h->n_unique;
-  if (tid == 0) {
-    const uint32_t b = atomicAdd(&counters[LC_PARTIALS], n);
-    a.h->row_base = b;
-    a.h->ok = 1;
-    slab_base[item] = b;
-    slab_count[item] = n;
-    if ((uint64_t)b + n > partial_capacity) {
-      a.h->ok = 0;
-      slab_count[item] = 0;
-      atomicExch(&counters[LC_PARTIAL_OVERFLOW], 1u);
+    if (item_list) {
+      seg += gridDim.x;
+    } else {
+      if (tid == 0) a.h->seg[it & 1u] = gridDim.x + atomicAdd(&counters[LC_SEGMENT], 1u);
+      __syncthreads();
+      seg = a.h->seg[it & 1u];
     }
-  }
-  __syncthreads();
-  if (!a.h->ok) return;
-  const size_t base = a.h->row_base;
-  const uint32_t WP = plan.WP;
-  for (uint32_t r = tid; r < n; r += kBlkThreads) {
-    slab_keys[base + r] = a.rkey[r];
-    const uint32_t* src = a.pool + r * WS;
-    uint4* dst = reinterpret_cast<uint4*>(slab_rows + (base + r) * WP);
-    uint32_t cnt = 0;
-    for (uint32_t q = 0; q < WP; q += 4) {
-      uint4 x;
-      x.x = src[q];
-      x.y = q + 1 < W ? src[q + 1] : 0u;
-      x.z = q + 2 < W ? src[q + 2] : 0u;
-      x.w = q + 3 < W ? src[q + 3] : 0u;
-      dst[q >> 2] = x;
-      cnt += __popc(x.x) + __popc(x.y) + __popc(x.z) + __popc(x.w);
-    }
-    slab_cnt[base + r] = cnt;
   }
 }
 

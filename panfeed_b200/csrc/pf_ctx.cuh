@@ -312,6 +312,7 @@ struct pf_ctx : BatchState {
   bool block_mode = false;       // S <= 1024 and not disabled: kA_block_aggregate + kB1..kB3
   uint32_t block_windows = 16;   // windows per position block (= kBlkRun)
   uint32_t blk_slots = 1024, blk_cap = 448, blk_cslots = 128;   // shared memory of kA: k-mer key slots / rows, chunk slots
+  uint32_t ka_seg_runs = 0;      // runs per kA segment (PF_KA_SEG_RUNS); 0: chosen from the batch
   uint32_t n_slices = 1, slice_samples = 0, Ws = 0;   // sample slices of the block engine (S > 1024): slices,
                                                        // samples per slice, bitset words of a partial row
   uint32_t block_fallbacks = 0;
@@ -599,9 +600,9 @@ constexpr uint32_t kBlkMaxSmem = 220u * 1024u;   // largest kA table we ask for
 enum { C_TICKET_N = 0, C_TICKET_W = 1, C_RUNS_N = 2, C_RUNS_W = 3, C_ERR = 4, C_ROWS_N = 5,
        C_ROWS_W = 6, C_NEW_KP = 7, C_NEW_CP = 8, C_TICKET_MARK_N = 9, C_TICKET_MARK_W = 10,
        C_LOCAL = 11 /* LC_COUNT words: rows, unique, table overflow, row overflow, rescue runs,
-                        partial rows, partial overflow */, C_TICKET_MERGE = 18,
+                        partial rows, partial overflow, kA segments */,
        C_X_UNIQUE_KP = 19, C_X_UNIQUE_CP = 20 /* owner-side unique counts of the exchange */, C_COUNT = 24 };
-static_assert(C_LOCAL + LC_COUNT <= C_TICKET_MERGE, "counter layout");
+static_assert(C_LOCAL + LC_COUNT <= C_X_UNIQUE_KP, "counter layout");
 
 bool keep_count(double maf, uint32_t c, uint32_t n) {
   double af = (double)c / (double)n;      // numpy: vec.sum() / vec.shape[0]

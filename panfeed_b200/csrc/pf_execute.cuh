@@ -416,11 +416,13 @@ BlkPlan block_plan(const pf_ctx* ctx) {
   bp.slice_samples = ctx->slice_samples;
   bp.slice_seq = ctx->n_slices > 1 ? ctx->d_slice_seq.as<uint32_t>() : nullptr;
   bp.item_desc = ctx->d_item_desc.as<uint4>();
+  bp.n_run_items = ctx->n_items;
   return bp;
 }
 
-// items == nullptr: all (cluster, block) items with the context's table size; else the listed
-// items (a rescue launch) with `slots` slots.  Items that overflow are appended to `rescue_out`.
+// items == nullptr: all (cluster, block) items with the context's table size, in segments of
+// consecutive runs; else the listed items (a rescue launch, one CTA and one run per item) with
+// `slots` slots.  Items that overflow are appended to `rescue_out`.
 int launch_block_aggregate(pf_ctx* ctx, const uint32_t* items, uint32_t n, uint32_t slots, uint32_t cap,
                            uint32_t cslots, uint32_t* rescue_out) {
   if (n == 0) return PF_OK;
@@ -432,15 +434,30 @@ int launch_block_aggregate(pf_ctx* ctx, const uint32_t* items, uint32_t n, uint3
   const uint32_t cap32 = (uint32_t)std::min<uint64_t>(ctx->partial_cap, 0xfffffff0u);
   uint32_t* counters = ctx->d_counters.as<uint32_t>() + C_LOCAL;
   const uint32_t smem = blkA_smem_bytes(slots, cap, cslots, ctx->Ws);
-#define PF_KA(CANON)                                                                                   \
-  kA_block_aggregate<CANON><<<n, kBlkThreads, smem, st>>>(                                             \
-      ctx->d_bases.as<uint64_t>(), ctx->d_ambbits.as<uint32_t>(), ctx->d_seq_lite.as<SeqLite>(), bp,   \
-      (int)ctx->prm.k, ctx->d_slab_keys.as<uint64_t>(), ctx->d_slab_rows.as<uint32_t>(),               \
-      ctx->d_slab_base.as<uint32_t>(), ctx->d_slab_count.as<uint32_t>(), ctx->d_slab_cnt.as<uint32_t>(), \
-      cap32, counters, items,                                                                          \
-      rescue_out)
-  if (ctx->prm.canonical) PF_KA(true); else PF_KA(false);
-#undef PF_KA
+  auto kernel = ctx->prm.canonical ? kA_block_aggregate<true> : kA_block_aggregate<false>;
+  uint32_t grid = n, n_segs = n, seg_runs = 1;
+  if (!items) {
+    // a grid of resident CTAs takes segments from counters[LC_SEGMENT] (zeroed with the other
+    // C_LOCAL words before kA).  Longer segments share more of the per-run set-up, but the GPU
+    // must stay full: segments are halved while there are fewer than 4 per resident CTA.
+    int sms = 0, dev = 0, per_sm = 0;
+    CU(cudaGetDevice(&dev));
+    CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kBlkThreads, smem));
+    const uint32_t resident = (uint32_t)std::max(1, sms * per_sm);
+    seg_runs = ctx->ka_seg_runs;
+    if (seg_runs == 0) {
+      seg_runs = 16;
+      while (seg_runs > 1 && (uint64_t)cdiv(ctx->n_items, seg_runs) * ctx->n_slices < 4ull * resident) seg_runs /= 2;
+    }
+    n_segs = cdiv(ctx->n_items, seg_runs) * ctx->n_slices;
+    grid = std::min(n_segs, resident);
+  }
+  kernel<<<grid, kBlkThreads, smem, st>>>(
+      ctx->d_bases.as<uint64_t>(), ctx->d_ambbits.as<uint32_t>(), ctx->d_seq_lite.as<SeqLite>(), bp,
+      (int)ctx->prm.k, ctx->d_slab_keys.as<uint64_t>(), ctx->d_slab_rows.as<uint32_t>(),
+      ctx->d_slab_base.as<uint32_t>(), ctx->d_slab_count.as<uint32_t>(), ctx->d_slab_cnt.as<uint32_t>(),
+      cap32, counters, items, n_segs, seg_runs, rescue_out);
   ctx->launches++;
   CU(cudaGetLastError());
   return PF_OK;
@@ -670,14 +687,14 @@ extern "C" int pf_execute(pf_ctx* ctx) {
           // sends runs down the direct path)
           uint32_t slots2 = slots * 2u, cap2 = 0;
           if (slots2 <= 8192u && blkA_smem_bytes(slots2, 0u, cslots, ctx->Ws) < kBlkMaxSmem) {
-            const uint32_t per_row = 8u + (ctx->Ws | 1u) * 4u;
+            const uint32_t per_row = 10u + (ctx->Ws | 1u) * 4u;   // rkey, rslot, bitset
             const uint32_t fit = (kBlkMaxSmem - blkA_smem_bytes(slots2, 0u, cslots, ctx->Ws)) / per_row;
             cap2 = std::min<uint32_t>(std::min<uint32_t>(fit, slots2 * 13u / 16u),
                                       std::max<uint32_t>(cap * 2u, slots2 * 5u / 8u));
           }
           if (cap2 <= cap) {        // no more rows with more slots: try all the rows the current slots allow
             slots2 = slots;
-            const uint32_t per_row = 8u + (ctx->Ws | 1u) * 4u;
+            const uint32_t per_row = 10u + (ctx->Ws | 1u) * 4u;   // rkey, rslot, bitset
             const uint32_t fit = (kBlkMaxSmem - blkA_smem_bytes(slots, 0u, cslots, ctx->Ws)) / per_row;
             cap2 = std::min<uint32_t>(fit, slots * 13u / 16u);
           }

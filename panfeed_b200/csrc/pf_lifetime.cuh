@@ -160,6 +160,10 @@ extern "C" int pf_create(pf_ctx** out, int device, const pf_params* p) {
     while (slots > 64u && blkA_smem_bytes(slots, cap, cslots, ctx->Ws) > kBlkMaxSmem) {
       slots /= 2; cap /= 2; cslots = std::max<uint32_t>(32u, cslots / 2);
     }
+    if (const char* e = getenv("PF_KA_SEG_RUNS")) {   // fixed segment length: tests of small batches, sweeps
+      const int v = atoi(e);
+      if (v >= 1 && v <= 4096) ctx->ka_seg_runs = (uint32_t)v;
+    }
     ctx->blk_slots = slots;
     ctx->blk_cap = cap;
     ctx->blk_cslots = cslots;
