@@ -29,14 +29,15 @@
 extern "C" {
 #endif
 
-#define PF_ABI_VERSION 1
+/* 2: pf_batch_result gained the xwide_row_* and pos_xwide_kmer fields (k = 33..64 with N/IUPAC) */
+#define PF_ABI_VERSION 2
 
 typedef enum pf_status {
   PF_OK = 0,
   PF_ERR_INVALID = -1,      /* bad argument / malformed batch              */
   PF_ERR_CUDA = -2,         /* CUDA runtime error (no device, launch, ...) */
   PF_ERR_NOMEM = -3,        /* host or device allocation failed            */
-  PF_ERR_UNSUPPORTED = -4,  /* e.g. k > 64                                 */
+  PF_ERR_UNSUPPORTED = -4,  /* k outside 1..64; a symbol outside PF_AMB_ALPHABET (packer) */
   PF_ERR_STATE = -5,        /* call order violated                         */
   PF_ERR_INTERNAL = -6      /* device-side watchdog / invariant violated   */
 } pf_status;
@@ -48,7 +49,9 @@ typedef struct pf_params {
   uint32_t abi_version;          /* PF_ABI_VERSION                                  */
   uint32_t k;                    /* -k/--kmer-length, 1..64: up to 32 a k-mer is one 64-bit word
                                     (all engines); 33..64 two words, through the 128-bit record
-                                    engine, rows come back as wide rows (2 bits per base)        */
+                                    engine, rows come back as wide rows (2 bits per base); there
+                                    a k-mer holding N/IUPAC symbols takes four words (4 bits per
+                                    symbol, 256-bit records) and comes back as an xwide row     */
   uint32_t n_samples;            /* S = number of strain columns of the panaroo CSV */
   uint32_t canonical;            /* 1 unless --non-canonical (panfeed.py:69-88)     */
   uint32_t consider_missing;     /* --consider-missing (panfeed.py:16-20,192-196)   */
@@ -162,9 +165,12 @@ typedef struct pf_batch_result {
   const int32_t*  pos_contig_start;/* contig_end  = contig_start + k (panfeed.py:91-99)          */
   const int32_t*  pos_gene_start;  /* gene_end    = gene_start + k   (panfeed.py:101-102)        */
   const uint8_t*  pos_flags;       /* bit0: reverse complement was the canonical one
-                                      (used_strand = -1); bit1: k-mer is ambiguous, then
-                                      pos_kmer holds an index into pos_wide_kmer              */
-  const uint64_t* pos_wide_kmer;   /* 2 words per ambiguous positional k-mer                  */
+                                      (used_strand = -1); bit1: two-word k-mer (N/IUPAC at
+                                      k <= 32, any k-mer at k > 32), pos_kmer holds an index
+                                      into pos_wide_kmer; bit2 (k > 32, k-mer holds N/IUPAC
+                                      symbols; bit1 is then clear): pos_kmer holds an index
+                                      into pos_xwide_kmer                                      */
+  const uint64_t* pos_wide_kmer;   /* 2 words per two-word positional k-mer                   */
   uint64_t        n_pos_wide;
   /* emit_positions == 2: n_pos still counts the instances, the pos_* arrays above are NULL and
    * bit (i & 31) of pos_strand_bits[i >> 5], i = pf_seq_desc.base_off + pos, is 1 iff the reverse
@@ -173,6 +179,16 @@ typedef struct pf_batch_result {
    * undefined; with canonical == 0 nothing is needed and the plane is empty. */
   const uint32_t* pos_strand_bits;
   uint64_t        n_pos_bit_words; /* pf_batch.n_words (one bit per base position), or 0      */
+  /* k = 33..64: rows whose k-mer holds N/IUPAC symbols, 4 bits per symbol (codes of
+     PF_AMB_ALPHABET), first symbol in the top used bits of [w0, w1, w2, w3].  Their patterns are
+     numbered with those of the other rows (one pattern, one id).  Empty (0 / NULL) otherwise. */
+  uint64_t        n_xwide_rows;
+  const uint32_t* xwide_row_cluster;
+  const uint64_t* xwide_row_kmer;  /* 4 words per row, most significant first                */
+  const uint32_t* xwide_row_count;
+  const uint32_t* xwide_row_pattern;
+  const uint64_t* pos_xwide_kmer;  /* 4 words per positional k-mer with pos_flags bit 2       */
+  uint64_t        n_pos_xwide;
 } pf_batch_result;
 
 typedef struct pf_stats {
@@ -287,13 +303,14 @@ int pf_format_patterns(const uint32_t* pattern_words, uint64_t n, uint32_t strid
 
 /* The kmers_to_hashes rows of a batch (panfeed.py:177 "<idx>\t\t<cluster hash>", :208
  * "<idx>\t<kmer>\t<hash>"): for every cluster of `result`, in order, the header row and then its
- * k-mer rows — the plain ones in alphabetical k-mer order, then those holding N/IUPAC symbols
- * (the reference's order inside a cluster is the insertion order of a Python dict; consumers
- * key on the k-mer).  tag_blob + tag_off[c .. c+1]: the text of the first column for cluster c.
+ * k-mer rows — the plain ones in alphabetical k-mer order, then the wide ones, then the xwide ones
+ * (k > 32 with N/IUPAC symbols), each group sorted (the reference's order inside a cluster is the
+ * insertion order of a Python dict; consumers key on the k-mer).  tag_blob + tag_off[c .. c+1]:
+ * the text of the first column for cluster c.
  * kmer_ids / cluster_ids: 24 characters per pattern, indexed by row_pattern / cluster_pattern
  * (all patterns numbered so far, e.g. from pf_pattern_ids + base64).  cluster_off (may be NULL):
  * [n_clusters + 1] byte offsets of every cluster's text.  out == NULL: only *out_len (and
- * cluster_off).  Uses row_*, wide_row_*, cluster_pattern and n_clusters of the result. */
+ * cluster_off).  Uses row_*, wide_row_*, xwide_row_*, cluster_pattern and n_clusters of the result. */
 int pf_format_kmer_rows(const pf_batch_result* result, uint32_t k, const char* tag_blob,
                         const uint64_t* tag_off, const char* kmer_ids, uint64_t n_kmer_ids,
                         const char* cluster_ids, uint64_t n_cluster_ids, char* out,

@@ -55,7 +55,8 @@ def get_options(argv=None):
     p.add_argument("-k", "--kmer-length", type=int, default=31,
                    help="K-mer length, 1..64 (a k-mer is packed into one or two 64-bit words; the "
                         "reference accepts longer k-mers, this build exits with an error).  33..64 run on "
-                        "the 128-bit record engine, several times slower than 1..32")
+                        "the 128-bit record engine, several times slower than 1..32; their k-mers holding "
+                        "N/IUPAC symbols take 256-bit records")
     p.add_argument("--maf", type=float, default=0.01, help="Minor allele frequency threshold")
     p.add_argument("--upstream", type=int, default=0)
     p.add_argument("--downstream", type=int, default=0)

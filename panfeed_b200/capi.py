@@ -14,7 +14,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 # PF_LIB_PATH: a differently built library (kernel A/B experiments); default = the in-tree build
 LIB_PATH = os.environ.get("PF_LIB_PATH") or os.path.join(HERE, "csrc", "libpanfeed_b200.so")
 
-PF_ABI_VERSION = 1
+PF_ABI_VERSION = 2
 PF_SEQ_TARGET = 1
 PF_SEQ_AMBIGUOUS = 2
 AMB_ALPHABET = "ABCDGHKMNRSTVWXY"
@@ -80,7 +80,14 @@ class BatchResult(C.Structure):
                 ("pos_wide_kmer", C.POINTER(C.c_uint64)),
                 ("n_pos_wide", C.c_uint64),
                 ("pos_strand_bits", C.POINTER(C.c_uint32)),
-                ("n_pos_bit_words", C.c_uint64)]
+                ("n_pos_bit_words", C.c_uint64),
+                ("n_xwide_rows", C.c_uint64),
+                ("xwide_row_cluster", C.POINTER(C.c_uint32)),
+                ("xwide_row_kmer", C.POINTER(C.c_uint64)),
+                ("xwide_row_count", C.POINTER(C.c_uint32)),
+                ("xwide_row_pattern", C.POINTER(C.c_uint32)),
+                ("pos_xwide_kmer", C.POINTER(C.c_uint64)),
+                ("n_pos_xwide", C.c_uint64)]
 
 
 class Stats(C.Structure):
@@ -385,9 +392,10 @@ def gzip_members(data, level=9, member_bytes=0, n_threads=0):
 
 def format_kmer_rows(r, k, tags, kmer_ids, cluster_ids, n_threads=0, raw=False):
     """kmers_to_hashes text of the batch result `r` (a dict as returned by Context.collect(), or
-    any dict with row_*, wide_row_* and cluster_pattern), formatted by the library's host threads
-    (pf_format_kmer_rows).  tags[c] = first column of cluster c (bytes); kmer_ids / cluster_ids:
-    numpy S24 arrays of all pattern ids numbered so far.  Returns (bytes, offsets[n_clusters+1])."""
+    any dict with row_*, wide_row_* (xwide_row_* if present) and cluster_pattern), formatted by
+    the library's host threads (pf_format_kmer_rows).  tags[c] = first column of cluster c (bytes);
+    kmer_ids / cluster_ids: numpy S24 arrays of all pattern ids numbered so far.  Returns (bytes,
+    offsets[n_clusters+1])."""
     lib = load()
     keep = []
 
@@ -412,6 +420,12 @@ def format_kmer_rows(r, k, tags, kmer_ids, cluster_ids, n_threads=0, raw=False):
         res.wide_row_kmer = ptr(wide, np.uint64, C.c_uint64)
         res.wide_row_cluster = ptr(r["wide_row_cluster"], np.uint32, C.c_uint32)
         res.wide_row_pattern = ptr(r["wide_row_pattern"], np.uint32, C.c_uint32)
+    xwide = np.ascontiguousarray(r.get("xwide_row_kmer", np.zeros((0, 4), np.uint64)), dtype=np.uint64).reshape(-1)
+    res.n_xwide_rows = xwide.size // 4
+    if xwide.size:
+        res.xwide_row_kmer = ptr(xwide, np.uint64, C.c_uint64)
+        res.xwide_row_cluster = ptr(r["xwide_row_cluster"], np.uint32, C.c_uint32)
+        res.xwide_row_pattern = ptr(r["xwide_row_pattern"], np.uint32, C.c_uint32)
     blob = b"".join(tags)
     off = np.zeros(nc + 1, np.uint64)
     np.cumsum([len(x) for x in tags], out=off[1:])
@@ -459,6 +473,10 @@ def format_positions(r, k, canonical, leads, seq_strand, n_threads=0):
         wide = np.zeros(2, np.uint64)
     res.pos_wide_kmer = ptr(wide, np.uint64, C.c_uint64)
     res.n_pos_wide = wide.size // 2
+    xwide = np.ascontiguousarray(r.get("pos_xwide_kmer", np.zeros((0, 4), np.uint64)), dtype=np.uint64).reshape(-1)
+    if xwide.size:                # (k > 32: positional k-mers holding N/IUPAC symbols, pos_flags bit 2)
+        res.pos_xwide_kmer = ptr(xwide, np.uint64, C.c_uint64)
+        res.n_pos_xwide = xwide.size // 4
     blob = b"".join(leads)
     off = np.zeros(len(leads) + 1, np.uint64)
     np.cumsum([len(x) for x in leads], out=off[1:])
@@ -651,6 +669,12 @@ class Context:
                                  np.uint64).reshape(-1, 2),
             "n_pos": int(r.n_pos),
             "pos_strand_bits": _np(r.pos_strand_bits, r.n_pos_bit_words, np.uint32),
+            # k > 32: rows / positional k-mers holding N/IUPAC symbols, 4 words (4 bits per symbol)
+            "xwide_row_cluster": _np(r.xwide_row_cluster, r.n_xwide_rows, np.uint32),
+            "xwide_row_kmer": _np(r.xwide_row_kmer, 4 * r.n_xwide_rows, np.uint64).reshape(-1, 4),
+            "xwide_row_count": _np(r.xwide_row_count, r.n_xwide_rows, np.uint32),
+            "xwide_row_pattern": _np(r.xwide_row_pattern, r.n_xwide_rows, np.uint32),
+            "pos_xwide_kmer": _np(r.pos_xwide_kmer, 4 * r.n_pos_xwide, np.uint64).reshape(-1, 4),
         }
         out["d2h_bytes"] = int(sum(v.nbytes for v in out.values()
                                    if isinstance(v, np.ndarray)))

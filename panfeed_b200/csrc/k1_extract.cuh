@@ -165,9 +165,13 @@ k1_strand_bits(const uint64_t* __restrict__ bases, const SeqDev* __restrict__ se
 // pipeline that the N/IUPAC windows use (radix sort of mixed keys + run reduction).  One warp
 // walks one sequence; lane l of iteration `it` owns the window starting at base 32 * it + l: the
 // three words it needs are the same for the whole warp.
+// A window of a sequence flagged ambiguous that touches a non-ACGT symbol (whose 2-bit code is
+// that of A) is written as a dead record here: k1_extract_wide<Key256> owns it, and runs after
+// this kernel on the same stream to correct its positional record / strand bit.
 template <bool CANON>
 __global__ void __launch_bounds__(kK1Warps * 32)
-k1_extract_long(const uint64_t* __restrict__ bases, const SeqDev* __restrict__ seqs, uint32_t n_seqs, int k,
+k1_extract_long(const uint64_t* __restrict__ bases, const uint32_t* __restrict__ ambbits,
+                const SeqDev* __restrict__ seqs, uint32_t n_seqs, int k,
                 Key128* __restrict__ keys, uint32_t* __restrict__ vals, PosOut pos,
                 uint64_t* __restrict__ pos_wide, uint32_t* __restrict__ strand_bits) {
   const uint32_t lane = lane_id();
@@ -180,10 +184,18 @@ k1_extract_long(const uint64_t* __restrict__ bases, const SeqDev* __restrict__ s
     const uint32_t nwin = d.len - (uint32_t)k + 1u;
     const uint64_t* w = bases + (d.base_off >> 5);
     const bool target = (d.flags & 1u) != 0u;
+    const uint32_t* ab = (d.flags & 2u) ? ambbits + (d.amb_off >> 5) : nullptr;
     for (uint32_t it = 0; it * 32u < nwin; ++it) {
       const uint32_t p = it * 32u + lane;
       const bool valid = p < nwin;
       const uint64_t w0 = __ldg(w + it), w1 = __ldg(w + it + 1), w2 = __ldg(w + it + 2);
+      bool is_amb = false;
+      if (ab && valid) {                   // any non-ACGT symbol in [p, p + k)?  (k <= 64: 3 bit words)
+        const uint32_t wi = p >> 5, bs = p & 31u;
+        const uint64_t two = ((uint64_t)ab[wi] << 32) | (uint64_t)ab[wi + 1];
+        const uint64_t x = (two << bs) | (((uint64_t)ab[wi + 2] << bs) >> 32);    // bits [p, p + 64)
+        is_amb = (k >= 64 ? x : x >> (64 - k)) != 0ull;
+      }
       const uint32_t sh = 2u * lane;
       // the 64 bases from base p, first base on top
       uint64_t hi = w0, lo = w1;
@@ -204,8 +216,8 @@ k1_extract_long(const uint64_t* __restrict__ bases, const SeqDev* __restrict__ s
       if (CANON) {
         const Key128 canon = use_rc ? r : f;
         const size_t rec = (size_t)d.wrec_off + p;
-        keys[rec] = mix128(canon);
-        vals[rec] = d.sample;
+        keys[rec] = is_amb ? Key128{0, 0} : mix128(canon);
+        vals[rec] = is_amb ? kInvalidSample : d.sample;
         if (target && pos.kmer) {
           const size_t q = (size_t)d.pos_off + p, wq = (size_t)d.pwide_off + p;
           pos.kmer[q] = (uint64_t)wq;
@@ -218,9 +230,9 @@ k1_extract_long(const uint64_t* __restrict__ bases, const SeqDev* __restrict__ s
         }
       } else {
         const size_t rec = (size_t)d.wrec_off + 2 * (size_t)p;
-        keys[rec] = mix128(f);
-        keys[rec + 1] = mix128(r);
-        vals[rec] = vals[rec + 1] = d.sample;
+        keys[rec] = is_amb ? Key128{0, 0} : mix128(f);
+        keys[rec + 1] = is_amb ? Key128{0, 0} : mix128(r);
+        vals[rec] = vals[rec + 1] = is_amb ? kInvalidSample : d.sample;
         if (target && pos.kmer) {
           const size_t q = (size_t)d.pos_off + p, wq = (size_t)d.pwide_off + p;
           pos.kmer[q] = (uint64_t)wq;
@@ -263,15 +275,44 @@ __device__ __forceinline__ uint32_t comp4(uint32_t c) {
   return (uint32_t)(kTable >> (4 * c)) & 15u;
 }
 
-// One thread per window of a flagged sequence; only windows that touch a
-// non-ACGT symbol produce a live record (the narrow kernel owns the others).
-template <bool CANON>
+// 4-bit keys, built one symbol at a time: push4 appends a symbol at the bottom (the forward
+// k-mer), set4 ORs a symbol into nibble i from the bottom (the reverse complement)
+__device__ __forceinline__ void push4(Key128& key, uint32_t c) {
+  key.hi = (key.hi << 4) | (key.lo >> 60);
+  key.lo = (key.lo << 4) | c;
+}
+__device__ __forceinline__ void push4(Key256& key, uint32_t c) {
+  key.w[0] = (key.w[0] << 4) | (key.w[1] >> 60);
+  key.w[1] = (key.w[1] << 4) | (key.w[2] >> 60);
+  key.w[2] = (key.w[2] << 4) | (key.w[3] >> 60);
+  key.w[3] = (key.w[3] << 4) | c;
+}
+__device__ __forceinline__ void set4(Key128& key, int i, uint64_t c) {
+  if (i < 16) key.lo |= c << (4 * i); else key.hi |= c << (4 * (i - 16));
+}
+__device__ __forceinline__ void set4(Key256& key, int i, uint64_t c) {
+  const uint64_t v = c << (4 * (i & 15));
+  const int j = i >> 4;                    // (a branch per word keeps the key in registers)
+  if (j == 0) key.w[3] |= v; else if (j == 1) key.w[2] |= v; else if (j == 2) key.w[1] |= v; else key.w[0] |= v;
+}
+__device__ __forceinline__ Key128 mix_key(const Key128& key) { return mix128(key); }
+__device__ __forceinline__ Key256 mix_key(const Key256& key) { return mix256(key); }
+
+// One thread per window of a flagged sequence; only windows that touch a non-ACGT symbol produce
+// a live record (the narrow kernel owns the others).  KeyT = Key128: k <= 32, records at wrec_off,
+// positional k-mers at pwide_off (pos_flags bit 1).  KeyT = Key256: k = 33..64, records at rec_off,
+// positional k-mers at pos_slot[list entry] (pos_flags bit 2; the positional record's k-mer index
+// is rewritten too) - after k1_extract_long, which wrote the windows' 2-bit records as dead ones.
+template <bool CANON, typename KeyT>
 __global__ void k1_extract_wide(const uint64_t* __restrict__ amb_codes,
                                 const SeqDev* __restrict__ seqs,
                                 const uint32_t* __restrict__ wide_seqs, uint32_t n_wide_seqs,
-                                int k, Key128* __restrict__ keys, uint32_t* __restrict__ vals,
+                                int k, KeyT* __restrict__ keys, uint32_t* __restrict__ vals,
                                 uint64_t* __restrict__ pos_wide, uint8_t* __restrict__ pos_flags,
-                                uint32_t* __restrict__ strand_bits /* compact positional form, else null */) {
+                                uint32_t* __restrict__ strand_bits /* compact positional form, else null */,
+                                uint64_t* __restrict__ pos_kmer = nullptr, const uint32_t* __restrict__ pos_slot = nullptr) {
+  constexpr bool kX = sizeof(KeyT) == sizeof(Key256);
+  constexpr uint8_t kFlag = kX ? 4u : 2u;
   const uint32_t lane = lane_id();
   const uint32_t warp = threadIdx.x >> 5;
   const uint32_t stride = gridDim.x * (blockDim.x >> 5);
@@ -281,49 +322,51 @@ __global__ void k1_extract_wide(const uint64_t* __restrict__ amb_codes,
     if (d.len < (uint32_t)k) continue;
     const uint32_t nwin = d.len - (uint32_t)k + 1u;
     const bool target = (d.flags & 1u) != 0u;
+    const uint32_t rec0 = kX ? d.rec_off : d.wrec_off;
+    const uint32_t slot0 = kX ? (pos_slot ? pos_slot[wsi] : 0u) : d.pwide_off;
     for (uint32_t p = lane; p < nwin; p += 32u) {
-      Key128 f{0, 0}, r{0, 0};
+      KeyT f = KeyTraits<KeyT>::zero(), r = KeyTraits<KeyT>::zero();
       bool is_amb = false;
       for (int i = 0; i < k; ++i) {
         const uint64_t sym = d.amb_off + p + (uint32_t)i;
         const uint32_t c = (uint32_t)(amb_codes[sym >> 4] >> (60 - 4 * (sym & 15u))) & 15u;
         is_amb |= !((c == 0u) | (c == 2u) | (c == 4u) | (c == 11u));
-        // forward: first symbol ends up in the top used nibble
-        f.hi = (f.hi << 4) | (f.lo >> 60);
-        f.lo = (f.lo << 4) | c;
-        // reverse complement: symbol i becomes nibble i from the bottom
-        const uint64_t cc = comp4(c);
-        if (i < 16) r.lo |= cc << (4 * i); else r.hi |= cc << (4 * (i - 16));
+        push4(f, c);                 // forward: first symbol ends up in the top used nibble
+        set4(r, i, comp4(c));        // reverse complement: symbol i becomes nibble i from the bottom
       }
-      // r currently has comp(sym_i) at nibble i (LSB side) = reversed order: top nibble
-      // (k-1) holds comp(sym_{k-1}) which is the first symbol of the reverse complement.
+      // r has comp(sym_i) at nibble i (LSB side) = reversed order: top nibble (k-1) holds
+      // comp(sym_{k-1}) which is the first symbol of the reverse complement.
+      const size_t slot = (size_t)slot0 + p;
       if (CANON) {
         const bool use_rc = r < f;
-        const Key128 canon = use_rc ? r : f;
-        const size_t rec = (size_t)d.wrec_off + p;
-        keys[rec] = is_amb ? mix128(canon) : Key128{0, 0};
+        const KeyT canon = use_rc ? r : f;
+        const size_t rec = (size_t)rec0 + p;
+        keys[rec] = is_amb ? mix_key(canon) : KeyTraits<KeyT>::zero();
         vals[rec] = is_amb ? d.sample : kInvalidSample;
         if (target && is_amb && strand_bits) {
-          // runs after k1_strand_bits on the same stream: the strand choice of an ambiguous
-          // window must come from the 4-bit comparison
+          // runs after k1_strand_bits / k1_extract_long on the same stream: the strand choice of
+          // an ambiguous window must come from the 4-bit comparison
           const uint64_t i = d.base_off + p;
           if (use_rc) atomicOr(&strand_bits[i >> 5], 1u << (i & 31u));
           else atomicAnd(&strand_bits[i >> 5], ~(1u << (i & 31u)));
         } else if (target && is_amb) {
-          pos_wide[2 * ((size_t)d.pwide_off + p)] = canon.hi;
-          pos_wide[2 * ((size_t)d.pwide_off + p) + 1] = canon.lo;
-          // runs after the narrow kernel on the same stream: the strand choice of an
+          store_kmer(pos_wide, slot, canon);
+          // runs after the narrow / long kernel on the same stream: the strand choice of an
           // ambiguous window must come from the 4-bit comparison
-          pos_flags[(size_t)d.pos_off + p] = (uint8_t)((use_rc ? 1u : 0u) | 2u);
+          pos_flags[(size_t)d.pos_off + p] = (uint8_t)((use_rc ? 1u : 0u) | kFlag);
+          if (kX) pos_kmer[(size_t)d.pos_off + p] = slot;
         }
       } else {
-        const size_t rec = (size_t)d.wrec_off + 2 * (size_t)p;
-        keys[rec] = is_amb ? mix128(f) : Key128{0, 0};
-        keys[rec + 1] = is_amb ? mix128(r) : Key128{0, 0};
+        const size_t rec = (size_t)rec0 + 2 * (size_t)p;
+        keys[rec] = is_amb ? mix_key(f) : KeyTraits<KeyT>::zero();
+        keys[rec + 1] = is_amb ? mix_key(r) : KeyTraits<KeyT>::zero();
         vals[rec] = vals[rec + 1] = is_amb ? d.sample : kInvalidSample;
         if (target && is_amb && pos_wide) {
-          pos_wide[2 * ((size_t)d.pwide_off + p)] = f.hi;
-          pos_wide[2 * ((size_t)d.pwide_off + p) + 1] = f.lo;
+          store_kmer(pos_wide, slot, f);
+          if (kX) {
+            pos_flags[(size_t)d.pos_off + p] = kFlag;
+            pos_kmer[(size_t)d.pos_off + p] = slot;
+          }
         }
       }
     }

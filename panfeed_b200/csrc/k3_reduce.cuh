@@ -124,9 +124,17 @@ __device__ __forceinline__ uint64_t shfl_key(uint64_t k, int src) { return __shf
 __device__ __forceinline__ Key128 shfl_key(const Key128& k, int src) {
   return Key128{__shfl_sync(kFull, k.hi, src), __shfl_sync(kFull, k.lo, src)};
 }
+__device__ __forceinline__ Key256 shfl_key(const Key256& k, int src) {
+  return Key256{{__shfl_sync(kFull, k.w[0], src), __shfl_sync(kFull, k.w[1], src),
+                 __shfl_sync(kFull, k.w[2], src), __shfl_sync(kFull, k.w[3], src)}};
+}
 __device__ __forceinline__ uint64_t shfl_xor_key(uint64_t k, int m) { return __shfl_xor_sync(kFull, k, m); }
 __device__ __forceinline__ Key128 shfl_xor_key(const Key128& k, int m) {
   return Key128{__shfl_xor_sync(kFull, k.hi, m), __shfl_xor_sync(kFull, k.lo, m)};
+}
+__device__ __forceinline__ Key256 shfl_xor_key(const Key256& k, int m) {
+  return Key256{{__shfl_xor_sync(kFull, k.w[0], m), __shfl_xor_sync(kFull, k.w[1], m),
+                 __shfl_xor_sync(kFull, k.w[2], m), __shfl_xor_sync(kFull, k.w[3], m)}};
 }
 // minimum over lanes whose `has` is set; returns whether any lane had one
 template <typename KeyT>
@@ -141,14 +149,11 @@ __device__ __forceinline__ bool warp_min_key(KeyT& key, bool has) {
 }
 __device__ __forceinline__ uint64_t unmix_key(uint64_t k) { return unmix64(k); }
 __device__ __forceinline__ Key128 unmix_key(const Key128& k) { return unmix128(k); }
-__device__ __forceinline__ void store_kmer(uint64_t* out, size_t row, uint64_t k) { out[row] = k; }
-__device__ __forceinline__ void store_kmer(uint64_t* out, size_t row, const Key128& k) {
-  out[2 * row] = k.hi; out[2 * row + 1] = k.lo;
-}
+__device__ __forceinline__ Key256 unmix_key(const Key256& k) { return unmix256(k); }
 
 struct RowOut {
   uint32_t* cluster;
-  uint64_t* kmer;          // 1 word per row (narrow) or 2 (wide)
+  uint64_t* kmer;          // 1 word per row (narrow), 2 (wide) or 4 (256-bit keys)
   uint32_t* count;
   uint32_t* cand;          // rows x key_words
   uint32_t key_words;      // W (+1 with consider_missing)
@@ -194,12 +199,14 @@ k3_runs(const KeyT* __restrict__ keys, const uint32_t* __restrict__ vals,
         const uint32_t* __restrict__ run_start, const uint32_t* __restrict__ run_seg,
         uint32_t n_runs, uint32_t n_records, const ClusterDev* __restrict__ clusters,
         uint32_t* __restrict__ nrows /* COUNT: out counts; EMIT: exclusive offsets (n_runs+1) */,
-        RowOut out) {
+        RowOut out,
+        uint32_t* __restrict__ n_unique = nullptr /* COUNT: += distinct live keys (may be null) */) {
   extern __shared__ uint32_t k3_smem[];
   const uint32_t lane = lane_id(), warp = threadIdx.x >> 5;
   const uint32_t W = out.pattern_words;
   uint32_t* bits = k3_smem + (size_t)warp * W;
   const uint32_t total_warps = gridDim.x * (blockDim.x >> 5);
+  uint32_t distinct = 0;                 // live keys of this warp's runs (n_unique only)
   for (uint32_t r = blockIdx.x * (blockDim.x >> 5) + warp; r < n_runs; r += total_warps) {
     uint32_t row0 = 0;
     if (EMIT) {
@@ -234,6 +241,7 @@ k3_runs(const KeyT* __restrict__ keys, const uint32_t* __restrict__ vals,
       clean = __all_sync(kFull, clean);
       if (same && clean) {
         if (lane == 0) nrows[r] = (cnt >= cl.lo && cnt <= cl.hi) ? 1u : 0u;
+        ++distinct;
         continue;
       }
     }
@@ -254,6 +262,7 @@ k3_runs(const KeyT* __restrict__ keys, const uint32_t* __restrict__ vals,
       if (!warp_min_key(best, has)) break;
       cur = best;
       have_cur = true;
+      ++distinct;
       const uint32_t c = build_bitset(keys, vals, a, b, cur, bits, W);
       if (c >= cl.lo && c <= cl.hi && c > 0u) {
         if (EMIT) {
@@ -273,6 +282,7 @@ k3_runs(const KeyT* __restrict__ keys, const uint32_t* __restrict__ vals,
     }
     if (!EMIT && lane == 0) nrows[r] = n_out;
   }
+  if (!EMIT && n_unique && lane == 0 && distinct) atomicAdd(n_unique, distinct);
 }
 
 // ---- in-place exclusive scan of a u32 array (three small kernels) ----------

@@ -73,6 +73,39 @@ __host__ __device__ __forceinline__ Key128 unmix128(Key128 k) {
   return k;
 }
 
+// 256-bit key for windows of 33..64 symbols holding N/IUPAC symbols: 4 bits per symbol (codes of
+// PF_AMB_ALPHABET), first symbol in the top used bits, w[0] the most significant word.  Unsigned
+// comparison over the words is the reference's string order, as for Key128.
+struct Key256 {
+  uint64_t w[4];
+};
+__host__ __device__ __forceinline__ bool operator==(const Key256& a, const Key256& b) {
+  return a.w[0] == b.w[0] && a.w[1] == b.w[1] && a.w[2] == b.w[2] && a.w[3] == b.w[3];
+}
+__host__ __device__ __forceinline__ bool operator!=(const Key256& a, const Key256& b) {
+  return !(a == b);
+}
+__host__ __device__ __forceinline__ bool operator<(const Key256& a, const Key256& b) {
+  if (a.w[0] != b.w[0]) return a.w[0] < b.w[0];
+  if (a.w[1] != b.w[1]) return a.w[1] < b.w[1];
+  if (a.w[2] != b.w[2]) return a.w[2] < b.w[2];
+  return a.w[3] < b.w[3];
+}
+// Bijection on 256 bits: the last word takes a hash of the first three, then the leading word a
+// hash of the (new) last one, which by then depends on all 256 bits.
+__host__ __device__ __forceinline__ Key256 mix256(Key256 k) {
+  k.w[3] ^= fmix64(k.w[0] + 0x9e3779b97f4a7c15ULL) ^ fmix64(k.w[1] + 0xd1b54a32d192ed03ULL) ^
+            fmix64(k.w[2] + 0x8cb92ba72f3d8dd7ULL);
+  k.w[0] ^= fmix64(k.w[3] + 0xa0761d6478bd642fULL);
+  return k;
+}
+__host__ __device__ __forceinline__ Key256 unmix256(Key256 k) {
+  k.w[0] ^= fmix64(k.w[3] + 0xa0761d6478bd642fULL);
+  k.w[3] ^= fmix64(k.w[0] + 0x9e3779b97f4a7c15ULL) ^ fmix64(k.w[1] + 0xd1b54a32d192ed03ULL) ^
+            fmix64(k.w[2] + 0x8cb92ba72f3d8dd7ULL);
+  return k;
+}
+
 // Leading `bits` of a key, right-aligned digit extraction for the radix passes.
 __device__ __forceinline__ uint32_t key_digit(uint64_t k, int shift) {
   return (uint32_t)(k >> shift) & 255u;
@@ -82,11 +115,26 @@ __device__ __forceinline__ uint32_t key_digit(const Key128& k, int shift) {
   // ones, so shift >= 64 whenever sort_bits <= 64 (always).
   return (uint32_t)(k.hi >> (shift - 64)) & 255u;
 }
+__device__ __forceinline__ uint32_t key_digit(const Key256& k, int shift) {
+  return (uint32_t)(k.w[0] >> (shift - 192)) & 255u;      // (the same on the leading word)
+}
 __device__ __forceinline__ uint64_t key_prefix(uint64_t k, int sort_bits) {
   return sort_bits >= 64 ? k : (k >> (64 - sort_bits));
 }
 __device__ __forceinline__ uint64_t key_prefix(const Key128& k, int sort_bits) {
   return sort_bits >= 64 ? k.hi : (k.hi >> (64 - sort_bits));
+}
+__device__ __forceinline__ uint64_t key_prefix(const Key256& k, int sort_bits) {
+  return sort_bits >= 64 ? k.w[0] : (k.w[0] >> (64 - sort_bits));
+}
+// k-mer `row` of an output array of 1, 2 or 4 words per k-mer, most significant word first
+__device__ __forceinline__ void store_kmer(uint64_t* out, size_t row, uint64_t k) { out[row] = k; }
+__device__ __forceinline__ void store_kmer(uint64_t* out, size_t row, const Key128& k) {
+  out[2 * row] = k.hi; out[2 * row + 1] = k.lo;
+}
+__device__ __forceinline__ void store_kmer(uint64_t* out, size_t row, const Key256& k) {
+#pragma unroll
+  for (int i = 0; i < 4; ++i) out[4 * row + i] = k.w[i];
 }
 template <typename K> struct KeyTraits;
 template <> struct KeyTraits<uint64_t> {
@@ -96,6 +144,10 @@ template <> struct KeyTraits<uint64_t> {
 template <> struct KeyTraits<Key128> {
   static constexpr int kBits = 128;
   __device__ static __forceinline__ Key128 zero() { return Key128{0, 0}; }
+};
+template <> struct KeyTraits<Key256> {
+  static constexpr int kBits = 256;
+  __device__ static __forceinline__ Key256 zero() { return Key256{{0, 0, 0, 0}}; }
 };
 
 // ---- relaxed gpu-scope accesses for the decoupled look-back chains --------
@@ -146,19 +198,21 @@ struct SeqDev {          // 64 bytes
   uint32_t cluster;      // batch-local
   uint32_t flags;
   int32_t start, end, offset, strand;
-  uint32_t rec_off;      // first record in the narrow record arrays
+  uint32_t rec_off;      // first record in the narrow record arrays; k > 32 (no narrow records):
+                         // first record in the 256-bit record arrays (sequences with N/IUPAC)
   uint32_t pos_off;      // first positional record
   uint32_t wrec_off;     // first record in the wide record arrays
   uint32_t pwide_off;    // first slot in the wide positional k-mer array (targets with N/IUPAC)
 };
 static_assert(sizeof(SeqDev) == 64, "SeqDev");
 
-struct ClusterDev {      // 32 bytes
+struct ClusterDev {      // 40 bytes
   uint32_t rec_start, rec_end;   // narrow record range (a segment of the sort)
   uint32_t id;
   uint32_t lo, hi;               // surviving sample counts, filters folded in
   uint32_t n_present;
   uint32_t wrec_start, wrec_end; // wide record range
+  uint32_t xrec_start, xrec_end; // 256-bit record range (k > 32, windows with N/IUPAC symbols)
 };
 
 struct TileDev {         // 16 bytes: one sort tile, never crossing a segment

@@ -5,12 +5,14 @@ namespace pf {
 // ---- planning helpers that run on the device (tile lists are pure functions of the
 //      per-cluster record ranges; generating them there saves host loops and H2D) -------
 __global__ void plan_expand_tiles(const ClusterDev* __restrict__ clusters, uint32_t n_clusters,
-                                  const uint32_t* __restrict__ tile_base, uint32_t tile_size, int wide,
+                                  const uint32_t* __restrict__ tile_base, uint32_t tile_size,
+                                  int width /* record range: 0 narrow, 1 wide, 2 256-bit */,
                                   TileDev* __restrict__ tiles) {
   const uint32_t c = blockIdx.x;
   if (c >= n_clusters) return;
-  const uint32_t lo = wide ? clusters[c].wrec_start : clusters[c].rec_start;
-  const uint32_t hi = wide ? clusters[c].wrec_end : clusters[c].rec_end;
+  const ClusterDev& cd = clusters[c];
+  const uint32_t lo = width == 2 ? cd.xrec_start : width ? cd.wrec_start : cd.rec_start;
+  const uint32_t hi = width == 2 ? cd.xrec_end : width ? cd.wrec_end : cd.rec_end;
   const uint32_t first = tile_base[c];
   const uint32_t n = (hi - lo + tile_size - 1) / tile_size;
   for (uint32_t i = threadIdx.x; i < n; i += blockDim.x) {
@@ -109,7 +111,7 @@ struct PatternSpace {
   const uint32_t* x_unique_mirror = nullptr;
 };
 
-struct WidthState {       // per key width (narrow u64 / wide Key128)
+struct WidthState {       // per key width (narrow u64 / wide Key128 / Key256)
   DevBuf keys[2], vals[2];
   DevBuf tiles, seg_start, seg_hist, lookback, cursors;
   DevBuf ltiles, tile_first_run;     // partition mode: 2048-record tiles of the local reduce
@@ -135,14 +137,16 @@ struct BatchState {
   bool have_batch = false, executed = false;
   uint32_t n_seqs = 0, n_clusters = 0, n_wide_seqs = 0;
   uint64_t n_words = 0, n_amb_words = 0, n_bases = 0;
-  uint32_t n_pos = 0, n_pos_wide = 0;
+  uint32_t n_pos = 0, n_pos_wide = 0, n_pos_xwide = 0;
   PinBuf h_seqs, h_clusters, h_wide_seqs;
-  DevBuf d_bases, d_amb, d_ambbits, d_seqs, d_clusters, d_wide_seqs, d_presence;
+  PinBuf h_xpos_slot;            // k > 32: first positional 256-bit slot of every listed ambiguous sequence
+  DevBuf d_bases, d_amb, d_ambbits, d_seqs, d_clusters, d_wide_seqs, d_presence, d_xpos_slot;
   WidthState nar, wid;
-  // rows (narrow first, then wide)
-  DevBuf d_row_cluster, d_row_kmer, d_wrow_kmer, d_row_count, d_row_pattern;
+  WidthState xwd;                // k > 32: the windows holding N/IUPAC symbols, Key256 records
+  // rows (narrow first, then wide, then 256-bit)
+  DevBuf d_row_cluster, d_row_kmer, d_wrow_kmer, d_xrow_kmer, d_row_count, d_row_pattern;
   DevBuf d_cl_pattern;
-  DevBuf d_pos_kmer, d_pos_seq, d_pos_cstart, d_pos_gstart, d_pos_flags, d_pos_wide;
+  DevBuf d_pos_kmer, d_pos_seq, d_pos_cstart, d_pos_gstart, d_pos_flags, d_pos_wide, d_pos_xwide;
   DevBuf d_pos_bits;             // compact positional form: used_strand bit plane, indexed like d_bases
   DevBuf d_seq_rec_off, d_tile_first_seq;
   PinBuf h_seq_rec_off, h_tile_first_seq;
@@ -328,9 +332,9 @@ struct pf_ctx : BatchState {
   uint32_t merge_slots = 49152;  // shared-memory merge table of kB1_local (PF_MERGE_SMEM_KB)
   PatternSpace kp, cp;     // k-mer patterns, cluster patterns
   // pinned results
-  PinBuf r_row_cluster, r_row_kmer, r_wrow_kmer, r_row_count, r_row_pattern, r_cl_pattern;
+  PinBuf r_row_cluster, r_row_kmer, r_wrow_kmer, r_xrow_kmer, r_row_count, r_row_pattern, r_cl_pattern;
   PinBuf r_new_kp, r_new_cp, r_pos_kmer, r_pos_seq, r_pos_cstart, r_pos_gstart, r_pos_flags,
-      r_pos_wide, r_pos_bits;
+      r_pos_wide, r_pos_xwide, r_pos_bits;
   PinBuf r_wrow_cluster, r_wrow_count, r_wrow_pattern;   // pipelined submit: wide rows apart
   cudaEvent_t ev_d2h[2]{};
   pf_stats stats{};
@@ -601,7 +605,11 @@ enum { C_TICKET_N = 0, C_TICKET_W = 1, C_RUNS_N = 2, C_RUNS_W = 3, C_ERR = 4, C_
        C_ROWS_W = 6, C_NEW_KP = 7, C_NEW_CP = 8, C_TICKET_MARK_N = 9, C_TICKET_MARK_W = 10,
        C_LOCAL = 11 /* LC_COUNT words: rows, unique, table overflow, row overflow, rescue runs,
                         partial rows, partial overflow, kA segments */,
-       C_X_UNIQUE_KP = 19, C_X_UNIQUE_CP = 20 /* owner-side unique counts of the exchange */, C_COUNT = 24 };
+       C_X_UNIQUE_KP = 19, C_X_UNIQUE_CP = 20 /* owner-side unique counts of the exchange */,
+       C_TICKET_X = 21, C_RUNS_X = 22, C_ROWS_X = 23, C_TICKET_MARK_X = 24 /* 256-bit keys (k > 32) */,
+       C_UNIQUE_WX = 25 /* distinct live keys of the wide and 256-bit records (k > 32 with N/IUPAC) */,
+       C_COUNT = 28 };
+static_assert(C_COUNT <= 32, "mirror_counters copies one warp's worth");
 static_assert(C_LOCAL + LC_COUNT <= C_X_UNIQUE_KP, "counter layout");
 
 bool keep_count(double maf, uint32_t c, uint32_t n) {

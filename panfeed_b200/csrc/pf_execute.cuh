@@ -131,8 +131,9 @@ int scan_inplace(pf_ctx* ctx, uint32_t* data, uint32_t n, uint32_t* total_dev, c
   return PF_OK;
 }
 
+// n_unique (COUNT pass, may be null): += the distinct live keys of the runs
 template <typename KeyT, bool EMIT>
-int runs_width(pf_ctx* ctx, WidthState& w, RowOut out) {
+int runs_width(pf_ctx* ctx, WidthState& w, RowOut out, uint32_t* n_unique = nullptr) {
   if (w.n_runs == 0) return PF_OK;
   cudaStream_t st = ctx->stream;
   const int other = w.final_buf ^ 1;
@@ -143,7 +144,7 @@ int runs_width(pf_ctx* ctx, WidthState& w, RowOut out) {
   const uint32_t grid = std::min<uint32_t>(cdiv(w.n_runs, 8), kGridPersist * 2);
   k3_runs<KeyT, EMIT><<<grid, 256, smem, st>>>(w.keys[w.final_buf].as<KeyT>(), w.vals[w.final_buf].as<uint32_t>(),
                                                run_start, run_seg, w.n_runs, w.n_records,
-                                               ctx->d_clusters.as<ClusterDev>(), nrows, out);
+                                               ctx->d_clusters.as<ClusterDev>(), nrows, out, n_unique);
   ctx->launches++;
   CU(cudaGetLastError());
   return PF_OK;
@@ -288,28 +289,51 @@ int launch_k1(pf_ctx* ctx) {
     const uint32_t grid = std::min<uint32_t>(cdiv(ctx->n_seqs, kK1Warps), 148 * 8);
     uint32_t* bits = compact && ctx->n_pos && P.canonical ? ctx->d_pos_bits.as<uint32_t>() : nullptr;
     if (P.canonical)
-      k1_extract_long<true><<<grid, kK1Warps * 32, 0, st>>>(ctx->d_bases.as<uint64_t>(), ctx->d_seqs.as<SeqDev>(), ctx->n_seqs,
+      k1_extract_long<true><<<grid, kK1Warps * 32, 0, st>>>(ctx->d_bases.as<uint64_t>(), ctx->d_ambbits.as<uint32_t>(),
+                                                            ctx->d_seqs.as<SeqDev>(), ctx->n_seqs,
                                                             (int)P.k, Wd.keys[0].as<Key128>(), Wd.vals[0].as<uint32_t>(), po,
                                                             ctx->d_pos_wide.as<uint64_t>(), bits);
     else
-      k1_extract_long<false><<<grid, kK1Warps * 32, 0, st>>>(ctx->d_bases.as<uint64_t>(), ctx->d_seqs.as<SeqDev>(), ctx->n_seqs,
+      k1_extract_long<false><<<grid, kK1Warps * 32, 0, st>>>(ctx->d_bases.as<uint64_t>(), ctx->d_ambbits.as<uint32_t>(),
+                                                             ctx->d_seqs.as<SeqDev>(), ctx->n_seqs,
                                                              (int)P.k, Wd.keys[0].as<Key128>(), Wd.vals[0].as<uint32_t>(), po,
                                                              ctx->d_pos_wide.as<uint64_t>(), nullptr);
     ctx->launches++;
+    WidthState& X = ctx->xwd;
+    if (ctx->n_wide_seqs && X.n_records) {
+      // windows holding N/IUPAC symbols: 256-bit records, and their positional records / strand
+      // bits corrected behind k1_extract_long (same stream)
+      const uint32_t xg = std::min<uint32_t>(cdiv(ctx->n_wide_seqs, 8), 148 * 8);
+      uint64_t* pk = compact ? nullptr : ctx->d_pos_kmer.as<uint64_t>();
+      uint64_t* px = compact ? nullptr : ctx->d_pos_xwide.as<uint64_t>();
+      if (P.canonical)
+        k1_extract_wide<true, Key256><<<xg, 256, 0, st>>>(ctx->d_amb.as<uint64_t>(), ctx->d_seqs.as<SeqDev>(),
+                                                          ctx->d_wide_seqs.as<uint32_t>(), ctx->n_wide_seqs, (int)P.k,
+                                                          X.keys[0].as<Key256>(), X.vals[0].as<uint32_t>(), px,
+                                                          ctx->d_pos_flags.as<uint8_t>(), bits, pk,
+                                                          ctx->d_xpos_slot.as<uint32_t>());
+      else
+        k1_extract_wide<false, Key256><<<xg, 256, 0, st>>>(ctx->d_amb.as<uint64_t>(), ctx->d_seqs.as<SeqDev>(),
+                                                           ctx->d_wide_seqs.as<uint32_t>(), ctx->n_wide_seqs, (int)P.k,
+                                                           X.keys[0].as<Key256>(), X.vals[0].as<uint32_t>(), px,
+                                                           ctx->d_pos_flags.as<uint8_t>(), nullptr, pk,
+                                                           ctx->d_xpos_slot.as<uint32_t>());
+      ctx->launches++;
+    }
   } else if (ctx->n_wide_seqs && Wd.n_records) {
     const uint32_t grid = std::min<uint32_t>(cdiv(ctx->n_wide_seqs, 8), 148 * 8);
     if (P.canonical)
-      k1_extract_wide<true><<<grid, 256, 0, st>>>(ctx->d_amb.as<uint64_t>(), ctx->d_seqs.as<SeqDev>(),
-                                                 ctx->d_wide_seqs.as<uint32_t>(), ctx->n_wide_seqs, (int)P.k,
-                                                 Wd.keys[0].as<Key128>(), Wd.vals[0].as<uint32_t>(),
-                                                 ctx->d_pos_wide.as<uint64_t>(), ctx->d_pos_flags.as<uint8_t>(),
-                                                 compact && ctx->n_pos ? ctx->d_pos_bits.as<uint32_t>() : nullptr);
+      k1_extract_wide<true, Key128><<<grid, 256, 0, st>>>(ctx->d_amb.as<uint64_t>(), ctx->d_seqs.as<SeqDev>(),
+                                                          ctx->d_wide_seqs.as<uint32_t>(), ctx->n_wide_seqs, (int)P.k,
+                                                          Wd.keys[0].as<Key128>(), Wd.vals[0].as<uint32_t>(),
+                                                          ctx->d_pos_wide.as<uint64_t>(), ctx->d_pos_flags.as<uint8_t>(),
+                                                          compact && ctx->n_pos ? ctx->d_pos_bits.as<uint32_t>() : nullptr);
     else
-      k1_extract_wide<false><<<grid, 256, 0, st>>>(ctx->d_amb.as<uint64_t>(), ctx->d_seqs.as<SeqDev>(),
-                                                  ctx->d_wide_seqs.as<uint32_t>(), ctx->n_wide_seqs, (int)P.k,
-                                                  Wd.keys[0].as<Key128>(), Wd.vals[0].as<uint32_t>(),
-                                                  compact ? nullptr : ctx->d_pos_wide.as<uint64_t>(),
-                                                  ctx->d_pos_flags.as<uint8_t>(), nullptr);
+      k1_extract_wide<false, Key128><<<grid, 256, 0, st>>>(ctx->d_amb.as<uint64_t>(), ctx->d_seqs.as<SeqDev>(),
+                                                           ctx->d_wide_seqs.as<uint32_t>(), ctx->n_wide_seqs, (int)P.k,
+                                                           Wd.keys[0].as<Key128>(), Wd.vals[0].as<uint32_t>(),
+                                                           compact ? nullptr : ctx->d_pos_wide.as<uint64_t>(),
+                                                           ctx->d_pos_flags.as<uint8_t>(), nullptr);
     ctx->launches++;
   }
   CU(cudaGetLastError());
@@ -574,6 +598,7 @@ extern "C" int pf_execute(pf_ctx* ctx) {
   const uint32_t launches0 = ctx->launches;
   WidthState& N = ctx->nar;
   WidthState& Wd = ctx->wid;
+  WidthState& X = ctx->xwd;      // k > 32, windows with N/IUPAC symbols (empty otherwise)
   uint32_t* counters = ctx->d_counters.as<uint32_t>();
   uint32_t* hcnt = ctx->h_counters.as<uint32_t>();
   ctx->executed = false;
@@ -595,6 +620,10 @@ extern "C" int pf_execute(pf_ctx* ctx) {
   for (int i = 0; i < 2; ++i) {
     TRY(dev_ensure(ctx, Wd.keys[i], ((size_t)Wd.n_records + 2) * 16));
     TRY(dev_ensure(ctx, Wd.vals[i], ((size_t)Wd.n_records + 2) * 4));
+    if (X.n_records) {
+      TRY(dev_ensure(ctx, X.keys[i], ((size_t)X.n_records + 2) * 32));
+      TRY(dev_ensure(ctx, X.vals[i], ((size_t)X.n_records + 2) * 4));
+    }
   }
   const bool compact_pos = ctx->prm.emit_positions == 2u;
   if (ctx->n_pos && compact_pos) {
@@ -607,6 +636,7 @@ extern "C" int pf_execute(pf_ctx* ctx) {
     TRY(dev_ensure(ctx, ctx->d_pos_flags, (size_t)ctx->n_pos));
   }
   if (ctx->n_pos_wide && !compact_pos) TRY(dev_ensure(ctx, ctx->d_pos_wide, (size_t)ctx->n_pos_wide * 16));
+  if (ctx->n_pos_xwide && !compact_pos) TRY(dev_ensure(ctx, ctx->d_pos_xwide, (size_t)ctx->n_pos_xwide * 32));
   TRY(dev_ensure(ctx, ctx->d_cl_pattern, std::max<size_t>(1, ctx->n_clusters) * 4));
   if (part) {
     uint64_t want_rows = std::max<uint64_t>(65536, (uint64_t)(ctx->row_ratio * 1.3 * (double)N.n_records) + 4096);
@@ -756,6 +786,7 @@ extern "C" int pf_execute(pf_ctx* ctx) {
       ctx->cp.n = ctx->cp_base + hcnt[C_NEW_CP];
       N.n_runs = 0;
       Wd.n_runs = Wd.n_records ? hcnt[C_RUNS_W] : 0;
+      X.n_runs = 0;
       if (hcnt[C_LOCAL + LC_PARTIAL_OVERFLOW]) {
         ctx->partial_cap = (uint64_t)hcnt[C_LOCAL + LC_PARTIALS] + 4096;
         continue;
@@ -777,10 +808,12 @@ extern "C" int pf_execute(pf_ctx* ctx) {
     CU(cudaEventRecord(ctx->ev[EV_EXTRACT], st));
     TRY(hist_width<uint64_t>(ctx, N, ctx->fused));
     TRY(hist_width<Key128>(ctx, Wd));
+    TRY(hist_width<Key256>(ctx, X));
     STAGE("k2_histogram");
     CU(cudaEventRecord(ctx->ev[EV_HIST], st));
     TRY(passes_width<uint64_t>(ctx, N, C_TICKET_N, part && ctx->use_direct, ctx->fused));
     TRY(passes_width<Key128>(ctx, Wd, C_TICKET_W));
+    TRY(passes_width<Key256>(ctx, X, C_TICKET_X));
     STAGE("k2_onesweep_pass");
     CU(cudaEventRecord(ctx->ev[EV_SORT], st));
     // ---- K3: runs -----------------------------------------------------------------
@@ -789,6 +822,7 @@ extern "C" int pf_execute(pf_ctx* ctx) {
     else TRY(mark_width<uint64_t>(ctx, N, C_TICKET_MARK_N, C_RUNS_N, part));
     STAGE("k3_mark_runs/k3_tiles_from_hist");
     TRY(mark_width<Key128>(ctx, Wd, C_TICKET_MARK_W, C_RUNS_W, false));
+    TRY(mark_width<Key256>(ctx, X, C_TICKET_MARK_X, C_RUNS_X, false));
     STAGE("k3_mark_runs<wide>");
     CU(cudaEventRecord(ctx->ev[EV_MARK], st));
     // local reduce (+ rescue launch of the direct variant), then one sync to read the counters
@@ -819,6 +853,7 @@ extern "C" int pf_execute(pf_ctx* ctx) {
     ctx->cp.n = ctx->cp_base + hcnt[C_NEW_CP];
     N.n_runs = N.n_records ? hcnt[C_RUNS_N] : 0;
     Wd.n_runs = Wd.n_records ? hcnt[C_RUNS_W] : 0;
+    X.n_runs = X.n_records ? hcnt[C_RUNS_X] : 0;
     if (!part || N.n_records == 0) break;
     if (attempt > 10) return fail(ctx, PF_ERR_INTERNAL, "partition mode did not converge");
     if (hcnt[C_LOCAL + LC_TABLE_OVERFLOW]) {
@@ -858,29 +893,37 @@ extern "C" int pf_execute(pf_ctx* ctx) {
   } else {
     TRY((runs_width<uint64_t, false>(ctx, N, ro)));
   }
-  TRY((runs_width<Key128, false>(ctx, Wd, ro)));
+  // with 256-bit records (k > 32, N/IUPAC symbols) both wide sections hold dead records of the
+  // windows the other one owns: their runs are counted by distinct live keys, not one per run
+  const bool exact_unique = X.n_records > 0;
+  TRY((runs_width<Key128, false>(ctx, Wd, ro, exact_unique ? counters + C_UNIQUE_WX : nullptr)));
+  TRY((runs_width<Key256, false>(ctx, X, ro, counters + C_UNIQUE_WX)));
   CU(cudaEventRecord(ctx->ev[EV_COUNTED], st));
-  const bool need_scan = (!part && N.n_runs) || Wd.n_runs;
+  const bool need_scan = (!part && N.n_runs) || Wd.n_runs || X.n_runs;
   if (need_scan) {
     if (!part && N.n_runs)
       TRY(scan_inplace(ctx, N.vals[N.final_buf ^ 1].as<uint32_t>(), N.n_runs, counters + C_ROWS_N));
     if (Wd.n_runs) TRY(scan_inplace(ctx, Wd.vals[Wd.final_buf ^ 1].as<uint32_t>(), Wd.n_runs, counters + C_ROWS_W));
+    if (X.n_runs) TRY(scan_inplace(ctx, X.vals[X.final_buf ^ 1].as<uint32_t>(), X.n_runs, counters + C_ROWS_X));
     mirror_counters<<<1, 32, 0, st>>>(hcnt, counters, C_COUNT);
     CU(cudaStreamSynchronize(st));
     if (!part) N.n_rows = N.n_runs ? hcnt[C_ROWS_N] : 0;
     Wd.n_rows = Wd.n_runs ? hcnt[C_ROWS_W] : 0;
+    X.n_rows = X.n_runs ? hcnt[C_ROWS_X] : 0;
   } else {
     if (!part) N.n_rows = 0;
     Wd.n_rows = 0;
+    X.n_rows = 0;
   }
   if (!part) ctx->unique_last = N.n_runs;
-  ctx->unique_last += Wd.n_runs;
-  const uint64_t rows = (uint64_t)N.n_rows + Wd.n_rows;
+  ctx->unique_last += exact_unique ? hcnt[C_UNIQUE_WX] : Wd.n_runs;
+  const uint64_t rows = (uint64_t)N.n_rows + Wd.n_rows + X.n_rows;
   if (rows >= (1ull << 31)) return fail(ctx, PF_ERR_INVALID, "batch yields 2^31 rows or more; split it");
 
-  if (!part || Wd.n_rows) TRY(ensure_rows(ctx, std::max<uint64_t>(rows, part ? ctx->row_cap : 0),
-                                          std::max<uint64_t>(N.n_rows, part ? ctx->row_cap : 0), part));
+  if (!part || Wd.n_rows || X.n_rows) TRY(ensure_rows(ctx, std::max<uint64_t>(rows, part ? ctx->row_cap : 0),
+                                                      std::max<uint64_t>(N.n_rows, part ? ctx->row_cap : 0), part));
   TRY(dev_ensure(ctx, ctx->d_wrow_kmer, std::max<size_t>(1, Wd.n_rows) * 16));
+  if (X.n_rows) TRY(dev_ensure(ctx, ctx->d_xrow_kmer, (size_t)X.n_rows * 32));
   ro.cluster = ctx->d_row_cluster.as<uint32_t>();
   ro.count = ctx->d_row_count.as<uint32_t>();
   ro.cand = ctx->d_cand.as<uint32_t>();
@@ -893,6 +936,11 @@ extern "C" int pf_execute(pf_ctx* ctx) {
     ro.kmer = ctx->d_wrow_kmer.as<uint64_t>();
     ro.row_base = N.n_rows;
     TRY((runs_width<Key128, true>(ctx, Wd, ro)));
+  }
+  if (X.n_rows) {             // after the wide rows: K4 numbers the patterns of all three sections at once
+    ro.kmer = ctx->d_xrow_kmer.as<uint64_t>();
+    ro.row_base = N.n_rows + Wd.n_rows;
+    TRY((runs_width<Key256, true>(ctx, X, ro)));
   }
   CU(cudaEventRecord(ctx->ev[EV_REDUCE], st));
 
@@ -910,6 +958,10 @@ extern "C" int pf_execute(pf_ctx* ctx) {
     CU(cudaMemcpyAsync(ctx->r_row_count.p, ctx->d_row_count.p, rows * 4, cudaMemcpyDeviceToHost, ctx->copy_stream));
     if (N.n_rows) CU(cudaMemcpyAsync(ctx->r_row_kmer.p, ctx->d_row_kmer.p, (size_t)N.n_rows * 8, cudaMemcpyDeviceToHost, ctx->copy_stream));
     if (Wd.n_rows) CU(cudaMemcpyAsync(ctx->r_wrow_kmer.p, ctx->d_wrow_kmer.p, (size_t)Wd.n_rows * 16, cudaMemcpyDeviceToHost, ctx->copy_stream));
+    if (X.n_rows) {
+      TRY(pin_ensure(ctx, ctx->r_xrow_kmer, (size_t)X.n_rows * 32));
+      CU(cudaMemcpyAsync(ctx->r_xrow_kmer.p, ctx->d_xrow_kmer.p, (size_t)X.n_rows * 32, cudaMemcpyDeviceToHost, ctx->copy_stream));
+    }
     ctx->rows_prefetched = true;
   }
 

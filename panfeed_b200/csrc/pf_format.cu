@@ -50,20 +50,16 @@ inline int len_int(int64_t v) {
   return len;
 }
 
-// text of a two-word k-mer [hi, lo], first symbol in the top used bits: 4 bits per symbol (N/IUPAC
-// k-mers, k <= 32) or, for k > 32, 2 bits per base
-inline void wide_kmer_text(const uint64_t* w, uint32_t k, char* out) {
-  if (k > 32) {
-    for (uint32_t s = 0; s < k; ++s) {
-      const uint32_t pos = 2 * (k - 1 - s);
-      out[s] = kAcgt[((pos < 64 ? w[1] >> pos : w[0] >> (pos - 64))) & 3u];
-    }
-    return;
-  }
+// text of a k-mer of n_words words (most significant first), first symbol in the top used bits:
+// 4 bits per symbol (codes of PF_AMB_ALPHABET) when k symbols fit that way (two words: N/IUPAC
+// k-mers of k <= 32; four words: k <= 64), else 2 bits per base (two words, k > 32)
+inline void wide_kmer_text(const uint64_t* w, uint32_t n_words, uint32_t k, char* out) {
+  const uint32_t bits = k <= 16 * n_words ? 4u : 2u;
+  const char* alphabet = bits == 4u ? kAmb : kAcgt;
+  const uint64_t mask = (1ull << bits) - 1ull;
   for (uint32_t s = 0; s < k; ++s) {
-    const uint32_t nib = k - 1 - s;
-    const uint64_t word = nib < 16 ? w[1] : w[0];
-    out[s] = kAmb[(word >> (4 * (nib % 16))) & 15u];
+    const uint32_t pos = bits * (k - 1 - s);              // from bit 0 of the last word
+    out[s] = alphabet[(w[n_words - 1 - pos / 64] >> (pos % 64)) & mask];
   }
 }
 
@@ -79,8 +75,10 @@ struct Job {
 // k-mer text of record i into `out` (k bytes)
 inline void kmer_text(const Job& j, uint64_t i, char* out) {
   const uint32_t k = j.k;
-  if (j.r->pos_flags[i] & 2u) {
-    wide_kmer_text(j.r->pos_wide_kmer + 2 * j.r->pos_kmer[i], k, out);
+  if (j.r->pos_flags[i] & 4u) {
+    wide_kmer_text(j.r->pos_xwide_kmer + 4 * j.r->pos_kmer[i], 4, k, out);
+  } else if (j.r->pos_flags[i] & 2u) {
+    wide_kmer_text(j.r->pos_wide_kmer + 2 * j.r->pos_kmer[i], 2, k, out);
   } else {
     const uint64_t v = j.r->pos_kmer[i];
     for (uint32_t s = 0; s < k; ++s) out[s] = kAcgt[(v >> (2 * (k - 1 - s))) & 3u];
@@ -601,13 +599,14 @@ extern "C" int pf_format_kmer_rows(const pf_batch_result* r, uint32_t k, const c
                                    const char* cluster_ids, uint64_t n_cluster_ids, char* out, uint64_t out_cap,
                                    uint64_t* out_len, uint64_t* cluster_off, uint32_t n_threads) {
   if (!r || !out_len || !tag_off || k == 0 || k > 64) return PF_ERR_INVALID;
-  const uint64_t nc = r->n_clusters, nn = r->n_rows, nw = r->n_wide_rows;
+  const uint64_t nc = r->n_clusters, nn = r->n_rows, nw = r->n_wide_rows, nx = r->n_xwide_rows;
   *out_len = 0;
-  if (nc >= (1ull << 32) || nn >= (1ull << 32) || nw >= (1ull << 32)) return PF_ERR_INVALID;
+  if (nc >= (1ull << 32) || nn >= (1ull << 32) || nw >= (1ull << 32) || nx >= (1ull << 32)) return PF_ERR_INVALID;
   if (nc && (!tag_blob || !cluster_ids || !r->cluster_pattern)) return PF_ERR_INVALID;
   if (nn && (!r->row_cluster || !r->row_kmer || !r->row_pattern || !kmer_ids)) return PF_ERR_INVALID;
   if (nw && (!r->wide_row_cluster || !r->wide_row_kmer || !r->wide_row_pattern || !kmer_ids)) return PF_ERR_INVALID;
-  if (nc == 0) return (nn || nw) ? PF_ERR_INVALID : PF_OK;
+  if (nx && (!r->xwide_row_cluster || !r->xwide_row_kmer || !r->xwide_row_pattern || !kmer_ids)) return PF_ERR_INVALID;
+  if (nc == 0) return (nn || nw || nx) ? PF_ERR_INVALID : PF_OK;
   if (nn && k > 32) return PF_ERR_INVALID;             // one-word k-mers hold at most 32 bases
   // rows of every cluster (narrow rows; the wide ones, few, below).  The block engine writes the
   // rows of a cluster as ONE run (a CTA per cluster reserves them with one atomic), clusters in any
@@ -640,19 +639,31 @@ extern "C" int pf_format_kmer_rows(const pf_batch_result* r, uint32_t k, const c
       ++first[r->row_cluster[i] + 1];
     }
   }
+  // the wide and xwide rows (few) of every cluster: a counting sort
+  std::vector<uint32_t> first_x(nx ? nc + 1 : 0, 0);
   for (uint64_t i = 0; i < nw; ++i) {
     if (r->wide_row_cluster[i] >= nc || r->wide_row_pattern[i] >= n_kmer_ids) return PF_ERR_INVALID;
     ++first_w[r->wide_row_cluster[i] + 1];
+  }
+  for (uint64_t i = 0; i < nx; ++i) {
+    if (r->xwide_row_cluster[i] >= nc || r->xwide_row_pattern[i] >= n_kmer_ids) return PF_ERR_INVALID;
+    ++first_x[r->xwide_row_cluster[i] + 1];
   }
   for (uint64_t c = 0; c < nc; ++c) {
     if (r->cluster_pattern[c] >= n_cluster_ids || tag_off[c + 1] < tag_off[c]) return PF_ERR_INVALID;
     first[c + 1] += first[c];
     first_w[c + 1] += first_w[c];
+    if (nx) first_x[c + 1] += first_x[c];
   }
-  std::vector<uint32_t> order_w(nw);
+  auto n_xrows = [&](uint64_t c) -> uint32_t { return nx ? first_x[c + 1] - first_x[c] : 0u; };
+  std::vector<uint32_t> order_w(nw), order_x(nx);
   {
     std::vector<uint32_t> at_w(first_w.begin(), first_w.end() - 1);
     for (uint64_t i = 0; i < nw; ++i) order_w[at_w[r->wide_row_cluster[i]]++] = (uint32_t)i;
+    if (nx) {
+      std::vector<uint32_t> at_x(first_x.begin(), first_x.end() - 1);
+      for (uint64_t i = 0; i < nx; ++i) order_x[at_x[r->xwide_row_cluster[i]]++] = (uint32_t)i;
+    }
     if (!direct) {
       order.resize(nn);
       std::vector<uint32_t> at(first.begin(), first.end() - 1);
@@ -663,7 +674,7 @@ extern "C" int pf_format_kmer_rows(const pf_batch_result* r, uint32_t k, const c
   std::vector<uint64_t> off(nc + 1, 0);
   for (uint64_t c = 0; c < nc; ++c) {
     const uint64_t tag = tag_off[c + 1] - tag_off[c];
-    const uint64_t rows = (uint64_t)(first[c + 1] - first[c]) + (first_w[c + 1] - first_w[c]);
+    const uint64_t rows = (uint64_t)(first[c + 1] - first[c]) + (first_w[c + 1] - first_w[c]) + n_xrows(c);
     off[c + 1] = off[c] + (tag + 2 + 24 + 1) + rows * (tag + 1 + k + 1 + 24 + 1);
   }
   *out_len = off[nc];
@@ -673,7 +684,7 @@ extern "C" int pf_format_kmer_rows(const pf_batch_result* r, uint32_t k, const c
   // clusters are taken one at a time by the threads (they differ in rows): sort, then write
   const uint32_t hw = pf_host_threads();
   uint32_t nt = n_threads ? n_threads : hw;
-  nt = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(nt, (nn + nw + nc + 16383) / 16384));
+  nt = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(nt, (nn + nw + nx + nc + 16383) / 16384));
   std::atomic<uint32_t> next{0};
   std::atomic<uint32_t> bad_pattern{0};
   auto work = [&]() {
@@ -696,15 +707,22 @@ extern "C" int pf_format_kmer_rows(const pf_batch_result* r, uint32_t k, const c
       for (uint32_t j = 0; j < n; ++j) ok &= r->row_pattern[keyed[j].row] < n_kmer_ids;
       if (!ok) { bad_pattern.store(1); continue; }
       sort_keyed(keyed, scratch, 2 * k);
+      // the k-mers of n_words words (most significant first) of rows `o`, sorted
+      auto sort_rows = [](uint32_t* o, uint32_t n_o, const uint64_t* kmers, uint32_t n_words) {
+        std::sort(o, o + n_o, [&](uint32_t a, uint32_t b) {
+          const uint64_t* x = kmers + (uint64_t)n_words * a;
+          const uint64_t* y = kmers + (uint64_t)n_words * b;
+          for (uint32_t i = 0; i < n_words; ++i)
+            if (x[i] != y[i]) return x[i] < y[i];
+          return a < b;
+        });
+      };
       uint32_t* ow = order_w.data() + first_w[c];
       const uint32_t n_w = first_w[c + 1] - first_w[c];
-      std::sort(ow, ow + n_w, [&](uint32_t a, uint32_t b) {
-        const uint64_t* x = r->wide_row_kmer + 2 * (uint64_t)a;
-        const uint64_t* y = r->wide_row_kmer + 2 * (uint64_t)b;
-        if (x[0] != y[0]) return x[0] < y[0];
-        if (x[1] != y[1]) return x[1] < y[1];
-        return a < b;
-      });
+      sort_rows(ow, n_w, r->wide_row_kmer, 2);
+      uint32_t* ox = nx ? order_x.data() + first_x[c] : nullptr;
+      const uint32_t n_x = n_xrows(c);
+      if (n_x) sort_rows(ox, n_x, r->xwide_row_kmer, 4);
       const char* tag = tag_blob + tag_off[c];
       const uint64_t tl = tag_off[c + 1] - tag_off[c];
       char* p = out + off[c];
@@ -725,16 +743,21 @@ extern "C" int pf_format_kmer_rows(const pf_batch_result* r, uint32_t k, const c
         memcpy(p, kmer_ids + (size_t)r->row_pattern[i] * 24, 24); p += 24;
         *p++ = '\n';
       }
-      for (uint32_t j = 0; j < n_w; ++j) {
-        const uint32_t i = ow[j];
-        memcpy(p, tag, tl); p += tl;
-        *p++ = '\t';
-        wide_kmer_text(r->wide_row_kmer + 2 * (uint64_t)i, k, p);
-        p += k;
-        *p++ = '\t';
-        memcpy(p, kmer_ids + (size_t)r->wide_row_pattern[i] * 24, 24); p += 24;
-        *p++ = '\n';
-      }
+      auto write_rows = [&](const uint32_t* o, uint32_t n_o, const uint64_t* kmers, const uint32_t* pattern,
+                            uint32_t n_words) {
+        for (uint32_t j = 0; j < n_o; ++j) {
+          const uint32_t i = o[j];
+          memcpy(p, tag, tl); p += tl;
+          *p++ = '\t';
+          wide_kmer_text(kmers + (uint64_t)n_words * i, n_words, k, p);
+          p += k;
+          *p++ = '\t';
+          memcpy(p, kmer_ids + (size_t)pattern[i] * 24, 24); p += 24;
+          *p++ = '\n';
+        }
+      };
+      write_rows(ow, n_w, r->wide_row_kmer, r->wide_row_pattern, 2);
+      if (n_x) write_rows(ox, n_x, r->xwide_row_kmer, r->xwide_row_pattern, 4);
     }
   };
   if (nt == 1) work();

@@ -50,7 +50,8 @@ extern "C" int pf_create(pf_ctx** out, int device, const pf_params* p) {
     return fail(nullptr, PF_ERR_INVALID, "pf_create: ABI version %u != %u", p->abi_version, PF_ABI_VERSION);
   if (p->k < 1 || p->k > 64)
     return fail(nullptr, PF_ERR_UNSUPPORTED, "k=%u unsupported: k-mers of 1..64 bases are packed into one or two 64-bit "
-                                             "words (1..32: all engines; 33..64: the 128-bit record engine)", p->k);
+                                             "words (1..32: all engines; 33..64: the 128-bit record engine, 256-bit "
+                                             "records for windows with N/IUPAC symbols)", p->k);
   if (p->n_samples < 1) return fail(nullptr, PF_ERR_INVALID, "n_samples must be >= 1");
   if (p->sort_bits != 0 && (p->sort_bits % 8 != 0 || p->sort_bits < 8 || p->sort_bits > 64))
     return fail(nullptr, PF_ERR_INVALID, "sort_bits must be 0 or a multiple of 8 in 8..64");
@@ -111,6 +112,8 @@ extern "C" int pf_create(pf_ctx** out, int device, const pf_params* p) {
                        (int)sizeof(SortSmem<uint64_t>));
   cudaFuncSetAttribute(k2_onesweep_pass<Key128>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                        (int)sizeof(SortSmem<Key128>));
+  cudaFuncSetAttribute(k2_onesweep_pass<Key256>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                       (int)sizeof(SortSmem<Key256>));
   cudaFuncSetAttribute(k2_scatter_pass<uint64_t>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                        (int)sizeof(ScatterSmem<uint64_t>));
   cudaFuncSetAttribute(k2_extract_scatter<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
@@ -190,6 +193,8 @@ extern "C" int pf_create(pf_ctx** out, int device, const pf_params* p) {
     cudaFuncSetAttribute(k3_runs<uint64_t, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, k3_smem);
     cudaFuncSetAttribute(k3_runs<Key128, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, k3_smem);
     cudaFuncSetAttribute(k3_runs<Key128, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, k3_smem);
+    cudaFuncSetAttribute(k3_runs<Key256, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, k3_smem);
+    cudaFuncSetAttribute(k3_runs<Key256, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, k3_smem);
   }
   if (k3_smem > 200 * 1024) {
     pf_destroy(ctx);
@@ -210,20 +215,21 @@ extern "C" void pf_destroy(pf_ctx* ctx) {
       if (*e) cudaEventDestroy(*e);
     for (auto& ev : bs->ev) if (ev) cudaEventDestroy(ev);
     for (DevBuf* b : {&bs->d_bases, &bs->d_amb, &bs->d_ambbits, &bs->d_seqs, &bs->d_clusters, &bs->d_wide_seqs,
+                      &bs->d_xpos_slot, &bs->d_xrow_kmer, &bs->d_pos_xwide,
                       &bs->d_presence, &bs->d_row_cluster, &bs->d_row_kmer, &bs->d_wrow_kmer, &bs->d_row_count,
                       &bs->d_row_pattern, &bs->d_cl_pattern, &bs->d_pos_kmer, &bs->d_pos_seq, &bs->d_pos_cstart,
                       &bs->d_pos_gstart, &bs->d_pos_flags, &bs->d_pos_wide, &bs->d_pos_bits, &bs->d_seq_rec_off,
                       &bs->d_tile_first_seq, &bs->d_seq_lite, &bs->d_cblk, &bs->d_item_base, &bs->d_item_cluster,
                       &bs->d_plan_total, &bs->d_bsum_slot, &bs->d_slice_seq, &bs->d_item_desc, &bs->d_raw, &bs->d_lite_tot})
       fd(*b);
-    for (WidthState* w : {&bs->nar, &bs->wid}) {
+    for (WidthState* w : {&bs->nar, &bs->wid, &bs->xwd}) {
       for (DevBuf* b : {&w->keys[0], &w->keys[1], &w->vals[0], &w->vals[1], &w->tiles, &w->seg_start,
                         &w->seg_hist, &w->lookback, &w->cursors, &w->ltiles, &w->tile_first_run,
                         &w->d_tile_base, &w->d_ltile_base})
         fd(*b);
       fp(w->h_tiles); fp(w->h_seg_start); fp(w->h_ltiles);
     }
-    for (PinBuf* b : {&bs->h_seqs, &bs->h_clusters, &bs->h_wide_seqs, &bs->h_seq_rec_off, &bs->h_tile_first_seq,
+    for (PinBuf* b : {&bs->h_seqs, &bs->h_clusters, &bs->h_wide_seqs, &bs->h_xpos_slot, &bs->h_seq_rec_off, &bs->h_tile_first_seq,
                       &bs->h_plan, &bs->h_done, &bs->h_raw, &bs->h_lite_tot})
       fp(*b);
   }
@@ -242,7 +248,8 @@ extern "C" void pf_destroy(pf_ctx* ctx) {
   for (PinBuf* b : {&ctx->h_counters, &ctx->r_row_cluster, &ctx->r_row_kmer, &ctx->r_wrow_kmer, &ctx->r_row_count,
                     &ctx->r_row_pattern, &ctx->r_cl_pattern, &ctx->r_new_kp, &ctx->r_new_cp, &ctx->r_pos_kmer,
                     &ctx->r_pos_seq, &ctx->r_pos_cstart, &ctx->r_pos_gstart, &ctx->r_pos_flags, &ctx->r_pos_wide,
-                    &ctx->r_wrow_cluster, &ctx->r_wrow_count, &ctx->r_wrow_pattern, &ctx->r_pos_bits})
+                    &ctx->r_wrow_cluster, &ctx->r_wrow_count, &ctx->r_wrow_pattern, &ctx->r_pos_bits,
+                    &ctx->r_xrow_kmer, &ctx->r_pos_xwide})
     fp(*b);
   for (auto& ev : ctx->ev_d2h) if (ev) cudaEventDestroy(ev);
   for (auto& e : ctx->dbg_ev) for (auto& x : e) if (x) cudaEventDestroy(x);

@@ -365,6 +365,7 @@ int collect_pipelined(pf_ctx* ctx, pf_batch_result* out) {
     out->wide_row_kmer = ctx->r_wrow_kmer.as<uint64_t>();
     out->wide_row_count = ctx->r_wrow_count.as<uint32_t>();
     out->wide_row_pattern = ctx->r_wrow_pattern.as<uint32_t>();
+    // (xwide_row_* / pos_xwide_kmer stay empty: batches with N/IUPAC symbols are not pipelined)
     out->n_clusters = ctx->pipe_clusters;
     out->cluster_pattern = ctx->r_cl_pattern.as<uint32_t>();
     out->kmer_pattern_base = ctx->pipe_kp_base;
@@ -417,7 +418,8 @@ extern "C" int pf_collect(pf_ctx* ctx, pf_batch_result* out) {
   TRY(check_device_error(ctx));
   WidthState& N = ctx->nar;
   WidthState& Wd = ctx->wid;
-  const uint64_t rows = (uint64_t)N.n_rows + Wd.n_rows;
+  WidthState& X = ctx->xwd;
+  const uint64_t rows = (uint64_t)N.n_rows + Wd.n_rows + X.n_rows;
   const uint64_t new_kp = hcnt[C_NEW_KP];
   const uint64_t new_cp = ctx->cp.n - ctx->cp_base;
   ctx->kp.n = ctx->kp_base + new_kp;
@@ -435,6 +437,7 @@ extern "C" int pf_collect(pf_ctx* ctx, pf_batch_result* out) {
     TRY(d2h(ctx->r_row_count, ctx->d_row_count.p, rows * 4));
     TRY(d2h(ctx->r_row_kmer, ctx->d_row_kmer.p, (size_t)N.n_rows * 8));
     TRY(d2h(ctx->r_wrow_kmer, ctx->d_wrow_kmer.p, (size_t)Wd.n_rows * 16));
+    if (X.n_rows) TRY(d2h(ctx->r_xrow_kmer, ctx->d_xrow_kmer.p, (size_t)X.n_rows * 32));
   }
   TRY(d2h(ctx->r_row_pattern, ctx->d_row_pattern.p, rows * 4));
   TRY(d2h(ctx->r_cl_pattern, ctx->d_cl_pattern.p, (size_t)ctx->n_clusters * 4));
@@ -451,6 +454,7 @@ extern "C" int pf_collect(pf_ctx* ctx, pf_batch_result* out) {
     TRY(d2h(ctx->r_pos_flags, ctx->d_pos_flags.p, (size_t)ctx->n_pos));
   }
   if (ctx->n_pos_wide && !compact) TRY(d2h(ctx->r_pos_wide, ctx->d_pos_wide.p, (size_t)ctx->n_pos_wide * 16));
+  if (ctx->n_pos_xwide && !compact) TRY(d2h(ctx->r_pos_xwide, ctx->d_pos_xwide.p, (size_t)ctx->n_pos_xwide * 32));
   CU(cudaEventRecord(ctx->ev_d2h[1], st));
   CU(cudaStreamSynchronize(st));
   if (ctx->rows_prefetched) CU(cudaStreamSynchronize(ctx->copy_stream));
@@ -484,6 +488,17 @@ extern "C" int pf_collect(pf_ctx* ctx, pf_batch_result* out) {
     out->pos_flags = ctx->r_pos_flags.as<uint8_t>();
     out->pos_wide_kmer = ctx->r_pos_wide.as<uint64_t>();
     out->n_pos_wide = ctx->n_pos_wide;
+    if (X.n_rows) {           // (rows of the 256-bit section follow the wide ones in the row arrays)
+      out->n_xwide_rows = X.n_rows;
+      out->xwide_row_cluster = out->row_cluster + N.n_rows + Wd.n_rows;
+      out->xwide_row_kmer = ctx->r_xrow_kmer.as<uint64_t>();
+      out->xwide_row_count = out->row_count + N.n_rows + Wd.n_rows;
+      out->xwide_row_pattern = out->row_pattern + N.n_rows + Wd.n_rows;
+    }
+    if (ctx->n_pos_xwide && !compact) {
+      out->pos_xwide_kmer = ctx->r_pos_xwide.as<uint64_t>();
+      out->n_pos_xwide = ctx->n_pos_xwide;
+    }
     if (compact) {
       out->pos_kmer = nullptr; out->pos_seq = nullptr; out->pos_contig_start = nullptr;
       out->pos_gene_start = nullptr; out->pos_flags = nullptr; out->pos_wide_kmer = nullptr;
@@ -498,7 +513,7 @@ extern "C" int pf_collect(pf_ctx* ctx, pf_batch_result* out) {
   pf_stats& s = ctx->stats;
   s.batches++;
   s.bases += ctx->n_bases;
-  s.instances += (uint64_t)N.n_records + Wd.n_records;
+  s.instances += (uint64_t)N.n_records + Wd.n_records + X.n_records;
   s.unique_kmers += ctx->unique_last;
   s.rows += rows;
   s.kmer_patterns = ctx->kp.n;

@@ -112,9 +112,9 @@ std::string describe_bad_seq(const pf_ctx* ctx, const pf_batch* b, uint32_t i, u
 }
 
 // ClusterDev of every cluster of the (sub-)batch: presence popcount, MAF window, filters folded in.
-// rec ranges stay zero unless `nr` / `wr` give them (record engines).
+// rec ranges stay zero unless `nr` / `wr` / `xr` give them (record engines).
 int build_clusters(pf_ctx* ctx, const pf_batch* b, ClusterDev* hc, const std::pair<uint32_t, uint32_t>* nr,
-                   const std::pair<uint32_t, uint32_t>* wr) {
+                   const std::pair<uint32_t, uint32_t>* wr, const std::pair<uint32_t, uint32_t>* xr = nullptr) {
   const pf_params& P = ctx->prm;
   const uint32_t S = P.n_samples, W = ctx->W;
   for (uint32_t c = 0; c < b->n_clusters; ++c) {
@@ -129,6 +129,7 @@ int build_clusters(pf_ctx* ctx, const pf_batch* b, ClusterDev* hc, const std::pa
     ClusterDev& d = hc[c];
     d.rec_start = nr ? nr[c].first : 0; d.rec_end = nr ? nr[c].second : 0;
     d.wrec_start = wr ? wr[c].first : 0; d.wrec_end = wr ? wr[c].second : 0;
+    d.xrec_start = xr ? xr[c].first : 0; d.xrec_end = xr ? xr[c].second : 0;
     d.id = b->clusters[c].id; d.n_present = np;
     const uint32_t n = P.consider_missing ? np : S;
     uint32_t lo, hi;
@@ -216,8 +217,8 @@ int upload_async_lite(pf_ctx* ctx, BatchState& B, const pf_batch* b, uint32_t rc
   mirror_counters<<<1, 32, 0, st>>>(B.h_lite_tot.as<uint32_t>(), B.d_lite_tot.as<uint32_t>(), 16);
   B.n_seqs = n; B.n_clusters = nc; B.n_wide_seqs = 0;
   B.n_words = b->n_words; B.n_amb_words = 0;
-  B.n_bases = 0; B.n_pos = 0; B.n_pos_wide = 0;         // totals: upload_finish*
-  B.nar.n_records = 0; B.wid.n_records = 0;
+  B.n_bases = 0; B.n_pos = 0; B.n_pos_wide = 0; B.n_pos_xwide = 0;   // totals: upload_finish*
+  B.nar.n_records = 0; B.wid.n_records = 0; B.xwd.n_records = 0; B.xwd.n_tiles = 0;
   B.nar.n_tiles = B.wid.n_tiles = 0; B.nar.n_ltiles = 0; B.nar.max_seg = B.wid.max_seg = 0;
   B.nar.passes = B.wid.passes = 1; B.nar.sort_bits = B.wid.sort_bits = 8;
   B.nar_ranges.clear();
@@ -290,7 +291,10 @@ int upload_async(pf_ctx* ctx, BatchState& B, const pf_batch* full, const SubRang
   uint32_t* hw = B.h_wide_seqs.as<uint32_t>();
 
   const uint32_t mult = P.canonical ? 1u : 2u;
-  const bool long_k = k > 32;          // two-word k-mers: every window is a record of the 128-bit pipeline
+  // two-word k-mers: every window is a record of the 128-bit pipeline; the windows of a sequence
+  // with N/IUPAC symbols are ALSO records of the 256-bit pipeline (4 bits per symbol), and each
+  // pipeline kills the records of the windows the other one owns
+  const bool long_k = k > 32;
   // the packed plane is the bulk of the transfer: start it before the host-side planning
   const size_t slack_words = 80;
   TRY(dev_ensure(ctx, B.d_bases, (b->n_words + slack_words) * 8));
@@ -304,9 +308,9 @@ int upload_async(pf_ctx* ctx, BatchState& B, const pf_batch* full, const SubRang
   // ---- planning, in parallel over chunks of sequences --------------------------------
   // phase A: validate + per-sequence sizes, per-chunk sums; phase B: prefix over chunks;
   // phase C: offsets.  Cluster ranges come from the first sequence of every cluster.
-  uint64_t rec = 0, wrec = 0, pos = 0, pwide = 0, bases = 0;
-  uint32_t n_wide = 0;
-  std::vector<std::pair<uint32_t, uint32_t>> nr(b->n_clusters), wr(b->n_clusters);
+  uint64_t rec = 0, wrec = 0, xrec = 0, pos = 0, pwide = 0, pxwide = 0, bases = 0;
+  uint32_t n_wide = 0;                 // sequences with N/IUPAC symbols (listed in h_wide_seqs)
+  std::vector<std::pair<uint32_t, uint32_t>> nr(b->n_clusters), wr(b->n_clusters), xr(b->n_clusters);
   {
     const uint32_t n = b->n_seqs;
     // PF_HOST_THREADS caps the planning threads (several contexts / ranks share the host's cores)
@@ -314,7 +318,7 @@ int upload_async(pf_ctx* ctx, BatchState& B, const pf_batch* full, const SubRang
                                             return v > 0 ? (uint32_t)v : 16u; }();
     const uint32_t n_thr = std::max(1u, std::min<uint32_t>(std::min(host_thr, std::thread::hardware_concurrency()),
                                                            (n + 16383u) / 16384u));
-    struct Part { uint64_t rec = 0, wrec = 0, pos = 0, pwide = 0, bases = 0; uint32_t wide = 0; std::string err; };
+    struct Part { uint64_t rec = 0, wrec = 0, xrec = 0, pos = 0, pwide = 0, pxwide = 0, bases = 0; uint32_t wide = 0; std::string err; };
     std::vector<Part> parts(n_thr);
     const uint32_t per = (n + n_thr - 1) / std::max(1u, n_thr);
     auto run = [&](const std::function<void(uint32_t)>& fn) { ctx->pool.parallel(n_thr, fn); };
@@ -340,7 +344,6 @@ int upload_async(pf_ctx* ctx, BatchState& B, const pf_batch* full, const SubRang
         if (q.base_off + q.len > b->n_words * 32ull) return errf(p, "seq %u: bases run past the packed plane", i);
         if (q.strand != 1 && q.strand != -1) return errf(p, "seq %u: strand must be +1/-1", i);
         const bool amb = (q.flags & PF_SEQ_AMBIGUOUS) != 0;
-        if (amb && long_k) return errf(p, "seq %u holds N/IUPAC symbols: not supported with k > 32", i);
         if (amb) {
           if (!b->amb_codes) return errf(p, "seq %u is ambiguous but amb_codes is NULL", i);
           if (q.amb_off & 31u) return errf(p, "seq %u: amb_off must be a multiple of 32", i);
@@ -350,22 +353,29 @@ int upload_async(pf_ctx* ctx, BatchState& B, const pf_batch* full, const SubRang
         const uint32_t nwin = q.len >= k ? q.len - k + 1 : 0;
         if (!long_k) p.rec += (uint64_t)nwin * mult;
         if (target) p.pos += nwin;
-        if (amb || long_k) { p.wrec += (uint64_t)nwin * mult; p.wide++; if (target) p.pwide += nwin; }
+        if (amb || long_k) { p.wrec += (uint64_t)nwin * mult; if (target) p.pwide += nwin; }
+        if (amb) {
+          p.wide++;
+          if (long_k) { p.xrec += (uint64_t)nwin * mult; if (target) p.pxwide += nwin; }
+        }
         p.bases += q.len;
       }
     });
     for (auto& p : parts) if (!p.err.empty()) return fail(ctx, PF_ERR_INVALID, "%s", p.err.c_str());
     std::vector<Part> base(n_thr);
     for (uint32_t t = 0; t < n_thr; ++t) {
-      base[t].rec = rec; base[t].wrec = wrec; base[t].pos = pos; base[t].pwide = pwide; base[t].wide = n_wide;
-      rec += parts[t].rec; wrec += parts[t].wrec; pos += parts[t].pos; pwide += parts[t].pwide;
-      n_wide += parts[t].wide; bases += parts[t].bases;
+      base[t].rec = rec; base[t].wrec = wrec; base[t].xrec = xrec; base[t].pos = pos; base[t].pwide = pwide;
+      base[t].pxwide = pxwide; base[t].wide = n_wide;
+      rec += parts[t].rec; wrec += parts[t].wrec; xrec += parts[t].xrec; pos += parts[t].pos; pwide += parts[t].pwide;
+      pxwide += parts[t].pxwide; n_wide += parts[t].wide; bases += parts[t].bases;
     }
-    if (rec >= (1ull << 32) - kSortTile || wrec >= (1ull << 32) - kSortTile)
+    if (rec >= (1ull << 32) - kSortTile || wrec >= (1ull << 32) - kSortTile || xrec >= (1ull << 32) - kSortTile)
       return fail(ctx, PF_ERR_INVALID, "batch holds more than 2^32 k-mer records; split it");
     if (pos >= (1ull << 32)) return fail(ctx, PF_ERR_INVALID, "more than 2^32 positional records; split the batch");
+    if (long_k && n_wide) TRY(pin_ensure(ctx, B.h_xpos_slot, (size_t)n_wide * sizeof(uint32_t)));
+    uint32_t* hxp = B.h_xpos_slot.as<uint32_t>();
     constexpr uint32_t kUnset = 0xffffffffu;
-    for (uint32_t c = 0; c < b->n_clusters; ++c) { nr[c] = {kUnset, kUnset}; wr[c] = {kUnset, kUnset}; }
+    for (uint32_t c = 0; c < b->n_clusters; ++c) { nr[c] = {kUnset, kUnset}; wr[c] = {kUnset, kUnset}; xr[c] = {kUnset, kUnset}; }
     run([&](uint32_t t) {
       Part o = base[t];
       const uint32_t i0 = std::min(n, t * per), i1 = std::min(n, i0 + per);
@@ -378,36 +388,49 @@ int upload_async(pf_ctx* ctx, BatchState& B, const pf_batch* full, const SubRang
         if (i == 0 || q.cluster + rc != b->seqs[i - 1].cluster) {     // first sequence of its cluster
           nr[q.cluster].first = (uint32_t)o.rec;
           wr[q.cluster].first = (uint32_t)o.wrec;
+          xr[q.cluster].first = (uint32_t)o.xrec;
         }
         SeqDev& d = hs[i];
         d.base_off = q.base_off; d.amb_off = amb ? q.amb_off : 0; d.len = q.len; d.sample = q.sample;
         d.cluster = q.cluster; d.flags = (target ? 1u : 0u) | (amb ? 2u : 0u);
         d.start = q.start; d.end = q.end; d.offset = q.offset; d.strand = q.strand;
-        d.rec_off = (uint32_t)o.rec; d.pos_off = (uint32_t)o.pos; d.wrec_off = (uint32_t)o.wrec;
+        d.rec_off = (uint32_t)(long_k ? o.xrec : o.rec); d.pos_off = (uint32_t)o.pos; d.wrec_off = (uint32_t)o.wrec;
         d.pwide_off = (uint32_t)o.pwide;
         if (!long_k) o.rec += (uint64_t)nwin * mult;
         if (target) o.pos += nwin;
-        if (amb || long_k) { o.wrec += (uint64_t)nwin * mult; hw[o.wide++] = i; if (target) o.pwide += nwin; }
+        if (amb || long_k) { o.wrec += (uint64_t)nwin * mult; if (target) o.pwide += nwin; }
+        if (amb) {
+          if (long_k) {
+            hxp[o.wide] = (uint32_t)o.pxwide;
+            o.xrec += (uint64_t)nwin * mult;
+            if (target) o.pxwide += nwin;
+          }
+          hw[o.wide++] = i;
+        }
       }
     });
     // clusters without sequences are empty ranges at the start of the next non-empty one
-    uint32_t next_n = (uint32_t)rec, next_w = (uint32_t)wrec;
+    uint32_t next_n = (uint32_t)rec, next_w = (uint32_t)wrec, next_x = (uint32_t)xrec;
     for (uint32_t c = b->n_clusters; c-- > 0;) {
-      if (nr[c].first == kUnset) { nr[c].first = next_n; wr[c].first = next_w; }
-      nr[c].second = next_n; wr[c].second = next_w;
-      next_n = nr[c].first; next_w = wr[c].first;
+      if (nr[c].first == kUnset) { nr[c].first = next_n; wr[c].first = next_w; xr[c].first = next_x; }
+      nr[c].second = next_n; wr[c].second = next_w; xr[c].second = next_x;
+      next_n = nr[c].first; next_w = wr[c].first; next_x = xr[c].first;
     }
   }
   const double t_dbg1 = now_ms();
-  TRY(build_clusters(ctx, b, hc, nr.data(), wr.data()));
+  TRY(build_clusters(ctx, b, hc, nr.data(), wr.data(), xr.data()));
 
   const double t_dbg2 = now_ms();
   B.n_seqs = b->n_seqs; B.n_clusters = b->n_clusters; B.n_wide_seqs = n_wide;
   B.n_words = b->n_words; B.n_amb_words = n_wide ? b->n_amb_words : 0; B.n_bases = bases;
-  B.n_pos = (uint32_t)pos; B.n_pos_wide = (uint32_t)pwide;
-  B.nar.n_records = (uint32_t)rec; B.wid.n_records = (uint32_t)wrec;
+  B.n_pos = (uint32_t)pos; B.n_pos_wide = (uint32_t)pwide; B.n_pos_xwide = (uint32_t)pxwide;
+  B.nar.n_records = (uint32_t)rec; B.wid.n_records = (uint32_t)wrec; B.xwd.n_records = (uint32_t)xrec;
   TRY(plan_tiles(ctx, B.nar, nr, true));
   TRY(plan_tiles(ctx, B.wid, wr, false));
+  // (the 256-bit width exists only for k > 32 batches with N/IUPAC symbols)
+  std::vector<WidthState*> widths{&B.nar, &B.wid};
+  if (xrec) { TRY(plan_tiles(ctx, B.xwd, xr, false)); widths.push_back(&B.xwd); }
+  else B.xwd.n_tiles = 0;
 
   // ---- device buffers + H2D ------------------------------------------------
   TRY(dev_ensure(ctx, B.d_seqs, std::max<size_t>(1, b->n_seqs) * sizeof(SeqDev)));
@@ -415,7 +438,7 @@ int upload_async(pf_ctx* ctx, BatchState& B, const pf_batch* full, const SubRang
   TRY(dev_ensure(ctx, B.d_presence, std::max<size_t>(1, (size_t)b->n_clusters * W) * 4));
   TRY(dev_ensure(ctx, ctx->d_counters, C_COUNT * 4));
   TRY(pin_ensure(ctx, ctx->h_counters, C_COUNT * 4 + 64 * 4));
-  for (WidthState* w : {&B.nar, &B.wid}) {
+  for (WidthState* w : widths) {
     TRY(dev_ensure(ctx, w->tiles, std::max<size_t>(1, w->n_tiles) * sizeof(TileDev)));
     TRY(dev_ensure(ctx, w->seg_start, std::max<size_t>(1, b->n_clusters) * 4));
     TRY(dev_ensure(ctx, w->seg_hist, std::max<size_t>(1, (size_t)b->n_clusters * w->passes * kRadix) * 4));
@@ -427,14 +450,14 @@ int upload_async(pf_ctx* ctx, BatchState& B, const pf_batch* full, const SubRang
     CU(cudaMemcpyAsync(B.d_presence.p, b->cluster_presence, (size_t)b->n_clusters * W * 4, cudaMemcpyHostToDevice, st));
   }
   // tile lists are generated on the device from the per-cluster record ranges
-  for (WidthState* w : {&B.nar, &B.wid}) {
+  for (WidthState* w : widths) {
     if (b->n_clusters) CU(cudaMemcpyAsync(w->seg_start.p, w->h_seg_start.p, b->n_clusters * 4, cudaMemcpyHostToDevice, st));
     if (w->n_tiles) {
       TRY(dev_ensure(ctx, w->d_tile_base, (size_t)b->n_clusters * 4));
       CU(cudaMemcpyAsync(w->d_tile_base.p, w->h_tiles.p, (size_t)b->n_clusters * 4, cudaMemcpyHostToDevice, st));
       plan_expand_tiles<<<b->n_clusters, 128, 0, st>>>(B.d_clusters.as<ClusterDev>(), b->n_clusters,
                                                        w->d_tile_base.as<uint32_t>(), kSortTile,
-                                                       w == &B.wid ? 1 : 0, w->tiles.as<TileDev>());
+                                                       w == &B.xwd ? 2 : w == &B.wid ? 1 : 0, w->tiles.as<TileDev>());
       ctx->launches++;
     }
   }
@@ -451,7 +474,7 @@ int upload_async(pf_ctx* ctx, BatchState& B, const pf_batch* full, const SubRang
         B.d_tile_first_seq.as<uint32_t>());
     ctx->launches += 2;
   }
-  if (n_wide && !long_k) {
+  if (n_wide) {
     const size_t bit_words = (b->n_amb_words + 1) / 2 + 4;
     TRY(dev_ensure(ctx, B.d_amb, (b->n_amb_words + 8) * 8));
     TRY(dev_ensure(ctx, B.d_ambbits, bit_words * 4));
@@ -459,6 +482,10 @@ int upload_async(pf_ctx* ctx, BatchState& B, const pf_batch* full, const SubRang
     CU(cudaMemcpyAsync(B.d_amb.p, b->amb_codes, b->n_amb_words * 8, cudaMemcpyHostToDevice, st));
     CU(cudaMemsetAsync((char*)B.d_amb.p + b->n_amb_words * 8, 0, 8 * 8, st));
     CU(cudaMemcpyAsync(B.d_wide_seqs.p, hw, n_wide * 4, cudaMemcpyHostToDevice, st));
+    if (long_k) {
+      TRY(dev_ensure(ctx, B.d_xpos_slot, n_wide * 4));
+      CU(cudaMemcpyAsync(B.d_xpos_slot.p, B.h_xpos_slot.p, n_wide * 4, cudaMemcpyHostToDevice, st));
+    }
     k1_amb_bits<<<cdiv(bit_words, 256), 256, 0, st>>>(B.d_amb.as<uint64_t>(), b->n_amb_words,
                                                        B.d_ambbits.as<uint32_t>(), bit_words);
     ctx->launches++;

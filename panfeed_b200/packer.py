@@ -215,21 +215,18 @@ def kmers_to_str(kmers, k):
     return np.ascontiguousarray(_ACGT[codes]).view(f"S{k}").ravel()
 
 
-def wide_kmers_to_str(kmers, k):
-    """[n,2] uint64 (hi, lo) two-word k-mers -> numpy bytes array S{k}: 4 bits per symbol
-    (N/IUPAC k-mers, k <= 32) or, for k > 32, 2 bits per base."""
-    kmers = np.asarray(kmers, np.uint64).reshape(-1, 2)
+def wide_kmers_to_str(kmers, k, n_words=2):
+    """[n, n_words] uint64 k-mers (most significant word first) -> numpy bytes array S{k}: 4 bits
+    per symbol (codes of AMB_ALPHABET) when k symbols fit that way - N/IUPAC k-mers of k <= 32 in
+    two words, of k <= 64 in four (xwide rows) - else 2 bits per base (two words, k > 32)."""
+    kmers = np.asarray(kmers, np.uint64).reshape(-1, n_words)
     if kmers.shape[0] == 0:
         return np.zeros(0, f"S{k}")
+    bits = 4 if k <= 16 * n_words else 2
+    alphabet = _AMB if bits == 4 else _ACGT
     out = np.zeros((kmers.shape[0], k), np.uint8)
-    if k > 32:
-        for i in range(k):
-            pos = 2 * (k - 1 - i)
-            word = kmers[:, 1] >> np.uint64(pos) if pos < 64 else kmers[:, 0] >> np.uint64(pos - 64)
-            out[:, i] = _ACGT[(word & np.uint64(3)).astype(np.uint8)]
-        return np.ascontiguousarray(out).view(f"S{k}").ravel()
     for i in range(k):
-        nib = k - 1 - i                    # nibble index from the bottom
-        word = kmers[:, 1] if nib < 16 else kmers[:, 0]
-        out[:, i] = _AMB[((word >> np.uint64(4 * (nib % 16))) & np.uint64(15)).astype(np.uint8)]
+        pos = bits * (k - 1 - i)           # bit offset from the bottom of the last word
+        word = kmers[:, n_words - 1 - pos // 64] >> np.uint64(pos % 64)
+        out[:, i] = alphabet[(word & np.uint64((1 << bits) - 1)).astype(np.uint8)]
     return np.ascontiguousarray(out).view(f"S{k}").ravel()
