@@ -18,9 +18,11 @@
 //                       (forward / reverse complement / canonical), each k-mer is looked up in
 //                       a shared-memory open-addressing table and takes the chunk's whole
 //                       W-word sample bitset.  The CTA ends by writing its distinct k-mers,
-//                       bitsets and popcounts ("partial rows") to a slab in HBM: ~1/30 of the
-//                       bytes the records would have taken, written once.  Every run keeps
-//                       its own slab, so the kernels after kA see per-run items.
+//                       popcounts and bitsets ("partial rows") to a slab in HBM: ~1/30 of the
+//                       bytes the records would have taken, written once.  A row of one sample
+//                       (most rows) is written as its key and a one-sample code, without the
+//                       bitset (see slab_cnt).  Every run keeps its own slab, so the kernels
+//                       after kA see per-run items.
 //   kB1/kB3             a k-mer can start in two runs (indels, clamped flanks, paralogs,
 //                       repeats), so the partial rows of one cluster are merged by FULL key in a
 //                       per-cluster open-addressing table in global memory: the first row of a
@@ -65,9 +67,29 @@ constexpr int kBlkThreads = PF_KA_THREADS;
 constexpr int kBlkWarps = kBlkThreads / 32;
 constexpr int kBlkRun = 16;                       // windows per task
 constexpr uint32_t kBlkOverflow = 0xffffffffu;    // slab count of a block that did not fit
-// slab_cnt[p]: popcount of partial row p as kA wrote it; after kB1: kCntDead = folded into an
-// earlier row of the same k-mer, kCntDirty = received another row's bits (recount from the row)
-constexpr uint32_t kCntDead = 0xfffffffeu, kCntDirty = 0xffffffffu;
+// slab_cnt[p], the state of partial row p:
+//   popcount           (kA) two or more samples: the bitset is in slab_rows
+//   kCntSingle | s     (kA) ONE sample, rank s < 1024 inside the slice: slab_rows holds nothing for p
+//   kCntDead           (kB1) folded into an earlier row of the same k-mer
+//   kCntDirty          (kB1) received another row's bits: recount from the row
+//   kCntLocked         (kB1, transient) a one-sample owner whose bitset is being written out
+constexpr uint32_t kCntSingle = 0x80000000u;
+constexpr uint32_t kCntLocked = 0xfffffffdu, kCntDead = 0xfffffffeu, kCntDirty = 0xffffffffu;
+__device__ __forceinline__ bool cnt_single(uint32_t code) { return (code & 0xfffffc00u) == kCntSingle; }
+// the count of partial row p from its slab_cnt code; kCntDead for a row folded into another.
+// Every reader of slab_cnt after kB1 goes through this.
+__device__ __forceinline__ uint32_t partial_row_count(const uint32_t* __restrict__ slab_rows, uint32_t code,
+                                                      size_t p, uint32_t WP) {
+  if (cnt_single(code)) return 1u;
+  if (code != kCntDirty) return code;          // popcount, or kCntDead
+  const uint4* row = reinterpret_cast<const uint4*>(slab_rows + p * WP);
+  uint32_t cnt = 0;
+  for (uint32_t q = 0; q < WP / 4; ++q) {
+    const uint4 x = row[q];
+    cnt += __popc(x.x) + __popc(x.y) + __popc(x.z) + __popc(x.w);
+  }
+  return cnt;
+}
 
 __global__ void plan_seq_lite(const SeqDev* __restrict__ seqs, uint32_t n, SeqLite* __restrict__ out) {
   const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -231,7 +253,7 @@ __global__ void plan_item_desc(const uint32_t* __restrict__ item_base, const uin
 // shared-memory table
 // ---------------------------------------------------------------------------
 struct BlkHead {           // 64 bytes at the start of kA's shared memory (see ARunView)
-  uint32_t n_unique, overflow, n_pass, row_base, ok, work, seg[2], pad[8];
+  uint32_t n_unique, overflow, n_pass, row_base, ok, work, seg[2], singles, pad[7];
 };
 __device__ __forceinline__ uint32_t ld_volatile_shared(const uint32_t* p) {
   return *reinterpret_cast<const volatile uint32_t*>(p);
@@ -405,7 +427,7 @@ kA_block_aggregate(const uint64_t* __restrict__ bases, const uint32_t* __restric
                    const SeqLite* __restrict__ seqs, BlkPlan plan, int k,
                    uint64_t* __restrict__ slab_keys, uint32_t* __restrict__ slab_rows,
                    uint32_t* __restrict__ slab_base, uint32_t* __restrict__ slab_count,
-                   uint32_t* __restrict__ slab_cnt /* popcount of every partial row */,
+                   uint32_t* __restrict__ slab_cnt /* popcount or one-sample code of every partial row */,
                    uint32_t partial_capacity, uint32_t* __restrict__ counters,
                    const uint32_t* __restrict__ item_list /* null: segments of seg_runs runs */,
                    uint32_t n_segs, uint32_t seg_runs,
@@ -422,7 +444,7 @@ kA_block_aggregate(const uint64_t* __restrict__ bases, const uint32_t* __restric
     for (uint32_t i = tid; i < a.ccap * WS; i += kBlkThreads) a.crows[i] = 0u;
   };
   clear_tables();
-  if (tid == 0) { a.h->n_unique = 0; a.h->overflow = 0; a.h->work = 0; a.h->n_pass = 0; }
+  if (tid == 0) { a.h->n_unique = 0; a.h->overflow = 0; a.h->work = 0; a.h->n_pass = 0; a.h->singles = 0; }
   __syncthreads();
 
   const uint32_t sh64 = 64u - 2u * (uint32_t)k;
@@ -609,27 +631,58 @@ kA_block_aggregate(const uint64_t* __restrict__ bases, const uint32_t* __restric
       __syncthreads();
       if (tid == 0) { a.h->n_unique = 0; a.h->overflow = 0; a.h->work = 0; a.h->n_pass = 0; }
       if (!overflow && a.h->ok) {
+        // a warp takes 32 rows: every lane writes its row's key and count code; a one-sample row
+        // (most of them: the k-mers of a private SNP) is only that code, its bitset is never
+        // written.  The other rows are listed (lane ids, in the chunk keys, which are dead until
+        // the next run: ccap >= 16 gives 32 bytes per warp) and copied by L = WP / 4 lanes each,
+        // one uint4 per lane, so a store instruction writes whole 16 * L-byte rows (W <= 32: L <= 8).
         const size_t base = a.h->row_base;
-        const uint32_t WP = plan.WP;
-        for (uint32_t r = tid; r < n; r += kBlkThreads) {
-          slab_keys[base + r] = a.rkey[r];
-          uint32_t* src = a.pool + r * WS;
-          uint4* dst = reinterpret_cast<uint4*>(slab_rows + (base + r) * WP);
-          uint32_t cnt = 0;
-          for (uint32_t q = 0; q < WP; q += 4) {
-            uint4 x;
-            x.x = src[q];
-            x.y = q + 1 < W ? src[q + 1] : 0u;
-            x.z = q + 2 < W ? src[q + 2] : 0u;
-            x.w = q + 3 < W ? src[q + 3] : 0u;
-            dst[q >> 2] = x;
-            cnt += __popc(x.x) + __popc(x.y) + __popc(x.z) + __popc(x.w);
+        const uint32_t WP = plan.WP, L = WP >> 2, lane = tid & 31u;
+        const uint32_t lrow = lane / L, lq = 4u * (lane - lrow * L), per = 32u / L;
+        uint8_t* list = reinterpret_cast<uint8_t*>(a.ckhi) + (tid & ~31u);
+        for (uint32_t r0 = tid & ~31u; r0 < n; r0 += kBlkThreads) {
+          const uint32_t r = r0 + lane;
+          bool multi = false;
+          if (r < n) {
+            slab_keys[base + r] = a.rkey[r];
+            uint32_t* src = a.pool + r * WS;
+            uint32_t cnt = 0, wq = 0, orx = 0;         // one sample: it is bit ffs(orx) of word wq
+            for (uint32_t q = 0; q < W; ++q) {
+              const uint32_t x = src[q], c = __popc(x);
+              cnt += c;
+              wq += c * q;
+              orx |= x;
+            }
+            multi = cnt != 1u;
+            if (multi) {
+              slab_cnt[base + r] = cnt;
+            } else {
+              slab_cnt[base + r] = kCntSingle | (wq << 5) | (uint32_t)(__ffs(orx) - 1);
+              src[wq] = 0u;
+            }
+            const uint32_t h = a.rslot[r];
+            a.keys[h] = ~0ull;
+            a.rowid[h] = 0xffffu;
           }
-          slab_cnt[base + r] = cnt;
-          for (uint32_t q = 0; q < W; ++q) src[q] = 0u;
-          const uint32_t h = a.rslot[r];
-          a.keys[h] = ~0ull;
-          a.rowid[h] = 0xffffu;
+          const uint32_t m = __ballot_sync(kFull, multi), nm = (uint32_t)__popc(m);
+          if (multi) list[__popc(m & lanemask_lt())] = (uint8_t)lane;
+          if (lane == 0 && nm < min(32u, n - r0)) atomicAdd(&a.h->singles, min(32u, n - r0) - nm);
+          __syncwarp();
+          for (uint32_t g = lrow; g < nm && lrow < per; g += per) {
+            const uint32_t rr = r0 + list[g];
+            uint32_t* src = a.pool + rr * WS + lq;
+            uint4 x;
+            x.x = src[0];                              // (lq < W: WP is W rounded up to 4)
+            x.y = lq + 1 < W ? src[1] : 0u;
+            x.z = lq + 2 < W ? src[2] : 0u;
+            x.w = lq + 3 < W ? src[3] : 0u;
+            reinterpret_cast<uint4*>(slab_rows + (base + rr) * WP + lq)[0] = x;
+            src[0] = 0u;
+            if (lq + 1 < W) src[1] = 0u;
+            if (lq + 2 < W) src[2] = 0u;
+            if (lq + 3 < W) src[3] = 0u;
+          }
+          __syncwarp();
         }
         for (uint32_t c = tid; c < n_chunks; c += kBlkThreads) a.cstate[a.cslot[c]] = kChunkEmpty;
         for (uint32_t i = tid; i < n_chunks * WS; i += kBlkThreads) a.crows[i] = 0u;
@@ -646,6 +699,7 @@ kA_block_aggregate(const uint64_t* __restrict__ bases, const uint32_t* __restric
       seg = a.h->seg[it & 1u];
     }
   }
+  if (tid == 0 && a.h->singles) atomicAdd(&counters[LC_SINGLES], a.h->singles);
 }
 
 // ---------------------------------------------------------------------------
@@ -719,6 +773,34 @@ __device__ __forceinline__ void fold_partial_row(uint32_t* __restrict__ slab_row
       if (v[u].w) atomicOr(d + 3, v[u].w);
     }
   }
+}
+
+// kB1: partial row p (a later row of the k-mer) goes into its owner q.  A one-sample row has no
+// bitset in slab_rows: p's is one atomicOr; q's is written out first, by the first row that folds
+// into it (single code -> kCntLocked by CAS, all WP words, kCntDirty), while other rows folding
+// into q at the same time wait for kCntDirty.
+__device__ __noinline__ void fold_into_owner(uint32_t* __restrict__ slab_rows, uint32_t* __restrict__ slab_cnt,
+                                             uint32_t p, uint32_t q, uint32_t WP) {
+  uint32_t* dst = slab_rows + (size_t)q * WP;
+  for (;;) {
+    const uint32_t code = *reinterpret_cast<volatile uint32_t*>(&slab_cnt[q]);
+    if (cnt_single(code)) {
+      if (atomicCAS(&slab_cnt[q], code, kCntLocked) != code) continue;
+      for (uint32_t w = 0; w < WP; w += 4) *reinterpret_cast<uint4*>(dst + w) = make_uint4(0u, 0u, 0u, 0u);
+      const uint32_t s = code & 0x3ffu;
+      dst[s >> 5] = 1u << (s & 31u);
+      __threadfence();
+      *reinterpret_cast<volatile uint32_t*>(&slab_cnt[q]) = kCntDirty;
+      break;
+    }
+    if (code != kCntLocked) { __threadfence(); break; }
+    __nanosleep(32);                          // (lets the writer run if it is a lane of this warp)
+  }
+  const uint32_t pc = slab_cnt[p];
+  if (cnt_single(pc)) atomicOr(dst + ((pc & 0x3ffu) >> 5), 1u << (pc & 31u));
+  else fold_partial_row(slab_rows, p, q, WP);
+  slab_cnt[p] = kCntDead;
+  slab_cnt[q] = kCntDirty;
 }
 
 // kB1 in shared memory: one CTA per (cluster, slice).  The partial rows of a cluster number a few
@@ -808,9 +890,7 @@ kB1_local(const uint64_t* __restrict__ slab_keys, uint32_t* __restrict__ slab_ro
     return slab_base[(size_t)(it0 + lo) * n_slices + slice] + (ql - prefix[lo]);
   };
   auto fold = [&](uint32_t p, uint32_t q) {
-    fold_partial_row(slab_rows, p, q, WP);
-    slab_cnt[p] = kCntDead;
-    slab_cnt[q] = kCntDirty;
+    fold_into_owner(slab_rows, slab_cnt, p, q, WP);
     ++dups;
   };
   // find-or-insert of one row: key, its index in the cluster's numbering, its partial-row index.
@@ -907,9 +987,7 @@ kB1_insert(const uint64_t* __restrict__ slab_keys, uint32_t* __restrict__ slab_r
       if ((uint32_t)(old >> 32) == fp) {
         const uint32_t q = (uint32_t)old;
         if (slab_keys[q] == key) {                          // an earlier row of the same k-mer
-          fold_partial_row(slab_rows, p, q, WP);
-          slab_cnt[p] = kCntDead;
-          slab_cnt[q] = kCntDirty;
+          fold_into_owner(slab_rows, slab_cnt, p, q, WP);
           atomicAdd(&counters[LC_RESCUE], 1u);              // (the rescue counter is free again after kA)
           break;
         }
@@ -942,16 +1020,8 @@ kB3_emit(const uint64_t* __restrict__ slab_keys, const uint32_t* __restrict__ sl
   if (n) cl = clusters[c];
   auto row_of = [&](uint32_t i) { return reinterpret_cast<const uint4*>(slab_rows + (size_t)(base + i) * WP); };
   auto count_of = [&](uint32_t i, bool& owner) {
-    uint32_t cnt = i < n ? slab_cnt[base + i] : kCntDead;
+    const uint32_t cnt = i < n ? partial_row_count(slab_rows, slab_cnt[base + i], base + i, WP) : kCntDead;
     owner = cnt != kCntDead;
-    if (cnt == kCntDirty) {                    // another row of the k-mer was folded in: recount
-      cnt = 0;
-      const uint4* row = row_of(i);
-      for (uint32_t q = 0; q < WP / 4; ++q) {
-        const uint4 x = row[q];
-        cnt += __popc(x.x) + __popc(x.y) + __popc(x.z) + __popc(x.w);
-      }
-    }
     return cnt;
   };
   // pass 1: rows this warp will write (verdicts of the first 256 partial rows stay in registers)
@@ -998,16 +1068,22 @@ kB3_emit(const uint64_t* __restrict__ slab_keys, const uint32_t* __restrict__ sl
       out.kmer[gi] = slab_keys[base + i];
       out.count[gi] = cnt;
       uint32_t* dst = out.cand + gi * out.key_words;
-      // (one row per half-warp through shuffles, so that loads and stores are coalesced segments,
-      //  was measured and is slower: kB 2.48 against 2.06 ms per config-2 step)
-      const uint4* row = row_of(i);
-      for (uint32_t q = 0; q < WP / 4; ++q) {
-        const uint4 x = row[q];
-        const uint32_t w = 4 * q;
-        if (w < W) dst[w] = x.x;
-        if (w + 1 < W) dst[w + 1] = x.y;
-        if (w + 2 < W) dst[w + 2] = x.z;
-        if (w + 3 < W) dst[w + 3] = x.w;
+      const uint32_t code = cnt == 1u ? slab_cnt[base + i] : 0u;
+      if (cnt_single(code)) {                  // one sample (a window with lo <= 1): no row to read
+        const uint32_t s = code & 0x3ffu;
+        for (uint32_t w = 0; w < W; ++w) dst[w] = w == (s >> 5) ? 1u << (s & 31u) : 0u;
+      } else {
+        // (one row per half-warp through shuffles, so that loads and stores are coalesced segments,
+        //  was measured and is slower: kB 2.48 against 2.06 ms per config-2 step)
+        const uint4* row = row_of(i);
+        for (uint32_t q = 0; q < WP / 4; ++q) {
+          const uint4 x = row[q];
+          const uint32_t w = 4 * q;
+          if (w < W) dst[w] = x.x;
+          if (w + 1 < W) dst[w + 1] = x.y;
+          if (w + 2 < W) dst[w + 2] = x.z;
+          if (w + 3 < W) dst[w + 3] = x.w;
+        }
       }
       if (out.key_words > W) dst[W] = out.cluster_pattern[c];
     }
@@ -1039,20 +1115,6 @@ struct LinkEntry {         // 16 bytes, memset to 0xff: key empty, row nil, coun
   uint32_t count;          // (sum of popcounts) - 1
 };
 
-__device__ __forceinline__ uint32_t partial_row_count(const uint32_t* __restrict__ slab_rows,
-                                                      const uint32_t* __restrict__ slab_cnt, uint32_t p, uint32_t WP) {
-  uint32_t cnt = slab_cnt[p];
-  if (cnt == kCntDirty) {                      // another row of the k-mer was folded in: recount
-    const uint4* row = reinterpret_cast<const uint4*>(slab_rows + (size_t)p * WP);
-    cnt = 0;
-    for (uint32_t q = 0; q < WP / 4; ++q) {
-      const uint4 x = row[q];
-      cnt += __popc(x.x) + __popc(x.y) + __popc(x.z) + __popc(x.w);
-    }
-  }
-  return cnt;
-}
-
 // one warp per kA work item, one row per lane and turn.  (Four rows per lane in flight measured
 // slower, 0.49 against 0.39 ms on 48 clusters of 10,000 samples: the registers cost occupancy, and
 // visiting the slices of a run far apart in time was slower still, 0.76 ms: the 20 slices of a
@@ -1071,7 +1133,7 @@ kB4_link(const uint64_t* __restrict__ slab_keys, const uint32_t* __restrict__ sl
   const uint32_t tb = table2_base[c] * 256u, ts = (table2_base[c + 1] - table2_base[c]) * 256u;
   const uint32_t base = slab_base[item];
   for (uint32_t i = lane_id(); i < n; i += 32u) {
-    const uint32_t cnt = partial_row_count(slab_rows, slab_cnt, base + i, WP);
+    const uint32_t cnt = partial_row_count(slab_rows, slab_cnt[base + i], base + i, WP);
     if (cnt == kCntDead) continue;              // folded into an earlier row of its slice
     const unsigned long long key = slab_keys[base + i];
     uint32_t s = __umulhi((uint32_t)(mix64(key) >> 32), ts);
@@ -1158,8 +1220,9 @@ kB6_scatter(const uint64_t* __restrict__ slab_keys, const uint32_t* __restrict__
   const uint32_t lane = lane_id();
   for (uint32_t i0 = 0; i0 < n; i0 += 32) {
     const uint32_t p = base + i0 + lane;
-    uint32_t g = 0xffffffffu;
-    if (i0 + lane < n && slab_cnt[p] != kCntDead) {      // (dead: folded into an earlier row of its slice)
+    uint32_t g = 0xffffffffu, code = 0;
+    if (i0 + lane < n) code = slab_cnt[p];
+    if (i0 + lane < n && partial_row_count(slab_rows, code, p, WP) != kCntDead) {   // (dead: folded into an earlier row of its slice)
       const unsigned long long key = slab_keys[p];
       uint32_t s = __umulhi((uint32_t)(mix64(key) >> 32), ts);
       if ((home_bits[(tb + s) >> 5] >> ((tb + s) & 31)) & 1u) {      // a survivor lives at this home slot
@@ -1170,8 +1233,14 @@ kB6_scatter(const uint64_t* __restrict__ slab_keys, const uint32_t* __restrict__
     }
     // the rows of survivors (a fifth of the partial rows: surviving k-mers sit in most slices) are
     // copied by half-warps, two rows per instruction, 64 B coalesced: ms_count of config 4 129.0
-    // against 135.7 ms with every lane copying its own row
-    uint32_t m = __ballot_sync(kFull, g != 0xffffffffu);
+    // against 135.7 ms with every lane copying its own row.  A one-sample row is one word: kB5
+    // cleared the k-mer's row and its slice has no other live row
+    const bool single = g != 0xffffffffu && cnt_single(code);
+    if (single) {
+      const uint32_t s = code & 0x3ffu;
+      out.cand[(size_t)g * out.key_words + w0 + (s >> 5)] = 1u << (s & 31u);
+    }
+    uint32_t m = __ballot_sync(kFull, g != 0xffffffffu && !single);
     while (m) {
       const int l0 = __ffs(m) - 1;
       m &= m - 1;

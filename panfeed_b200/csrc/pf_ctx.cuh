@@ -604,10 +604,10 @@ constexpr uint32_t kBlkMaxSmem = 220u * 1024u;   // largest kA table we ask for
 enum { C_TICKET_N = 0, C_TICKET_W = 1, C_RUNS_N = 2, C_RUNS_W = 3, C_ERR = 4, C_ROWS_N = 5,
        C_ROWS_W = 6, C_NEW_KP = 7, C_NEW_CP = 8, C_TICKET_MARK_N = 9, C_TICKET_MARK_W = 10,
        C_LOCAL = 11 /* LC_COUNT words: rows, unique, table overflow, row overflow, rescue runs,
-                        partial rows, partial overflow, kA segments */,
-       C_X_UNIQUE_KP = 19, C_X_UNIQUE_CP = 20 /* owner-side unique counts of the exchange */,
-       C_TICKET_X = 21, C_RUNS_X = 22, C_ROWS_X = 23, C_TICKET_MARK_X = 24 /* 256-bit keys (k > 32) */,
-       C_UNIQUE_WX = 25 /* distinct live keys of the wide and 256-bit records (k > 32 with N/IUPAC) */,
+                        partial rows, partial overflow, kA segments, one-sample partial rows */,
+       C_X_UNIQUE_KP = 20, C_X_UNIQUE_CP = 21 /* owner-side unique counts of the exchange */,
+       C_TICKET_X = 22, C_RUNS_X = 23, C_ROWS_X = 24, C_TICKET_MARK_X = 25 /* 256-bit keys (k > 32) */,
+       C_UNIQUE_WX = 26 /* distinct live keys of the wide and 256-bit records (k > 32 with N/IUPAC) */,
        C_COUNT = 28 };
 static_assert(C_COUNT <= 32, "mirror_counters copies one warp's worth");
 static_assert(C_LOCAL + LC_COUNT <= C_X_UNIQUE_KP, "counter layout");

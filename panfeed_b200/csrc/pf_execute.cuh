@@ -704,9 +704,10 @@ extern "C" int pf_execute(pf_ctx* ctx) {
       bool too_big = false;
       static const bool dbg = getenv("PF_DEBUG_BLOCK") != nullptr;
       if (dbg)
-        fprintf(stderr, "[pf] kA: items %u slots %u cap %u cslots %u -> overflow %u rescue %u partials %u part_ovf %u\n",
-                ctx->n_items, ctx->blk_slots, ctx->blk_cap, ctx->blk_cslots, hcnt[C_LOCAL + LC_TABLE_OVERFLOW],
-                hcnt[C_LOCAL + LC_RESCUE], hcnt[C_LOCAL + LC_PARTIALS], hcnt[C_LOCAL + LC_PARTIAL_OVERFLOW]);
+        fprintf(stderr, "[pf] kA: items %u slots %u cap %u cslots %u -> overflow %u rescue %u partials %u (one-sample %u) "
+                "part_ovf %u\n", ctx->n_items, ctx->blk_slots, ctx->blk_cap, ctx->blk_cslots,
+                hcnt[C_LOCAL + LC_TABLE_OVERFLOW], hcnt[C_LOCAL + LC_RESCUE], hcnt[C_LOCAL + LC_PARTIALS],
+                hcnt[C_LOCAL + LC_SINGLES], hcnt[C_LOCAL + LC_PARTIAL_OVERFLOW]);
       {
         uint32_t slots = ctx->blk_slots, cap = ctx->blk_cap, cslots = ctx->blk_cslots;
         int cur = 0;
@@ -739,8 +740,9 @@ extern "C" int pf_execute(pf_ctx* ctx) {
           mirror_counters<<<1, 32, 0, st>>>(hcnt, counters, C_COUNT);
           CU(cudaStreamSynchronize(st));
           if (dbg)
-            fprintf(stderr, "[pf] kA rescue: %u items slots %u cap %u cslots %u -> overflow %u rescue %u\n", n_resc, slots,
-                    cap, cslots, hcnt[C_LOCAL + LC_TABLE_OVERFLOW], hcnt[C_LOCAL + LC_RESCUE]);
+            fprintf(stderr, "[pf] kA rescue: %u items slots %u cap %u cslots %u -> overflow %u rescue %u partials %u "
+                    "(one-sample %u)\n", n_resc, slots, cap, cslots, hcnt[C_LOCAL + LC_TABLE_OVERFLOW],
+                    hcnt[C_LOCAL + LC_RESCUE], hcnt[C_LOCAL + LC_PARTIALS], hcnt[C_LOCAL + LC_SINGLES]);
         }
         // many rescued blocks: start the next batches with more rows (and key slots to match)
         if (!too_big && first_rescue > n_ka_items / 8u) {
