@@ -27,7 +27,8 @@
 //                       repeats), so the partial rows of one cluster are merged by FULL key in a
 //                       per-cluster open-addressing table in global memory: the first row of a
 //                       key owns it, later ones OR their bitset into the owner's; owners are
-//                       filtered on their popcount with the integer MAF window and emitted.
+//                       filtered on their popcount with the integer MAF window and emitted,
+//                       one CTA per cluster, with the cluster's distinct bitsets as K4's candidates.
 //   kB4/kB5             with sample slices (S > 1024) kB1 merges per (cluster, slice); kB4
 //                       links the slices of a k-mer and sums their popcounts, kB5 filters on the
 //                       sum and assembles the full-width bitsets of the survivors.
@@ -997,106 +998,235 @@ kB1_insert(const uint64_t* __restrict__ slab_keys, uint32_t* __restrict__ slab_r
   }
 }
 
-// kB3: one warp per slab; owners are counted, filtered and written out as rows.  Rows are
-// handed out with ONE global atomic per CTA (a counter shared by 300,000 warps serialises).
-__global__ void __launch_bounds__(256)
-kB3_emit(const uint64_t* __restrict__ slab_keys, const uint32_t* __restrict__ slab_rows,
-         const uint32_t* __restrict__ slab_base, const uint32_t* __restrict__ slab_count,
-         const uint32_t* __restrict__ item_cluster, uint32_t n_items,
-         const uint32_t* __restrict__ slab_cnt, const ClusterDev* __restrict__ clusters, RowOut out,
-         uint32_t row_capacity, uint32_t* __restrict__ counters, uint32_t W, uint32_t WP) {
-  __shared__ uint32_t w_pass[8];
-  __shared__ uint32_t cta_base, cta_ok;
-  const uint32_t item = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  const uint32_t lane = lane_id(), warp = threadIdx.x >> 5;
-  uint32_t n = 0, c = 0, base = 0;
-  if (item < n_items) {
-    n = slab_count[item];
-    if (n == kBlkOverflow) n = 0;
-    c = item_cluster[item];
-    base = slab_base[item];
+// kB3: one CTA per cluster; owners are counted, filtered and written out as rows, and the rows'
+// bitsets are deduplicated inside the cluster before K4 sees them.  All k-mers of a stretch of a
+// cluster carry the same sample set until a SNP enters or leaves the window, so ~4 surviving rows
+// share each pattern; patterns of different clusters rarely coincide.  K4 gets one candidate per
+// pattern of a cluster instead of one per row (row_cand maps a row to its candidate) and still
+// deduplicates the candidates globally on the full key, so the result does not depend on how
+// many rows share a candidate.
+//   pass 1  verdict of every partial row (owner, count in [lo, hi]); the survivors are listed in
+//           shared memory; ONE atomic takes the cluster's rows
+//   pass 2  the rows, one survivor per thread; each bitset is found or inserted in a
+//           shared-memory table of the cluster's patterns (entry: 16-bit hash fingerprint |
+//           candidate id; a candidate remembers the survivor that created it, and a match is
+//           confirmed on all words: nothing is merged on a hash).  Lanes of a warp with equal
+//           hashes (neighbouring k-mers of one stretch) compare with their leader instead.
+//   pass 3  ONE atomic takes the candidates; their bitsets and row_cand are written
+// A cluster with more survivors than the list takes (PF_PATTERN_SMEM_KB) makes every row its own
+// candidate, written on a second walk over its partial rows.
+constexpr uint32_t kEmitThreads = 512;
+constexpr uint32_t kEmitWarps = kEmitThreads / 32;
+constexpr uint32_t kPatEmpty = 0xffffffffu, kPatLocked = 0xfffffffeu;
+constexpr uint32_t kPatMaxCand = 0xfff0u;          // candidate ids stay below the two marks' low halves
+constexpr uint32_t kNoOne = 0xffffu;               // a survivor whose bitset is a row of slab_rows
+// survivors of a cluster that `smem` bytes take: per survivor its partial row (4 bytes), count and
+// one-sample code (4), 1.5 table slots (6) and, as a candidate, the survivor that created it (2)
+__host__ __device__ inline uint32_t pattern_table_rows(uint32_t smem) {
+  const uint32_t n = smem >= 16u ? (smem - 16u) / 16u : 0u;
+  return n < kPatMaxCand ? n : kPatMaxCand;
+}
+
+// words 4q .. 4q + 3 of a pattern: partial row p of slab_rows (W rounded up to WP with zeros),
+// or the one-hot bitset of sample `one` (a one-sample row has no bitset in slab_rows)
+__device__ __forceinline__ uint4 pattern_quad(const uint32_t* __restrict__ slab_rows, uint32_t p, uint32_t one,
+                                              uint32_t q, uint32_t WP) {
+  if (one == kNoOne) return __ldg(reinterpret_cast<const uint4*>(slab_rows + (size_t)p * WP) + q);
+  uint4 x = make_uint4(0u, 0u, 0u, 0u);
+  if ((one >> 7) == q) {
+    const uint32_t b = 1u << (one & 31u);
+    switch ((one >> 5) & 3u) {
+      case 0: x.x = b; break;
+      case 1: x.y = b; break;
+      case 2: x.z = b; break;
+      default: x.w = b; break;
+    }
   }
-  ClusterDev cl{};
-  if (n) cl = clusters[c];
-  auto row_of = [&](uint32_t i) { return reinterpret_cast<const uint4*>(slab_rows + (size_t)(base + i) * WP); };
-  auto count_of = [&](uint32_t i, bool& owner) {
-    const uint32_t cnt = i < n ? partial_row_count(slab_rows, slab_cnt[base + i], base + i, WP) : kCntDead;
-    owner = cnt != kCntDead;
-    return cnt;
-  };
-  // pass 1: rows this warp will write (verdicts of the first 256 partial rows stay in registers)
-  uint32_t my = 0;
-  uint32_t verdict[8];
+  return x;
+}
+
+__global__ void __launch_bounds__(kEmitThreads)
+kB3_cluster_emit(const uint64_t* __restrict__ slab_keys, const uint32_t* __restrict__ slab_rows,
+                 const uint32_t* __restrict__ slab_base, const uint32_t* __restrict__ slab_count,
+                 const uint32_t* __restrict__ item_base /* [n_clusters + 1] */,
+                 const uint32_t* __restrict__ slab_cnt, const ClusterDev* __restrict__ clusters, RowOut out,
+                 uint32_t row_capacity, uint32_t* __restrict__ counters, uint32_t W, uint32_t WP,
+                 uint32_t cap /* pattern_table_rows(dynamic shared memory) */) {
+  extern __shared__ uint32_t pat_sm[];
+  __shared__ uint32_t s_total, s_emit, s_row_base, s_mode, s_cand_base, s_n_cand;
+  const uint32_t c = blockIdx.x, tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
+  const uint32_t it0 = item_base[c], it1 = item_base[c + 1];
+  const ClusterDev cl = clusters[c];
+  const uint32_t NQ = WP >> 2;
+  uint32_t* list_p = pat_sm;                  // [cap] partial row of survivor j
+  uint32_t* list_c = list_p + cap;            // [cap] one-sample code << 16 | count (pass 2: | candidate)
+  if (tid == 0) { s_total = 0; s_emit = 0; s_n_cand = 0; }
+  __syncthreads();
+
+  // every survivor of the cluster: visit(partial row, count, one-sample code, index j from *next).
+  // A warp takes every kEmitWarps-th slab, 128 rows per turn (four loads in flight per lane).
+  auto walk = [&](uint32_t* next, auto&& visit) {
+    for (uint32_t it = it0 + warp; it < it1; it += kEmitWarps) {
+      uint32_t n = slab_count[it];
+      if (n == kBlkOverflow) n = 0;
+      const uint32_t base = slab_base[it];
+      for (uint32_t i0 = 0; i0 < n; i0 += 128) {
+        uint32_t code[4];
 #pragma unroll
-  for (int it = 0; it < 8; ++it) {
-    verdict[it] = 0u;
-    if ((uint32_t)it * 32u < n) {
-      bool owner;
-      const uint32_t cnt = count_of((uint32_t)it * 32u + lane, owner);
-      const bool pass = owner && cnt >= cl.lo && cnt <= cl.hi;
-      verdict[it] = pass ? (0x80000000u | cnt) : 0u;
-      my += __popc(__ballot_sync(kFull, pass));
-    }
-  }
-  for (uint32_t i0 = 256; i0 < n; i0 += 32) {
-    bool owner;
-    const uint32_t cnt = count_of(i0 + lane, owner);
-    my += __popc(__ballot_sync(kFull, owner && cnt >= cl.lo && cnt <= cl.hi));
-  }
-  if (lane == 0) w_pass[warp] = my;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    uint32_t total = 0;
-    for (int w = 0; w < 8; ++w) { const uint32_t x = w_pass[w]; w_pass[w] = total; total += x; }
-    uint32_t b = 0, ok = 1;
-    if (total) {
-      b = atomicAdd(&counters[LC_ROWS], total);
-      if ((uint64_t)b + total > row_capacity) { ok = 0; atomicExch(&counters[LC_ROW_OVERFLOW], 1u); }
-    }
-    cta_base = b;
-    cta_ok = ok;
-  }
-  __syncthreads();
-  if (!cta_ok || my == 0) return;
-  // pass 2: write them (the bitsets come back from L2)
-  uint32_t g = cta_base + w_pass[warp];
-  auto emit = [&](uint32_t i, bool pass, uint32_t cnt) {
-    const uint32_t mp = __ballot_sync(kFull, pass);
-    if (pass) {
-      const size_t gi = (size_t)g + __popc(mp & lanemask_lt());
-      out.cluster[gi] = cl.id;
-      out.kmer[gi] = slab_keys[base + i];
-      out.count[gi] = cnt;
-      uint32_t* dst = out.cand + gi * out.key_words;
-      const uint32_t code = cnt == 1u ? slab_cnt[base + i] : 0u;
-      if (cnt_single(code)) {                  // one sample (a window with lo <= 1): no row to read
-        const uint32_t s = code & 0x3ffu;
-        for (uint32_t w = 0; w < W; ++w) dst[w] = w == (s >> 5) ? 1u << (s & 31u) : 0u;
-      } else {
-        // (one row per half-warp through shuffles, so that loads and stores are coalesced segments,
-        //  was measured and is slower: kB 2.48 against 2.06 ms per config-2 step)
-        const uint4* row = row_of(i);
-        for (uint32_t q = 0; q < WP / 4; ++q) {
-          const uint4 x = row[q];
-          const uint32_t w = 4 * q;
-          if (w < W) dst[w] = x.x;
-          if (w + 1 < W) dst[w + 1] = x.y;
-          if (w + 2 < W) dst[w + 2] = x.z;
-          if (w + 3 < W) dst[w + 3] = x.w;
+        for (int u = 0; u < 4; ++u) {
+          const uint32_t i = i0 + 32u * u + lane;
+          code[u] = i < n ? slab_cnt[base + i] : kCntDead;
+        }
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+          const uint32_t p = base + i0 + 32u * u + lane;
+          const uint32_t cnt = partial_row_count(slab_rows, code[u], p, WP);     // kCntDead past n
+          const bool pass = cnt != kCntDead && cnt >= cl.lo && cnt <= cl.hi;
+          const uint32_t mp = __ballot_sync(kFull, pass);
+          if (!mp) continue;
+          uint32_t b = 0;
+          if (lane == 0) b = atomicAdd(next, (uint32_t)__popc(mp));
+          b = __shfl_sync(kFull, b, 0);
+          if (pass) visit(p, cnt, cnt_single(code[u]) ? (code[u] & 0x3ffu) : kNoOne, b + __popc(mp & lanemask_lt()));
         }
       }
-      if (out.key_words > W) dst[W] = out.cluster_pattern[c];
     }
-    g += __popc(mp);
   };
-#pragma unroll
-  for (int it = 0; it < 8; ++it)
-    if ((uint32_t)it * 32u < n) emit((uint32_t)it * 32u + lane, (verdict[it] >> 31) != 0u, verdict[it] & 0x7fffffffu);
-  for (uint32_t i0 = 256; i0 < n; i0 += 32) {
-    bool owner;
-    const uint32_t cnt = count_of(i0 + lane, owner);
-    emit(i0 + lane, owner && cnt >= cl.lo && cnt <= cl.hi, cnt);
+  auto write_row = [&](uint32_t gi, uint32_t p, uint32_t cnt) {
+    out.cluster[gi] = cl.id;
+    out.kmer[gi] = slab_keys[p];
+    out.count[gi] = cnt;
+  };
+  auto write_cand = [&](uint32_t id, uint32_t p, uint32_t one) {
+    uint32_t* dst = out.cand + (size_t)id * out.key_words;
+    for (uint32_t q = 0; q < NQ; ++q) {
+      const uint4 x = pattern_quad(slab_rows, p, one, q, WP);
+      const uint32_t w = 4 * q;
+      if (w < W) dst[w] = x.x;
+      if (w + 1 < W) dst[w + 1] = x.y;
+      if (w + 2 < W) dst[w + 2] = x.z;
+      if (w + 3 < W) dst[w + 3] = x.w;
+    }
+    if (out.key_words > W) dst[W] = out.cluster_pattern[c];       // the same word for every row of c
+  };
+
+  // ---- pass 1: list the survivors ----------------------------------------------------------------
+  walk(&s_total, [&](uint32_t p, uint32_t cnt, uint32_t one, uint32_t j) {
+    if (j < cap) { list_p[j] = p; list_c[j] = (one << 16) | cnt; }
+  });
+  __syncthreads();
+  if (tid == 0) {
+    const uint32_t total = s_total;
+    uint32_t b = 0, mode = 0;                       // 0: nothing to write, 1: table, 2: a candidate per row
+    if (total) {
+      b = atomicAdd(&counters[LC_ROWS], total);
+      if ((uint64_t)b + total > row_capacity) atomicExch(&counters[LC_ROW_OVERFLOW], 1u);
+      else if (total <= cap) mode = 1;
+      else { mode = 2; s_cand_base = atomicAdd(&counters[LC_CAND], total); }
+    }
+    s_row_base = b;
+    s_mode = mode;
   }
+  __syncthreads();
+  const uint32_t mode = s_mode, total = s_total, row_base = s_row_base;
+  if (mode == 0) return;
+  if (mode == 2) {                                  // too many survivors: walk again, rows are candidates
+    const uint32_t cand_base = s_cand_base;
+    walk(&s_emit, [&](uint32_t p, uint32_t cnt, uint32_t one, uint32_t j) {
+      write_row(row_base + j, p, cnt);
+      write_cand(cand_base + j, p, one);
+      out.row_cand[row_base + j] = cand_base + j;
+    });
+    return;
+  }
+
+  // ---- pass 2: rows, and the candidate of each ------------------------------------------------
+  const uint32_t slots = total + (total >> 1) + 1u;
+  uint32_t* tab = list_c + cap;                                     // [slots]
+  uint16_t* cand = reinterpret_cast<uint16_t*>(tab + slots);        // [<= total] survivor that created it
+  for (uint32_t i = tid; i < slots; i += kEmitThreads) tab[i] = kPatEmpty;
+  __syncthreads();
+  auto same = [&](uint32_t p, uint32_t one, uint32_t p2, uint32_t one2) {
+    if (one != kNoOne && one2 != kNoOne) return one == one2;
+    for (uint32_t q = 0; q < NQ; ++q) {
+      const uint4 a = pattern_quad(slab_rows, p, one, q, WP), b = pattern_quad(slab_rows, p2, one2, q, WP);
+      if (a.x != b.x || a.y != b.y || a.z != b.z || a.w != b.w) return false;
+    }
+    return true;
+  };
+  auto new_cand = [&](uint32_t j) {
+    const uint32_t id = atomicAdd(&s_n_cand, 1u);   // each survivor takes at most one: ids < total
+    cand[id] = (uint16_t)j;
+    return id;
+  };
+  // local candidate id of survivor j's pattern (inserted if new)
+  auto find_or_insert = [&](uint32_t j, uint32_t p, uint32_t one, uint64_t h) -> uint32_t {
+    const uint32_t fp = (uint32_t)h & 0xffffu;
+    uint32_t s = __umulhi((uint32_t)(h >> 32), slots);
+    for (uint32_t probes = 0, spins = 0; probes < slots;) {
+      const uint32_t e = ld_volatile_shared(&tab[s]);
+      if (e == kPatEmpty) {
+        if (atomicCAS(&tab[s], kPatEmpty, kPatLocked) == kPatEmpty) {
+          const uint32_t id = new_cand(j);
+          __threadfence_block();
+          *reinterpret_cast<volatile uint32_t*>(&tab[s]) = (fp << 16) | id;
+          return id;
+        }
+        continue;
+      }
+      if (e == kPatLocked) {                    // its owner publishes it in a few cycles
+        if (++spins > (1u << 14)) break;
+        __nanosleep(20);
+        continue;
+      }
+      if ((e >> 16) == fp) {
+        const uint32_t id = e & 0xffffu;
+        const uint32_t j2 = *reinterpret_cast<volatile uint16_t*>(&cand[id]);
+        if (same(p, one, list_p[j2], list_c[j2] >> 16)) return id;
+      }
+      if (++s == slots) s = 0;
+      ++probes;
+    }
+    return new_cand(j);                         // no slot: a candidate of its own (K4 merges it)
+  };
+  for (uint32_t j0 = warp * 32u; j0 < total; j0 += kEmitThreads) {
+    const uint32_t j = j0 + lane;
+    const bool live = j < total;
+    uint32_t p = 0, one = kNoOne;
+    uint64_t h = ~0ull;
+    if (live) {
+      p = list_p[j];
+      const uint32_t lc = list_c[j];
+      one = lc >> 16;
+      write_row(row_base + j, p, lc & 0xffffu);
+      h = 0;
+      for (uint32_t q = 0; q < NQ; ++q) {
+        const uint4 x = pattern_quad(slab_rows, p, one, q, WP);
+        h += word_hash(x.x, 4 * q) + word_hash(x.y, 4 * q + 1) + word_hash(x.z, 4 * q + 2) + word_hash(x.w, 4 * q + 3);
+      }
+      h = fmix64(h);
+    }
+    const uint32_t lm = __ballot_sync(kFull, live);
+    uint32_t leader = lane;
+    if (live) leader = __ffs(__match_any_sync(lm, h)) - 1;
+    uint32_t id = 0;
+    if (live && lane == leader) id = find_or_insert(j, p, one, h);
+    const uint32_t lid = __shfl_sync(kFull, id, leader);
+    const uint32_t lp = __shfl_sync(kFull, p, leader), lone = __shfl_sync(kFull, one, leader);
+    if (live && lane != leader) id = same(p, one, lp, lone) ? lid : find_or_insert(j, p, one, h);
+    if (live) list_c[j] = (one << 16) | id;     // (the count is written; readers use the high half)
+  }
+  __syncthreads();
+
+  // ---- pass 3: the candidates ---------------------------------------------------------------------
+  if (tid == 0) s_cand_base = atomicAdd(&counters[LC_CAND], s_n_cand);
+  __syncthreads();
+  const uint32_t cand_base = s_cand_base, n_cand = s_n_cand;
+  for (uint32_t id = tid; id < n_cand; id += kEmitThreads) {
+    const uint32_t j = cand[id];
+    write_cand(cand_base + id, list_p[j], list_c[j] >> 16);
+  }
+  for (uint32_t j = tid; j < total; j += kEmitThreads) out.row_cand[row_base + j] = cand_base + (list_c[j] & 0xffffu);
 }
 
 

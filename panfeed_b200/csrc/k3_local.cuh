@@ -42,7 +42,8 @@ constexpr uint64_t kEmptyKey = ~0ull;
 constexpr uint32_t kNoRow = 0xffffffffu;
 enum { LC_ROWS = 0, LC_UNIQUE = 1, LC_TABLE_OVERFLOW = 2, LC_ROW_OVERFLOW = 3, LC_RESCUE = 4,
        LC_PARTIALS = 5, LC_PARTIAL_OVERFLOW = 6, LC_SEGMENT = 7 /* kA's segment counter */,
-       LC_SINGLES = 8 /* one-sample partial rows kA wrote */, LC_COUNT = 9 };
+       LC_SINGLES = 8 /* one-sample partial rows kA wrote */,
+       LC_CAND = 9 /* K4 candidates of kB3_cluster_emit: patterns distinct within a cluster */, LC_COUNT = 10 };
 
 // prefix-runs of one radix pass are the digit buckets: their starts are the
 // scanned histogram itself.  first_run[t] = first bucket starting at or after tile t.

@@ -160,6 +160,8 @@ struct RowOut {
   uint32_t pattern_words;  // W
   const uint32_t* cluster_pattern;   // batch-local cluster -> cluster-pattern id (or null)
   uint32_t row_base;       // first row of this key width in the shared row arrays
+  uint32_t cand_base;      // first candidate of this key width: row_base, or less after a per-cluster emit
+  uint32_t* row_cand;      // kB3_cluster_emit: candidate of every row (rows share candidates); else null
 };
 
 // OR the sample bits of every live record of [a,b) whose key equals `cur` into
@@ -272,7 +274,7 @@ k3_runs(const KeyT* __restrict__ keys, const uint32_t* __restrict__ vals,
             store_kmer(out.kmer, row, unmix_key(cur));
             out.count[out.row_base + row] = c;
           }
-          uint32_t* dst = out.cand + (out.row_base + row) * out.key_words;
+          uint32_t* dst = out.cand + (out.cand_base + row) * out.key_words;
           for (uint32_t w = lane; w < W; w += 32) dst[w] = bits[w];
           if (out.key_words > W && lane == 0) dst[W] = out.cluster_pattern[seg];
         }

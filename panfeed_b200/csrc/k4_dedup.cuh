@@ -133,6 +133,16 @@ k4_commit(const uint32_t* __restrict__ cand, uint32_t n_rows, uint32_t key_words
   }
 }
 
+// pattern id of every row from its candidate's: the first n_mapped rows (kB3_cluster_emit) name
+// their candidate in row_cand, row r after them owns candidate r - shift
+__global__ void __launch_bounds__(256)
+k4_gather(const uint32_t* __restrict__ row_cand, uint32_t n_mapped, uint32_t shift,
+          const uint32_t* __restrict__ cand_pattern, uint32_t n_rows, uint32_t* __restrict__ row_pattern) {
+  const uint32_t r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= n_rows) return;
+  row_pattern[r] = cand_pattern[r < n_mapped ? row_cand[r] : r - shift];
+}
+
 // re-insert pool entries [0, n) into a fresh (larger) table; entries are distinct
 __global__ void __launch_bounds__(256)
 k4_rehash(const uint32_t* __restrict__ pool, uint32_t n, uint32_t key_words,

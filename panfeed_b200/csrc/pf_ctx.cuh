@@ -298,6 +298,8 @@ struct pf_ctx : BatchState {
   PinBuf h_counters;
   DevBuf d_bsum;
   DevBuf d_cand;
+  DevBuf d_row_cand, d_cand_pattern;   // block engine without slices: row -> K4 candidate -> pattern id
+  uint32_t n_cand_block = 0;     // candidates kB3_cluster_emit wrote for the last batch (0: a row is a candidate)
   DevBuf d_rep, d_slot_of, d_winner;
   DevBuf d_cl_rep, d_cl_slot, d_cl_winner;
   bool partition = true;   // mode 0: few radix passes + shared-memory hash grouping (k3_local)
@@ -330,6 +332,7 @@ struct pf_ctx : BatchState {
       d_spill /* (cluster, slice) merged in the global table */;
   uint32_t merge_fp_mask = 0x7fffu;   // PF_MERGE_FP_BITS (tests: a 1-bit fingerprint exercises the mismatch path)
   uint32_t merge_slots = 49152;  // shared-memory merge table of kB1_local (PF_MERGE_SMEM_KB)
+  uint32_t pattern_smem = 96u * 1024u;   // pattern table of kB3_cluster_emit, bytes (PF_PATTERN_SMEM_KB)
   PatternSpace kp, cp;     // k-mer patterns, cluster patterns
   // pinned results
   PinBuf r_row_cluster, r_row_kmer, r_wrow_kmer, r_xrow_kmer, r_row_count, r_row_pattern, r_cl_pattern;
@@ -604,11 +607,12 @@ constexpr uint32_t kBlkMaxSmem = 220u * 1024u;   // largest kA table we ask for
 enum { C_TICKET_N = 0, C_TICKET_W = 1, C_RUNS_N = 2, C_RUNS_W = 3, C_ERR = 4, C_ROWS_N = 5,
        C_ROWS_W = 6, C_NEW_KP = 7, C_NEW_CP = 8, C_TICKET_MARK_N = 9, C_TICKET_MARK_W = 10,
        C_LOCAL = 11 /* LC_COUNT words: rows, unique, table overflow, row overflow, rescue runs,
-                        partial rows, partial overflow, kA segments, one-sample partial rows */,
-       C_X_UNIQUE_KP = 20, C_X_UNIQUE_CP = 21 /* owner-side unique counts of the exchange */,
-       C_TICKET_X = 22, C_RUNS_X = 23, C_ROWS_X = 24, C_TICKET_MARK_X = 25 /* 256-bit keys (k > 32) */,
-       C_UNIQUE_WX = 26 /* distinct live keys of the wide and 256-bit records (k > 32 with N/IUPAC) */,
-       C_COUNT = 28 };
+                        partial rows, partial overflow, kA segments, one-sample partial rows,
+                        K4 candidates */,
+       C_X_UNIQUE_KP = 21, C_X_UNIQUE_CP = 22 /* owner-side unique counts of the exchange */,
+       C_TICKET_X = 23, C_RUNS_X = 24, C_ROWS_X = 25, C_TICKET_MARK_X = 26 /* 256-bit keys (k > 32) */,
+       C_UNIQUE_WX = 27 /* distinct live keys of the wide and 256-bit records (k > 32 with N/IUPAC) */,
+       C_COUNT = 29 };
 static_assert(C_COUNT <= 32, "mirror_counters copies one warp's worth");
 static_assert(C_LOCAL + LC_COUNT <= C_X_UNIQUE_KP, "counter layout");
 

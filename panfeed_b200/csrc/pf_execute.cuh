@@ -254,6 +254,7 @@ int ensure_rows(pf_ctx* ctx, uint64_t rows, uint64_t narrow_rows, bool keep) {
   TRY(dev_ensure(ctx, ctx->d_row_pattern, std::max<size_t>(1, rows) * 4, keep));
   TRY(dev_ensure(ctx, ctx->d_row_kmer, std::max<size_t>(1, narrow_rows) * 8, keep));
   TRY(dev_ensure(ctx, ctx->d_cand, std::max<size_t>(1, rows) * ctx->Wk * 4, keep));
+  if (ctx->block_mode && ctx->n_slices == 1) TRY(dev_ensure(ctx, ctx->d_row_cand, std::max<size_t>(1, rows) * 4, keep));
   return PF_OK;
 }
 
@@ -532,10 +533,12 @@ int launch_block_merge(pf_ctx* ctx, RowOut ro, uint32_t n_partials) {
                                  ctx->d_spill.as<uint8_t>());
   const uint32_t cap = (uint32_t)std::min<uint64_t>(ctx->row_cap, 0x7fffffffu);
   if (ns == 1) {
-    kB3_emit<<<g0, 256, 0, st>>>(ctx->d_slab_keys.as<uint64_t>(), ctx->d_slab_rows.as<uint32_t>(),
-                                 ctx->d_slab_base.as<uint32_t>(), ctx->d_slab_count.as<uint32_t>(),
-                                 ctx->d_item_cluster.as<uint32_t>(), ctx->n_items, ctx->d_slab_cnt.as<uint32_t>(),
-                                 ctx->d_clusters.as<ClusterDev>(), ro, cap, counters + C_LOCAL, ctx->W, WP);
+    ro.row_cand = ctx->d_row_cand.as<uint32_t>();
+    kB3_cluster_emit<<<nc, kEmitThreads, ctx->pattern_smem, st>>>(
+        ctx->d_slab_keys.as<uint64_t>(), ctx->d_slab_rows.as<uint32_t>(), ctx->d_slab_base.as<uint32_t>(),
+        ctx->d_slab_count.as<uint32_t>(), ctx->d_item_base.as<uint32_t>(), ctx->d_slab_cnt.as<uint32_t>(),
+        ctx->d_clusters.as<ClusterDev>(), ro, cap, counters + C_LOCAL, ctx->W, WP,
+        pattern_table_rows(ctx->pattern_smem));
     ctx->launches += 2;
     CU(cudaGetLastError());
     return PF_OK;
@@ -602,6 +605,7 @@ extern "C" int pf_execute(pf_ctx* ctx) {
   uint32_t* counters = ctx->d_counters.as<uint32_t>();
   uint32_t* hcnt = ctx->h_counters.as<uint32_t>();
   ctx->executed = false;
+  ctx->n_cand_block = 0;
   ctx->cp_base = ctx->cp.n;
   const bool part = ctx->partition;
 
@@ -799,6 +803,10 @@ extern "C" int pf_execute(pf_ctx* ctx) {
         continue;
       }
       ctx->used_block = true;
+      if (ctx->n_slices == 1) ctx->n_cand_block = hcnt[C_LOCAL + LC_CAND];
+      if (dbg)
+        fprintf(stderr, "[pf] kB: rows %u candidates %u (one-sample partial rows %u)\n", hcnt[C_LOCAL + LC_ROWS],
+                hcnt[C_LOCAL + LC_CAND], hcnt[C_LOCAL + LC_SINGLES]);
       ctx->partials_last = hcnt[C_LOCAL + LC_PARTIALS];
       if (n_windows) ctx->partial_ratio = std::max(1e-4, (double)ctx->partials_last / (double)n_windows);
       break;
@@ -929,19 +937,26 @@ extern "C" int pf_execute(pf_ctx* ctx) {
   ro.cluster = ctx->d_row_cluster.as<uint32_t>();
   ro.count = ctx->d_row_count.as<uint32_t>();
   ro.cand = ctx->d_cand.as<uint32_t>();
+  // K4's candidates: one per row, except that the block rows of kB3_cluster_emit share theirs
+  // (n_cand_block of them); the wide and 256-bit rows' candidates follow right after those
+  const bool cand_map = ctx->used_block && ctx->n_slices == 1;
+  const uint32_t cand_shift = cand_map ? N.n_rows - ctx->n_cand_block : 0u;
   if (!part && N.n_rows) {
     ro.kmer = ctx->d_row_kmer.as<uint64_t>();
     ro.row_base = 0;
+    ro.cand_base = 0;
     TRY((runs_width<uint64_t, true>(ctx, N, ro)));
   }
   if (Wd.n_rows) {
     ro.kmer = ctx->d_wrow_kmer.as<uint64_t>();
     ro.row_base = N.n_rows;
+    ro.cand_base = N.n_rows - cand_shift;
     TRY((runs_width<Key128, true>(ctx, Wd, ro)));
   }
   if (X.n_rows) {             // after the wide rows: K4 numbers the patterns of all three sections at once
     ro.kmer = ctx->d_xrow_kmer.as<uint64_t>();
     ro.row_base = N.n_rows + Wd.n_rows;
+    ro.cand_base = N.n_rows + Wd.n_rows - cand_shift;
     TRY((runs_width<Key256, true>(ctx, X, ro)));
   }
   CU(cudaEventRecord(ctx->ev[EV_REDUCE], st));
@@ -973,8 +988,22 @@ extern "C" int pf_execute(pf_ctx* ctx) {
   // once since): fold its pattern count in, then number this batch's patterns behind it
   TRY(finalize_pending(ctx));
   ctx->kp_base = ctx->kp.n;
-  TRY(dedup(ctx, ctx->kp, ctx->d_cand.as<uint32_t>(), (uint32_t)rows, ctx->d_rep, ctx->d_slot_of,
-            ctx->d_winner, ctx->d_row_pattern.as<uint32_t>(), C_NEW_KP));
+  if (cand_map) {
+    const uint32_t n_cand = (uint32_t)rows - cand_shift;
+    TRY(dev_ensure(ctx, ctx->d_cand_pattern, std::max<size_t>(1, n_cand) * 4));
+    TRY(dedup(ctx, ctx->kp, ctx->d_cand.as<uint32_t>(), n_cand, ctx->d_rep, ctx->d_slot_of,
+              ctx->d_winner, ctx->d_cand_pattern.as<uint32_t>(), C_NEW_KP));
+    if (rows) {
+      k4_gather<<<cdiv(rows, 256), 256, 0, st>>>(ctx->d_row_cand.as<uint32_t>(), N.n_rows, cand_shift,
+                                                 ctx->d_cand_pattern.as<uint32_t>(), (uint32_t)rows,
+                                                 ctx->d_row_pattern.as<uint32_t>());
+      ctx->launches++;
+      CU(cudaGetLastError());
+    }
+  } else {
+    TRY(dedup(ctx, ctx->kp, ctx->d_cand.as<uint32_t>(), (uint32_t)rows, ctx->d_rep, ctx->d_slot_of,
+              ctx->d_winner, ctx->d_row_pattern.as<uint32_t>(), C_NEW_KP));
+  }
   STAGE("k4 k-mer rows");
   CU(cudaEventRecord(ctx->ev[EV_DEDUP], st));
   TRY(pin_ensure(ctx, ctx->h_done, 16));

@@ -182,6 +182,11 @@ extern "C" int pf_create(pf_ctx** out, int device, const pf_params* p) {
     }
     cudaFuncSetAttribute(kB1_local, cudaFuncAttributeMaxDynamicSharedMemorySize,
                          (int)merge_local_smem_bytes(ctx->merge_slots));
+    if (const char* e = getenv("PF_PATTERN_SMEM_KB")) {     // 0: every row its own K4 candidate
+      const long kb = atol(e);
+      if (kb >= 0 && kb <= 200) ctx->pattern_smem = (uint32_t)(kb * 1024);
+    }
+    cudaFuncSetAttribute(kB3_cluster_emit, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ctx->pattern_smem);
     cudaFuncSetAttribute(kA_block_aggregate<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBlkMaxSmem);
     cudaFuncSetAttribute(kA_block_aggregate<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBlkMaxSmem);
   }
@@ -233,7 +238,7 @@ extern "C" void pf_destroy(pf_ctx* ctx) {
                       &bs->h_plan, &bs->h_done, &bs->h_raw, &bs->h_lite_tot})
       fp(*b);
   }
-  for (DevBuf* b : {&ctx->d_counters, &ctx->d_bsum, &ctx->d_cand, &ctx->d_rep, &ctx->d_slot_of, &ctx->d_winner,
+  for (DevBuf* b : {&ctx->d_counters, &ctx->d_bsum, &ctx->d_cand, &ctx->d_row_cand, &ctx->d_cand_pattern, &ctx->d_rep, &ctx->d_slot_of, &ctx->d_winner,
                     &ctx->d_cl_rep, &ctx->d_cl_slot, &ctx->d_cl_winner, &ctx->d_digests, &ctx->d_slab_base,
                     &ctx->d_slab_count, &ctx->d_slab_keys, &ctx->d_slab_rows, &ctx->d_group_base, &ctx->d_mtable,
                     &ctx->d_rescue[0], &ctx->d_rescue[1], &ctx->d_table2_base, &ctx->d_table2,
