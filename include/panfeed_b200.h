@@ -262,7 +262,7 @@ int pf_pattern_ids(pf_ctx* ctx, int cluster_namespace, uint64_t first, uint64_t 
 int pf_stats_get(pf_ctx* ctx, pf_stats* out);
 /* sizeof of the ABI structs as the library was built: 0 pf_params, 1 pf_seq_desc,
  * 2 pf_cluster_desc, 3 pf_batch, 4 pf_batch_result, 5 pf_stats, 6 pf_synth_params,
- * 7 pf_cut_result; 0 for an unknown id.  Lets a binding check its own struct mirrors. */
+ * 7 pf_cut_result, 8 pf_cut_planes, 9 pf_comm, 10 pf_exchange_result; 0 for an unknown id.  Lets a binding check its own struct mirrors. */
 uint32_t pf_struct_size(int which);
 /* CUDA stream the context launches on, as an opaque handle (cudaStream_t). */
 void* pf_stream(pf_ctx* ctx);
@@ -423,6 +423,72 @@ int pf_exchange_scatter(pf_ctx* ctx, int cluster_namespace, uint32_t world,
                         const uint32_t* mask_remap_dev, void* const* dest_ptrs /* [world]: device
                         pointers, the own buffer or pf_exchange_open_peer mappings */,
                         const uint64_t* dest_row0 /* [world] */);
+
+/* ---- the whole exchange in one call ----
+ * pf_exchange_run numbers the patterns of every rank globally, both namespaces, over collectives
+ * the caller provides (pf_comm: NCCL, torch.distributed, or pf_comm_local for the threads of one
+ * process).  Every rank calls it, each on its own pf_ctx; everything it enqueues goes on the
+ * context's stream (pf_stream), which the collectives receive as `stream`.  Order of the work:
+ *   1. owners and bucket positions of the local patterns (both namespaces at once; with
+ *      consider_missing the cluster namespace first, then the k-mer keys rewritten with its
+ *      local_to_global, then the k-mer namespace: steps 1-6 run once per namespace)
+ *   2. all_gather of one record per rank: bucket sizes, receive capacity, host identity,
+ *      device ordinal, receive buffer (raw pointer and CUDA IPC handle), flags; the one host sync
+ *      before the keys move.  Ranks that disagree on world, rank or consider_missing all return
+ *      PF_ERR_INVALID here.
+ *   3. transport: peer memory unless a rank set PF_EXCHANGE_NO_PEER or an earlier call fell back.
+ *      Receive buffers that are too small grow to need * 5/4 + 1024 rows: mappings of them are
+ *      closed, every rank passes a barrier, the owners reallocate, the record is gathered again.
+ *      Peers in the same process are written through their raw pointers (peer access enabled
+ *      between devices), peers in other processes through cached CUDA IPC mappings.  When the
+ *      mappings were (re)opened, every rank's "ok" is all-gathered: if one rank could not get
+ *      or map a buffer, all ranks take the all-to-all transport, now and in later calls, or all
+ *      return PF_ERR_UNSUPPORTED when a rank has no all_to_all_v.
+ *   4. peer memory: the keys go straight into the owners' buffers; a one-word all_gather is the
+ *      barrier after it.  All-to-all: keys packed by owner, all_to_all_v.
+ *   5. owner-side dedup; all_gather of the unique counts; owner_base = their exclusive scan (on
+ *      the device)
+ *   6. the unique index of every local key comes back (peer memory: copied from the owner's
+ *      buffer; otherwise all_to_all_v), local_to_global = owner_base[owner] + index
+ *   7. the final counts to the host (one sync).
+ * A collective that returns non-zero makes the call return PF_ERR_STATE; the caller then aborts
+ * its communicator (pf_comm_local_abort, ncclCommAbort) so that no other rank waits for ever. */
+
+/* Collectives the caller provides.  Both run on DEVICE buffers, are enqueued on `stream`
+ * (the context's, pf_stream) and have NCCL's semantics: a collective on a stream completes only
+ * after every rank's stream has reached it.  Return 0 on success. */
+typedef struct pf_comm {
+  uint32_t rank, world;
+  void*    user;
+  int (*all_gather)(const void* send, void* recv, uint64_t bytes_per_rank, void* stream, void* user);
+  /* may be NULL: then only the peer-memory transport is available */
+  int (*all_to_all_v)(const void* send, const uint64_t* send_bytes /*[world]*/, void* recv,
+                      const uint64_t* recv_bytes /*[world]*/, void* stream, void* user);
+} pf_comm;
+
+typedef struct pf_exchange_ns {      /* one namespace (cluster, k-mer) */
+  uint64_t n_local, n_global, n_owned, owned_base, bytes_sent;
+  const uint32_t* local_to_global;   /* device, [n_local], library-owned: valid until the next
+                                        pf_exchange_run / pf_reset_patterns / pf_destroy       */
+  const uint8_t*  writer;            /* device, [n_local], or NULL without PF_EXCHANGE_WRITER  */
+} pf_exchange_ns;
+typedef struct pf_exchange_result { pf_exchange_ns cluster, kmer; } pf_exchange_result;
+
+/* PF_EXCHANGE_WRITER: writer flags (1 on exactly one rank per global pattern: that rank writes its
+ * hashes_to_patterns row).  PF_EXCHANGE_KEEP_UNIQUE: the owner keeps its unique keys for
+ * pf_exchange_unique_export.  PF_EXCHANGE_NO_PEER: the all-to-all transport only. */
+enum { PF_EXCHANGE_WRITER = 1, PF_EXCHANGE_KEEP_UNIQUE = 2, PF_EXCHANGE_NO_PEER = 4 };
+
+int pf_exchange_run(pf_ctx* ctx, const pf_comm* comm, uint32_t flags, pf_exchange_result* out);
+int pf_exchange_release(pf_ctx* ctx, const pf_comm* comm);   /* collective: unmap the peers' buffers */
+
+/* Communicator for the threads of ONE process (one pf_ctx per thread, same or different devices):
+ * no NCCL, no daemon.  pf_comm_local_get fills a pf_comm for `rank`. */
+typedef struct pf_comm_local pf_comm_local;
+int  pf_comm_local_create(uint32_t world, pf_comm_local** out);
+int  pf_comm_local_get(pf_comm_local* g, uint32_t rank, pf_comm* out);
+void pf_comm_local_abort(pf_comm_local* g);      /* wakes every waiting rank with an error */
+void pf_comm_local_destroy(pf_comm_local* g);
 
 /* Pattern ids as text (host threads): out[24 * i ..] = base64 of the 16-byte digest i, as
  * binascii.b2a_base64(md5(...).digest())[:24] gives them (panfeed.py:175-176, 206-207). */

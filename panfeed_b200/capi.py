@@ -141,6 +141,31 @@ class CutPlanes(C.Structure):
                 ("amb_off", C.POINTER(C.c_uint64)), ("bad_symbol", C.c_int32)]
 
 
+ALL_GATHER_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p)
+ALL_TO_ALL_V_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.POINTER(C.c_uint64), C.c_void_p, C.POINTER(C.c_uint64),
+                              C.c_void_p, C.c_void_p)
+
+
+class Comm(C.Structure):
+    """pf_comm: the collectives pf_exchange_run runs over (device buffers, the context's stream)."""
+    _fields_ = [("rank", C.c_uint32), ("world", C.c_uint32), ("user", C.c_void_p),
+                ("all_gather", ALL_GATHER_FN), ("all_to_all_v", ALL_TO_ALL_V_FN)]
+
+
+class ExchangeNs(C.Structure):
+    """pf_exchange_ns: one namespace of a pf_exchange_run result."""
+    _fields_ = [("n_local", C.c_uint64), ("n_global", C.c_uint64), ("n_owned", C.c_uint64),
+                ("owned_base", C.c_uint64), ("bytes_sent", C.c_uint64),
+                ("local_to_global", C.c_void_p), ("writer", C.c_void_p)]
+
+
+class ExchangeResult(C.Structure):
+    _fields_ = [("cluster", ExchangeNs), ("kmer", ExchangeNs)]
+
+
+PF_EXCHANGE_WRITER, PF_EXCHANGE_KEEP_UNIQUE, PF_EXCHANGE_NO_PEER = 1, 2, 4
+
+
 EXPORTS = ["pf_create", "pf_destroy", "pf_last_error", "pf_abi_version",
            "pf_upload", "pf_execute", "pf_submit", "pf_collect",
            "pf_reset_patterns", "pf_pattern_words", "pf_kmer_pattern_words",
@@ -156,7 +181,8 @@ EXPORTS = ["pf_create", "pf_destroy", "pf_last_error", "pf_abi_version",
            "pf_synth_plan", "pf_synth_fill", "pf_exchange_pack",
            "pf_exchange_dedup", "pf_exchange_unique_count", "pf_exchange_unique_export",
            "pf_exchange_unpack", "pf_exchange_classify", "pf_exchange_recv_buffer", "pf_exchange_open_peer",
-           "pf_exchange_close_peer", "pf_exchange_scatter"]
+           "pf_exchange_close_peer", "pf_exchange_scatter", "pf_exchange_run", "pf_exchange_release",
+           "pf_comm_local_create", "pf_comm_local_get", "pf_comm_local_abort", "pf_comm_local_destroy"]
 
 _lib = None
 
@@ -247,6 +273,16 @@ def load():
     lib.pf_exchange_open_peer.argtypes = [vp, C.POINTER(C.c_ubyte), C.POINTER(vp)]
     lib.pf_exchange_close_peer.argtypes = [vp, vp]
     lib.pf_exchange_scatter.argtypes = [vp, C.c_int, u32, vp, C.POINTER(vp), C.POINTER(u64)]
+    lib.pf_exchange_run.argtypes = [vp, C.POINTER(Comm), u32, C.POINTER(ExchangeResult)]
+    lib.pf_exchange_release.argtypes = [vp, C.POINTER(Comm)]
+    lib.pf_comm_local_create.argtypes = [u32, C.POINTER(vp)]
+    lib.pf_comm_local_get.argtypes = [vp, u32, C.POINTER(Comm)]
+    lib.pf_comm_local_abort.argtypes = [vp]
+    lib.pf_comm_local_abort.restype = None
+    lib.pf_comm_local_destroy.argtypes = [vp]
+    lib.pf_comm_local_destroy.restype = None
+    lib.pf_struct_size.argtypes = [C.c_int]
+    lib.pf_struct_size.restype = u32
     if lib.pf_abi_version() != PF_ABI_VERSION:
         raise PfError(-1, "ABI version mismatch")
     _lib = lib
@@ -707,6 +743,63 @@ class Context:
 
     def stream_handle(self):
         return self.lib.pf_stream(self.h)
+
+    def exchange_run(self, comm, flags=0):
+        """pf_exchange_run over `comm` (a Comm, e.g. LocalComm.get(rank)): the global numbering of the
+        patterns of every rank.  -> {"cluster": ..., "kmer": ...}, each a dict of the counts and the
+        DEVICE addresses of local_to_global (uint32 [n_local]) and writer (uint8 [n_local] or 0),
+        owned by the context until its next exchange_run / reset_patterns / close."""
+        out = ExchangeResult()
+        self._check(self.lib.pf_exchange_run(self.h, C.byref(comm), int(flags), C.byref(out)))
+        return {name: {f: (getattr(ns, f) or 0) for f, _ in ExchangeNs._fields_}
+                for name, ns in (("cluster", out.cluster), ("kmer", out.kmer))}
+
+    def exchange_release(self, comm):
+        """pf_exchange_release: collective, unmaps the peers' receive buffers."""
+        self._check(self.lib.pf_exchange_release(self.h, C.byref(comm)))
+
+    def exchange_unique_keys(self, cluster_namespace):
+        """The owner-side unique keys of the last exchange (PF_EXCHANGE_KEEP_UNIQUE)."""
+        n = C.c_uint64()
+        self._check(self.lib.pf_exchange_unique_count(self.h, int(cluster_namespace), C.byref(n)))
+        out = np.zeros((n.value, self.W if cluster_namespace else self.Wk), np.uint32)
+        self._check(self.lib.pf_exchange_unique_export(self.h, int(cluster_namespace), out.ctypes.data))
+        return out
+
+
+class LocalComm:
+    """pf_comm_local: collectives between the threads of this process, one Context per thread (same
+    or different devices).  get(rank) is the Comm of one rank."""
+
+    def __init__(self, world):
+        self.lib = load()
+        self.h = C.c_void_p()
+        rc = self.lib.pf_comm_local_create(int(world), C.byref(self.h))
+        if rc != 0:
+            raise PfError(rc, f"pf_comm_local_create({world}) failed")
+        self.world = int(world)
+
+    def get(self, rank):
+        c = Comm()
+        rc = self.lib.pf_comm_local_get(self.h, int(rank), C.byref(c))
+        if rc != 0:
+            raise PfError(rc, f"pf_comm_local_get: no rank {rank} in a world of {self.world}")
+        return c
+
+    def abort(self):
+        """Every rank waiting in (or later entering) a collective returns an error."""
+        self.lib.pf_comm_local_abort(self.h)
+
+    def close(self):
+        if self.h:
+            self.lib.pf_comm_local_destroy(self.h)
+            self.h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
 
 
 class SynthArena:

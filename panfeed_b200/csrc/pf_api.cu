@@ -3,7 +3,7 @@
 // kernel sequencing, result staging.  One translation unit; the parts, in order:
 //   kernels      k1_*.cuh k2_*.cuh k3_*.cuh k4_dedup.cuh k5_md5.cuh synth.cuh
 //   host side    pf_ctx.cuh pf_lifetime.cuh pf_upload.cuh pf_execute.cuh pf_pipeline.cuh
-//                pf_synth_api.cuh pf_exchange.cuh
+//                pf_synth_api.cuh pf_exchange.cuh pf_exchange_run.cuh
 // (pf_format.cu, the native text formatter, is a second, host-only translation unit.)
 #include <cuda.h>            // driver types for the virtual-memory pool (entry points are fetched at run time)
 #include <cuda_runtime.h>
@@ -21,6 +21,7 @@
 #include <mutex>
 #include <string>
 #include <thread>
+#include <unistd.h>
 #include <unordered_map>
 #include <vector>
 
@@ -44,3 +45,4 @@ using namespace pf;
 #include "pf_pipeline.cuh"
 #include "pf_synth_api.cuh"
 #include "pf_exchange.cuh"
+#include "pf_exchange_run.cuh"

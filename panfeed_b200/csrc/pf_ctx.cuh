@@ -278,6 +278,8 @@ class AsyncWorker {
   bool busy_ = false, stop_ = false;
 };
 
+namespace { struct XRunState; }    // pf_exchange_run's own state (pf_exchange_run.cuh)
+
 struct pf_ctx : BatchState {
   pf_params prm{};
   int device = 0;
@@ -364,9 +366,12 @@ struct pf_ctx : BatchState {
   uint32_t pipe_target_seqs = 262144;   // sequences per sub-batch
   uint32_t pipe_first_seqs = 98304;     // ... of the first one (its upload is not hidden)
   bool lite_ok = true;           // device-side planning of uploads (PF_LITE=0 disables; off after a record fall-back)
+  XRunState* xrun = nullptr;     // created by the first pf_exchange_run
 };
 
 namespace {
+
+void xrun_free(pf_ctx* ctx);    // pf_exchange_run.cuh
 
 int fail(pf_ctx* c, int code, const char* fmt, ...) {
   char buf[512];

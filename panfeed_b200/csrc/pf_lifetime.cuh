@@ -33,6 +33,8 @@ extern "C" uint32_t pf_struct_size(int which) {
     case 6: return (uint32_t)sizeof(pf_synth_params);
     case 7: return (uint32_t)sizeof(pf_cut_result);
     case 8: return (uint32_t)sizeof(pf_cut_planes);
+    case 9: return (uint32_t)sizeof(pf_comm);
+    case 10: return (uint32_t)sizeof(pf_exchange_result);
     default: return 0;
   }
 }
@@ -245,6 +247,7 @@ extern "C" void pf_destroy(pf_ctx* ctx) {
                     &ctx->d_home_bits, &ctx->d_cta_cluster, &ctx->d_slab_cnt, &ctx->d_spill})
     fd(*b);
   ctx->grower.join();
+  xrun_free(ctx);                      // pf_exchange_run's buffers and peer mappings
   for (PatternSpace* s : {&ctx->kp, &ctx->cp}) pool_free(s->pool);
   for (PatternSpace* s : {&ctx->kp, &ctx->cp})
     for (DevBuf* b : {&s->table, &s->x_owner, &s->x_pos, &s->x_perm, &s->x_counts, &s->x_unique,

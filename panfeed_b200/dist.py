@@ -376,3 +376,104 @@ class PatternExchange:
                 #  of ctx->cp / ctx->kp - so the k-mer exchange has not overwritten the cluster namespace's)
                 out[name]["owned_keys"] = be.unique_keys(p["ns"])
         return out
+
+
+class _DeviceBytes:
+    """A device buffer of the library (raw address) as seen by torch: __cuda_array_interface__."""
+
+    def __init__(self, ptr, n, typestr="|u1"):
+        self.__cuda_array_interface__ = {"shape": (int(n),), "typestr": typestr, "data": (int(ptr), False),
+                                         "version": 2}
+
+
+def _device_view(ptr, n, device, typestr="|u1", dtype=torch.uint8):
+    if n == 0 or not ptr:
+        return torch.empty(0, dtype=dtype, device=device)
+    return torch.as_tensor(_DeviceBytes(ptr, n, typestr), device=device)
+
+
+class NativePatternExchange:
+    """The same global numbering as PatternExchange, in ONE library call (pf_exchange_run): the
+    transport choice, the peer mappings and the agreement points are the library's; this class only
+    hands it the collectives of torch.distributed (NCCL) as a pf_comm.  `run()` returns what
+    PatternExchange.run returns."""
+
+    def __init__(self, ctx, device, group=None):
+        from . import capi
+        self.ctx, self.device, self.group = ctx, device, group
+        self.world = dist.get_world_size(group) if dist.is_initialized() else 1
+        self.rank = dist.get_rank(group) if dist.is_initialized() else 0
+        self._error = None
+        # (the ctypes callbacks must stay referenced as long as the library may call them)
+        self._ag = capi.ALL_GATHER_FN(self._all_gather)
+        self._a2a = capi.ALL_TO_ALL_V_FN(self._all_to_all_v)
+        self.comm = capi.Comm(self.rank, self.world, None, self._ag, self._a2a)
+        self._ran = False
+
+    def _on(self, stream):
+        return torch.cuda.stream(torch.cuda.ExternalStream(stream, device=self.device))
+
+    def _all_gather(self, send, recv, nbytes, stream, user):
+        try:
+            with self._on(stream):
+                inp = _device_view(send, nbytes, self.device)
+                out = _device_view(recv, nbytes * self.world, self.device)
+                if self.world == 1:
+                    out.copy_(inp)
+                else:
+                    dist.all_gather_into_tensor(out, inp, group=self.group)
+            return 0
+        except Exception as e:          # (no exception may cross the C frames)
+            self._error = e
+            return -1
+
+    def _all_to_all_v(self, send, send_bytes, recv, recv_bytes, stream, user):
+        try:
+            sb = [int(send_bytes[r]) for r in range(self.world)]
+            rb = [int(recv_bytes[r]) for r in range(self.world)]
+            with self._on(stream):
+                inp = _device_view(send, sum(sb), self.device)
+                out = _device_view(recv, sum(rb), self.device)
+                if self.world == 1:
+                    out.copy_(inp)
+                else:
+                    dist.all_to_all_single(out, inp, output_split_sizes=rb, input_split_sizes=sb, group=self.group)
+            return 0
+        except Exception as e:
+            self._error = e
+            return -1
+
+    def run(self, want_unique=False, want_writer=False, flags=0):
+        import time
+        from . import capi
+        t0 = time.perf_counter()
+        flags |= (capi.PF_EXCHANGE_WRITER if want_writer else 0) | (capi.PF_EXCHANGE_KEEP_UNIQUE if want_unique else 0)
+        self._error = None
+        try:
+            res = self.ctx.exchange_run(self.comm, flags)
+        except capi.PfError:
+            if self._error is not None:
+                raise RuntimeError(f"pattern exchange: a collective failed: {self._error!r}") from self._error
+            raise
+        self._ran = True
+        ms = (time.perf_counter() - t0) * 1e3
+        out = {}
+        for name, ns in (("cluster", CLUSTER), ("kmer", KMER)):
+            r = res[name]
+            n = int(r["n_local"])
+            # copies: the library's tables are reused by its next exchange
+            l2g = _device_view(r["local_to_global"], n, self.device, "<i4", torch.int32).clone()
+            writer = _device_view(r["writer"], n, self.device).clone() if want_writer else None
+            out[name] = {"local_to_global": l2g, "writer": writer, "n_global": int(r["n_global"]),
+                         "n_owned": int(r["n_owned"]), "owned_base": int(r["owned_base"]),
+                         "bytes_sent": int(r["bytes_sent"]), "ms": {"total_both_namespaces": ms, "stages": None}}
+            if want_unique:
+                out[name]["owned_keys"] = self.ctx.exchange_unique_keys(ns == CLUSTER)
+        return out
+
+    def close(self):
+        """Collective, like PatternExchange.close: the peers' buffers are unmapped on every rank
+        before any rank goes on to destroy its context."""
+        if self._ran:
+            self.ctx.exchange_release(self.comm)
+            self._ran = False

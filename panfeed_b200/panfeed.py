@@ -155,7 +155,11 @@ class PatternStore:
         # (a context may bring its own exchange primitives and device: the CPU tests' stand-in does)
         dev = getattr(ctx, "exchange_device", None) or torch.device("cuda", device)
         backend = ctx.exchange_backend() if hasattr(ctx, "exchange_backend") else None
-        exchange = pfdist.PatternExchange(ctx, dev, backend=backend)
+        if os.environ.get("PF_EXCHANGE_IMPL", "") == "native":
+            # the whole exchange in one library call (pf_exchange_run) over torch.distributed
+            exchange = pfdist.NativePatternExchange(ctx, dev)
+        else:
+            exchange = pfdist.PatternExchange(ctx, dev, backend=backend)
         out = exchange.run(want_writer=True)
         exchange.close()
         W = (S + 31) // 32
