@@ -14,15 +14,18 @@
 //                       windows cover as ONE 128-bit chunk; identical chunks (same haplotype)
 //                       meet in a shared-memory chunk table and only OR one sample bit there:
 //                       ~25 instructions per sequence and run instead of per window.
-//                       Level 2: the few dozen DISTINCT chunks are cut into their 16 k-mers
+//                       A chunk's key carries the run's live-window mask (ragged tails, N /
+//                       IUPAC symbols), so every sequence takes this path.
+//                       Level 2: the few dozen DISTINCT chunks are cut into their live k-mers
 //                       (forward / reverse complement / canonical), each k-mer is looked up in
-//                       a shared-memory open-addressing table and takes the chunk's whole
-//                       W-word sample bitset.  The CTA ends by writing its distinct k-mers,
-//                       popcounts and bitsets ("partial rows") to a slab in HBM: ~1/30 of the
-//                       bytes the records would have taken, written once.  A row of one sample
-//                       (most rows) is written as its key and a one-sample code, without the
-//                       bitset (see slab_cnt).  Every run keeps its own slab, so the kernels
-//                       after kA see per-run items.
+//                       a shared-memory open-addressing table and the (chunk, window) pair is
+//                       pushed onto the k-mer row's list.  The CTA ends by writing its distinct
+//                       k-mers, popcounts and bitsets ("partial rows", a bitset being the OR of
+//                       the listed chunks' bitsets) to a slab in HBM: ~1/30 of the bytes the
+//                       records would have taken, written once.  A row of one sample (most
+//                       rows) is written as its key and a one-sample code, without the bitset
+//                       (see slab_cnt).  Every run keeps its own slab, so the kernels after kA
+//                       see per-run items.
 //   kB1/kB3             a k-mer can start in two runs (indels, clamped flanks, paralogs,
 //                       repeats), so the partial rows of one cluster are merged by FULL key in a
 //                       per-cluster open-addressing table in global memory: the first row of a
@@ -287,65 +290,78 @@ struct BlkPlan {
 // Shared memory of kA.  Both tables hand out DENSE row ids on insertion, so the epilogue needs
 // no compaction pass.  The tables are cleared once per CTA; after a run only what it touched is
 // undone: the key slot of every k-mer row (rslot) and the state slot of every chunk id (cslot)
-// are recorded on insertion, the pool rows are zeroed as they are copied out, and the chunk rows
-// 0..n_chunks-1 are cleared.  An overflowing run may have claimed slots without a row; after it
-// everything is cleared.
+// are recorded on insertion, row lists are emptied as the epilogue reads them, and the chunk
+// rows 0..n_chunks-1 are cleared.  An overflowing run may have claimed slots without
+// a row; after it everything is cleared.
 //
 // chunk table: the R = k + 15 bases that the 16 windows of a run cover, as a 128-bit key
-//   (top-aligned).  Sequences of a cluster are copies of a few haplotypes, so the ~500
+//   (top-aligned, bases past the sequence's end zero) whose free low 16 bits hold the run's
+//   live-window mask.  Sequences of a cluster are copies of a few haplotypes, so the ~500
 //   sequences of a run collapse into a few dozen distinct chunks; only those are cut into
-//   k-mers.  A slot's state word goes empty -> locked -> (full | chunk id).
+//   k-mers.  A chunk keeps the sample bitset of its sequences and its first sequence's sample,
+//   or kChunkMixed once a sequence of another sample joins it.  A slot's state word goes
+//   empty -> locked -> (full | chunk id).
 // k-mer table: 64-bit keys claimed with one CAS; rowid[slot] is published afterwards
-//   (0xffff = not yet), readers of a freshly claimed slot spin for those few cycles.
+//   (0xffff = not yet), readers of a freshly claimed slot spin for those few cycles.  A row
+//   holds no bitset, only a list of the (chunk, window[, strand]) nodes that carry its k-mer:
+//   rhead[row] -> pnext[node] -> ... -> kNodeNil.  Node = chunk * 16 + window (canonical) or
+//   2 * (chunk * 16 + window) + strand (--non-canonical).
 constexpr uint32_t kChunkEmpty = 0u, kChunkLocked = 1u, kChunkFull = 0x80000000u;
+constexpr uint32_t kNodeNil = 0xffffu, kChunkMixed = 0xffffu;
+constexpr uint32_t kBlkRowBytes = 14u;   // shared memory of a k-mer row: rkey, rhead, rslot
 struct ARunView {
   BlkHead* h;              // n_unique = k-mer rows handed out, work = chunk ids handed out
+  uint32_t* crows;         // [ccap * WP]  sample bitset of chunk id (16-byte aligned rows)
   uint64_t* keys;          // [slots]
-  uint64_t* rkey;          // [cap + 1]   key of row id
+  uint64_t* rkey;          // [cap + 1]   key of row id (row `cap`: scratch of an overflowing run)
   uint64_t* ckhi;          // [ccap]
-  uint64_t* cklo;          // [ccap]
+  uint64_t* cklo;          // [ccap]      low 16 bits: live-window mask
   uint32_t* cstate;        // [cslots]
-  uint32_t* pool;          // [(cap + 1) * WS]   row `cap` takes the ORs of an overflowing block
-  uint32_t* crows;         // [ccap * WS]
+  uint32_t* rhead;         // [cap]       first node of row id's list
   uint16_t* rowid;         // [slots]
-  uint16_t* cmeta;         // [ccap]  low byte: bitset word of the chunk's first sample; bit 15: other words too
-  uint16_t* rslot;         // [cap + 1]  key slot of row id
-  uint16_t* cslot;         // [ccap]     state slot of chunk id
+  uint16_t* rslot;         // [cap + 1]   key slot of row id
+  uint16_t* cslot;         // [ccap]      state slot of chunk id
+  uint16_t* csample;       // [ccap]      sample rank of chunk id's sequences, or kChunkMixed
+  uint16_t* pnext;         // [ccap * 16 * (CANON ? 1 : 2)]  next node of a row's list
   uint32_t mask, shift, cmask, cshift, cap, ccap;
 };
 __host__ __device__ inline uint32_t blkA_ccap(uint32_t cslots) { return cslots * 3u / 4u; }
 // slots: k-mer key slots (power of two); cap: k-mer rows (<= 13/16 slots); cslots: chunk slots
-__host__ __device__ inline uint32_t blkA_smem_bytes(uint32_t slots, uint32_t cap, uint32_t cslots, uint32_t W) {
-  const uint32_t ccap = blkA_ccap(cslots), WS = W | 1u;
-  return (uint32_t)sizeof(BlkHead) + slots * 8u + (cap + 1u) * 8u + ccap * 16u + cslots * 4u +
-         (cap + 1u) * WS * 4u + ccap * WS * 4u + slots * 2u + ccap * 2u + (cap + 1u) * 2u + ccap * 2u + 16u;
+// (power of two, <= 2048 so that node ids fit 16 bits); canon: one list node per (chunk, window)
+__host__ __device__ inline uint32_t blkA_smem_bytes(uint32_t slots, uint32_t cap, uint32_t cslots, uint32_t W,
+                                                   bool canon) {
+  const uint32_t ccap = blkA_ccap(cslots), WP = (W + 3u) & ~3u;
+  return (uint32_t)sizeof(BlkHead) + ccap * WP * 4u + slots * 8u + (cap + 1u) * 8u + ccap * 16u + cslots * 4u +
+         cap * 4u + slots * 2u + (cap + 1u) * 2u + ccap * 4u +
+         ccap * (uint32_t)kBlkRun * (canon ? 2u : 4u) + 16u;
 }
 __device__ __forceinline__ ARunView arun_view(unsigned char* raw, uint32_t slots, uint32_t cap, uint32_t cslots, uint32_t W) {
   ARunView a;
-  const uint32_t WS = W | 1u;
+  const uint32_t WP = (W + 3u) & ~3u;
   a.cap = cap;
   a.ccap = blkA_ccap(cslots);
   a.h = reinterpret_cast<BlkHead*>(raw);
-  a.keys = reinterpret_cast<uint64_t*>(raw + sizeof(BlkHead));
+  a.crows = reinterpret_cast<uint32_t*>(raw + sizeof(BlkHead));
+  a.keys = reinterpret_cast<uint64_t*>(a.crows + a.ccap * WP);
   a.rkey = a.keys + slots;
   a.ckhi = a.rkey + (a.cap + 1u);
   a.cklo = a.ckhi + a.ccap;
   a.cstate = reinterpret_cast<uint32_t*>(a.cklo + a.ccap);
-  a.pool = a.cstate + cslots;
-  a.crows = a.pool + (a.cap + 1u) * WS;
-  a.rowid = reinterpret_cast<uint16_t*>(a.crows + a.ccap * WS);
-  a.cmeta = a.rowid + slots;
-  a.rslot = a.cmeta + a.ccap;
+  a.rhead = a.cstate + cslots;
+  a.rowid = reinterpret_cast<uint16_t*>(a.rhead + a.cap);
+  a.rslot = a.rowid + slots;
   a.cslot = a.rslot + (a.cap + 1u);
+  a.csample = a.cslot + a.ccap;
+  a.pnext = a.csample + a.ccap;
   a.mask = slots - 1u;
   a.shift = 32u - (uint32_t)__popc(a.mask);
   a.cmask = cslots - 1u;
   a.cshift = 32u - (uint32_t)__popc(a.cmask);
   return a;
 }
-// chunk id of (hi, lo); 0xffffffff if the chunk table is full (the caller then cuts the run
-// into k-mers itself)
-__device__ __noinline__ uint32_t chunk_find_or_insert(const ARunView a, uint64_t hi, uint64_t lo, uint32_t wofs) {
+// chunk id of (hi, lo), created with `sample` if new; 0xffffffff if the chunk table is full (the
+// run then overflows)
+__device__ __noinline__ uint32_t chunk_find_or_insert(const ARunView a, uint64_t hi, uint64_t lo, uint32_t sample) {
   const uint64_t m = (hi ^ (hi >> 29)) * 0x9e3779b97f4a7c15ULL + (lo ^ (lo >> 31)) * 0xc2b2ae3d27d4eb4fULL;
   uint32_t s = (uint32_t)(m >> 32) >> a.cshift;
   uint32_t spins = 0;
@@ -367,8 +383,8 @@ __device__ __noinline__ uint32_t chunk_find_or_insert(const ARunView a, uint64_t
           *reinterpret_cast<volatile uint32_t*>(&a.cstate[s]) = kChunkEmpty;
           return 0xffffffffu;
         }
-        a.cmeta[id] = (uint16_t)wofs;
         a.cslot[id] = (uint16_t)s;
+        a.csample[id] = (uint16_t)sample;
         *reinterpret_cast<volatile uint64_t*>(&a.ckhi[id]) = hi;
         *reinterpret_cast<volatile uint64_t*>(&a.cklo[id]) = lo;
         __threadfence_block();
@@ -383,7 +399,7 @@ __device__ __noinline__ uint32_t chunk_find_or_insert(const ARunView a, uint64_t
   return 0xffffffffu;
 }
 // row id of a k-mer (insert if new); a.cap = the scratch row when the block overflows
-__device__ __noinline__ uint32_t kmer_row_slow(const ARunView a, uint64_t key, uint32_t h, uint32_t WS) {
+__device__ __noinline__ uint32_t kmer_row_slow(const ARunView a, uint64_t key, uint32_t h) {
   const uint32_t limit = min(a.mask, 96u);
   bool found = false;
   for (uint32_t probes = 0; probes < limit; ++probes) {
@@ -414,14 +430,14 @@ __device__ __noinline__ uint32_t kmer_row_slow(const ARunView a, uint64_t key, u
 }
 
 #ifndef PF_KA_MIN_CTAS
-#define PF_KA_MIN_CTAS 4
+#define PF_KA_MIN_CTAS 5      // 5 x 256 threads at 48 registers; ~30 KB of shared memory per CTA at S = 500
 #endif
 // A CTA walks SEGMENTS: `seg_runs` consecutive (cluster, run) items of one slice (item =
 // run_item * n_slices + slice), taken from counters[LC_SEGMENT] after the first one; with an
 // item list (a rescue launch) a segment is one listed item.  Every run still gets its own slab.
 // Across the runs of a segment a thread keeps its first two sequences of the (cluster, slice) in
-// registers: descriptor and the 64-bit words wi, wi + 1 of the run plus wi + 2, requested a run
-// ahead of its use.  A run starts at a multiple of 16, so its R <= 47 bases lie in two words.
+// registers: descriptor and the 64-bit words wi, wi + 1 of the run.  A run starts at a multiple
+// of 16, so its R <= 47 bases lie in two words.
 template <bool CANON>
 __global__ void __launch_bounds__(kBlkThreads, PF_KA_MIN_CTAS)
 kA_block_aggregate(const uint64_t* __restrict__ bases, const uint32_t* __restrict__ ambbits,
@@ -434,15 +450,15 @@ kA_block_aggregate(const uint64_t* __restrict__ bases, const uint32_t* __restric
                    uint32_t n_segs, uint32_t seg_runs,
                    uint32_t* __restrict__ rescue_items /* out: items whose table overflowed */) {
   extern __shared__ __align__(16) unsigned char blk_raw[];
-  const uint32_t W = plan.W, WS = W | 1u;
+  const uint32_t W = plan.W, WP = plan.WP;
   const ARunView a = arun_view(blk_raw, plan.slots, plan.cap, plan.cslots, W);
   const uint32_t tid = threadIdx.x;
 
   auto clear_tables = [&]() {
     for (uint32_t i = tid; i < plan.slots; i += kBlkThreads) { a.keys[i] = ~0ull; a.rowid[i] = 0xffffu; }
     for (uint32_t i = tid; i < plan.cslots; i += kBlkThreads) a.cstate[i] = kChunkEmpty;
-    for (uint32_t i = tid; i < (a.cap + 1u) * WS; i += kBlkThreads) a.pool[i] = 0u;
-    for (uint32_t i = tid; i < a.ccap * WS; i += kBlkThreads) a.crows[i] = 0u;
+    for (uint32_t i = tid; i < a.cap; i += kBlkThreads) a.rhead[i] = kNodeNil;
+    for (uint32_t i = tid; i < a.ccap * WP; i += kBlkThreads) a.crows[i] = 0u;
   };
   clear_tables();
   if (tid == 0) { a.h->n_unique = 0; a.h->overflow = 0; a.h->work = 0; a.h->n_pass = 0; a.h->singles = 0; }
@@ -454,30 +470,21 @@ kA_block_aggregate(const uint64_t* __restrict__ bases, const uint32_t* __restric
   const uint64_t cm_hi = R >= 32u ? ~0ull : (~0ull << (64u - 2u * R));
   const uint64_t cm_lo = R > 32u ? (~0ull << (64u - 2u * (R - 32u))) : 0ull;
 
-  // one k-mer (in the low 2k bits) -> row, OR `nw` words starting at src into it
-  auto put_bits = [&](uint64_t key, const uint32_t* src, uint32_t first_word, uint32_t nw) {
+  // one k-mer (in the low 2k bits) -> row, `node` pushed onto the row's list
+  auto put_node = [&](uint64_t key, uint32_t node) {
     const uint32_t h = blk_hash((uint32_t)(key >> 32), (uint32_t)key, a.shift);
     uint32_t id = 0xffffu;
     if (*reinterpret_cast<const volatile uint64_t*>(&a.keys[h]) == key)
       id = *reinterpret_cast<const volatile uint16_t*>(&a.rowid[h]);
-    if (id == 0xffffu) id = kmer_row_slow(a, key, h, WS);
-    uint32_t* dst = a.pool + id * WS + first_word;
-    for (uint32_t w = 0; w < nw; ++w) {
-      const uint32_t x = src[w];
-      if (x) atomicOr(dst + w, x);
-    }
-  };
-  auto put_kmer = [&](uint64_t fwd, const uint32_t* src, uint32_t first_word, uint32_t nw) {
-    const uint64_t rc = revcomp2(fwd, k);
-    if (CANON) put_bits(rc < fwd ? rc : fwd, src, first_word, nw);
-    else { put_bits(fwd, src, first_word, nw); put_bits(rc, src, first_word, nw); }
+    if (id == 0xffffu) id = kmer_row_slow(a, key, h);
+    if (id < a.cap) a.pnext[node] = (uint16_t)atomicExch(&a.rhead[id], node);
   };
 
   // the thread's sequences j = 0, 1 of the (cluster, slice) whose first sequence is st_lo, at
   // word index st_wi: window count (0: none), sample | ambiguity flag, first word, words
   uint32_t st_lo = 0xffffffffu, st_wi = 0;
   uint32_t nw0 = 0, nw1 = 0, sf0 = 0, sf1 = 0, wo0 = 0, wo1 = 0;
-  uint64_t c0 = 0, n0 = 0, p0 = 0, c1 = 0, n1 = 0, p1 = 0;
+  uint64_t c0 = 0, n0 = 0, c1 = 0, n1 = 0;
 
   uint32_t seg = blockIdx.x;
   for (uint32_t it = 0; seg < n_segs; ++it) {
@@ -500,17 +507,16 @@ kA_block_aggregate(const uint64_t* __restrict__ bases, const uint32_t* __restric
 
       // ---- the register-held sequences at this run: new (cluster, slice) or position -> load,
       //      next word -> slide by one word and request the one after ---------------------------
-      auto fetch = [&](uint32_t nw, uint32_t wo, uint64_t& c, uint64_t& n, uint64_t& p) {
-        c = 0; n = 0; p = 0;
+      auto fetch = [&](uint32_t nw, uint32_t wo, uint64_t& c, uint64_t& n) {
+        c = 0; n = 0;
         if (s_rel < nw) {
           const uint64_t* w = bases + wo + wi;
           c = __ldg(w); n = __ldg(w + 1);
-          if (32u * (wi + 1u) < nw) p = __ldg(w + 2);
         }
       };
-      auto slide = [&](uint32_t nw, uint32_t wo, uint64_t& c, uint64_t& n, uint64_t& p) {
-        c = n; n = p; p = 0;
-        if (32u * (wi + 1u) < nw) p = __ldg(bases + wo + wi + 2u);
+      auto slide = [&](uint32_t nw, uint32_t wo, uint64_t& c, uint64_t& n) {
+        c = n; n = 0;
+        if (s_rel < nw) n = __ldg(bases + wo + wi + 1u);
       };
       if (seq_lo != st_lo) {
         nw0 = 0; nw1 = 0;
@@ -524,17 +530,17 @@ kA_block_aggregate(const uint64_t* __restrict__ bases, const uint32_t* __restric
         }
       }
       if (seq_lo == st_lo && wi == st_wi + 1u) {
-        slide(nw0, wo0, c0, n0, p0);
-        slide(nw1, wo1, c1, n1, p1);
+        slide(nw0, wo0, c0, n0);
+        slide(nw1, wo1, c1, n1);
       } else if (seq_lo != st_lo || wi != st_wi) {
-        fetch(nw0, wo0, c0, n0, p0);
-        fetch(nw1, wo1, c1, n1, p1);
+        fetch(nw0, wo0, c0, n0);
+        fetch(nw1, wo1, c1, n1);
       }
       st_lo = seq_lo;
       st_wi = wi;
 
-      // ---- phase 1: every sequence's run -> chunk table (or, for ragged / ambiguous runs and a
-      //      full chunk table, straight into the k-mer table) ----------------------------------
+      // ---- phase 1: every sequence's run -> chunk table: the bases its live windows cover and
+      //      the mask of those windows (a ragged tail, windows over N / IUPAC symbols) ---------
       for (uint32_t j = 0, si = seq_lo + tid; si < seq_hi; ++j, si += kBlkThreads) {
         uint32_t nwin, sf;
         uint64_t w0, w1;
@@ -550,53 +556,54 @@ kA_block_aggregate(const uint64_t* __restrict__ bases, const uint32_t* __restric
         if (s_rel >= nwin) continue;
         const uint32_t nv = min((uint32_t)kBlkRun, nwin - s_rel);
         const uint32_t sample = (sf & 0x7fffffffu) - sample0;      // rank inside the slice
-        const bool amb = (sf >> 31) != 0u;
-        const uint32_t wofs = sample >> 5, bit = 1u << (sample & 31u);
         const uint32_t o0 = s_rel & 31u;
+        uint32_t live = (1u << nv) - 1u;                 // bit q: window s_rel + q exists, no N in it
+        if (sf >> 31) {                                  // ambiguous: the N / IUPAC bit plane, MSB first
+          const uint32_t* ab = ambbits + seqs[si].amb_word_off + wi;
+          const uint64_t t = (((uint64_t)ab[0] << 32) | (uint64_t)ab[1]) << o0;
+          for (uint32_t q = 0; q < nv; ++q)
+            if ((t << q) >> (64 - k)) live &= ~(1u << q);
+          if (!live) continue;
+        }
         uint64_t hi = w0, lo = w1;
         if (o0) {
           hi = (w0 << (2u * o0)) | (w1 >> (64u - 2u * o0));
           lo = w1 << (2u * o0);
         }
-        uint32_t cs = 0xffffffffu;
-        if (nv == (uint32_t)kBlkRun && !amb) cs = chunk_find_or_insert(a, hi & cm_hi, lo & cm_lo, wofs);
-        if (cs != 0xffffffffu) {
-          atomicOr(&a.crows[cs * WS + wofs], bit);
-          const uint16_t meta = a.cmeta[cs];            // most chunks are one sample's: remember if not
-          if ((meta & 0xffu) != wofs && !(meta & 0x8000u)) a.cmeta[cs] = meta | 0x8000u;
+        // the bases the run covers (top-aligned; those past the sequence's end cleared, so
+        // equal ragged tails meet) and the live-window mask in the free low bits of lo
+        if (nv == (uint32_t)kBlkRun) {
+          hi &= cm_hi; lo &= cm_lo;
         } else {
-          const uint32_t* ab = amb ? ambbits + seqs[si].amb_word_off : nullptr;
-          for (uint32_t q = 0; q < nv; ++q) {
-            bool dead = false;
-            if (amb) {
-              const uint32_t p = s_rel + q;
-              const uint32_t wj = p >> 5, bs = p & 31u;
-              const uint64_t two = ((uint64_t)ab[wj] << 32) | (uint64_t)ab[wj + 1];
-              dead = ((two << bs) >> (64 - k)) != 0ull;
-            }
-            if (!dead) {
-              const uint64_t x = q ? ((hi << (2u * q)) | (lo >> (64u - 2u * q))) : hi;
-              put_kmer(x >> sh64, &bit, wofs, 1u);
-            }
-          }
+          const uint32_t nb = nv + (uint32_t)k - 1u;
+          hi &= nb >= 32u ? ~0ull : ~0ull << (64u - 2u * nb);
+          lo &= nb > 32u ? ~0ull << (64u - 2u * (nb - 32u)) : 0ull;
         }
+        const uint32_t cs = chunk_find_or_insert(a, hi, lo | live, sample);
+        if (cs == 0xffffffffu) { a.h->overflow = 1u; continue; }
+        atomicOr(&a.crows[cs * WP + (sample >> 5)], 1u << (sample & 31u));
+        if (a.csample[cs] != sample) a.csample[cs] = (uint16_t)kChunkMixed;   // (a paralog of the same sample is not)
       }
       __syncthreads();
 
-      // ---- phase 2: distinct chunks x 16 windows -> k-mer table, whole sample bitsets at a time ----
+      // ---- phase 2: distinct chunks x live windows -> k-mer table; a (chunk, window) pair only
+      //      adds itself to its k-mer row's list -------------------------------------------------
       const uint32_t n_chunks = min(a.h->work, a.ccap);
-      const uint32_t n_pairs = n_chunks * (uint32_t)kBlkRun;
-      // pairs cost very different amounts (a new k-mer is an insertion, a many-sample chunk ORs W
-      // words): the first round is static, after it the warps take 32 pairs at a time from a counter
+      const uint32_t n_pairs = a.h->overflow ? 0u : n_chunks * (uint32_t)kBlkRun;
+      // pairs cost very different amounts (a new k-mer is an insertion): the first round is
+      // static, after it the warps take 32 pairs at a time from a counter
       for (uint32_t q0 = (tid & ~31u);;) {
         const uint32_t p = q0 + (tid & 31u);
         if (p < n_pairs) {
           const uint32_t cs = p >> 4, q = p & 15u;
-          const uint64_t hi = a.ckhi[cs], lo = a.cklo[cs];
-          const uint64_t x = q ? ((hi << (2u * q)) | (lo >> (64u - 2u * q))) : hi;
-          const uint16_t meta = a.cmeta[cs];
-          if (meta & 0x8000u) put_kmer(x >> sh64, a.crows + cs * WS, 0u, W);
-          else put_kmer(x >> sh64, a.crows + cs * WS + (meta & 0xffu), meta & 0xffu, 1u);
+          const uint64_t lo = a.cklo[cs];
+          if ((lo >> q) & 1u) {
+            const uint64_t hi = a.ckhi[cs];
+            const uint64_t x = q ? ((hi << (2u * q)) | (lo >> (64u - 2u * q))) : hi;
+            const uint64_t fwd = x >> sh64, rc = revcomp2(fwd, k);
+            if (CANON) put_node(rc < fwd ? rc : fwd, p);
+            else { put_node(fwd, 2u * p); put_node(rc, 2u * p + 1u); }
+          }
         }
         __syncwarp();
         uint32_t nx = 0;
@@ -632,61 +639,71 @@ kA_block_aggregate(const uint64_t* __restrict__ bases, const uint32_t* __restric
       __syncthreads();
       if (tid == 0) { a.h->n_unique = 0; a.h->overflow = 0; a.h->work = 0; a.h->n_pass = 0; }
       if (!overflow && a.h->ok) {
-        // a warp takes 32 rows: every lane writes its row's key and count code; a one-sample row
-        // (most of them: the k-mers of a private SNP) is only that code, its bitset is never
-        // written.  The other rows are listed (lane ids, in the chunk keys, which are dead until
-        // the next run: ccap >= 16 gives 32 bytes per warp) and copied by L = WP / 4 lanes each,
-        // one uint4 per lane, so a store instruction writes whole 16 * L-byte rows (W <= 32: L <= 8).
+        // a warp takes 32 rows: every lane writes its row's key, takes its list and empties it.
+        // A list of ONE node whose chunk has one sample (most rows: the k-mers of a private SNP)
+        // is a one-sample row: its code comes from the chunk, no bitset is read or written.  The
+        // other rows are listed (lane ids, in the chunk keys, which are dead until the next run:
+        // ccap >= 16 gives 32 bytes per warp) and built by L lanes each, L = WP / 4 rounded up to
+        // a power of two: they walk the row's list together, OR one uint4 slice of every listed
+        // chunk's row, and sum the popcount by shuffles.  A row whose OR has one bit (two chunks
+        // of one sample's paralogs) is still written as a one-sample code.
         const size_t base = a.h->row_base;
-        const uint32_t WP = plan.WP, L = WP >> 2, lane = tid & 31u;
-        const uint32_t lrow = lane / L, lq = 4u * (lane - lrow * L), per = 32u / L;
+        const uint32_t L = WP > 16u ? 8u : WP > 8u ? 4u : WP > 4u ? 2u : 1u, lane = tid & 31u;
+        const uint32_t lrow = lane / L, lq = 4u * (lane & (L - 1u)), per = 32u / L;
+        const uint32_t nsh = CANON ? 4u : 5u;            // node -> chunk id
         uint8_t* list = reinterpret_cast<uint8_t*>(a.ckhi) + (tid & ~31u);
+        uint32_t singles = 0;
         for (uint32_t r0 = tid & ~31u; r0 < n; r0 += kBlkThreads) {
           const uint32_t r = r0 + lane;
           bool multi = false;
+          uint32_t head = kNodeNil;
           if (r < n) {
             slab_keys[base + r] = a.rkey[r];
-            uint32_t* src = a.pool + r * WS;
-            uint32_t cnt = 0, wq = 0, orx = 0;         // one sample: it is bit ffs(orx) of word wq
-            for (uint32_t q = 0; q < W; ++q) {
-              const uint32_t x = src[q], c = __popc(x);
-              cnt += c;
-              wq += c * q;
-              orx |= x;
-            }
-            multi = cnt != 1u;
-            if (multi) {
-              slab_cnt[base + r] = cnt;
-            } else {
-              slab_cnt[base + r] = kCntSingle | (wq << 5) | (uint32_t)(__ffs(orx) - 1);
-              src[wq] = 0u;
-            }
+            head = a.rhead[r];
+            a.rhead[r] = kNodeNil;
+            const uint32_t c = head >> nsh;
+            const uint32_t s1 = a.csample[c];
+            multi = a.pnext[head] != kNodeNil || s1 == kChunkMixed;
+            if (!multi) slab_cnt[base + r] = kCntSingle | s1;
             const uint32_t h = a.rslot[r];
             a.keys[h] = ~0ull;
             a.rowid[h] = 0xffffu;
           }
           const uint32_t m = __ballot_sync(kFull, multi), nm = (uint32_t)__popc(m);
           if (multi) list[__popc(m & lanemask_lt())] = (uint8_t)lane;
-          if (lane == 0 && nm < min(32u, n - r0)) atomicAdd(&a.h->singles, min(32u, n - r0) - nm);
+          singles += min(32u, n - r0) - nm;
           __syncwarp();
-          for (uint32_t g = lrow; g < nm && lrow < per; g += per) {
-            const uint32_t rr = r0 + list[g];
-            uint32_t* src = a.pool + rr * WS + lq;
-            uint4 x;
-            x.x = src[0];                              // (lq < W: WP is W rounded up to 4)
-            x.y = lq + 1 < W ? src[1] : 0u;
-            x.z = lq + 2 < W ? src[2] : 0u;
-            x.w = lq + 3 < W ? src[3] : 0u;
-            reinterpret_cast<uint4*>(slab_rows + (base + rr) * WP + lq)[0] = x;
-            src[0] = 0u;
-            if (lq + 1 < W) src[1] = 0u;
-            if (lq + 2 < W) src[2] = 0u;
-            if (lq + 3 < W) src[3] = 0u;
+          for (uint32_t g0 = 0; g0 < nm; g0 += per) {
+            const uint32_t g = g0 + lrow;
+            const uint32_t src = g < nm ? list[g] : 0u;
+            uint32_t node = __shfl_sync(kFull, head, src);
+            uint4 x = make_uint4(0u, 0u, 0u, 0u);
+            if (g < nm && lq < WP) {
+              for (; node != kNodeNil; node = a.pnext[node]) {
+                const uint4 y = *reinterpret_cast<const uint4*>(a.crows + (node >> nsh) * WP + lq);
+                x.x |= y.x; x.y |= y.y; x.z |= y.z; x.w |= y.w;
+              }
+            }
+            uint32_t cnt = __popc(x.x) + __popc(x.y) + __popc(x.z) + __popc(x.w);
+            uint32_t one = x.x ? 32u * lq + __ffs(x.x) - 1u : x.y ? 32u * (lq + 1u) + __ffs(x.y) - 1u
+                         : x.z ? 32u * (lq + 2u) + __ffs(x.z) - 1u : x.w ? 32u * (lq + 3u) + __ffs(x.w) - 1u : 0u;
+            for (uint32_t o = 1; o < L; o <<= 1) {
+              cnt += __shfl_xor_sync(kFull, cnt, o);
+              one |= __shfl_xor_sync(kFull, one, o);
+            }
+            singles += __popc(__ballot_sync(kFull, g < nm && lq == 0u && cnt == 1u));
+            if (g < nm) {
+              const size_t p = base + r0 + src;
+              if (lq == 0u) slab_cnt[p] = cnt == 1u ? kCntSingle | one : cnt;
+              if (cnt != 1u && lq < WP) reinterpret_cast<uint4*>(slab_rows + p * WP + lq)[0] = x;
+            }
           }
           __syncwarp();
         }
+        if (lane == 0 && singles) atomicAdd(&a.h->singles, singles);
+        __syncthreads();                                 // chunk rows are read until here
         for (uint32_t c = tid; c < n_chunks; c += kBlkThreads) a.cstate[a.cslot[c]] = kChunkEmpty;
-        for (uint32_t i = tid; i < n_chunks * WS; i += kBlkThreads) a.crows[i] = 0u;
+        for (uint32_t i = tid; i < n_chunks * WP; i += kBlkThreads) a.crows[i] = 0u;
       } else {
         clear_tables();
       }

@@ -320,6 +320,7 @@ struct pf_ctx : BatchState {
   bool block_mode = false;       // S <= 1024 and not disabled: kA_block_aggregate + kB1..kB3
   uint32_t block_windows = 16;   // windows per position block (= kBlkRun)
   uint32_t blk_slots = 1024, blk_cap = 448, blk_cslots = 128;   // shared memory of kA: k-mer key slots / rows, chunk slots
+  uint32_t blk_rescue_cslots = 1024;   // chunk slots of a rescue launch of kA
   uint32_t ka_seg_runs = 0;      // runs per kA segment (PF_KA_SEG_RUNS); 0: chosen from the batch
   uint32_t n_slices = 1, slice_samples = 0, Ws = 0;   // sample slices of the block engine (S > 1024): slices,
                                                        // samples per slice, bitset words of a partial row

@@ -458,7 +458,7 @@ int launch_block_aggregate(pf_ctx* ctx, const uint32_t* items, uint32_t n, uint3
   bp.cslots = cslots;
   const uint32_t cap32 = (uint32_t)std::min<uint64_t>(ctx->partial_cap, 0xfffffff0u);
   uint32_t* counters = ctx->d_counters.as<uint32_t>() + C_LOCAL;
-  const uint32_t smem = blkA_smem_bytes(slots, cap, cslots, ctx->Ws);
+  const uint32_t smem = blkA_smem_bytes(slots, cap, cslots, ctx->Ws, ctx->prm.canonical);
   auto kernel = ctx->prm.canonical ? kA_block_aggregate<true> : kA_block_aggregate<false>;
   uint32_t grid = n, n_segs = n, seg_runs = 1;
   if (!items) {
@@ -718,24 +718,23 @@ extern "C" int pf_execute(pf_ctx* ctx) {
         const uint32_t first_rescue = hcnt[C_LOCAL + LC_RESCUE];
         while (hcnt[C_LOCAL + LC_TABLE_OVERFLOW] == 1u) {
           const uint32_t n_resc = hcnt[C_LOCAL + LC_RESCUE];
-          // twice the key slots, as many rows as then fit (the chunk table stays: a full one only
-          // sends runs down the direct path)
+          // the rescue chunk table (a full chunk table overflows a run too), twice the key slots
+          // and as many rows as then fit
+          const uint32_t cslots2 = ctx->blk_rescue_cslots;
+          auto rows_fit = [&](uint32_t s) -> uint32_t {
+            const uint32_t fixed = blkA_smem_bytes(s, 0u, cslots2, ctx->Ws, ctx->prm.canonical);
+            return fixed < kBlkMaxSmem ? std::min<uint32_t>((kBlkMaxSmem - fixed) / kBlkRowBytes, s * 13u / 16u) : 0u;
+          };
           uint32_t slots2 = slots * 2u, cap2 = 0;
-          if (slots2 <= 8192u && blkA_smem_bytes(slots2, 0u, cslots, ctx->Ws) < kBlkMaxSmem) {
-            const uint32_t per_row = 10u + (ctx->Ws | 1u) * 4u;   // rkey, rslot, bitset
-            const uint32_t fit = (kBlkMaxSmem - blkA_smem_bytes(slots2, 0u, cslots, ctx->Ws)) / per_row;
-            cap2 = std::min<uint32_t>(std::min<uint32_t>(fit, slots2 * 13u / 16u),
-                                      std::max<uint32_t>(cap * 2u, slots2 * 5u / 8u));
-          }
+          if (slots2 <= 8192u) cap2 = std::min<uint32_t>(rows_fit(slots2), std::max<uint32_t>(cap * 2u, slots2 * 5u / 8u));
           if (cap2 <= cap) {        // no more rows with more slots: try all the rows the current slots allow
             slots2 = slots;
-            const uint32_t per_row = 10u + (ctx->Ws | 1u) * 4u;   // rkey, rslot, bitset
-            const uint32_t fit = (kBlkMaxSmem - blkA_smem_bytes(slots, 0u, cslots, ctx->Ws)) / per_row;
-            cap2 = std::min<uint32_t>(fit, slots * 13u / 16u);
+            cap2 = rows_fit(slots);
           }
-          if (cap2 <= cap) { too_big = true; break; }
+          if (cap2 <= cap && cslots2 == cslots) { too_big = true; break; }
           slots = slots2;
           cap = cap2;
+          cslots = cslots2;
           CU(cudaMemsetAsync(counters + C_LOCAL + LC_TABLE_OVERFLOW, 0, 4, st));
           CU(cudaMemsetAsync(counters + C_LOCAL + LC_RESCUE, 0, 4, st));
           TRY(launch_block_aggregate(ctx, ctx->d_rescue[cur].as<uint32_t>(), n_resc, slots, cap, cslots,
@@ -752,7 +751,7 @@ extern "C" int pf_execute(pf_ctx* ctx) {
         if (!too_big && first_rescue > n_ka_items / 8u) {
           uint32_t ns = ctx->blk_slots, ncap = ctx->blk_cap + ctx->blk_cap / 2;
           while (ncap > ns * 13u / 16u) ns *= 2;
-          if (ns <= 8192u && blkA_smem_bytes(ns, ncap, ctx->blk_cslots, ctx->Ws) <= kBlkMaxSmem) {
+          if (ns <= 8192u && blkA_smem_bytes(ns, ncap, ctx->blk_cslots, ctx->Ws, ctx->prm.canonical) <= kBlkMaxSmem) {
             ctx->blk_slots = ns;
             ctx->blk_cap = ncap;
           }

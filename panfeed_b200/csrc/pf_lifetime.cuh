@@ -140,9 +140,9 @@ extern "C" int pf_create(pf_ctx** out, int device, const pf_params* p) {
     }
     if (const char* e = getenv("PF_BLOCK_SLICED")) if (atoi(e) == 0 && ctx->n_slices > 1) ctx->block_mode = false;
     if (const char* e = getenv("PF_BLOCK_MODE")) ctx->block_mode = ctx->block_mode && atoi(e) != 0;
-    // tables of kA: one k-mer slot per expected distinct k-mer of a 16-window run at ~50 % load
-    // (about one haplotype per 30 samples and position), a quarter as many chunk slots;
-    // overflowing blocks are rerun with both doubled
+    // tables of kA: two k-mer slots per sample of a 16-window run (about one haplotype per 30
+    // samples and position), an eighth as many chunk slots; overflowing runs are rerun with the
+    // rescue chunk table and twice the key slots
     ctx->block_windows = (uint32_t)kBlkRun;
     // (about one new k-mer per sample and run of 16 windows, plus the haplotypes' own)
     uint32_t slots = 256;
@@ -152,7 +152,7 @@ extern "C" int pf_create(pf_ctx** out, int device, const pf_params* p) {
       const int v = atoi(e);
       if (v >= 64 && v <= 8192 && (v & (v - 1)) == 0) slots = (uint32_t)v;
     }
-    uint32_t cap = std::min<uint32_t>(slots * 13u / 16u, std::max<uint32_t>(96u, s_eff * 9u / 10u));
+    uint32_t cap = slots * 13u / 16u;              // a row costs 14 bytes: as many as the key slots allow
     if (const char* e = getenv("PF_BLOCK_CAP")) {
       const int v = atoi(e);
       if (v >= 32 && (uint32_t)v <= slots * 13u / 16u) cap = (uint32_t)v;
@@ -162,9 +162,16 @@ extern "C" int pf_create(pf_ctx** out, int device, const pf_params* p) {
       const int v = atoi(e);
       if (v >= 32 && v <= 8192 && (v & (v - 1)) == 0) cslots = (uint32_t)v;
     }
-    while (slots > 64u && blkA_smem_bytes(slots, cap, cslots, ctx->Ws) > kBlkMaxSmem) {
+    const bool canon = p->canonical != 0;
+    while (slots > 64u && blkA_smem_bytes(slots, cap, cslots, ctx->Ws, canon) > kBlkMaxSmem) {
       slots /= 2; cap /= 2; cslots = std::max<uint32_t>(32u, cslots / 2);
     }
+    // a rescue launch gives every sequence of a work item its own chunk (at one sequence per
+    // sample), while 2048 key slots and their rows still fit next to the chunk table
+    uint32_t rcs = 32u;
+    while (blkA_ccap(rcs) < s_eff && rcs < 2048u) rcs *= 2;
+    while (rcs > cslots && blkA_smem_bytes(2048u, 1664u, rcs, ctx->Ws, canon) > kBlkMaxSmem) rcs /= 2;
+    ctx->blk_rescue_cslots = std::max(rcs, cslots);
     if (const char* e = getenv("PF_KA_SEG_RUNS")) {   // fixed segment length: tests of small batches, sweeps
       const int v = atoi(e);
       if (v >= 1 && v <= 4096) ctx->ka_seg_runs = (uint32_t)v;
