@@ -260,9 +260,43 @@ int pf_patterns_export(pf_ctx* ctx, int cluster_namespace, uint64_t first,
 int pf_pattern_ids(pf_ctx* ctx, int cluster_namespace, uint64_t first, uint64_t count,
                    uint8_t* host_digests);
 int pf_stats_get(pf_ctx* ctx, pf_stats* out);
+
+/* ---- --associations: the post-GWAS join of a second pass on the device ----
+ * What panfeed-get-kmers does with a run's kmers_to_hashes.tsv and kmers.tsv (get_kmers.py:108-145:
+ * the passing associations inner-joined to the hashes, then joined to the positional rows on
+ * (cluster, k-mer)), computed while the batch is still on the device, so that only the rows of
+ * the answer leave it.
+ *
+ * pf_assoc_load: the set of passing patterns, as the 16-byte MD5 digests their ids encode (an id is
+ * base64(digest)[:24]); digest i is association row i.  An open-addressing table in device memory
+ * keyed on the whole 128-bit digest.  Once per run (a second call replaces the set); equal digests
+ * are refused.  While a set is loaded, pf_submit runs every batch whole (no pipelined sub-batches).
+ *
+ * pf_assoc_collect: after the pf_collect of a batch (the context must have emit_positions == 2).
+ * Every pattern numbered since the last call is looked up by its MD5 (both namespaces, K5's digest),
+ * then every window of the batch's PF_SEQ_TARGET sequences is joined to the batch's rows on
+ * (cluster, k-mer): the k-mer of the strand the canonical k-mer came from (canonical), or both
+ * strands (canonical == 0: kmers.tsv has a row for each).  The arrays are the context's and stay
+ * valid until its next pf_assoc_collect. */
+#define PF_ASSOC_NONE 0xffffffffu
+typedef struct pf_assoc_result {
+  uint64_t n_windows;              /* window rows whose (cluster, k-mer) pattern passes, any order:      */
+  const uint64_t* window;          /*   (base_off + pos) << 1 | (1 for the reverse-complement row, canonical == 0) */
+  const uint32_t* window_assoc;    /*   their association row                                              */
+  uint32_t n_clusters;             /* per cluster of the batch:                                            */
+  const uint8_t* cluster_pass;     /*   1 if any of its hashes passes, its own cluster-row hash included   */
+  const uint32_t* cluster_assoc;   /*   association row of its cluster-row hash, or PF_ASSOC_NONE          */
+  uint64_t n_rows;                 /* rows of pf_collect whose pattern passes, any order:                  */
+  const uint32_t* row;             /*   row index (narrow rows, then wide, then 256-bit, as pf_collect)    */
+  const uint32_t* row_assoc;       /*   association row                                                    */
+  const uint8_t* row_seen;         /*   1 if a target window carries it                                    */
+} pf_assoc_result;
+int pf_assoc_load(pf_ctx* ctx, const uint8_t* digests /* [n][16] */, uint64_t n);
+int pf_assoc_collect(pf_ctx* ctx, pf_assoc_result* out);
+
 /* sizeof of the ABI structs as the library was built: 0 pf_params, 1 pf_seq_desc,
  * 2 pf_cluster_desc, 3 pf_batch, 4 pf_batch_result, 5 pf_stats, 6 pf_synth_params,
- * 7 pf_cut_result, 8 pf_cut_planes, 9 pf_comm, 10 pf_exchange_result; 0 for an unknown id.  Lets a binding check its own struct mirrors. */
+ * 7 pf_cut_result, 8 pf_cut_planes, 9 pf_comm, 10 pf_exchange_result, 11 pf_assoc_result; 0 for an unknown id.  Lets a binding check its own struct mirrors. */
 uint32_t pf_struct_size(int which);
 /* CUDA stream the context launches on, as an opaque handle (cudaStream_t). */
 void* pf_stream(pf_ctx* ctx);
@@ -291,6 +325,29 @@ int pf_format_positions_compact(const pf_batch* batch, const uint32_t* strand_bi
                                 int canonical, uint32_t seq_first, uint32_t seq_count,
                                 const char* lead_blob, const uint64_t* lead_off, char* out,
                                 uint64_t out_cap, uint64_t* out_len, uint32_t n_threads);
+
+/* The lines of panfeed-get-kmers (get_kmers.py:108-145) for one batch, from the compact positional
+ * form and a pf_assoc_collect result:
+ *   {cluster}\t{k-mer}\t{snippet}\t{strain}\t{gene_id}\t{contig}\t{strand}\t{truestart}\t{trueend}\t{genestart}\t{geneend}\t{used_strand}\n
+ * snippet = snip_blob[snip_off[a], snip_off[a + 1]) for association row a: the hashed_pattern and
+ * association columns as the caller wants them printed ("id\tcol\t..."), snip_fields fields;
+ * where the k-mer's pattern does not pass, snip_fields - 1 tabs.  tag_blob / tag_off: the cluster
+ * column, per cluster of the batch; lead_blob / lead_off: "strain\tgene_id\tcontig\t" per sequence.
+ *   flags 0 (right join, the default of get-kmers): every window row of the clusters that have a
+ *     passing hash.
+ *   PF_ANNOT_ONLY_PASSING (left join, --only-passing): the passing window rows, then every passing row
+ *     of `rows` that no window carries and every passing cluster-row hash, with empty positional
+ *     fields (a cluster-row line has an empty k-mer).
+ *   PF_ANNOT_FLOAT_POSITIONS: the six integer positional fields printed as floats ("361.0"), as pandas
+ *     prints them once one line of the frame has them empty.
+ * out == NULL: only *out_len.  n_threads == 0: all host cores. */
+#define PF_ANNOT_ONLY_PASSING 1u
+#define PF_ANNOT_FLOAT_POSITIONS 2u
+int pf_format_annotated(const pf_batch* batch, const uint32_t* strand_bits, uint32_t k, int canonical,
+                        const pf_batch_result* rows, const pf_assoc_result* assoc, const char* tag_blob,
+                        const uint64_t* tag_off, const char* lead_blob, const uint64_t* lead_off,
+                        const char* snip_blob, const uint64_t* snip_off, uint64_t n_snips, uint32_t snip_fields,
+                        uint32_t flags, char* out, uint64_t out_cap, uint64_t* out_len, uint32_t n_threads);
 
 /* The hashes_to_patterns rows of n patterns (panfeed.py:183-187,217-223): ids (n x 24 chars,
  * e.g. from pf_pattern_ids + base64), then per sample a tab and '0' / '1' — or nothing where

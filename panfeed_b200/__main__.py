@@ -76,6 +76,20 @@ def get_options(argv=None):
     p.add_argument("-ql", "--queue-limit", type=int, default=3,
                    help="accepted for compatibility (GPU build)")
     p.add_argument("--stop-on-missing", action="store_true", default=False)
+    # (the association options exist in the parsed namespace only when given: without them a run is
+    #  the reference's, option for option)
+    assoc = p.add_argument_group("post-GWAS annotation (panfeed-get-kmers in the same run)")
+    assoc.add_argument("--associations", default=argparse.SUPPRESS,
+                       help="pyseer-style associations table (tab-separated, a header, the pattern id in the first "
+                            "column): write <output>/annotated_kmers.tsv, the table panfeed-get-kmers would print "
+                            "for this run's kmers_to_hashes.tsv and kmers.tsv, instead of kmers.tsv.  The join runs "
+                            "on the GPU; kmers_to_hashes.tsv and hashes_to_patterns.tsv are written as usual")
+    assoc.add_argument("--association-threshold", type=float, default=argparse.SUPPRESS,
+                       help="p-value threshold (get-kmers -t, default 1)")
+    assoc.add_argument("--association-column", default=argparse.SUPPRESS,
+                       help="p-value column (get-kmers -c, default lrt-pvalue)")
+    assoc.add_argument("--only-passing", action="store_true", default=argparse.SUPPRESS,
+                       help="only the passing k-mers (get-kmers --only-passing)")
     p.add_argument("--device", type=int, default=0, help="CUDA device")
     p.add_argument("-v", action="count", default=0)
     p.add_argument("--version", action="version", version="%(prog)s " + __version__)
@@ -84,6 +98,10 @@ def get_options(argv=None):
 
 def main(argv=None):
     args = get_options(argv)
+    for name, default in (("associations", None), ("association_threshold", 1.0),
+                          ("association_column", "lrt-pvalue"), ("only_passing", False)):
+        if not hasattr(args, name):
+            setattr(args, name, default)
     set_logging(args.v)
     klength = args.kmer_length
     if args.downstream_start_codon and args.upstream + args.downstream < klength:
@@ -100,6 +118,10 @@ def main(argv=None):
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     sharded = world > 1
+    if args.associations is not None and (args.multiple_files or sharded):
+        logger.error("--associations runs on one GPU and writes one file: it cannot be combined with "
+                     "--multiple-files or several ranks (torchrun)")
+        sys.exit(1)
     if sharded:
         import torch
         import torch.distributed as tdist
@@ -125,6 +147,16 @@ def main(argv=None):
         not args.multiple_files, args.compress, make_outputs=not sharded,
         native_table=not args.python_feeder)
     all_columns = genepres
+    annotate = None
+    if args.associations is not None:
+        from .assoc import AnnotatedWriter, load_passing
+        a, digests = load_passing(args.associations, args.association_column, args.association_threshold)
+        logger.info(f"{len(a)} patterns pass the association threshold {args.association_threshold}")
+        # annotated_kmers.tsv takes the place of kmers.tsv
+        kmer_stroi.close()
+        os.remove(os.path.join(args.output, "kmers.tsv.gz" if args.compress else "kmers.tsv"))
+        kmer_stroi = None
+        annotate = AnnotatedWriter(args.output, a, digests, args.only_passing, args.compress)
     if sharded:
         if rank == 0:
             os.mkdir(args.output)
@@ -168,7 +200,7 @@ def main(argv=None):
     func_w = partial(pattern_hasher, kmer_stroi=kmer_stroi, hash_pat=hash_pat,
                      kmer_hash=kmer_hash, genepres=all_columns, patfilt=not args.no_filter,
                      maf=args.maf, consider_missing_cluster=args.consider_missing,
-                     output=args.output, compress=args.compress, device=args.device)
+                     output=args.output, compress=args.compress, device=args.device, annotate=annotate)
     # one streaming call: the generator packs clusters while the GPU batches them
     patterns = func_w(cut_clusters, patterns=patterns)
     if patterns.sharded:
@@ -177,6 +209,8 @@ def main(argv=None):
         logger.info(f"rank {rank}: wrote {info['written_here']} of {info['cluster_patterns_global']} + "
                     f"{info['kmer_patterns_global']} patterns")
     patterns.close()
+    if annotate is not None:
+        annotate.close()
 
     for handle in (kmer_stroi, hash_pat, kmer_hash):
         if handle is not None:

@@ -166,6 +166,19 @@ class ExchangeResult(C.Structure):
 PF_EXCHANGE_WRITER, PF_EXCHANGE_KEEP_UNIQUE, PF_EXCHANGE_NO_PEER = 1, 2, 4
 
 
+class AssocResult(C.Structure):
+    """pf_assoc_result: the device join of one batch against the passing associations."""
+    _fields_ = [("n_windows", C.c_uint64), ("window", C.POINTER(C.c_uint64)),
+                ("window_assoc", C.POINTER(C.c_uint32)), ("n_clusters", C.c_uint32),
+                ("cluster_pass", C.POINTER(C.c_uint8)), ("cluster_assoc", C.POINTER(C.c_uint32)),
+                ("n_rows", C.c_uint64), ("row", C.POINTER(C.c_uint32)),
+                ("row_assoc", C.POINTER(C.c_uint32)), ("row_seen", C.POINTER(C.c_uint8))]
+
+
+PF_ASSOC_NONE = 0xFFFFFFFF
+PF_ANNOT_ONLY_PASSING, PF_ANNOT_FLOAT_POSITIONS = 1, 2
+
+
 EXPORTS = ["pf_create", "pf_destroy", "pf_last_error", "pf_abi_version",
            "pf_upload", "pf_execute", "pf_submit", "pf_collect",
            "pf_reset_patterns", "pf_pattern_words", "pf_kmer_pattern_words",
@@ -182,7 +195,8 @@ EXPORTS = ["pf_create", "pf_destroy", "pf_last_error", "pf_abi_version",
            "pf_exchange_dedup", "pf_exchange_unique_count", "pf_exchange_unique_export",
            "pf_exchange_unpack", "pf_exchange_classify", "pf_exchange_recv_buffer", "pf_exchange_open_peer",
            "pf_exchange_close_peer", "pf_exchange_scatter", "pf_exchange_run", "pf_exchange_release",
-           "pf_comm_local_create", "pf_comm_local_get", "pf_comm_local_abort", "pf_comm_local_destroy"]
+           "pf_comm_local_create", "pf_comm_local_get", "pf_comm_local_abort", "pf_comm_local_destroy",
+           "pf_assoc_load", "pf_assoc_collect", "pf_format_annotated"]
 
 _lib = None
 
@@ -281,6 +295,11 @@ def load():
     lib.pf_comm_local_abort.restype = None
     lib.pf_comm_local_destroy.argtypes = [vp]
     lib.pf_comm_local_destroy.restype = None
+    lib.pf_assoc_load.argtypes = [vp, vp, u64]
+    lib.pf_assoc_collect.argtypes = [vp, C.POINTER(AssocResult)]
+    lib.pf_format_annotated.argtypes = [C.POINTER(Batch), vp, u32, C.c_int, C.POINTER(BatchResult),
+                                        C.POINTER(AssocResult), C.c_char_p, vp, C.c_char_p, vp, C.c_char_p, vp,
+                                        u64, u32, u32, vp, u64, C.POINTER(u64), u32]
     lib.pf_struct_size.argtypes = [C.c_int]
     lib.pf_struct_size.restype = u32
     if lib.pf_abi_version() != PF_ABI_VERSION:
@@ -561,6 +580,94 @@ def format_positions_compact(hb, strand_bits, k, canonical, leads, n_threads=0, 
     return out[:int(need.value)] if raw else out[:int(need.value)].tobytes()
 
 
+def id_digests(ids):
+    """Pattern ids (base64(md5)[:24], the first column of an associations file) -> ([n, 16] uint8
+    digests, positions in `ids` of the ones that decode).  An id that is not 24 characters of
+    base64 for 16 bytes names no pattern and is skipped."""
+    import binascii
+    out, keep = [], []
+    for i, x in enumerate(ids):
+        x = x.decode() if isinstance(x, bytes) else str(x)
+        if len(x) != 24 or not x.endswith("=="):
+            continue
+        try:
+            d = binascii.a2b_base64(x)
+        except (binascii.Error, ValueError):
+            continue
+        if len(d) != 16 or binascii.b2a_base64(d).decode()[:24] != x:
+            continue
+        out.append(d)
+        keep.append(i)
+    return np.frombuffer(b"".join(out), np.uint8).reshape(-1, 16).copy(), np.array(keep, np.int64)
+
+
+def _blob(parts):
+    """bytes joined + uint64 offsets [n + 1]"""
+    off = np.zeros(len(parts) + 1, np.uint64)
+    if parts:
+        np.cumsum(np.fromiter((len(x) for x in parts), np.uint64, len(parts)), out=off[1:])
+    return b"".join(parts), off
+
+
+def format_annotated(hb, strand_bits, k, canonical, r, assoc, tags, leads, snippets, snip_fields, flags,
+                     n_threads=0, raw=False):
+    """panfeed-get-kmers lines of one batch (pf_format_annotated): hb = the batch's HostBatch, r its
+    collect() dict, assoc its Context.assoc_collect() dict, tags[c] = cluster column (bytes) per
+    cluster, leads[i] = b"strain\tgene_id\tcontig\t" per sequence, snippets[a] = the hashed_pattern
+    and association fields of association row a (bytes, snip_fields fields), flags = PF_ANNOT_*."""
+    lib = load()
+    keep = []
+
+    def ptr(a, dtype, ctype):
+        a = np.ascontiguousarray(a, dtype=dtype)
+        keep.append(a)
+        return a.ctypes.data_as(C.POINTER(ctype))
+
+    b = hb.struct()
+    res = BatchResult()
+    res.n_clusters = len(hb.clusters)
+    res.n_rows = len(r["row_kmer"])
+    res.row_cluster = ptr(r["row_cluster"][:res.n_rows], np.uint32, C.c_uint32)
+    res.row_kmer = ptr(r["row_kmer"], np.uint64, C.c_uint64)
+    res.n_wide_rows = len(r["wide_row_kmer"])
+    res.wide_row_cluster = ptr(r["wide_row_cluster"], np.uint32, C.c_uint32)
+    res.wide_row_kmer = ptr(r["wide_row_kmer"].reshape(-1), np.uint64, C.c_uint64)
+    res.n_xwide_rows = len(r["xwide_row_kmer"])
+    res.xwide_row_cluster = ptr(r["xwide_row_cluster"], np.uint32, C.c_uint32)
+    res.xwide_row_kmer = ptr(r["xwide_row_kmer"].reshape(-1), np.uint64, C.c_uint64)
+    a = AssocResult()
+    a.n_windows = len(assoc["window"])
+    a.window = ptr(assoc["window"], np.uint64, C.c_uint64)
+    a.window_assoc = ptr(assoc["window_assoc"], np.uint32, C.c_uint32)
+    a.n_clusters = len(assoc["cluster_pass"])
+    a.cluster_pass = ptr(assoc["cluster_pass"], np.uint8, C.c_uint8)
+    a.cluster_assoc = ptr(assoc["cluster_assoc"], np.uint32, C.c_uint32)
+    a.n_rows = len(assoc["row"])
+    a.row = ptr(assoc["row"], np.uint32, C.c_uint32)
+    a.row_assoc = ptr(assoc["row_assoc"], np.uint32, C.c_uint32)
+    a.row_seen = ptr(assoc["row_seen"], np.uint8, C.c_uint8)
+    tag_blob, tag_off = _blob(tags)
+    lead_blob, lead_off = _blob(leads)
+    snip_blob, snip_off = _blob(snippets)
+    bits = None
+    if canonical and len(hb.seqs):
+        bits = np.ascontiguousarray(strand_bits, dtype=np.uint32)
+        if bits.size < hb.packed.size:
+            raise ValueError("strand bit plane is shorter than the packed plane")
+    need = C.c_uint64()
+    args = (C.byref(b), bits.ctypes.data if bits is not None else None, int(k), int(bool(canonical)), C.byref(res),
+            C.byref(a), tag_blob, tag_off.ctypes.data, lead_blob, lead_off.ctypes.data, snip_blob,
+            snip_off.ctypes.data, len(snippets), int(snip_fields), int(flags))
+    rc = lib.pf_format_annotated(*args, None, 0, C.byref(need), int(n_threads))
+    if rc != 0:
+        raise PfError(rc, "pf_format_annotated (sizing) failed")
+    out = _scratch("annotated", need.value)
+    rc = lib.pf_format_annotated(*args, out.ctypes.data, out.size, C.byref(need), int(n_threads))
+    if rc != 0:
+        raise PfError(rc, "pf_format_annotated failed")
+    return out[:int(need.value)] if raw else out[:int(need.value)].tobytes()
+
+
 def _np(ptr, n, dtype, copy=True):
     if n == 0:
         return np.zeros(0, dtype)
@@ -740,6 +847,23 @@ class Context:
         self._check(self.lib.pf_pattern_ids(self.h, int(cluster_namespace), first, count,
                                             dig.ctypes.data))
         return base64_ids(dig)
+
+    def assoc_load(self, digests):
+        """pf_assoc_load: the passing patterns ([n, 16] uint8 MD5 digests; row i = association row i)."""
+        d = np.ascontiguousarray(digests, dtype=np.uint8).reshape(-1, 16)
+        self._check(self.lib.pf_assoc_load(self.h, d.ctypes.data if len(d) else None, len(d)))
+
+    def assoc_collect(self):
+        """pf_assoc_collect after collect(): the join of the batch, as copies."""
+        a = AssocResult()
+        self._check(self.lib.pf_assoc_collect(self.h, C.byref(a)))
+        return {"window": _np(a.window, a.n_windows, np.uint64),
+                "window_assoc": _np(a.window_assoc, a.n_windows, np.uint32),
+                "cluster_pass": _np(a.cluster_pass, a.n_clusters, np.uint8),
+                "cluster_assoc": _np(a.cluster_assoc, a.n_clusters, np.uint32),
+                "row": _np(a.row, a.n_rows, np.uint32),
+                "row_assoc": _np(a.row_assoc, a.n_rows, np.uint32),
+                "row_seen": _np(a.row_seen, a.n_rows, np.uint8)}
 
     def stream_handle(self):
         return self.lib.pf_stream(self.h)

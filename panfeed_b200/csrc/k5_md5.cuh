@@ -41,17 +41,11 @@ __device__ __forceinline__ void md5_block(uint32_t (&s)[4], const uint32_t (&m)[
   s[0] += a; s[1] += b; s[2] += c; s[3] += d;
 }
 
-// pool: n x key_words.  as_int64: cluster namespace.  nan_pool / nan_words: cluster pattern
-// pool used for the NaN plane when key_words == W + 1 (consider_missing).
-__global__ void __launch_bounds__(128)
-k5_md5_ids(const uint32_t* __restrict__ pool, uint32_t first, uint32_t count, uint32_t key_words,
-           uint32_t W, uint32_t S, int as_int64, const uint32_t* __restrict__ nan_pool,
-           uint8_t* __restrict__ digests) {
-  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= count) return;
-  const uint32_t* bits = pool + (size_t)(first + i) * key_words;
-  const uint32_t* present = (key_words > W && nan_pool) ? nan_pool + (size_t)bits[W] * W : nullptr;
-  uint32_t st[4] = {0x67452301u, 0xefcdab89u, 0x98badcfeu, 0x10325476u};
+// MD5 state of one pattern: its bits expanded on the fly into the 8-byte little-endian images the
+// reference hashes.  present (may be null): the NaN plane of a k-mer pattern under --consider-missing.
+__device__ __forceinline__ void md5_pattern(const uint32_t* __restrict__ bits, const uint32_t* __restrict__ present,
+                                            uint32_t S, int as_int64, uint32_t (&st)[4]) {
+  st[0] = 0x67452301u; st[1] = 0xefcdab89u; st[2] = 0x98badcfeu; st[3] = 0x10325476u;
   uint32_t m[16];
   const uint64_t total_bytes = (uint64_t)S * 8;
   const uint32_t n_blocks = (uint32_t)((total_bytes + 9 + 63) / 64);     // message + 0x80 + 64-bit length
@@ -80,6 +74,20 @@ k5_md5_ids(const uint32_t* __restrict__ pool, uint32_t first, uint32_t count, ui
     }
     md5_block(st, m);
   }
+}
+
+// pool: n x key_words.  as_int64: cluster namespace.  nan_pool / nan_words: cluster pattern
+// pool used for the NaN plane when key_words == W + 1 (consider_missing).
+__global__ void __launch_bounds__(128)
+k5_md5_ids(const uint32_t* __restrict__ pool, uint32_t first, uint32_t count, uint32_t key_words,
+           uint32_t W, uint32_t S, int as_int64, const uint32_t* __restrict__ nan_pool,
+           uint8_t* __restrict__ digests) {
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= count) return;
+  const uint32_t* bits = pool + (size_t)(first + i) * key_words;
+  const uint32_t* present = (key_words > W && nan_pool) ? nan_pool + (size_t)bits[W] * W : nullptr;
+  uint32_t st[4];
+  md5_pattern(bits, present, S, as_int64, st);
   uint32_t* out = reinterpret_cast<uint32_t*>(digests + (size_t)i * 16);
   out[0] = st[0]; out[1] = st[1]; out[2] = st[2]; out[3] = st[3];
 }

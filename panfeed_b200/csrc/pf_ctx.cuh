@@ -280,6 +280,18 @@ class AsyncWorker {
 
 namespace { struct XRunState; }    // pf_exchange_run's own state (pf_exchange_run.cuh)
 
+// --associations (pf_assoc_load / pf_assoc_collect, pf_assoc.cuh)
+struct AssocState {
+  bool loaded = false;
+  bool batch_ready = false;      // the last batch was collected whole: its rows and windows are on the device
+  uint32_t mask = 0;             // digest table: mask + 1 slots
+  DevBuf d_key, d_val;           // uint4 / u32 per slot
+  DevBuf d_kp, d_cp;             // association row of every pattern of the pools (kAssocNone: not passing)
+  uint64_t kp_done = 0, cp_done = 0;   // patterns looked up so far
+  DevBuf d_table, d_row_seen, d_cl_pass, d_cl_assoc, d_win, d_win_assoc, d_prow, d_prow_assoc, d_prow_seen, d_count;
+  PinBuf h_count, r_win, r_win_assoc, r_cl_pass, r_cl_assoc, r_prow, r_prow_assoc, r_prow_seen;
+};
+
 struct pf_ctx : BatchState {
   pf_params prm{};
   int device = 0;
@@ -368,6 +380,7 @@ struct pf_ctx : BatchState {
   uint32_t pipe_first_seqs = 98304;     // ... of the first one (its upload is not hidden)
   bool lite_ok = true;           // device-side planning of uploads (PF_LITE=0 disables; off after a record fall-back)
   XRunState* xrun = nullptr;     // created by the first pf_exchange_run
+  AssocState assoc;
 };
 
 namespace {

@@ -342,6 +342,234 @@ extern "C" int pf_format_positions_compact(const pf_batch* b, const uint32_t* st
 }
 
 // ---------------------------------------------------------------------------
+// --associations: the lines of panfeed-get-kmers (get_kmers.py:108-145) from the compact positional
+// form and the device join (pf_assoc_collect).  The association columns arrive as one text snippet
+// per passing association, formatted by the caller (pandas prints them, so pandas formats them);
+// a line is a concatenation of the cluster tag, the k-mer, a snippet and the positional fields.
+// ---------------------------------------------------------------------------
+namespace {
+struct AJob {
+  const pf_batch* b;
+  const uint32_t* bits;
+  uint32_t k;
+  int canonical;
+  const pf_batch_result* rows;
+  const pf_assoc_result* a;
+  const char* tag_blob;
+  const uint64_t* tag_off;
+  const char* lead_blob;
+  const uint64_t* lead_off;
+  const char* snip_blob;
+  const uint64_t* snip_off;
+  uint32_t empty_snip;          // tabs of a snippet where nothing passes
+  bool only_passing, floats;
+  std::vector<std::pair<uint64_t, uint32_t>> win;     // (window, association row), sorted
+};
+
+inline uint64_t snip_len(const AJob& j, uint32_t a) {
+  return a == PF_ASSOC_NONE ? j.empty_snip : j.snip_off[a + 1] - j.snip_off[a];
+}
+inline char* put_snip(const AJob& j, uint32_t a, char* p) {
+  if (a == PF_ASSOC_NONE) { memset(p, '\t', j.empty_snip); return p + j.empty_snip; }
+  const uint64_t n = j.snip_off[a + 1] - j.snip_off[a];
+  memcpy(p, j.snip_blob + j.snip_off[a], n);
+  return p + n;
+}
+inline char* put_num(const AJob& j, char* p, int64_t v) {
+  p += put_int(p, v);
+  if (j.floats) { *p++ = '.'; *p++ = '0'; }
+  return p;
+}
+// the window entries of sequence q: [lo, hi) of j.win
+inline std::pair<size_t, size_t> seq_windows(const AJob& j, const pf_seq_desc& q) {
+  auto lo = std::lower_bound(j.win.begin(), j.win.end(), std::make_pair(q.base_off << 1, 0u));
+  auto hi = std::lower_bound(lo, j.win.end(), std::make_pair((q.base_off + q.len) << 1, 0u));
+  return {(size_t)(lo - j.win.begin()), (size_t)(hi - j.win.begin())};
+}
+// Bytes (out == NULL) or the lines of target sequence si.  Right join: every window row of a
+// passing cluster; left join: the passing ones.
+inline uint64_t annot_seq(const AJob& j, uint32_t si, char* out) {
+  const pf_seq_desc& q = j.b->seqs[si];
+  if (!(q.flags & PF_SEQ_TARGET) || q.len < j.k || !j.a->cluster_pass[q.cluster]) return 0;
+  const uint32_t k = j.k, nwin = q.len - k + 1;
+  auto range = seq_windows(j, q);
+  if (j.only_passing && range.first == range.second) return 0;
+  const uint64_t tl = j.tag_off[q.cluster + 1] - j.tag_off[q.cluster];
+  const char* tag = j.tag_blob + j.tag_off[q.cluster];
+  const uint64_t ll = j.lead_off[si + 1] - j.lead_off[si];
+  const char* lead = j.lead_blob + j.lead_off[si];
+  const uint32_t fl = j.floats ? 2 : 0;
+  std::vector<char> text, rc_text;
+  if (out) {
+    text.resize(q.len);
+    rc_text.resize(q.len);
+    if (q.flags & PF_SEQ_AMBIGUOUS) {
+      for (uint32_t s = 0; s < q.len; ++s) {
+        const uint64_t i = q.amb_off + s;
+        text[s] = kAmb[(j.b->amb_codes[i >> 4] >> (60 - 4 * (i & 15u))) & 15u];
+      }
+    } else {
+      for (uint32_t s = 0; s < q.len; ++s) {
+        const uint64_t i = q.base_off + s;
+        text[s] = kAcgt[(j.b->packed_bases[i >> 5] >> (62 - 2 * (i & 31u))) & 3u];
+      }
+    }
+    for (uint32_t s = 0; s < q.len; ++s) rc_text[s] = comp_symbol(text[q.len - 1 - s]);
+  }
+  uint64_t total = 0;
+  char* p = out;
+  size_t at = range.first;
+  auto line = [&](uint32_t w, bool rc, int64_t used, uint32_t a) {
+    const int64_t c0 = q.strand > 0 ? (int64_t)q.start + w : (int64_t)q.end - w - k, g0 = (int64_t)w - q.offset;
+    if (!out) {
+      total += tl + 1 + k + 1 + snip_len(j, a) + 1 + ll + len_int(q.strand) + len_int(c0) + len_int(c0 + k) +
+               len_int(g0) + len_int(g0 + k) + len_int(used) + 6 * fl + 6;
+      return;
+    }
+    memcpy(p, tag, tl); p += tl; *p++ = '\t';
+    memcpy(p, rc ? rc_text.data() + (q.len - w - k) : text.data() + w, k); p += k; *p++ = '\t';
+    p = put_snip(j, a, p); *p++ = '\t';
+    memcpy(p, lead, ll); p += ll;
+    p = put_num(j, p, q.strand); *p++ = '\t';
+    p = put_num(j, p, c0); *p++ = '\t';
+    p = put_num(j, p, c0 + k); *p++ = '\t';
+    p = put_num(j, p, g0); *p++ = '\t';
+    p = put_num(j, p, g0 + k); *p++ = '\t';
+    p = put_num(j, p, used); *p++ = '\n';
+  };
+  auto emit = [&](uint32_t w, uint32_t o) {          // window w, row o (canonical: the one row)
+    const uint64_t id = ((q.base_off + w) << 1) | o;
+    while (at < range.second && j.win[at].first < id) ++at;
+    const uint32_t a = at < range.second && j.win[at].first == id ? j.win[at].second : PF_ASSOC_NONE;
+    if (j.only_passing && a == PF_ASSOC_NONE) return;
+    if (j.canonical) {
+      const uint64_t i = q.base_off + w;
+      const bool rc = (j.bits[i >> 5] >> (i & 31u)) & 1u;
+      line(w, rc, rc ? -1 : 1, a);
+    } else {
+      line(w, o == 1, o == 1 ? -(int64_t)q.strand : (int64_t)q.strand, a);
+    }
+  };
+  if (j.only_passing) {                               // only the listed windows
+    for (size_t e = range.first; e < range.second; ++e) {
+      if (e > range.first && j.win[e].first == j.win[e - 1].first) continue;
+      const uint64_t id = j.win[e].first;
+      emit((uint32_t)((id >> 1) - q.base_off), (uint32_t)(id & 1u));
+    }
+  } else {
+    for (uint32_t w = 0; w < nwin; ++w)
+      for (uint32_t o = 0; o < (j.canonical ? 1u : 2u); ++o) emit(w, o);
+  }
+  return out ? (uint64_t)(p - out) : total;
+}
+// --only-passing: the passing rows no window carries and the passing cluster-row hashes
+inline uint64_t annot_unseen(const AJob& j, char* out) {
+  const pf_batch_result* r = j.rows;
+  const uint64_t nn = r->n_rows, nw = r->n_wide_rows;
+  uint64_t total = 0;
+  char* p = out;
+  auto line = [&](uint32_t c, const char* kmer, uint32_t a) {
+    const uint64_t tl = j.tag_off[c + 1] - j.tag_off[c];
+    const uint64_t kl = kmer ? j.k : 0;
+    if (!out) { total += tl + 1 + kl + 1 + snip_len(j, a) + 9 + 1; return; }
+    memcpy(p, j.tag_blob + j.tag_off[c], tl); p += tl; *p++ = '\t';
+    if (kmer) { memcpy(p, kmer, kl); p += kl; }
+    *p++ = '\t';
+    p = put_snip(j, a, p);
+    memset(p, '\t', 9); p += 9;
+    *p++ = '\n';
+  };
+  char km[72];
+  for (uint64_t e = 0; e < j.a->n_rows; ++e) {
+    if (j.a->row_seen[e]) continue;
+    const uint64_t i = j.a->row[e];
+    uint32_t c;
+    if (i < nn) {
+      c = r->row_cluster[i];
+      for (uint32_t s = 0; s < j.k; ++s) km[s] = kAcgt[(r->row_kmer[i] >> (2 * (j.k - 1 - s))) & 3u];
+    } else if (i < nn + nw) {
+      c = r->wide_row_cluster[i - nn];
+      wide_kmer_text(r->wide_row_kmer + 2 * (i - nn), 2, j.k, km);
+    } else {
+      c = r->xwide_row_cluster[i - nn - nw];
+      wide_kmer_text(r->xwide_row_kmer + 4 * (i - nn - nw), 4, j.k, km);
+    }
+    line(c, km, j.a->row_assoc[e]);
+  }
+  for (uint32_t c = 0; c < j.a->n_clusters; ++c)
+    if (j.a->cluster_assoc[c] != PF_ASSOC_NONE) line(c, nullptr, j.a->cluster_assoc[c]);
+  return out ? (uint64_t)(p - out) : total;
+}
+}  // namespace
+
+extern "C" int pf_format_annotated(const pf_batch* b, const uint32_t* strand_bits, uint32_t k, int canonical,
+                                   const pf_batch_result* rows, const pf_assoc_result* assoc, const char* tag_blob,
+                                   const uint64_t* tag_off, const char* lead_blob, const uint64_t* lead_off,
+                                   const char* snip_blob, const uint64_t* snip_off, uint64_t n_snips,
+                                   uint32_t snip_fields, uint32_t flags, char* out, uint64_t out_cap,
+                                   uint64_t* out_len, uint32_t n_threads) {
+  if (!b || !rows || !assoc || !out_len || k < 1 || k > 64 || snip_fields < 1) return PF_ERR_INVALID;
+  *out_len = 0;
+  if (assoc->n_clusters != b->n_clusters || rows->n_clusters != b->n_clusters) return PF_ERR_INVALID;
+  if (b->n_clusters && (!tag_blob || !tag_off || !assoc->cluster_pass || !assoc->cluster_assoc)) return PF_ERR_INVALID;
+  if (b->n_seqs && (!b->seqs || !b->packed_bases || !lead_blob || !lead_off || (canonical && !strand_bits)))
+    return PF_ERR_INVALID;
+  if (n_snips && (!snip_blob || !snip_off)) return PF_ERR_INVALID;
+  if (assoc->n_windows && (!assoc->window || !assoc->window_assoc)) return PF_ERR_INVALID;
+  if (assoc->n_rows && (!assoc->row || !assoc->row_assoc || !assoc->row_seen)) return PF_ERR_INVALID;
+  const uint64_t n_all_rows = rows->n_rows + rows->n_wide_rows + rows->n_xwide_rows;
+  for (uint64_t e = 0; e < assoc->n_windows; ++e) if (assoc->window_assoc[e] >= n_snips) return PF_ERR_INVALID;
+  for (uint64_t e = 0; e < assoc->n_rows; ++e)
+    if (assoc->row_assoc[e] >= n_snips || assoc->row[e] >= n_all_rows) return PF_ERR_INVALID;
+  for (uint32_t c = 0; c < b->n_clusters; ++c) {
+    const uint32_t a = assoc->cluster_assoc[c];
+    if ((a != PF_ASSOC_NONE && a >= n_snips) || tag_off[c + 1] < tag_off[c]) return PF_ERR_INVALID;
+  }
+  for (uint32_t i = 0; i < b->n_seqs; ++i) {
+    const pf_seq_desc& q = b->seqs[i];
+    if (q.cluster >= b->n_clusters) return PF_ERR_INVALID;
+    if ((q.flags & PF_SEQ_TARGET) && (q.flags & PF_SEQ_AMBIGUOUS) && !b->amb_codes) return PF_ERR_INVALID;
+  }
+  AJob j{b, strand_bits, k, canonical, rows, assoc, tag_blob, tag_off, lead_blob, lead_off, snip_blob, snip_off,
+         snip_fields - 1, (flags & PF_ANNOT_ONLY_PASSING) != 0, (flags & PF_ANNOT_FLOAT_POSITIONS) != 0, {}};
+  j.win.resize(assoc->n_windows);
+  for (uint64_t e = 0; e < assoc->n_windows; ++e) j.win[e] = {assoc->window[e], assoc->window_assoc[e]};
+  std::sort(j.win.begin(), j.win.end());
+  const uint32_t n = b->n_seqs;
+  const uint32_t hw = pf_host_threads();
+  uint32_t nt = n_threads ? n_threads : hw;
+  nt = std::max(1u, std::min<uint32_t>(nt, (n + 63u) / 64u));
+  const uint32_t per = (n + nt - 1) / nt;
+  auto run = [&](auto&& fn) {
+    if (nt == 1) { fn(0u); return; }
+    std::vector<std::thread> th;
+    for (uint32_t t = 0; t < nt; ++t) th.emplace_back(fn, t);
+    for (auto& x : th) x.join();
+  };
+  std::vector<uint64_t> bytes(nt + 1, 0);
+  run([&](uint32_t t) {
+    const uint32_t a = std::min(n, t * per), e = std::min(n, (t + 1) * per);
+    uint64_t s = 0;
+    for (uint32_t i = a; i < e; ++i) s += annot_seq(j, i, nullptr);
+    bytes[t] = s;
+  });
+  if (j.only_passing) bytes[nt] = annot_unseen(j, nullptr);
+  std::vector<uint64_t> start(nt + 1, 0);
+  uint64_t total = 0;
+  for (uint32_t t = 0; t <= nt; ++t) { start[t] = total; total += bytes[t]; }
+  *out_len = total;
+  if (!out) return PF_OK;
+  if (out_cap < total) return PF_ERR_NOMEM;
+  run([&](uint32_t t) {
+    const uint32_t a = std::min(n, t * per), e = std::min(n, (t + 1) * per);
+    char* p = out + start[t];
+    for (uint32_t i = a; i < e; ++i) p += annot_seq(j, i, p);
+  });
+  if (j.only_passing) annot_unseen(j, out + start[nt]);
+  return PF_OK;
+}
+
+// ---------------------------------------------------------------------------
 // Native packer: ASCII sequences -> the 2-bit / 4-bit planes of a pf_batch (what
 // panfeed_b200/packer.py:pack_batch does with numpy look-up tables), host threads.
 // ---------------------------------------------------------------------------

@@ -35,6 +35,7 @@ extern "C" uint32_t pf_struct_size(int which) {
     case 8: return (uint32_t)sizeof(pf_cut_planes);
     case 9: return (uint32_t)sizeof(pf_comm);
     case 10: return (uint32_t)sizeof(pf_exchange_result);
+    case 11: return (uint32_t)sizeof(pf_assoc_result);
     default: return 0;
   }
 }
@@ -253,6 +254,15 @@ extern "C" void pf_destroy(pf_ctx* ctx) {
                     &ctx->d_rescue[0], &ctx->d_rescue[1], &ctx->d_table2_base, &ctx->d_table2,
                     &ctx->d_home_bits, &ctx->d_cta_cluster, &ctx->d_slab_cnt, &ctx->d_spill})
     fd(*b);
+  {
+    AssocState& a = ctx->assoc;
+    for (DevBuf* b : {&a.d_key, &a.d_val, &a.d_kp, &a.d_cp, &a.d_table, &a.d_row_seen, &a.d_cl_pass, &a.d_cl_assoc,
+                      &a.d_win, &a.d_win_assoc, &a.d_prow, &a.d_prow_assoc, &a.d_prow_seen, &a.d_count})
+      fd(*b);
+    for (PinBuf* b : {&a.h_count, &a.r_win, &a.r_win_assoc, &a.r_cl_pass, &a.r_cl_assoc, &a.r_prow, &a.r_prow_assoc,
+                      &a.r_prow_seen})
+      fp(*b);
+  }
   ctx->grower.join();
   xrun_free(ctx);                      // pf_exchange_run's buffers and peer mappings
   for (PatternSpace* s : {&ctx->kp, &ctx->cp}) pool_free(s->pool);

@@ -308,7 +308,11 @@ extern "C" int pf_submit(pf_ctx* ctx, const pf_batch* batch) {
   if (!ctx) return PF_ERR_INVALID;
   if (!batch) return fail(ctx, PF_ERR_INVALID, "pf_submit: null batch");
   if (ctx->pipe_pending) return fail(ctx, PF_ERR_STATE, "pf_submit: results of the previous pf_submit were not collected");
-  if (batch->n_seqs >= ctx->pipe_min_seqs && batch->n_amb_words == 0 && batch->seqs && batch->n_clusters > 1) {
+  ctx->assoc.batch_ready = false;
+  // with an association table the join (pf_assoc_collect) reads the batch's rows and windows on the
+  // device after pf_collect: such batches run whole, as batches with N/IUPAC symbols do
+  if (batch->n_seqs >= ctx->pipe_min_seqs && batch->n_amb_words == 0 && batch->seqs && batch->n_clusters > 1 &&
+      !ctx->assoc.loaded) {
     CU(cudaSetDevice(ctx->device));
     const std::vector<SubRange> subs = split_batch(batch, ctx->pipe_target_seqs, ctx->pipe_first_seqs);
     if (subs.size() > 1) return submit_pipelined(ctx, batch, subs);
@@ -459,6 +463,7 @@ extern "C" int pf_collect(pf_ctx* ctx, pf_batch_result* out) {
   CU(cudaStreamSynchronize(st));
   if (ctx->rows_prefetched) CU(cudaStreamSynchronize(ctx->copy_stream));
   ctx->rows_prefetched = false;
+  ctx->assoc.batch_ready = true;        // its rows and windows stay on the device until the next upload
 
   if (out) {
     memset(out, 0, sizeof *out);
@@ -541,6 +546,7 @@ extern "C" int pf_reset_patterns(pf_ctx* ctx) {
   }
   ctx->kp_base = ctx->cp_base = 0;
   ctx->stats.kmer_patterns = ctx->stats.cluster_patterns = 0;
+  ctx->assoc.kp_done = ctx->assoc.cp_done = 0;
   CU(cudaStreamSynchronize(ctx->stream));
   return PF_OK;
 }

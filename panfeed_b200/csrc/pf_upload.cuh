@@ -553,6 +553,7 @@ extern "C" int pf_upload(pf_ctx* ctx, const pf_batch* b) {
   if (!b) return fail(ctx, PF_ERR_INVALID, "pf_upload: null batch");
   CU(cudaSetDevice(ctx->device));
   if (ctx->pipe_pending) return fail(ctx, PF_ERR_STATE, "pf_upload: results of the previous pf_submit were not collected");
+  ctx->assoc.batch_ready = false;
   SubRange r{0, b->n_seqs, 0, b->n_clusters, 0, b->n_words, 0, b->n_amb_words};
   TRY(upload_async(ctx, *ctx, b, r, ctx->stream));
   // caller buffers may be pageable: upload_finish makes sure the copies have consumed them

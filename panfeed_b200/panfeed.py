@@ -199,7 +199,7 @@ def write_text(handle, data):
         handle.write(bytes(data).decode())
 
 
-def _run_batch(store, ctx, hb, meta, idxs, S, k, canonical, consider_missing):
+def _run_batch(store, ctx, hb, meta, idxs, S, k, canonical, consider_missing, annotate=None):
     """One GPU batch (`hb`: the capi.HostBatch; meta(i) -> (strain, feature id, contig) of its
     sequence i; idxs: the names of its clusters) -> (kmers.tsv text, list of hashes_to_patterns
     texts, kmers_to_hashes text) as bytes / uint8 arrays; the arrays are the formatters' reused
@@ -245,7 +245,10 @@ def _run_batch(store, ctx, hb, meta, idxs, S, k, canonical, consider_missing):
     #      many for Python.  Only the target sequences need their leading fields (and with them
     #      their lazily built metadata). ----
     pos_text = b""
-    if r["n_pos"]:
+    if annotate is not None:
+        # --associations: the get-kmers lines instead of kmers.tsv, joined on the device (assoc.py)
+        annotate.batch(hb, r, ctx.assoc_collect(), k, canonical, idxs, meta)
+    elif r["n_pos"]:
         leads = [b""] * len(hb.seqs)
         cl, strand = hb.seqs["cluster"], hb.seqs["strand"]
         for i in np.nonzero(hb.seqs["flags"] & capi.PF_SEQ_TARGET)[0].tolist():
@@ -256,10 +259,12 @@ def _run_batch(store, ctx, hb, meta, idxs, S, k, canonical, consider_missing):
 
 def pattern_hasher(cluster_dict_iter, kmer_stroi, hash_pat, kmer_hash, genepres, patfilt, maf,
                    output, patterns=None, consider_missing_cluster=False, compress=False,
-                   device=0, sort_bits=0):
+                   device=0, sort_bits=0, annotate=None):
     """Consumes `cluster_cutter` results, runs K1..K4 on the GPU in batches of
     whole clusters and writes the three files exactly as the reference does
-    (panfeed.py:152-233).  Returns the updated `patterns` (a PatternStore)."""
+    (panfeed.py:152-233).  Returns the updated `patterns` (a PatternStore).
+    annotate (an assoc.AnnotatedWriter, --associations): the positional rows are joined to the
+    passing associations on the device and written there instead of to kmer_stroi."""
     multiple_files = hash_pat is None or kmer_hash is None
     if patterns is None or isinstance(patterns, set):
         patterns = PatternStore()
@@ -283,8 +288,11 @@ def pattern_hasher(cluster_dict_iter, kmer_stroi, hash_pat, kmer_hash, genepres,
             return
         ctx = patterns.context(first.k, S, first.canonical, bool(consider_missing_cluster),
                                patfilt == False, maf, device, sort_bits)  # noqa: E712
+        if annotate is not None and not annotate.loaded:
+            ctx.assoc_load(annotate.digests)
+            annotate.loaded = True
         pos_text, pat_texts, hash_text = _run_batch(patterns, ctx, hb, meta, idxs, S, first.k,
-                                                    first.canonical, bool(consider_missing_cluster))
+                                                    first.canonical, bool(consider_missing_cluster), annotate)
         if multiple_files:
             path = os.path.join(output, idxs[0])
             if not os.path.exists(path):
