@@ -10,7 +10,9 @@ that owns the `patterns` set (`__main__.py:299-344`, `:70`); here whole clusters
 over the ranks (greedy by number of genes), every rank writes header-less pieces of
 kmers.tsv / kmers_to_hashes for its clusters, one NCCL exchange (dist.PatternExchange) decides
 which rank writes each pattern's hashes_to_patterns row, and rank 0 joins the pieces into the
-same three files a single process writes."""
+same three files a single process writes.  With --associations every rank writes a piece of
+annotated_kmers.tsv instead of kmers.tsv (assoc.AnnotatedWriter: the ranks OR their upcast facts
+once, just before the exchange)."""
 import argparse
 import logging
 import os
@@ -20,7 +22,7 @@ from functools import partial
 import numpy as np
 
 from . import __version__
-from .input import (KMERS_TSV_HEADER, clean_up_fasta, create_part_files, iter_gene_clusters,
+from .input import (KMERS_TSV_HEADER, OUTPUT_NAMES, clean_up_fasta, create_part_files, iter_gene_clusters,
                     merge_part_files, prep_data_n_fasta, set_input_output, what_are_my_inputfiles)
 from .panfeed import PatternStore, cluster_cutter, pattern_hasher, write_headers
 
@@ -83,7 +85,9 @@ def get_options(argv=None):
                        help="pyseer-style associations table (tab-separated, a header, the pattern id in the first "
                             "column): write <output>/annotated_kmers.tsv, the table panfeed-get-kmers would print "
                             "for this run's kmers_to_hashes.tsv and kmers.tsv, instead of kmers.tsv.  The join runs "
-                            "on the GPU; kmers_to_hashes.tsv and hashes_to_patterns.tsv are written as usual")
+                            "on the GPU (under torchrun every rank joins its own clusters and rank 0 writes the one "
+                            "file); kmers_to_hashes.tsv and hashes_to_patterns.tsv are written as usual.  Not with "
+                            "--multiple-files")
     assoc.add_argument("--association-threshold", type=float, default=argparse.SUPPRESS,
                        help="p-value threshold (get-kmers -t, default 1)")
     assoc.add_argument("--association-column", default=argparse.SUPPRESS,
@@ -118,9 +122,8 @@ def main(argv=None):
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     sharded = world > 1
-    if args.associations is not None and (args.multiple_files or sharded):
-        logger.error("--associations runs on one GPU and writes one file: it cannot be combined with "
-                     "--multiple-files or several ranks (torchrun)")
+    if args.associations is not None and args.multiple_files:
+        logger.error("--associations writes one file: it cannot be combined with --multiple-files")
         sys.exit(1)
     if sharded:
         import torch
@@ -152,16 +155,20 @@ def main(argv=None):
         from .assoc import AnnotatedWriter, load_passing
         a, digests = load_passing(args.associations, args.association_column, args.association_threshold)
         logger.info(f"{len(a)} patterns pass the association threshold {args.association_threshold}")
-        # annotated_kmers.tsv takes the place of kmers.tsv
-        kmer_stroi.close()
-        os.remove(os.path.join(args.output, "kmers.tsv.gz" if args.compress else "kmers.tsv"))
-        kmer_stroi = None
-        annotate = AnnotatedWriter(args.output, a, digests, args.only_passing, args.compress)
+        if not sharded:
+            # annotated_kmers.tsv takes the place of kmers.tsv
+            kmer_stroi.close()
+            os.remove(os.path.join(args.output, "kmers.tsv.gz" if args.compress else "kmers.tsv"))
+            kmer_stroi = None
+            annotate = AnnotatedWriter(args.output, a, digests, args.only_passing, args.compress)
     if sharded:
         if rank == 0:
             os.mkdir(args.output)
         tdist.barrier()
-        if not args.multiple_files:
+        if args.associations is not None:          # a piece of annotated_kmers.tsv in place of kmers.tsv's
+            hash_pat, kmer_hash = create_part_files(args.output, rank, args.compress, OUTPUT_NAMES[1:])
+            annotate = AnnotatedWriter(args.output, a, digests, args.only_passing, args.compress, rank=rank)
+        elif not args.multiple_files:
             kmer_stroi, hash_pat, kmer_hash = create_part_files(args.output, rank, args.compress)
         # whole clusters to ranks, greedy by the number of genes (cells) of the rows that will be cut
         from .dist import shard_clusters
@@ -203,14 +210,22 @@ def main(argv=None):
                      output=args.output, compress=args.compress, device=args.device, annotate=annotate)
     # one streaming call: the generator packs clusters while the GPU batches them
     patterns = func_w(cut_clusters, patterns=patterns)
+    if annotate is not None:
+        # the upcast facts over every rank (one process: its own).  Sharded, a collective: every rank
+        # calls it exactly once, here, after its last batch and before the pattern exchange,
+        # whether it had clusters or not
+        any_rank = bool
+        if sharded:
+            from .dist import any_rank as or_over_ranks
+            dev = torch.device("cuda", args.device) if tdist.get_backend() == "nccl" else torch.device("cpu")
+            any_rank = partial(or_over_ranks, device=dev)
+        annotate.finish(any_rank)
     if patterns.sharded:
         info = patterns.finish_sharded(hash_pat, klength, len(all_columns.columns), not args.non_canonical,
                                        args.consider_missing, args.no_filter, args.maf, args.device)
         logger.info(f"rank {rank}: wrote {info['written_here']} of {info['cluster_patterns_global']} + "
                     f"{info['kmer_patterns_global']} patterns")
     patterns.close()
-    if annotate is not None:
-        annotate.close()
 
     for handle in (kmer_stroi, hash_pat, kmer_hash):
         if handle is not None:
@@ -219,9 +234,14 @@ def main(argv=None):
         tdist.barrier()
         if rank == 0 and not args.multiple_files:
             import io
+            import time
             hp, kh = io.StringIO(), io.StringIO()
             write_headers(hp, kh, all_columns)
-            merge_part_files(args.output, world, (KMERS_TSV_HEADER, hp.getvalue(), kh.getvalue()), args.compress)
+            first = (KMERS_TSV_HEADER, OUTPUT_NAMES[0]) if annotate is None else (annotate.header, annotate.NAME)
+            t0 = time.perf_counter()
+            merge_part_files(args.output, world, (first[0], hp.getvalue(), kh.getvalue()), args.compress,
+                             (first[1],) + OUTPUT_NAMES[1:])
+            logger.info(f"rank 0: merged the pieces of {world} ranks in {time.perf_counter() - t0:.2f} s")
         tdist.barrier()
         tdist.destroy_process_group()
     logger.info("Removing temporary fasta files and faidx indices")

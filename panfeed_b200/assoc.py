@@ -17,6 +17,8 @@ on them are held back until they are known:
   - --only-passing (left join): a passing k-mer without a target window, or a passing cluster-row
     hash, has empty positional fields, which makes pandas print all integer positional columns as
     floats ("361.0").
+Each fact is an OR over the batches, so a sharded run (torchrun, whole clusters per rank) ORs the
+ranks' facts once after their last batch; every rank writes a piece, rank 0 merges them.
 """
 import io
 import logging
@@ -25,7 +27,7 @@ import os
 import numpy as np
 
 from . import capi
-from .input import GzipTextWriter
+from .input import GzipTextWriter, part_path
 
 logger = logging.getLogger("panfeed.assoc")
 
@@ -65,11 +67,20 @@ def snippets(a, upcast):
 
 
 class AnnotatedWriter:
-    """<out>/annotated_kmers.tsv(.gz): the header, then the lines of every batch."""
+    """<out>/annotated_kmers.tsv(.gz): the header, then the lines of every batch.
 
-    def __init__(self, output, a, digests, only_passing, compress):
+    rank (a sharded run, one process per GPU): this rank's header-less piece of that file under
+    <out>/.parts/ instead; rank 0 merges the pieces after `header`.  The upcast fact is then the OR
+    over the ranks: a rank holds both variants of its batches until `finish` has learnt it."""
+
+    NAME = "annotated_kmers.tsv"
+
+    def __init__(self, output, a, digests, only_passing, compress, rank=None):
         self.only_passing = bool(only_passing)
-        path = os.path.join(output, "annotated_kmers.tsv" + (".gz" if compress else ""))
+        if rank is None:
+            path = os.path.join(output, self.NAME + (".gz" if compress else ""))
+        else:
+            path = part_path(output, self.NAME, rank, compress)
         self.handle = GzipTextWriter(path) if compress else open(path, "wb")
         self.digests = digests
         self.loaded = False              # pf_assoc_load on the run's context (pattern_hasher, first batch)
@@ -80,8 +91,9 @@ class AnnotatedWriter:
         self.upcast = False
         self.pending = []
         self.bytes = 0
-        header = "\t".join(["cluster", "k-mer", "hashed_pattern"] + [str(c) for c in a.columns] + POSITIONAL)
-        self._write((header + "\n").encode())
+        self.header = "\t".join(["cluster", "k-mer", "hashed_pattern"] + [str(c) for c in a.columns] + POSITIONAL) + "\n"
+        if rank is None:
+            self._write(self.header.encode())
 
     def _write(self, data):
         if len(data):
@@ -125,8 +137,12 @@ class AnnotatedWriter:
         else:
             self.pending.append((bytes(self._format(job, False)), bytes(self._format(job, True))))
 
-    def close(self):
-        for text, _ in self.pending:
-            self._write(text)
+    def finish(self, any_rank=bool):
+        """After the last batch: any_rank(local fact) -> the fact over all ranks (a collective in a
+        sharded run, which every rank must call exactly once, batches or not), then the held
+        batches in the variant it selects, and the file is closed."""
+        upcast = any_rank(self.upcast)
+        for text, up in self.pending:
+            self._write(up if upcast else text)
         self.pending = []
         self.handle.close()

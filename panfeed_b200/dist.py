@@ -53,6 +53,15 @@ def shard_clusters(weights, world):
     return [sorted(s) for s in shards]
 
 
+def any_rank(flag, device):
+    """True on every rank if `flag` is true on any rank: an all_reduce (MAX) over the default
+    group, on `device` (the rank's GPU under NCCL, the CPU under gloo).  A collective: every
+    rank calls it at the same point."""
+    t = torch.tensor([1 if flag else 0], dtype=torch.int32, device=device)
+    dist.all_reduce(t, op=dist.ReduceOp.MAX)
+    return bool(t.item())
+
+
 class DeviceBackend:
     """pf_exchange_* on one pf_ctx; buffers are torch tensors on its device."""
 

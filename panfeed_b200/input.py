@@ -208,33 +208,36 @@ def create_kmer_stroi(output, compress=False):
 OUTPUT_NAMES = ("kmers.tsv", "hashes_to_patterns.tsv", "kmers_to_hashes.tsv")
 
 
-def create_part_files(output, rank, compress=False):
-    """Sharded run: this rank's header-less pieces of the three outputs
-    (kmers.tsv, hashes_to_patterns, kmers_to_hashes) under <output>/.parts/.  With --compress
-    every piece is a complete gzip stream, so the merged file is a run of gzip members."""
-    parts = os.path.join(output, ".parts")
-    os.makedirs(parts, exist_ok=True)
+def part_path(output, name, rank, compress=False):
+    """<output>/.parts/<name>[.gz].<rank>: a rank's header-less piece of output file `name`."""
+    return os.path.join(output, ".parts", f"{name}{'.gz' if compress else ''}.{rank}")
+
+
+def create_part_files(output, rank, compress=False, names=OUTPUT_NAMES):
+    """Sharded run: this rank's header-less pieces of the outputs `names` (by default kmers.tsv,
+    hashes_to_patterns, kmers_to_hashes) under <output>/.parts/.  With --compress every piece is
+    a complete gzip stream, so the merged file is a run of gzip members."""
+    os.makedirs(os.path.join(output, ".parts"), exist_ok=True)
     handles = []
-    for name in OUTPUT_NAMES:
-        path = os.path.join(parts, f"{name}{'.gz' if compress else ''}.{rank}")
+    for name in names:
+        path = part_path(output, name, rank, compress)
         handles.append(GzipTextWriter(path) if compress else open(path, "w"))
     return tuple(handles)
 
 
-def merge_part_files(output, world, headers, compress=False):
+def merge_part_files(output, world, headers, compress=False, names=OUTPUT_NAMES):
     """Rank 0, after every rank closed its pieces: header + the pieces in rank order -> the
-    three output files; the pieces are removed."""
+    output files `names`; the pieces are removed."""
     import shutil
     from . import capi
-    parts = os.path.join(output, ".parts")
-    for name, header in zip(OUTPUT_NAMES, headers):
+    for name, header in zip(names, headers, strict=True):
         final = os.path.join(output, name + (".gz" if compress else ""))
         with open(final, "wb") as out:
             out.write(capi.gzip_members(header.encode(), 9) if compress else header.encode())
             for r in range(world):
-                with open(os.path.join(parts, f"{name}{'.gz' if compress else ''}.{r}"), "rb") as piece:
+                with open(part_path(output, name, r, compress), "rb") as piece:
                     shutil.copyfileobj(piece, out, 16 << 20)
-    shutil.rmtree(parts)
+    shutil.rmtree(os.path.join(output, ".parts"))
 
 
 def create_hash_files(output, compress=False):
