@@ -421,67 +421,8 @@ int pf_synth_fill(int device, const pf_synth_params* p, pf_seq_desc* seqs,
                   uint64_t* packed_bases);
 
 /* ---- multi-GPU global pattern dedup (SURVEY.md §8(e)) ----
- * Clusters are sharded over ranks; the only global state is the reference's
- * `patterns` set (__main__.py:70).  Owner of a pattern = hash(bitset) % world.
- * The caller moves the buffers between ranks (NCCL all-to-all on the context's
- * stream, see pf_stream); all pointers in this group are DEVICE pointers owned
- * by the caller unless named *_host.  Order of one namespace:
- *   pf_exchange_pack      local patterns bucketed by owner -> send buffer; bucket sizes on the host
- *                         (the one host sync: they are the split sizes of the all-to-all)
- *   [all-to-all of the keys]
- *   pf_exchange_dedup     owner side: unique index of every received key (bit 31 set on the first
- *                         copy of a pattern: its sender is the one that writes the pattern row),
- *                         the number of unique keys to a device word (asynchronous) and/or the host
- *   [all-gather of the unique counts -> exclusive scan = owner_base; reverse all-to-all of the indices]
- *   pf_exchange_unpack    local_to_global[i] = owner_base[owner(i)] + unique index; writer[i] = bit 31
- *                         (asynchronous on the context's stream) */
-int pf_exchange_pack(pf_ctx* ctx, int cluster_namespace, uint32_t world,
-                     const uint32_t* mask_remap_dev, /* local->global cluster-pattern ids, or NULL */
-                     uint32_t* send_words_dev, uint64_t capacity_patterns,
-                     uint64_t* counts_host /* [world] */);
-int pf_exchange_dedup(pf_ctx* ctx, int cluster_namespace,
-                      const uint32_t* recv_words_dev, uint64_t n_recv,
-                      uint32_t* recv_unique_index_dev,
-                      uint32_t* n_unique_dev /* one word, may be NULL */,
-                      uint64_t* n_unique_host /* may be NULL: then the call does not synchronise */,
-                      uint32_t keep_unique_keys /* 1: keep the owner-side unique keys (n_unique x words
-                                                   of device memory) for pf_exchange_unique_export */);
-int pf_exchange_unique_count(pf_ctx* ctx, int cluster_namespace, uint64_t* n_unique_host);
-int pf_exchange_unique_export(pf_ctx* ctx, int cluster_namespace,
-                              uint32_t* host_out /* n_unique x words */);
-int pf_exchange_unpack(pf_ctx* ctx, int cluster_namespace,
-                       const uint32_t* returned_ids_dev, /* in send order */
-                       const uint32_t* owner_base_dev /* [world] or NULL (ids already global) */,
-                       uint32_t* local_to_global_dev /* [n local patterns] */,
-                       uint8_t* writer_dev /* [n local patterns] or NULL */);
-
-/* The same exchange over peer memory (ranks of one box): the keys go straight from the local
- * pattern pool into the OWNER's receive buffer with NVLink peer stores - no send buffer, no
- * all-to-all of the keys.  Order of one namespace:
- *   pf_exchange_classify     owners and bucket positions of the local patterns; bucket sizes on
- *                            the host (one sync)
- *   [all-gather of every rank's bucket sizes: rank r's bucket for owner o starts at row
- *    sum of counts[r' -> o] over r' < r of o's receive buffer, which holds sum over all r']
- *   pf_exchange_recv_buffer  this rank's receive buffer (library-owned, grows; a growth
- *                            invalidates earlier handles: peers close their mappings first) and
- *                            its CUDA IPC handle, which the caller passes to the peers
- *   pf_exchange_open_peer    map a peer's receive buffer (cudaIpcOpenMemHandle); cache the result
- *   pf_exchange_scatter      every local key to owner_buffer[owner] + (row0[owner] + position);
- *                            asynchronous on the context's stream
- *   [a barrier of all ranks on that stream: every scatter has completed]
- *   pf_exchange_dedup on the receive buffer, then as above */
-int pf_exchange_classify(pf_ctx* ctx, int cluster_namespace, uint32_t world,
-                         const uint32_t* mask_remap_dev, uint64_t* counts_host /* [world] */);
-int pf_exchange_recv_buffer(pf_ctx* ctx, int cluster_namespace, uint64_t min_rows, void** dev_ptr,
-                            uint64_t* capacity_rows, unsigned char* ipc_handle_out /* 64 bytes */);
-int pf_exchange_open_peer(pf_ctx* ctx, const unsigned char* ipc_handle /* 64 bytes */, void** mapped);
-int pf_exchange_close_peer(pf_ctx* ctx, void* mapped);
-int pf_exchange_scatter(pf_ctx* ctx, int cluster_namespace, uint32_t world,
-                        const uint32_t* mask_remap_dev, void* const* dest_ptrs /* [world]: device
-                        pointers, the own buffer or pf_exchange_open_peer mappings */,
-                        const uint64_t* dest_row0 /* [world] */);
-
-/* ---- the whole exchange in one call ----
+ * Clusters are sharded over ranks; the only global state is the reference's `patterns` set
+ * (__main__.py:70).  Owner of a pattern = hash(full key) % world.
  * pf_exchange_run numbers the patterns of every rank globally, both namespaces, over collectives
  * the caller provides (pf_comm: NCCL, torch.distributed, or pf_comm_local for the threads of one
  * process).  Every rank calls it, each on its own pf_ctx; everything it enqueues goes on the
@@ -538,6 +479,11 @@ enum { PF_EXCHANGE_WRITER = 1, PF_EXCHANGE_KEEP_UNIQUE = 2, PF_EXCHANGE_NO_PEER 
 
 int pf_exchange_run(pf_ctx* ctx, const pf_comm* comm, uint32_t flags, pf_exchange_result* out);
 int pf_exchange_release(pf_ctx* ctx, const pf_comm* comm);   /* collective: unmap the peers' buffers */
+/* After a pf_exchange_run with PF_EXCHANGE_KEEP_UNIQUE: the owner's unique keys of a namespace
+ * (n_unique = that call's n_owned; global id = owned_base + row), copied to the host. */
+int pf_exchange_unique_count(pf_ctx* ctx, int cluster_namespace, uint64_t* n_unique_host);
+int pf_exchange_unique_export(pf_ctx* ctx, int cluster_namespace,
+                              uint32_t* host_out /* n_unique x words */);
 
 /* Communicator for the threads of ONE process (one pf_ctx per thread, same or different devices):
  * no NCCL, no daemon.  pf_comm_local_get fills a pf_comm for `rank`. */

@@ -8,7 +8,8 @@ Several GPUs: `torchrun --nproc-per-node N -m panfeed_b200 <same options>` (one 
 GPU).  The reference's parallel mode is a reader, N-2 `cluster_cutter` workers and ONE writer
 that owns the `patterns` set (`__main__.py:299-344`, `:70`); here whole clusters are sharded
 over the ranks (greedy by number of genes), every rank writes header-less pieces of
-kmers.tsv / kmers_to_hashes for its clusters, one NCCL exchange (dist.PatternExchange) decides
+kmers.tsv / kmers_to_hashes for its clusters, one exchange (dist.PatternExchange, the library's
+pf_exchange_run over NCCL) decides
 which rank writes each pattern's hashes_to_patterns row, and rank 0 joins the pieces into the
 same three files a single process writes.  With --associations every rank writes a piece of
 annotated_kmers.tsv instead of kmers.tsv (assoc.AnnotatedWriter: the ranks OR their upcast facts

@@ -191,10 +191,8 @@ EXPORTS = ["pf_create", "pf_destroy", "pf_last_error", "pf_abi_version",
            "pf_table_create", "pf_table_destroy", "pf_table_last_error", "pf_table_load", "pf_table_shape",
            "pf_table_names", "pf_table_row_counts", "pf_table_cells",
            "pf_tsv_filter", "pf_free",
-           "pf_synth_plan", "pf_synth_fill", "pf_exchange_pack",
-           "pf_exchange_dedup", "pf_exchange_unique_count", "pf_exchange_unique_export",
-           "pf_exchange_unpack", "pf_exchange_classify", "pf_exchange_recv_buffer", "pf_exchange_open_peer",
-           "pf_exchange_close_peer", "pf_exchange_scatter", "pf_exchange_run", "pf_exchange_release",
+           "pf_synth_plan", "pf_synth_fill", "pf_exchange_unique_count", "pf_exchange_unique_export",
+           "pf_exchange_run", "pf_exchange_release",
            "pf_comm_local_create", "pf_comm_local_get", "pf_comm_local_abort", "pf_comm_local_destroy",
            "pf_assoc_load", "pf_assoc_collect", "pf_format_annotated"]
 
@@ -277,16 +275,8 @@ def load():
     lib.pf_stream.restype = vp
     lib.pf_synth_plan.argtypes = [C.POINTER(SynthParams), C.POINTER(u32), C.POINTER(u64)]
     lib.pf_synth_fill.argtypes = [C.c_int, C.POINTER(SynthParams), vp, vp, vp, vp]
-    lib.pf_exchange_pack.argtypes = [vp, C.c_int, u32, vp, vp, u64, C.POINTER(u64)]
-    lib.pf_exchange_dedup.argtypes = [vp, C.c_int, vp, u64, vp, vp, C.POINTER(u64), u32]
     lib.pf_exchange_unique_count.argtypes = [vp, C.c_int, C.POINTER(u64)]
     lib.pf_exchange_unique_export.argtypes = [vp, C.c_int, vp]
-    lib.pf_exchange_unpack.argtypes = [vp, C.c_int, vp, vp, vp, vp]
-    lib.pf_exchange_classify.argtypes = [vp, C.c_int, u32, vp, C.POINTER(u64)]
-    lib.pf_exchange_recv_buffer.argtypes = [vp, C.c_int, u64, C.POINTER(vp), C.POINTER(u64), C.POINTER(C.c_ubyte)]
-    lib.pf_exchange_open_peer.argtypes = [vp, C.POINTER(C.c_ubyte), C.POINTER(vp)]
-    lib.pf_exchange_close_peer.argtypes = [vp, vp]
-    lib.pf_exchange_scatter.argtypes = [vp, C.c_int, u32, vp, C.POINTER(vp), C.POINTER(u64)]
     lib.pf_exchange_run.argtypes = [vp, C.POINTER(Comm), u32, C.POINTER(ExchangeResult)]
     lib.pf_exchange_release.argtypes = [vp, C.POINTER(Comm)]
     lib.pf_comm_local_create.argtypes = [u32, C.POINTER(vp)]

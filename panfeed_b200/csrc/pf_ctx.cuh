@@ -104,11 +104,9 @@ struct PatternSpace {
   DevBuf table;           // table_size x u32
   uint32_t table_size = 0;
   // exchange state
-  DevBuf x_owner, x_pos, x_perm, x_counts, x_unique, x_table, x_rep, x_slot, x_winner, x_recv;
+  DevBuf x_owner, x_pos, x_perm, x_counts, x_unique, x_table, x_rep, x_slot, x_winner;
   uint64_t x_n_unique = 0;
   bool x_have_unique = false;           // x_unique holds the owner-side unique keys of the last exchange
-  bool x_unique_pending = false;        // x_n_unique still sits in the pinned mirror below
-  const uint32_t* x_unique_mirror = nullptr;
 };
 
 struct WidthState {       // per key width (narrow u64 / wide Key128 / Key256)
@@ -628,12 +626,11 @@ enum { C_TICKET_N = 0, C_TICKET_W = 1, C_RUNS_N = 2, C_RUNS_W = 3, C_ERR = 4, C_
        C_LOCAL = 11 /* LC_COUNT words: rows, unique, table overflow, row overflow, rescue runs,
                         partial rows, partial overflow, kA segments, one-sample partial rows,
                         K4 candidates */,
-       C_X_UNIQUE_KP = 21, C_X_UNIQUE_CP = 22 /* owner-side unique counts of the exchange */,
        C_TICKET_X = 23, C_RUNS_X = 24, C_ROWS_X = 25, C_TICKET_MARK_X = 26 /* 256-bit keys (k > 32) */,
        C_UNIQUE_WX = 27 /* distinct live keys of the wide and 256-bit records (k > 32 with N/IUPAC) */,
        C_COUNT = 29 };
 static_assert(C_COUNT <= 32, "mirror_counters copies one warp's worth");
-static_assert(C_LOCAL + LC_COUNT <= C_X_UNIQUE_KP, "counter layout");
+static_assert(C_LOCAL + LC_COUNT <= C_TICKET_X, "counter layout");
 
 bool keep_count(double maf, uint32_t c, uint32_t n) {
   double af = (double)c / (double)n;      // numpy: vec.sum() / vec.shape[0]

@@ -1,4 +1,5 @@
-// pf_exchange.cuh — multi-GPU pattern exchange kernels and the pf_exchange_* entry points.
+// pf_exchange.cuh — multi-GPU pattern exchange kernels, the classify and owner-side dedup steps
+// pf_exchange_run.cuh sequences, and the export of the owner's unique keys.
 // Part of libpanfeed_b200.so's single translation unit: included once, in order, by pf_api.cu.
 
 // ---------------------------------------------------------------------------
@@ -150,282 +151,96 @@ __global__ void x_unpack(const uint32_t* __restrict__ returned, const uint32_t* 
 }  // namespace pf
 
 namespace {
-// owners, bucket positions and bucket sizes of the local patterns of one namespace; the sizes
-// come back to the host (one sync: they size the receive side)
-int exchange_classify(pf_ctx* ctx, PatternSpace& s, bool cluster_namespace, uint32_t world,
-                      const uint32_t* mask_remap_dev, std::vector<uint32_t>& counts) {
+// One instantiation per lanes-per-key L: short keys would leave most of a warp idle (as in K4).
+template <typename F>
+void xr_launch_by_width(uint32_t key_words, F&& f) {
+  const int L = key_words <= 16 ? 4 : key_words <= 32 ? 8 : key_words <= 64 ? 16 : 32;
+  if (L == 4) f(std::integral_constant<int, 4>());
+  else if (L == 8) f(std::integral_constant<int, 8>());
+  else if (L == 16) f(std::integral_constant<int, 16>());
+  else f(std::integral_constant<int, 32>());
+}
+
+// owners, bucket positions, bucket sizes (x_counts[0, world)) and bucket offsets
+// (x_counts[world, 2 world)) of the local patterns of one namespace, on the stream
+int exchange_classify(pf_ctx* ctx, PatternSpace& s, uint32_t world, const uint32_t* mask_remap_dev) {
   cudaStream_t st = ctx->stream;
   const uint32_t n = (uint32_t)s.n;
-  if (mask_remap_dev && (cluster_namespace || !ctx->prm.consider_missing))
-    return fail(ctx, PF_ERR_INVALID, "mask_remap only applies to k-mer patterns with consider_missing");
-  if (world > 32) return fail(ctx, PF_ERR_UNSUPPORTED, "exchange over more than 32 ranks");
   TRY(dev_ensure(ctx, s.x_owner, std::max<size_t>(1, n) * 4));
   TRY(dev_ensure(ctx, s.x_pos, std::max<size_t>(1, n) * 4));
   TRY(dev_ensure(ctx, s.x_perm, std::max<size_t>(1, n) * 4));
   TRY(dev_ensure(ctx, s.x_counts, (size_t)world * 2 * 4));
   CU(cudaMemsetAsync(s.x_counts.p, 0, (size_t)world * 2 * 4, st));
-  counts.assign(world, 0);
   if (n == 0) return PF_OK;
-  TRY(pin_ensure(ctx, ctx->h_counters, C_COUNT * 4 + 64 * 4));
-  uint32_t* hx = ctx->h_counters.as<uint32_t>() + C_COUNT;
-  const int L = s.key_words <= 16 ? 4 : s.key_words <= 32 ? 8 : s.key_words <= 64 ? 16 : 32;
-  const uint32_t cgrid = std::min<uint32_t>(cdiv(n, 256), kGridPersist * 2);
-#define PF_XC(LL)                                                                                        \
-  x_classify<LL><<<cgrid, 256, 0, st>>>(s.pool.as<uint32_t>(), n, s.key_words, mask_remap_dev, world,    \
-                                        s.x_owner.as<uint32_t>(), s.x_pos.as<uint32_t>(),                \
-                                        s.x_counts.as<uint32_t>())
-  if (L == 4) PF_XC(4); else if (L == 8) PF_XC(8); else if (L == 16) PF_XC(16); else PF_XC(32);
-#undef PF_XC
+  xr_launch_by_width(s.key_words, [&](auto LL) {
+    constexpr int L = decltype(LL)::value;
+    x_classify<L><<<std::min<uint32_t>(cdiv(n, 256), kGridPersist * 2), 256, 0, st>>>(
+        s.pool.as<uint32_t>(), n, s.key_words, mask_remap_dev, world, s.x_owner.as<uint32_t>(),
+        s.x_pos.as<uint32_t>(), s.x_counts.as<uint32_t>());
+  });
   x_offsets<<<1, 32, 0, st>>>(s.x_counts.as<uint32_t>(), world);
-  mirror_counters<<<1, 32, 0, st>>>(hx, s.x_counts.as<uint32_t>(), world);
-  ctx->launches += 3;
+  ctx->launches += 2;
   CU(cudaGetLastError());
   return PF_OK;
 }
-int exchange_counts_to_host(pf_ctx* ctx, uint32_t world, std::vector<uint32_t>& counts) {
-  CU(cudaStreamSynchronize(ctx->stream));        // the only sync: bucket sizes for the receive side
-  const uint32_t* hx = ctx->h_counters.as<uint32_t>() + C_COUNT;
-  for (uint32_t r = 0; r < world; ++r) counts[r] = hx[r];
+
+// owner side of one namespace, on the stream: the unique index of every received key (bit 31 set
+// on the first copy of a pattern: its sender writes the pattern row) and their number to
+// *n_unique_dev; keep_unique: the unique keys stay in s.x_unique for pf_exchange_unique_export
+int exchange_dedup(pf_ctx* ctx, PatternSpace& s, const uint32_t* recv, uint64_t n_recv, uint32_t* unique_index,
+                   uint32_t* n_unique_dev, bool keep_unique) {
+  cudaStream_t st = ctx->stream;
+  s.x_n_unique = 0;                   // (pf_exchange_run sets it once the count is on the host)
+  if (n_recv == 0) {
+    CU(cudaMemsetAsync(n_unique_dev, 0, 4, st));
+    return PF_OK;
+  }
+  if (n_recv >= (1ull << 30)) return fail(ctx, PF_ERR_INVALID, "too many received patterns");
+  const uint32_t n = (uint32_t)n_recv;
+  uint32_t size = 1024;
+  while (size < 2ull * n + 16) size *= 2;
+  // scratch kept across calls: no cudaMalloc in the steady state
+  TRY(dev_ensure(ctx, s.x_table, (size_t)size * 4));
+  TRY(dev_ensure(ctx, s.x_rep, (size_t)n * 4));
+  TRY(dev_ensure(ctx, s.x_slot, (size_t)n * 4));
+  TRY(dev_ensure(ctx, s.x_winner, ((size_t)n + 1) * 4));
+  if (keep_unique) TRY(dev_ensure(ctx, s.x_unique, (size_t)n * s.key_words * 4));
+  s.x_have_unique = keep_unique;
+  CU(cudaMemsetAsync(s.x_table.p, 0xff, (size_t)size * 4, st));
+  xr_launch_by_width(s.key_words, [&](auto LL) {
+    constexpr int L = decltype(LL)::value;
+    k4_probe<L><<<std::min<uint32_t>(cdiv(n, 256 / L), kGridPersist * 4), 256, 0, st>>>(
+        recv, n, s.key_words, nullptr, s.x_table.as<uint32_t>(), size - 1, s.x_rep.as<uint32_t>(),
+        s.x_slot.as<uint32_t>(), s.x_winner.as<uint32_t>());
+  });
+  TRY(scan_inplace(ctx, s.x_winner.as<uint32_t>(), n, n_unique_dev));
+  xr_launch_by_width(s.key_words, [&](auto LL) {
+    constexpr int L = decltype(LL)::value;
+    x_finish<L><<<std::min<uint32_t>(cdiv(n, 256 / L), kGridPersist * 4), 256, 0, st>>>(
+        recv, n, s.key_words, s.x_rep.as<uint32_t>(), s.x_winner.as<uint32_t>(), unique_index,
+        keep_unique ? s.x_unique.as<uint32_t>() : nullptr);
+  });
+  ctx->launches += 2;
+  CU(cudaGetLastError());
   return PF_OK;
 }
 }  // namespace
 
-extern "C" int pf_exchange_pack(pf_ctx* ctx, int cluster_namespace, uint32_t world,
-                                const uint32_t* mask_remap_dev, uint32_t* send_words_dev,
-                                uint64_t capacity_patterns, uint64_t* counts_host) {
-  if (!ctx || !counts_host || world == 0) return PF_ERR_INVALID;
-  CU(cudaSetDevice(ctx->device));
-  TRY(finalize_pending(ctx));
-  PatternSpace& s = cluster_namespace ? ctx->cp : ctx->kp;
-  cudaStream_t st = ctx->stream;
-  const uint32_t n = (uint32_t)s.n;
-  if (n > capacity_patterns) return fail(ctx, PF_ERR_INVALID, "send buffer too small: %u patterns", n);
-  if (n && !send_words_dev) return fail(ctx, PF_ERR_INVALID, "null send buffer");
-  std::vector<uint32_t> counts;
-  TRY(exchange_classify(ctx, s, cluster_namespace != 0, world, mask_remap_dev, counts));
-  if (n) {
-    const int L = s.key_words <= 16 ? 4 : s.key_words <= 32 ? 8 : s.key_words <= 64 ? 16 : 32;
-    const uint32_t pgrid = std::min<uint32_t>(cdiv(n, 256 / L), kGridPersist * 4);
-#define PF_XC(LL)                                                                                        \
-    x_pack<LL><<<pgrid, 256, 0, st>>>(s.pool.as<uint32_t>(), n, s.key_words, mask_remap_dev,             \
-                                      s.x_owner.as<uint32_t>(), s.x_pos.as<uint32_t>(),                  \
-                                      s.x_counts.as<uint32_t>() + world, send_words_dev,                 \
-                                      s.x_perm.as<uint32_t>())
-    if (L == 4) PF_XC(4); else if (L == 8) PF_XC(8); else if (L == 16) PF_XC(16); else PF_XC(32);
-#undef PF_XC
-    ctx->launches++;
-    CU(cudaGetLastError());
-    TRY(exchange_counts_to_host(ctx, world, counts));
-  }
-  for (uint32_t r = 0; r < world; ++r) counts_host[r] = counts[r];
-  return PF_OK;
-}
-
-// ---- the same exchange over peer memory: classify -> [the caller gathers the bucket sizes of
-//      all ranks and maps the owners' receive buffers] -> scatter -> [barrier] -> dedup ----
-extern "C" int pf_exchange_classify(pf_ctx* ctx, int cluster_namespace, uint32_t world,
-                                    const uint32_t* mask_remap_dev, uint64_t* counts_host) {
-  if (!ctx || !counts_host || world == 0) return PF_ERR_INVALID;
-  CU(cudaSetDevice(ctx->device));
-  TRY(finalize_pending(ctx));
-  PatternSpace& s = cluster_namespace ? ctx->cp : ctx->kp;
-  std::vector<uint32_t> counts;
-  TRY(exchange_classify(ctx, s, cluster_namespace != 0, world, mask_remap_dev, counts));
-  if (s.n) TRY(exchange_counts_to_host(ctx, world, counts));
-  for (uint32_t r = 0; r < world; ++r) counts_host[r] = counts[r];
-  return PF_OK;
-}
-
-extern "C" int pf_exchange_recv_buffer(pf_ctx* ctx, int cluster_namespace, uint64_t min_rows, void** dev_ptr,
-                                       uint64_t* capacity_rows, unsigned char* ipc_handle_out /* 64 bytes */) {
-  if (!ctx || !dev_ptr || !capacity_rows || !ipc_handle_out) return PF_ERR_INVALID;
-  CU(cudaSetDevice(ctx->device));
-  PatternSpace& s = cluster_namespace ? ctx->cp : ctx->kp;
-  const size_t row = (size_t)s.key_words * 4;
-  if (!s.x_recv.p || s.x_recv.cap < min_rows * row) {
-    // (peers that mapped the old buffer have closed it: the caller's protocol, see dist.py)
-    CU(cudaStreamSynchronize(ctx->stream));
-    if (s.x_recv.p) { CU(cudaFree(s.x_recv.p)); s.x_recv.p = nullptr; s.x_recv.cap = 0; }      // (contents are scratch)
-    TRY(dev_ensure(ctx, s.x_recv, std::max<size_t>(row, min_rows * row)));
-  }
-  static_assert(sizeof(cudaIpcMemHandle_t) == 64, "IPC handle size");
-  cudaIpcMemHandle_t h;
-  if (cudaIpcGetMemHandle(&h, s.x_recv.p) != cudaSuccess) {
-    cudaGetLastError();
-    return fail(ctx, PF_ERR_CUDA, "cudaIpcGetMemHandle failed on the receive buffer");
-  }
-  memcpy(ipc_handle_out, &h, 64);
-  *dev_ptr = s.x_recv.p;
-  *capacity_rows = s.x_recv.cap / row;
-  return PF_OK;
-}
-
-extern "C" int pf_exchange_open_peer(pf_ctx* ctx, const unsigned char* ipc_handle /* 64 bytes */, void** mapped) {
-  if (!ctx || !ipc_handle || !mapped) return PF_ERR_INVALID;
-  CU(cudaSetDevice(ctx->device));
-  cudaIpcMemHandle_t h;
-  memcpy(&h, ipc_handle, 64);
-  void* p = nullptr;
-  if (cudaIpcOpenMemHandle(&p, h, cudaIpcMemLazyEnablePeerAccess) != cudaSuccess) {
-    cudaGetLastError();
-    return fail(ctx, PF_ERR_CUDA, "cudaIpcOpenMemHandle failed: no peer access to the owner's receive buffer");
-  }
-  *mapped = p;
-  return PF_OK;
-}
-
-extern "C" int pf_exchange_close_peer(pf_ctx* ctx, void* mapped) {
-  if (!ctx) return PF_ERR_INVALID;
-  if (!mapped) return PF_OK;
-  CU(cudaSetDevice(ctx->device));
-  if (cudaIpcCloseMemHandle(mapped) != cudaSuccess) { cudaGetLastError(); return fail(ctx, PF_ERR_CUDA, "cudaIpcCloseMemHandle failed"); }
-  return PF_OK;
-}
-
-extern "C" int pf_exchange_scatter(pf_ctx* ctx, int cluster_namespace, uint32_t world,
-                                   const uint32_t* mask_remap_dev, void* const* dest_ptrs /* [world] */,
-                                   const uint64_t* dest_row0 /* [world] */) {
-  if (!ctx || !dest_ptrs || !dest_row0 || world == 0 || world > 32) return PF_ERR_INVALID;
-  CU(cudaSetDevice(ctx->device));
-  PatternSpace& s = cluster_namespace ? ctx->cp : ctx->kp;
-  cudaStream_t st = ctx->stream;
-  const uint32_t n = (uint32_t)s.n;
-  if (n == 0) return PF_OK;
-  if (!s.x_owner.p || !s.x_pos.p) return fail(ctx, PF_ERR_STATE, "pf_exchange_scatter before pf_exchange_classify");
-  const uint32_t* hx = ctx->h_counters.as<uint32_t>() + C_COUNT;      // bucket sizes of the classify call
-  XDest d{};
-  uint32_t run = 0;
-  for (uint32_t r = 0; r < world; ++r) {
-    if (hx[r] && !dest_ptrs[r]) return fail(ctx, PF_ERR_INVALID, "no receive buffer of rank %u", r);
-    if (dest_row0[r] + hx[r] >= (1ull << 32)) return fail(ctx, PF_ERR_INVALID, "receive buffer of rank %u too large", r);
-    d.ptr[r] = static_cast<uint32_t*>(dest_ptrs[r]);
-    d.row0[r] = (uint32_t)dest_row0[r];
-    d.send0[r] = run;
-    run += hx[r];
-  }
-  const int L = s.key_words <= 16 ? 4 : s.key_words <= 32 ? 8 : s.key_words <= 64 ? 16 : 32;
-  const uint32_t pgrid = std::min<uint32_t>(cdiv(n, 256 / L), kGridPersist * 4);
-#define PF_XS(LL)                                                                                        \
-  x_scatter<LL><<<pgrid, 256, 0, st>>>(s.pool.as<uint32_t>(), n, s.key_words, mask_remap_dev,            \
-                                       s.x_owner.as<uint32_t>(), s.x_pos.as<uint32_t>(), d, s.x_perm.as<uint32_t>())
-  if (L == 4) PF_XS(4); else if (L == 8) PF_XS(8); else if (L == 16) PF_XS(16); else PF_XS(32);
-#undef PF_XS
-  ctx->launches++;
-  CU(cudaGetLastError());
-  return PF_OK;
-}
-
-extern "C" int pf_exchange_dedup(pf_ctx* ctx, int cluster_namespace, const uint32_t* recv_words_dev,
-                                 uint64_t n_recv, uint32_t* recv_unique_index_dev, uint32_t* n_unique_dev,
-                                 uint64_t* n_unique_host, uint32_t keep_unique_keys) {
-  if (!ctx || (!n_unique_host && !n_unique_dev)) return PF_ERR_INVALID;
-  CU(cudaSetDevice(ctx->device));
-  PatternSpace& s = cluster_namespace ? ctx->cp : ctx->kp;
-  cudaStream_t st = ctx->stream;
-  if (n_unique_host) *n_unique_host = 0;
-  s.x_n_unique = 0;
-  s.x_unique_pending = false;
-  if (n_recv == 0) {
-    if (n_unique_dev) CU(cudaMemsetAsync(n_unique_dev, 0, 4, st));
-    return PF_OK;
-  }
-  if (n_recv >= (1ull << 30)) return fail(ctx, PF_ERR_INVALID, "too many received patterns");
-  if (!recv_words_dev || !recv_unique_index_dev) return fail(ctx, PF_ERR_INVALID, "null exchange buffer");
-  const uint32_t n = (uint32_t)n_recv;
-  uint32_t size = 1024;
-  while (size < 2ull * n + 16) size *= 2;
-  DevBuf& table = s.x_table;          // scratch kept across calls: no cudaMalloc in the steady state
-  DevBuf& rep = s.x_rep;
-  DevBuf& slot_of = s.x_slot;
-  DevBuf& winner = s.x_winner;
-  TRY(dev_ensure(ctx, table, (size_t)size * 4));
-  TRY(dev_ensure(ctx, rep, (size_t)n * 4));
-  TRY(dev_ensure(ctx, slot_of, (size_t)n * 4));
-  TRY(dev_ensure(ctx, winner, ((size_t)n + 1) * 4));
-  if (keep_unique_keys) TRY(dev_ensure(ctx, s.x_unique, (size_t)n * s.key_words * 4));
-  s.x_have_unique = keep_unique_keys != 0;
-  CU(cudaMemsetAsync(table.p, 0xff, (size_t)size * 4, st));
-  uint32_t* counters = ctx->d_counters.p ? ctx->d_counters.as<uint32_t>() : nullptr;
-  if (!counters) { TRY(dev_ensure(ctx, ctx->d_counters, C_COUNT * 4)); TRY(pin_ensure(ctx, ctx->h_counters, C_COUNT * 4 + 64 * 4)); counters = ctx->d_counters.as<uint32_t>(); }
-  const uint32_t grid = std::min<uint32_t>(cdiv(n, 8), kGridPersist * 2);
-  {
-    // lanes per pattern as in K4: short keys would leave most of a warp idle
-    const int L = s.key_words <= 16 ? 4 : s.key_words <= 32 ? 8 : s.key_words <= 64 ? 16 : 32;
-    const uint32_t pgrid = std::min<uint32_t>(cdiv(n, 256 / L), kGridPersist * 4);
-#define PF_XP(LL)                                                                                          \
-    k4_probe<LL><<<pgrid, 256, 0, st>>>(recv_words_dev, n, s.key_words, nullptr, table.as<uint32_t>(), size - 1, \
-                                        rep.as<uint32_t>(), slot_of.as<uint32_t>(), winner.as<uint32_t>())
-    if (L == 4) PF_XP(4); else if (L == 8) PF_XP(8); else if (L == 16) PF_XP(16); else PF_XP(32);
-#undef PF_XP
-  }
-  uint32_t* total_dev = counters + (cluster_namespace ? C_X_UNIQUE_CP : C_X_UNIQUE_KP);
-  TRY(scan_inplace(ctx, winner.as<uint32_t>(), n, total_dev));
-  {
-    const int L = s.key_words <= 16 ? 4 : s.key_words <= 32 ? 8 : s.key_words <= 64 ? 16 : 32;
-    const uint32_t fgrid = std::min<uint32_t>(cdiv(n, 256 / L), kGridPersist * 4);
-#define PF_XF(LL)                                                                                          \
-    x_finish<LL><<<fgrid, 256, 0, st>>>(recv_words_dev, n, s.key_words, rep.as<uint32_t>(), winner.as<uint32_t>(), \
-                                        recv_unique_index_dev, keep_unique_keys ? s.x_unique.as<uint32_t>() : nullptr)
-    if (L == 4) PF_XF(4); else if (L == 8) PF_XF(8); else if (L == 16) PF_XF(16); else PF_XF(32);
-#undef PF_XF
-  }
-  ctx->launches += 2;
-  TRY(pin_ensure(ctx, ctx->h_counters, C_COUNT * 4 + 64 * 4));
-  // pinned mirror of the unique count, one word per namespace (behind the pack counts)
-  uint32_t* hx = ctx->h_counters.as<uint32_t>() + C_COUNT + 32 + (cluster_namespace ? 1 : 0);
-  mirror_counters<<<1, 32, 0, st>>>(hx, total_dev, 1);
-  if (n_unique_dev) CU(cudaMemcpyAsync(n_unique_dev, total_dev, 4, cudaMemcpyDeviceToDevice, st));
-  ctx->launches++;
-  CU(cudaGetLastError());
-  s.x_unique_pending = true;          // x_n_unique is read from the mirror once the stream has passed
-  s.x_unique_mirror = hx;
-  if (n_unique_host) {                // the caller wants the count now: one sync
-    CU(cudaStreamSynchronize(st));
-    s.x_n_unique = hx[0];
-    s.x_unique_pending = false;
-    *n_unique_host = hx[0];
-  }
-  return PF_OK;
-}
-
+// the owner-side unique keys of the last pf_exchange_run with PF_EXCHANGE_KEEP_UNIQUE
 extern "C" int pf_exchange_unique_count(pf_ctx* ctx, int cluster_namespace, uint64_t* n_unique_host) {
   if (!ctx || !n_unique_host) return PF_ERR_INVALID;
-  PatternSpace& s = cluster_namespace ? ctx->cp : ctx->kp;
-  CU(cudaSetDevice(ctx->device));
-  if (s.x_unique_pending) {
-    CU(cudaStreamSynchronize(ctx->stream));
-    s.x_n_unique = s.x_unique_mirror[0];
-    s.x_unique_pending = false;
-  }
-  *n_unique_host = s.x_n_unique;
+  *n_unique_host = (cluster_namespace ? ctx->cp : ctx->kp).x_n_unique;
   return PF_OK;
 }
 
 extern "C" int pf_exchange_unique_export(pf_ctx* ctx, int cluster_namespace, uint32_t* host_out) {
   if (!ctx) return PF_ERR_INVALID;
-  uint64_t n = 0;
-  TRY(pf_exchange_unique_count(ctx, cluster_namespace, &n));
   PatternSpace& s = cluster_namespace ? ctx->cp : ctx->kp;
+  const uint64_t n = s.x_n_unique;
   if (n == 0) return PF_OK;
   if (!host_out) return PF_ERR_INVALID;
-  if (!s.x_have_unique) return fail(ctx, PF_ERR_STATE, "pf_exchange_dedup was not asked to keep the unique keys");
-  CU(cudaMemcpy(host_out, s.x_unique.p, n * s.key_words * 4, cudaMemcpyDeviceToHost));
-  return PF_OK;
-}
-
-extern "C" int pf_exchange_unpack(pf_ctx* ctx, int cluster_namespace, const uint32_t* returned_ids_dev,
-                                  const uint32_t* owner_base_dev, uint32_t* local_to_global_dev,
-                                  uint8_t* writer_dev) {
-  if (!ctx) return PF_ERR_INVALID;
+  if (!s.x_have_unique) return fail(ctx, PF_ERR_STATE, "pf_exchange_run was not asked to keep the unique keys");
   CU(cudaSetDevice(ctx->device));
-  PatternSpace& s = cluster_namespace ? ctx->cp : ctx->kp;
-  const uint32_t n = (uint32_t)s.n;
-  if (n == 0) return PF_OK;
-  if (!returned_ids_dev || !local_to_global_dev) return fail(ctx, PF_ERR_INVALID, "null exchange buffer");
-  // asynchronous on the context's stream: the caller synchronises when it reads the table
-  x_unpack<<<cdiv(n, 256), 256, 0, ctx->stream>>>(returned_ids_dev, s.x_perm.as<uint32_t>(), s.x_owner.as<uint32_t>(),
-                                                  owner_base_dev, n, local_to_global_dev, writer_dev);
-  ctx->launches++;
-  CU(cudaGetLastError());
+  CU(cudaMemcpy(host_out, s.x_unique.p, n * s.key_words * 4, cudaMemcpyDeviceToHost));
   return PF_OK;
 }

@@ -1,7 +1,7 @@
 // pf_exchange_run.cuh — pf_exchange_run / pf_exchange_release: the multi-GPU pattern exchange of
 // pf_exchange.cuh in one call, over collectives the caller provides (pf_comm), and pf_comm_local,
 // a communicator for the threads of one process.  The kernels are those of pf_exchange.cuh
-// (x_classify, x_scatter, x_pack, the K4 dedup of pf_exchange_dedup, x_unpack); the only new device
+// (x_classify, x_scatter, x_pack, the K4 dedup of exchange_dedup, x_unpack); the only new device
 // code is the scan of the unique counts.
 // Part of libpanfeed_b200.so's single translation unit: included once, in order, by pf_api.cu.
 
@@ -284,15 +284,6 @@ int xr_peer_setup(pf_ctx* ctx, const pf_comm* c, XRunState& x, uint32_t flags, c
   return PF_OK;
 }
 
-template <typename F>
-void xr_launch_by_width(uint32_t key_words, F&& f) {
-  const int L = key_words <= 16 ? 4 : key_words <= 32 ? 8 : key_words <= 64 ? 16 : 32;
-  if (L == 4) f(std::integral_constant<int, 4>());
-  else if (L == 8) f(std::integral_constant<int, 8>());
-  else if (L == 16) f(std::integral_constant<int, 16>());
-  else f(std::integral_constant<int, 32>());
-}
-
 // owner side + ids back + unpack of one namespace, either transport; recv: the received keys
 int xr_finish(pf_ctx* ctx, const pf_comm* c, XRunState& x, int ns, uint32_t flags, const XRec* all, bool peer,
               const uint32_t* recv, uint64_t n_recv, uint32_t* uniq) {
@@ -301,7 +292,7 @@ int xr_finish(pf_ctx* ctx, const pf_comm* c, XRunState& x, int ns, uint32_t flag
   XNs& n = x.ns[ns];
   cudaStream_t st = ctx->stream;
   const uint32_t nl = (uint32_t)n.n_local;
-  TRY(pf_exchange_dedup(ctx, ns, recv, n_recv, uniq, xs_nu(x, ns), nullptr, (flags & PF_EXCHANGE_KEEP_UNIQUE) ? 1u : 0u));
+  TRY(exchange_dedup(ctx, s, recv, n_recv, uniq, xs_nu(x, ns), (flags & PF_EXCHANGE_KEEP_UNIQUE) != 0));
   // every owner's unique count; on the peer path also the barrier before the indices are read back
   TRY(xr_gather(ctx, c, xs_nu(x, ns), xs_all_nu(x, ns), 4));
   x_owner_base<<<1, 32, 0, st>>>(xs_all_nu(x, ns), world, xs_base(x, ns));
@@ -345,14 +336,13 @@ int xr_step(pf_ctx* ctx, const pf_comm* c, XRunState& x, uint32_t flags, const i
             const uint32_t* mask_remap) {
   const uint32_t world = c->world, rank = c->rank;
   cudaStream_t st = ctx->stream;
-  std::vector<uint32_t> unused;
   for (int i = 0; i < n_ns; ++i) {
     const int ns = nss[i];
     PatternSpace& s = ns ? ctx->cp : ctx->kp;
     if (s.n >= (1ull << 31)) return fail(ctx, PF_ERR_INVALID, "too many local patterns for the exchange");
     x.ns[ns].n_local = s.n;
     x.ns[ns].bytes_sent = s.n * s.key_words * 4;
-    TRY(exchange_classify(ctx, s, ns != 0, world, ns ? nullptr : mask_remap, unused));
+    TRY(exchange_classify(ctx, s, world, ns ? nullptr : mask_remap));
     if (!x.ns[ns].recv.p && !(flags & PF_EXCHANGE_NO_PEER) && !x.peer_failed)
       xr_grow(ctx, x.ns[ns], s.key_words, 1);
   }
@@ -491,6 +481,7 @@ extern "C" int pf_exchange_run(pf_ctx* ctx, const pf_comm* comm, uint32_t flags,
       if (r < comm->rank) o.owned_base += c[r];
     }
     o.n_owned = c[comm->rank];
+    (ns ? ctx->cp : ctx->kp).x_n_unique = o.n_owned;       // for pf_exchange_unique_export
     o.local_to_global = n.l2g.as<uint32_t>();
     o.writer = (flags & PF_EXCHANGE_WRITER) ? n.writer.as<uint8_t>() : nullptr;
   }

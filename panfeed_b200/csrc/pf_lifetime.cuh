@@ -268,7 +268,7 @@ extern "C" void pf_destroy(pf_ctx* ctx) {
   for (PatternSpace* s : {&ctx->kp, &ctx->cp}) pool_free(s->pool);
   for (PatternSpace* s : {&ctx->kp, &ctx->cp})
     for (DevBuf* b : {&s->table, &s->x_owner, &s->x_pos, &s->x_perm, &s->x_counts, &s->x_unique,
-                      &s->x_table, &s->x_rep, &s->x_slot, &s->x_winner, &s->x_recv})
+                      &s->x_table, &s->x_rep, &s->x_slot, &s->x_winner})
       fd(*b);
   for (PinBuf* b : {&ctx->h_counters, &ctx->r_row_cluster, &ctx->r_row_kmer, &ctx->r_wrow_kmer, &ctx->r_row_count,
                     &ctx->r_row_pattern, &ctx->r_cl_pattern, &ctx->r_new_kp, &ctx->r_new_cp, &ctx->r_pos_kmer,

@@ -201,7 +201,7 @@ int upload_async_lite(pf_ctx* ctx, BatchState& B, const pf_batch* b, uint32_t rc
   TRY(dev_ensure(ctx, B.d_clusters, std::max<size_t>(1, nc) * sizeof(ClusterDev)));
   TRY(dev_ensure(ctx, B.d_presence, std::max<size_t>(1, (size_t)nc * W) * 4));
   TRY(dev_ensure(ctx, ctx->d_counters, C_COUNT * 4));
-  TRY(pin_ensure(ctx, ctx->h_counters, C_COUNT * 4 + 64 * 4));
+  TRY(pin_ensure(ctx, ctx->h_counters, C_COUNT * 4));
   TRY(dev_ensure(ctx, B.d_lite_tot, sizeof(LiteTotals)));
   TRY(pin_ensure(ctx, B.h_lite_tot, sizeof(LiteTotals)));
   CU(cudaMemcpyAsync(B.d_clusters.p, B.h_clusters.p, (size_t)nc * sizeof(ClusterDev), cudaMemcpyHostToDevice, st));
@@ -437,7 +437,7 @@ int upload_async(pf_ctx* ctx, BatchState& B, const pf_batch* full, const SubRang
   TRY(dev_ensure(ctx, B.d_clusters, std::max<size_t>(1, b->n_clusters) * sizeof(ClusterDev)));
   TRY(dev_ensure(ctx, B.d_presence, std::max<size_t>(1, (size_t)b->n_clusters * W) * 4));
   TRY(dev_ensure(ctx, ctx->d_counters, C_COUNT * 4));
-  TRY(pin_ensure(ctx, ctx->h_counters, C_COUNT * 4 + 64 * 4));
+  TRY(pin_ensure(ctx, ctx->h_counters, C_COUNT * 4));
   for (WidthState* w : widths) {
     TRY(dev_ensure(ctx, w->tiles, std::max<size_t>(1, w->n_tiles) * sizeof(TileDev)));
     TRY(dev_ensure(ctx, w->seg_start, std::max<size_t>(1, b->n_clusters) * 4));

@@ -145,21 +145,18 @@ class PatternStore:
     def finish_sharded(self, hash_pat, k, S, canonical, consider_missing, cluster_equal_filter, maf,
                        device, chunk=1 << 16):
         """After the last batch of a sharded run: the global pattern exchange
-        (dist.PatternExchange over NCCL), then the hashes_to_patterns rows of the patterns THIS
+        (dist.PatternExchange: pf_exchange_run over NCCL), then the hashes_to_patterns rows of the patterns THIS
         rank is the writer of (the owner of a pattern names the first rank that sent it), so
         that the ranks together write every pattern once - the job of the reference's single
         writer process and its `patterns` set (__main__.py:67-81, panfeed.py:210-212)."""
         import torch
         from . import dist as pfdist
         ctx = self.context(k, S, canonical, consider_missing, cluster_equal_filter, maf, device)
-        # (a context may bring its own exchange primitives and device: the CPU tests' stand-in does)
-        dev = getattr(ctx, "exchange_device", None) or torch.device("cuda", device)
-        backend = ctx.exchange_backend() if hasattr(ctx, "exchange_backend") else None
-        if os.environ.get("PF_EXCHANGE_IMPL", "") == "native":
-            # the whole exchange in one library call (pf_exchange_run) over torch.distributed
-            exchange = pfdist.NativePatternExchange(ctx, dev)
+        # (a context may bring its own exchange: the CPU tests' stand-in does)
+        if hasattr(ctx, "exchange"):
+            exchange = ctx.exchange(device)
         else:
-            exchange = pfdist.PatternExchange(ctx, dev, backend=backend)
+            exchange = pfdist.PatternExchange(ctx, torch.device("cuda", device))
         out = exchange.run(want_writer=True)
         exchange.close()
         W = (S + 31) // 32

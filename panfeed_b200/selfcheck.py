@@ -2,8 +2,8 @@
 
 The reference keeps ONE `patterns` set in its single writer process
 (`/root/reference/panfeed/__main__.py:70`, `panfeed.py:210-212`); here every
-rank numbers its own patterns (K4) and `dist.PatternExchange` makes the
-numbering global over NCCL.  `check_exchange` proves, on the ranks and the
+rank numbers its own patterns (K4) and `dist.PatternExchange` (pf_exchange_run)
+makes the numbering global over NCCL.  `check_exchange` proves, on the ranks and the
 communicator that are actually running, that the global numbering is the one a
 single context over all clusters would produce:
 
@@ -13,6 +13,10 @@ single context over all clusters would produce:
   2. the global table holds every full (ternary) pattern exactly once;
   3. rank 0 runs ALL clusters of the sample through one context: the same
      number of patterns in both namespaces and the same set of full patterns.
+
+With more_clusters_per_rank, the same contexts then take that many clusters more per rank and
+the same PatternExchange runs again: the receive buffers the first exchange sized (and the
+other ranks mapped) have to grow, and the checks apply to the second result.
 
 Used by `bench.py` before the timed region at N > 1 and by
 `tests/test_gpu_multirank.py`; works at world size 1 too (degenerate routing).
@@ -34,15 +38,16 @@ def _gather(obj, world):
 
 
 def check_exchange(local_device, consider_missing, seed=20261018, n_samples=256,
-                   clusters_per_rank=6, gene_len=400, k=31, maf=0.01):
+                   clusters_per_rank=6, gene_len=400, k=31, maf=0.01, more_clusters_per_rank=0):
     """Raises AssertionError on any mismatch; returns the pattern counts."""
     world = dist.get_world_size() if dist.is_initialized() else 1
     rank = dist.get_rank() if dist.is_initialized() else 0
     dev = torch.device("cuda", local_device)
-    S, cpr = n_samples, clusters_per_rank
+    S, cpr, more = n_samples, clusters_per_rank, more_clusters_per_rank
     W = (S + 31) // 32
+    total = world * (cpr + more)
     hb = capi.synth_batch(local_device, seed, S, cpr, first_cluster=rank * cpr,
-                          total_clusters=world * cpr, gene_len=gene_len)
+                          total_clusters=total, gene_len=gene_len)
     ctx = capi.Context(k, S, consider_missing=consider_missing, maf=maf, device=local_device)
     ex = None
     try:
@@ -50,8 +55,18 @@ def check_exchange(local_device, consider_missing, seed=20261018, n_samples=256,
         ctx.collect()
         ex = PatternExchange(ctx, dev)
         out = ex.run(want_unique=True)
-        n_cl = ex.backend.n_local(1)
-        n_km = ex.backend.n_local(0)
+        grown = {}
+        if more:
+            grown = {"kmer_patterns_local_first_exchange": len(out["kmer"]["local_to_global"])}
+            ctx.submit(capi.synth_batch(local_device, seed, S, more, first_cluster=world * cpr + rank * more,
+                                        total_clusters=total, gene_len=gene_len))
+            ctx.collect()
+            out = ex.run(want_unique=True)
+        # the transport asked for: pf_exchange_run still falls back to the all-to-all on every rank
+        # when a peer buffer cannot be mapped
+        transport = "local copy" if world == 1 else "nccl all-to-all" if ex.no_peer else "peer memory"
+        n_cl = len(out["cluster"]["local_to_global"])
+        n_km = len(out["kmer"]["local_to_global"])
         local_cl = ctx.export_patterns(True, 0, n_cl)
         local_km = ctx.export_patterns(False, 0, n_km)
         l2g_cl = out["cluster"]["local_to_global"].cpu().numpy().astype(np.int64)
@@ -80,8 +95,8 @@ def check_exchange(local_device, consider_missing, seed=20261018, n_samples=256,
 
         # 3. one context over all clusters (rank 0)
         if rank == 0:
-            hb_all = capi.synth_batch(local_device, seed, S, cpr * world, first_cluster=0,
-                                      total_clusters=world * cpr, gene_len=gene_len)
+            hb_all = capi.synth_batch(local_device, seed, S, total, first_cluster=0,
+                                      total_clusters=total, gene_len=gene_len)
             one = capi.Context(k, S, consider_missing=consider_missing, maf=maf, device=local_device)
             try:
                 one.submit(hb_all)
@@ -98,7 +113,7 @@ def check_exchange(local_device, consider_missing, seed=20261018, n_samples=256,
         return {"world": world, "consider_missing": bool(consider_missing),
                 "cluster_patterns_global": int(len(glob_cl)), "kmer_patterns_global": int(len(glob_km)),
                 "kmer_patterns_local": int(n_km), "ok": True,
-                "transport": "peer memory" if ex.peer else ("nccl all-to-all" if world > 1 else "local copy")}
+                "transport": transport, **grown}
     finally:
         if ex is not None:
             ex.close()

@@ -199,69 +199,68 @@ class OracleContext:
     def close(self):
         pass
 
-    # ---- sharded runs: the pattern exchange over gloo with host primitives ----
-    @property
-    def exchange_device(self):
-        import torch
-        return torch.device("cpu")
-
-    def exchange_backend(self):
-        return HostExchangeBackend(self)
+    # ---- sharded runs: the pattern exchange over gloo on host arrays ----
+    def exchange(self, device):
+        return HostExchange(self)
 
 
-class HostExchangeBackend:
-    """pf_exchange_pack / dedup / unpack on host arrays (the all-to-all transport), over the
-    pattern pools of an OracleContext: lets `PatternStore.finish_sharded` and dist.PatternExchange
-    run their real choreography between CPU processes."""
+class HostExchange:
+    """The global numbering pf_exchange_run gives, on host arrays between CPU processes (gloo):
+    every rank's keys go to every rank (all_gather_object); owner = a hash of the full key mod
+    world; the first sender in rank order writes the pattern; global id = the owner's base + the
+    pattern's order at its owner.  Lets `PatternStore.finish_sharded` run between CPU processes
+    and returns what dist.PatternExchange.run returns."""
 
     def __init__(self, ctx):
-        self.ctx, self.consider_missing = ctx, ctx.consider_missing
-        self.perm, self.owner, self.uniq = {}, {}, {}
+        self.ctx = ctx
 
-    def _pool(self, ns):
-        rows = self.ctx._cp_rows if ns == 1 else self.ctx._kp_rows
-        w = self.ctx.W if ns == 1 else self.ctx.Wk
-        return np.stack(rows).astype(np.uint32) if rows else np.zeros((0, w), np.uint32)
-
-    def key_words(self, ns):
-        return self.ctx.W if ns == 1 else self.ctx.Wk
-
-    def n_local(self, ns):
-        return len(self.ctx._cp_rows if ns == 1 else self.ctx._kp_rows)
-
-    def pack(self, ns, world, mask_remap, send):
-        import torch
+    def _number(self, keys, world, rank):
         import zlib
-        keys = self._pool(ns)
-        if mask_remap is not None:
-            keys[:, -1] = mask_remap.numpy().astype(np.uint32)[keys[:, -1]]
-        owner = np.array([zlib.crc32(k.tobytes()) % world for k in keys], np.int64)
-        order = np.argsort(owner, kind="stable")
-        perm = np.empty(len(keys), np.int64)
-        perm[order] = np.arange(len(keys))
-        self.perm[ns], self.owner[ns] = perm, owner
-        send.copy_(torch.from_numpy(keys[order].astype(np.int32).reshape(send.shape)))
-        return [int((owner == r).sum()) for r in range(world)]
+        import torch.distributed as dist
+        every = [keys]
+        if dist.is_initialized():
+            every = [None] * world
+            dist.all_gather_object(every, keys)
+        at_owner = [{} for _ in range(world)]           # owner -> {key: (order, first sender)}
+        for r, rk in enumerate(every):
+            for k in rk:
+                b = k.tobytes()
+                d = at_owner[zlib.crc32(b) % world]
+                d.setdefault(b, (len(d), r))
+        n_owned = [len(d) for d in at_owner]
+        base = np.concatenate([[0], np.cumsum(n_owned)]).astype(np.int64)
+        l2g = np.zeros(len(keys), np.int32)
+        writer = np.zeros(len(keys), np.uint8)
+        for i, k in enumerate(keys):
+            b = k.tobytes()
+            o = zlib.crc32(b) % world
+            order, first = at_owner[o][b]
+            l2g[i] = base[o] + order
+            writer[i] = first == rank
+        owned = np.array([np.frombuffer(b, np.uint32) for b in at_owner[rank]], np.uint32).reshape(
+            n_owned[rank], keys.shape[1])
+        return l2g, writer, n_owned, int(base[rank]), owned
 
-    def dedup(self, ns, recv, unique_index, n_unique, keep_unique=False):
+    def run(self, want_unique=False, want_writer=False):
         import torch
-        keys = recv.numpy().astype(np.uint32)
-        seen, idx = {}, []
-        for k in keys:
-            first = k.tobytes() not in seen
-            u = seen.setdefault(k.tobytes(), len(seen))
-            idx.append(u - (1 << 31) if first else u)        # bit 31: the first copy names the writer
-        unique_index.copy_(torch.tensor(idx, dtype=torch.int32))
-        self.uniq[ns] = np.array([np.frombuffer(b, np.uint32) for b in seen], np.uint32).reshape(len(seen), keys.shape[1])
-        n_unique.fill_(len(seen))
+        import torch.distributed as dist
+        world = dist.get_world_size() if dist.is_initialized() else 1
+        rank = dist.get_rank() if dist.is_initialized() else 0
+        out, cl_l2g = {}, None
+        for name, rows, w in (("cluster", self.ctx._cp_rows, self.ctx.W), ("kmer", self.ctx._kp_rows, self.ctx.Wk)):
+            keys = np.stack(rows).astype(np.uint32) if rows else np.zeros((0, w), np.uint32)
+            if name == "kmer" and self.ctx.consider_missing and len(keys):
+                keys[:, -1] = cl_l2g[keys[:, -1]]       # the NaN plane by its GLOBAL cluster-pattern id
+            l2g, writer, n_owned, base, owned = self._number(keys, world, rank)
+            if name == "cluster":
+                cl_l2g = l2g.astype(np.uint32)
+            out[name] = {"local_to_global": torch.from_numpy(l2g),
+                         "writer": torch.from_numpy(writer) if want_writer else None,
+                         "n_global": int(sum(n_owned)), "n_owned": n_owned[rank], "owned_base": base,
+                         "bytes_sent": int(keys.nbytes), "ms": {"total_both_namespaces": 0.0, "stages": None}}
+            if want_unique:
+                out[name]["owned_keys"] = owned
+        return out
 
-    def unique_keys(self, ns):
-        return self.uniq[ns]
-
-    def unpack(self, ns, returned, owner_base, l2g, writer):
-        import torch
-        v = returned[torch.from_numpy(self.perm[ns])].numpy().astype(np.int64) & 0xffffffff
-        base = owner_base.numpy().astype(np.int64)[self.owner[ns]]
-        l2g.copy_(torch.from_numpy(((v & 0x7fffffff) + base).astype(np.int32)))
-        if writer is not None:
-            writer.copy_(torch.from_numpy((v >> 31).astype(np.uint8)))
+    def close(self):
+        pass

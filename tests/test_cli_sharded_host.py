@@ -1,8 +1,8 @@
 """The sharded CLI (`torchrun -m panfeed_b200`, one process per GPU) on the CPU: two processes
 over gloo, each with the oracle-backed stand-in for its GPU context (tests/cpu_context.py) and
-host primitives for the pattern exchange.  Everything else is the product's own code: cluster
-sharding, per-rank piece files, `PatternStore.finish_sharded` (dist.PatternExchange: counts,
-keys to the owners, ids back, writer flags), the merge on rank 0.  The three files must equal
+a host model of the pattern exchange (its `exchange`, in place of dist.PatternExchange).
+Everything else is the product's own code: cluster sharding, per-rank piece files,
+`PatternStore.finish_sharded` (the writer flags, the hashes_to_patterns rows), the merge on rank 0.  The three files must equal
 the unmodified reference's goldens, as tests/test_gpu_multirank.py demands on real ranks."""
 import gzip
 import os

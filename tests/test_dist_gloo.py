@@ -1,20 +1,9 @@
-"""Host-side logic of the multi-GPU path on CPU: cluster sharding and the
-choreography of the global pattern dedup over gloo, for both transports of the
-keys - the all-to-all (world_size 2) and the peer-memory scatter (world_size 2 and
-3, with receive buffers that have to grow between exchanges).
-The device primitives (pf_exchange_*) are replaced by a numpy model HERE (test
-double only; the product has no CPU path): a "receive buffer another rank can
-map" is a file in a shared directory.  So the collective plumbing, bucket offsets,
-handle rounds, id bases and remap tables can be checked without a GPU."""
-import os
-import subprocess
-import sys
-
+"""Host-side logic of the multi-GPU path on CPU: the sharding of the clusters over the ranks.
+(The pattern exchange itself is the library's pf_exchange_run: tests/test_gpu_exchange_run.py and
+tests/test_gpu_multirank.py.)"""
 import numpy as np
 
 from panfeed_b200 import dist as pfdist
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def test_shard_clusters_balanced_and_complete():
@@ -26,199 +15,3 @@ def test_shard_clusters_balanced_and_complete():
         loads = [int(w[s].sum()) for s in shards]
         assert max(loads) - min(loads) <= int(w.max())
         assert all(s == sorted(s) for s in shards)
-
-
-WORKER = r'''
-import os, sys
-import numpy as np, torch, torch.distributed as dist
-sys.path.insert(0, sys.argv[1])
-from panfeed_b200 import dist as pfdist
-
-class NumpyBackend:
-    """Model of pf_exchange_pack/dedup/unpack on host arrays."""
-    def __init__(self, pools, consider_missing):
-        self.pools, self.consider_missing, self.perm, self.uniq = pools, consider_missing, {}, {}
-    def key_words(self, ns): return self.pools[ns].shape[1]
-    def n_local(self, ns): return self.pools[ns].shape[0]
-    def _keys(self, ns, mask_remap):
-        keys = self.pools[ns].copy()
-        if mask_remap is not None:
-            keys[:, -1] = mask_remap.numpy().astype(np.uint32)[keys[:, -1]]
-        return keys
-    def pack(self, ns, world, mask_remap, send):
-        keys = self._keys(ns, mask_remap)
-        owner = np.array([hash(k.tobytes()) % world for k in keys], dtype=np.int64) if len(keys) else np.zeros(0, np.int64)
-        order = np.argsort(owner, kind="stable")
-        perm = np.empty(len(keys), np.int64); perm[order] = np.arange(len(keys))
-        self.perm[ns] = perm
-        self.owner = getattr(self, "owner", {}); self.owner[ns] = owner
-        send.copy_(torch.from_numpy(keys[order].astype(np.int32).reshape(send.shape)))
-        return [int((owner == r).sum()) for r in range(world)]
-    def dedup(self, ns, recv, unique_index, n_unique, keep_unique=False):
-        if isinstance(recv, tuple):
-            keys = np.array(self.maps[recv[0]][:recv[1]], dtype=np.uint32)
-        else:
-            keys = recv.numpy().astype(np.uint32)
-        seen, idx = {}, []
-        for k in keys:
-            first = k.tobytes() not in seen
-            u = seen.setdefault(k.tobytes(), len(seen))
-            idx.append(u - (1 << 31) if first else u)        # bit 31 (int32): first copy = writer
-        unique_index.copy_(torch.tensor(idx, dtype=torch.int32))
-        self.uniq[ns] = np.array([np.frombuffer(b, np.uint32) for b in seen], dtype=np.uint32).reshape(len(seen), keys.shape[1])
-        n_unique.fill_(len(seen))
-    def unique_keys(self, ns): return self.uniq[ns]
-    # -- peer-memory primitives: receive buffers are .npy files in a shared directory, mapped
-    #    with np.load(mmap_mode="r+"); "pointers" index self.maps; a handle is the file name --
-    def classify(self, ns, world, mask_remap):
-        keys = self._keys(ns, mask_remap)
-        owner = np.array([hash(k.tobytes()) % world for k in keys], dtype=np.int64) if len(keys) else np.zeros(0, np.int64)
-        pos = np.zeros(len(keys), np.int64)
-        for r in range(world):
-            sel = np.nonzero(owner == r)[0]
-            pos[sel] = np.arange(len(sel))
-        self.cls = getattr(self, "cls", {}); self.cls[ns] = (keys, owner, pos)
-        self.owner = getattr(self, "owner", {}); self.owner[ns] = owner
-        return [int((owner == r).sum()) for r in range(world)]
-    def _register(self, arr):
-        self.maps = getattr(self, "maps", {}); self.next_ptr = getattr(self, "next_ptr", 1000) + 1
-        self.maps[self.next_ptr] = arr
-        return self.next_ptr
-    def recv_buffer(self, ns, min_rows):
-        self.bufs = getattr(self, "bufs", {}); self.gen = getattr(self, "gen", 0)
-        cur = self.bufs.get(ns)
-        if cur is None or cur[1] < min_rows:
-            if cur is not None:                      # the peers have closed their mappings by now
-                del self.maps[cur[0]]
-                os.unlink(os.path.join(SHARED, cur[2]))
-                self.regrown = getattr(self, "regrown", 0) + 1
-            self.gen += 1
-            name = f"recv_r{dist.get_rank()}_n{ns}_g{self.gen}.npy"
-            arr = np.lib.format.open_memmap(os.path.join(SHARED, name), mode="w+", dtype=np.uint32,
-                                            shape=(max(1, int(min_rows)), self.key_words(ns)))
-            self.bufs[ns] = (self._register(arr), max(1, int(min_rows)), name)
-        ptr, rows, name = self.bufs[ns]
-        return ptr, rows, name.encode().ljust(64, b"\0")
-    def open_peer(self, handle):
-        self.opened = getattr(self, "opened", 0) + 1
-        return self._register(np.load(os.path.join(SHARED, handle.rstrip(b"\0").decode()), mmap_mode="r+"))
-    def close_peer(self, mapped):
-        self.closed = getattr(self, "closed", 0) + 1
-        self.maps.pop(mapped).flush()
-    def scatter(self, ns, world, mask_remap, ptrs, row0):
-        keys, owner, pos = self.cls[ns]
-        assert np.array_equal(keys, self._keys(ns, mask_remap))
-        counts = [int((owner == r).sum()) for r in range(world)]
-        send0 = np.concatenate([[0], np.cumsum(counts)[:-1]]).astype(np.int64)
-        for e in range(len(keys)):
-            self.maps[ptrs[owner[e]]][row0[owner[e]] + pos[e]] = keys[e]
-        for a in self.maps.values():
-            a.flush()
-        self.perm[ns] = send0[owner] + pos if len(keys) else np.zeros(0, np.int64)
-    def unpack(self, ns, returned, owner_base, l2g, writer):
-        v = returned[torch.from_numpy(self.perm[ns])].numpy().astype(np.int64) & 0xffffffff
-        base = owner_base.numpy().astype(np.int64)[self.owner[ns]]
-        l2g.copy_(torch.from_numpy(((v & 0x7fffffff) + base).astype(np.int32)))
-        if writer is not None:
-            writer.copy_(torch.from_numpy((v >> 31).astype(np.uint8)))
-
-os.environ["PYTHONHASHSEED"] = "0"
-dist.init_process_group("gloo")
-rank, world = dist.get_rank(), dist.get_world_size()
-cm = sys.argv[2] == "1"
-peer = sys.argv[3] == "1"
-SHARED = sys.argv[4]
-rng = np.random.default_rng(7)            # same stream on every rank
-W = 3
-universe_c = rng.integers(0, 2**32, (6, W), dtype=np.uint64).astype(np.uint32)
-universe_k = rng.integers(0, 2**32, (40, W), dtype=np.uint64).astype(np.uint32)
-pick = np.random.default_rng(100 + rank)
-cl_all = universe_c[pick.choice(6, 4, replace=False)]
-rows = pick.choice(40, 25, replace=False)
-if cm:
-    kp_all = np.concatenate([universe_k[rows], pick.integers(0, 4, (25, 1)).astype(np.uint32)], axis=1)
-else:
-    kp_all = universe_k[rows]
-def gather(obj):
-    lst = [None] * world
-    dist.all_gather_object(lst, obj)
-    return lst
-be = NumpyBackend({}, cm)
-ex = pfdist.PatternExchange(None, torch.device("cpu"), backend=be, peer_memory=True if peer else None)
-assert ex.peer == peer
-ex.recv_slack_rows = 0          # (so that 25 patterns after 8 outgrow the buffers)
-# three exchanges on growing pattern pools (as pf_reset_patterns / further batches give): the
-# receive buffers of the peer-memory transport are mapped once, reused, and regrown
-for n_k in (8, 8, 25):
-    cl_local, kp_local = cl_all, kp_all[:n_k]
-    be.pools = {pfdist.CLUSTER: cl_local, pfdist.KMER: kp_local}
-    out = ex.run(want_unique=True, want_writer=True)
-    cl_g = out["cluster"]["local_to_global"].numpy()
-    km_g = out["kmer"]["local_to_global"].numpy()
-    true_k = kp_local.copy()
-    if cm:
-        true_k[:, -1] = cl_g[kp_local[:, -1]]
-    all_cl = gather((cl_local, cl_g, out["cluster"]["owned_keys"], out["cluster"]["owned_base"], out["cluster"]["writer"].numpy()))
-    all_km = gather((true_k, km_g, out["kmer"]["owned_keys"], out["kmer"]["owned_base"], out["kmer"]["writer"].numpy()))
-    for name, allx, total in (("cluster", all_cl, out["cluster"]["n_global"]), ("kmer", all_km, out["kmer"]["n_global"])):
-        key_to_id = {}
-        for keys, ids, _, _, _ in allx:
-            for k, i in zip(keys, ids):
-                assert key_to_id.setdefault(k.tobytes(), int(i)) == int(i), name + ": same key, two ids"
-        assert len(set(key_to_id.values())) == len(key_to_id), name + ": two keys share an id"
-        assert sorted(key_to_id.values()) == list(range(total)), name + ": ids not dense"
-        # the owner's exported unique keys sit at owned_base + index
-        for _, _, owned, base, _ in allx:
-            for j, k in enumerate(owned):
-                assert key_to_id[k.tobytes()] == base + j
-        # every global pattern has exactly one writer over all ranks
-        written = [int(i) for _, ids, _, _, wr in allx for i, w in zip(ids, wr) if w]
-        assert sorted(written) == list(range(total)), name + ": writer flags"
-if peer:
-    assert ex.peer, "fell back to the all-to-all"
-    stats = gather((getattr(be, "opened", 0), getattr(be, "closed", 0), getattr(be, "regrown", 0)))
-    assert all(o >= 2 * (world - 1) for o, _, _ in stats), stats        # every peer buffer mapped, both namespaces
-    assert sum(g for _, _, g in stats) > 0 and sum(c for _, c, _ in stats) > 0, stats   # 8 -> 25 patterns: regrown
-    ex.close()
-    assert not any(ex._peer_maps.values())
-print(f"rank {rank} ok cm={cm} peer={peer} clusters={out['cluster']['n_global']} kmers={out['kmer']['n_global']}")
-dist.destroy_process_group()
-'''
-
-
-def _run(cm, peer=0, world=2, tmp_path=None):
-    import tempfile
-    with tempfile.NamedTemporaryFile("w", suffix=".py", delete=False) as f:
-        f.write(WORKER)
-        path = f.name
-    shared = tempfile.mkdtemp(prefix="pf_peer_")
-    env = dict(os.environ, PYTHONHASHSEED="0")
-    try:
-        r = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1",
-                            "--nproc-per-node", str(world), "--master-addr", "127.0.0.1",
-                            "--master-port", str(29540 + cm + 2 * peer + 4 * (world - 2)), path, ROOT, str(cm),
-                            str(peer), shared],
-                           capture_output=True, text=True, timeout=300, env=env)
-    finally:
-        os.unlink(path)
-        import shutil
-        shutil.rmtree(shared, ignore_errors=True)
-    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-3000:]
-    assert r.stdout.count(" ok ") == world, r.stdout
-
-
-def test_exchange_world2_gloo():
-    _run(0)
-
-
-def test_exchange_world2_gloo_consider_missing():
-    _run(1)
-
-
-def test_exchange_peer_memory_protocol_world2():
-    """Bucket offsets, handle rounds, cached mappings and the regrowth of a receive buffer."""
-    _run(0, peer=1)
-
-
-def test_exchange_peer_memory_protocol_world3_consider_missing():
-    _run(1, peer=1, world=3)

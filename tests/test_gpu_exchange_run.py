@@ -2,15 +2,14 @@
 
 Contexts own disjoint cluster shards and run the exchange from one host thread each over the
 in-process communicator (capi.LocalComm), on one GPU or on several; the invariants are those of
-test_gpu_exchange.py and selfcheck.check_exchange:
+selfcheck.check_exchange:
   * local key == the owner's unique key at the returned global id;
   * the global pattern sets equal those of ONE context that saw every cluster;
   * exactly one writer per distinct pattern across ranks;
   * n_global, n_owned and owned_base agree on every rank.
-Also: a C program driving the call from pthreads, and (two GPUs or more) real ranks over NCCL."""
+Also: a C program driving the call from pthreads.  Real ranks over NCCL: tests/test_gpu_multirank.py."""
 import os
 import subprocess
-import sys
 import threading
 
 import numpy as np
@@ -18,8 +17,7 @@ import pytest
 import torch
 
 import gpu_util  # noqa: F401  (path setup)
-from panfeed_b200 import capi, dist as pfdist
-from test_gpu_exchange import _submit
+from panfeed_b200 import capi, dist as pfdist, packer
 from test_gpu_parity import _random_items
 
 pytestmark = pytest.mark.gpu
@@ -27,6 +25,13 @@ pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 S, K = 48, 21
 FLAGS = capi.PF_EXCHANGE_WRITER | capi.PF_EXCHANGE_KEEP_UNIQUE
+
+
+def _submit(ctx, items, stroi, base):
+    pcs = [packer.PackedCluster(c, idx, pa, stroi) for c, idx, pa in items]
+    hb, _, _ = packer.pack_batch(pcs, list(range(base, base + len(items))))
+    ctx.submit(hb)
+    return ctx.collect()
 
 
 def _threads(world, fn, comm=None, timeout=600):
@@ -283,30 +288,3 @@ def test_c_program_runs_the_exchange_from_threads(tmp_path, world, spread):
     assert (int(got["kmer_global"]), int(got["cluster_global"])) == (km, cl)
     assert km > 0 and cl > 0
 
-
-# ---- real ranks (torchrun, NCCL) ----
-needs_two = pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs")
-
-
-@needs_two
-@pytest.mark.parametrize("mode", ["basic", "considermissing", "cm_nofilter_up", "secondpass"])
-def test_cli_ranks_native_exchange_match_reference(mode, tmp_path):
-    import helpers
-    import test_gpu_multirank as mr
-    extra = dict(mr.CASES)[mode]
-    out = str(tmp_path / "out")
-    args = ["-m", "panfeed_b200"] + list(helpers.modes()[mode]) + extra + ["--output", out]
-    mr._torchrun(args, 29710 + ["basic", "considermissing", "cm_nofilter_up", "secondpass"].index(mode),
-                 helpers.GOLDEN, extra_env={"PF_EXCHANGE_IMPL": "native"})
-    for name in helpers.FILES:
-        got = mr._read(os.path.join(out, name))
-        assert helpers.sorted_lines(got) == helpers.sorted_lines(helpers.golden(mode, name)), (mode, name)
-
-
-@needs_two
-@pytest.mark.parametrize("cm", [0, 1])
-def test_native_and_python_exchange_agree_on_real_ranks(cm, tmp_path):
-    import test_gpu_multirank as mr
-    script = os.path.join(ROOT, "tests", "exchange_native_rank.py")
-    r = mr._torchrun([script, str(cm)], 29720 + cm, ROOT)
-    assert "native == python" in r.stdout, r.stdout[-2000:]

@@ -7,9 +7,12 @@
     the same sorted comparison: its row order is nondeterministic);
   * `selfcheck.check_exchange`: local keys == the owners' keys under the returned global ids, no
     duplicate in the global tables, and the same pattern sets as ONE context over all clusters,
-    with and without the cluster-absent encoding.
+    with and without the cluster-absent encoding, for both transports of the keys; also after a
+    second exchange on the same contexts whose receive buffers, mapped by the other processes over
+    CUDA IPC, have to grow.
 """
 import gzip
+import json
 import os
 import subprocess
 import sys
@@ -118,8 +121,9 @@ from panfeed_b200 import selfcheck
 local = int(os.environ["LOCAL_RANK"])
 torch.cuda.set_device(local)
 dist.init_process_group("nccl", device_id=torch.device("cuda", local))
+more = int(sys.argv[5]) if len(sys.argv) > 5 else 0
 res = [selfcheck.check_exchange(local, cm, n_samples=int(sys.argv[2]), clusters_per_rank=int(sys.argv[3]),
-                                gene_len=int(sys.argv[4])) for cm in (False, True)]
+                                gene_len=int(sys.argv[4]), more_clusters_per_rank=more) for cm in (False, True)]
 if dist.get_rank() == 0:
     print("SELFCHECK " + json.dumps(res))
 dist.barrier()
@@ -142,6 +146,28 @@ def test_exchange_two_ranks_nccl(samples, clusters, gene_len, peer, tmp_path):
     print(line)
     if peer == "0":
         assert "nccl all-to-all" in line
+
+
+@needs_two
+@pytest.mark.parametrize("peer", ["1", "0"])
+def test_exchange_two_ranks_regrows_mapped_buffers(peer, tmp_path):
+    """One exchange, then twenty times the clusters on the same contexts and a second exchange with
+    the same PatternExchange: every owner's receive buffer (need * 5/4 + 1024 rows after the first
+    call) has to grow; with peer = 1 the other process has it mapped over CUDA IPC and must drop
+    and reopen its mapping.  The self-check then holds for the second result."""
+    path = tmp_path / "worker.py"
+    path.write_text(WORKER)
+    r = _torchrun([str(path), ROOT, "256", "2", "400", "40"], 29670 + int(peer), ROOT,
+                  extra_env={"PF_EXCHANGE_PEER": peer})
+    line = [x for x in r.stdout.splitlines() if x.startswith("SELFCHECK")][0]
+    print(line)
+    for res in json.loads(line[len("SELFCHECK "):]):
+        assert res["ok"]
+        assert res["transport"] == ("peer memory" if peer == "1" else "nccl all-to-all")
+        # (rank 0's patterns as the measure of every owner's need: the second call's exceeds the
+        #  first call's receive capacity)
+        first, second = res["kmer_patterns_local_first_exchange"], res["kmer_patterns_local"]
+        assert second > 1.25 * first + 1024, (first, second)
 
 
 def test_exchange_selfcheck_single_rank():

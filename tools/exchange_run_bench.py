@@ -1,12 +1,9 @@
 """Time pf_exchange_run (one library call per rank, one host thread per rank, in-process
-communicator) at world 2..N in ONE process, against dist.PatternExchange on the same contexts.
+communicator) at world 1..N in ONE process, for both transports of the keys.
 
 Every rank holds the patterns of config 2's shape (bench.py --config 2: 500 genomes, 4,000 gene
 clusters per rank of a 4,000*N-cluster synthetic pangenome, pf_synth batches).  Ranks go round-robin
-over the visible GPUs (--devices 1: all on cuda:0).  PatternExchange needs one process per rank
-(torch.distributed): in one process it runs at world 1, so its line is the time ONE rank's exchange
-takes through the Python choreography over its own patterns; the native call is timed at world 1 on
-the same context for the like-for-like number.  Prints one JSON line per measurement.
+over the visible GPUs (--devices 1: all on cuda:0).  Prints one JSON line per measurement.
 
     python tools/exchange_run_bench.py --max-world 4 [--clusters 4000] [--reps 3] [--devices N]
 """
@@ -23,7 +20,7 @@ sys.path.insert(0, ROOT)
 
 import torch  # noqa: E402
 
-from panfeed_b200 import capi, dist as pfdist  # noqa: E402
+from panfeed_b200 import capi  # noqa: E402
 
 SEED = 20261018 + 2          # bench.py config 2
 
@@ -97,19 +94,6 @@ def main():
             ms, n_global = timed(world, flags)
             print(json.dumps(dict(base, impl=name, world=world, ms_median=round(ms, 2),
                                   kmer_global=int(n_global))), flush=True)
-    # PatternExchange (Python choreography) at world 1 on rank 0's context
-    dev = torch.device("cuda", 0)
-    times = []
-    for _ in range(a.reps + 1):
-        torch.cuda.synchronize(0)
-        t0 = time.perf_counter()
-        ex = pfdist.PatternExchange(ctxs[0], dev)
-        out = ex.run(want_writer=True)
-        times.append((time.perf_counter() - t0) * 1e3)
-        ex.close()
-    print(json.dumps(dict(base, impl="python_PatternExchange", world=1,
-                          ms_median=round(sorted(times[1:])[len(times[1:]) // 2], 2),
-                          kmer_global=int(out["kmer"]["n_global"]))), flush=True)
     for c in ctxs:
         c.close()
 
