@@ -95,41 +95,33 @@ __device__ __forceinline__ uint32_t partial_row_count(const uint32_t* __restrict
   return cnt;
 }
 
-__global__ void plan_seq_lite(const SeqDev* __restrict__ seqs, uint32_t n, SeqLite* __restrict__ out) {
-  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  const SeqDev d = seqs[i];
-  SeqLite l;
-  l.word_off = (uint32_t)(d.base_off >> 5);
-  l.len = d.len;
-  l.sample_flags = d.sample | ((d.flags & 2u) ? 0x80000000u : 0u);
-  l.amb_word_off = (uint32_t)(d.amb_off >> 5);
-  out[i] = l;
-}
-
 // ---------------------------------------------------------------------------
-// Device-side planning of an upload ("lite" upload): the caller's pf_seq_desc array goes to the
-// device as it is and ONE kernel does what the host planner does per sequence - validation
-// (include/panfeed_b200.h: pf_seq_desc), rebasing to the sub-range, the 64-byte SeqDev and the
-// 16-byte SeqLite - plus the batch totals.  The host then touches no descriptor at all: with
-// several ranks sharing the host's cores the per-sequence planning (~15 ns per sequence and
-// thread) was what bounded the end-to-end rate.  Only the block engine can run from it (no
-// record offsets are computed); a batch that falls back to the record engine is re-planned on
-// the host from the device copy of the descriptors.
+// Device-side planning of an upload: the caller's pf_seq_desc array goes to the device as it is
+// and ONE kernel validates every descriptor (include/panfeed_b200.h: pf_seq_desc), rebases it to
+// the sub-range and writes the 64-byte SeqDev, the 16-byte SeqLite and the batch totals.  The host
+// touches no descriptor: with several ranks sharing the host's cores, per-sequence host planning
+// (~15 ns per sequence and thread) was what bounded the end-to-end rate.  The block engine runs
+// from this alone; a batch that runs a record width also needs record offsets and tile lists,
+// which plan_records (pf_upload.cuh) derives on the device from the SeqDev array.
 // ---------------------------------------------------------------------------
-struct LiteTotals {          // 64 bytes, zeroed (err = all ones) before the kernel
+struct PlanTotals {          // 128 bytes, zeroed (err = all ones) before plan_from_raw
   unsigned long long bases, windows, pos_windows;
   unsigned long long err;    // min over bad sequences of (index << 32 | code); ~0 = none
-  uint32_t pad[8];
+  // plan_records: totals of the per-sequence offsets (kOff* order), then per record width
+  // (narrow, wide, 256-bit) the largest cluster and the sort tiles, and the local-reduce tiles
+  uint32_t seq_tot[6], max_seg[3], n_tiles[3], n_ltiles;
+  uint32_t pad[11];
 };
-enum : uint32_t { kLiteErrCluster = 1, kLiteErrClusterOrder, kLiteErrSample, kLiteErrSampleOrder, kLiteErrPresence,
-                  kLiteErrAlign, kLiteErrPlane, kLiteErrStrand, kLiteErrAmbiguous, kLiteErrOrder };
+static_assert(sizeof(PlanTotals) == 128, "PlanTotals");
+enum : uint32_t { kPlanErrCluster = 1, kPlanErrClusterOrder, kPlanErrSample, kPlanErrSampleOrder, kPlanErrPresence,
+                  kPlanErrAlign, kPlanErrPlane, kPlanErrStrand, kPlanErrNoAmbPlane, kPlanErrAmbAlign,
+                  kPlanErrAmbPlane };
 
 __global__ void __launch_bounds__(256)
 plan_from_raw(const pf_seq_desc* __restrict__ raw, uint32_t n, uint32_t cluster_base, uint64_t base_rebase,
-              uint32_t n_clusters, uint32_t S, uint32_t W, const uint32_t* __restrict__ presence,
-              uint64_t plane_bases, int k, uint32_t emit_positions, SeqDev* __restrict__ out,
-              SeqLite* __restrict__ lite, LiteTotals* __restrict__ tot) {
+              uint64_t amb_rebase, uint32_t n_clusters, uint32_t S, uint32_t W, const uint32_t* __restrict__ presence,
+              uint64_t plane_bases, bool has_amb_plane, uint64_t amb_plane_symbols, int k, uint32_t emit_positions,
+              SeqDev* __restrict__ out, SeqLite* __restrict__ lite, PlanTotals* __restrict__ tot) {
   __shared__ unsigned long long s_sum[3][8];
   const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
   unsigned long long bases = 0, windows = 0, posw = 0;
@@ -138,30 +130,36 @@ plan_from_raw(const pf_seq_desc* __restrict__ raw, uint32_t n, uint32_t cluster_
     uint32_t err = 0;
     const uint32_t cluster = q.cluster - cluster_base;
     const uint64_t base_off = q.base_off - base_rebase;
-    if (q.cluster < cluster_base || cluster >= n_clusters) err = kLiteErrCluster;
-    else if (q.sample >= S) err = kLiteErrSample;
-    else if (!((presence[(size_t)cluster * W + (q.sample >> 5)] >> (q.sample & 31u)) & 1u)) err = kLiteErrPresence;
-    else if (q.base_off < base_rebase || (base_off & 63u)) err = kLiteErrAlign;
-    else if (base_off + q.len > plane_bases) err = kLiteErrPlane;
-    else if (q.strand != 1 && q.strand != -1) err = kLiteErrStrand;
-    else if (q.flags & PF_SEQ_AMBIGUOUS) err = kLiteErrAmbiguous;
+    const bool amb = (q.flags & PF_SEQ_AMBIGUOUS) != 0;
+    const uint64_t amb_off = amb ? q.amb_off - amb_rebase : 0;
+    if (q.cluster < cluster_base || cluster >= n_clusters) err = kPlanErrCluster;
+    else if (q.sample >= S) err = kPlanErrSample;
+    else if (!((presence[(size_t)cluster * W + (q.sample >> 5)] >> (q.sample & 31u)) & 1u)) err = kPlanErrPresence;
+    else if (q.base_off < base_rebase || (base_off & 63u)) err = kPlanErrAlign;
+    else if (base_off + q.len > plane_bases) err = kPlanErrPlane;
+    else if (q.strand != 1 && q.strand != -1) err = kPlanErrStrand;
+    else if (amb && !has_amb_plane) err = kPlanErrNoAmbPlane;
+    else if (amb && (amb_off & 31u)) err = kPlanErrAmbAlign;
+    else if (amb && amb_off + q.len > amb_plane_symbols) err = kPlanErrAmbPlane;
     else if (i) {
       const pf_seq_desc p = raw[i - 1];
-      if (q.cluster < p.cluster) err = kLiteErrClusterOrder;
-      else if (q.cluster == p.cluster && q.sample < p.sample) err = kLiteErrSampleOrder;
+      if (q.cluster < p.cluster) err = kPlanErrClusterOrder;
+      else if (q.cluster == p.cluster && q.sample < p.sample) err = kPlanErrSampleOrder;
     }
     if (err) {
       atomicMin(&tot->err, ((unsigned long long)i << 32) | err);
     } else {
       const bool target = emit_positions && (q.flags & PF_SEQ_TARGET);
       SeqDev d;
-      d.base_off = base_off; d.amb_off = 0; d.len = q.len; d.sample = q.sample; d.cluster = cluster;
-      d.flags = target ? 1u : 0u;
+      d.base_off = base_off; d.amb_off = amb_off; d.len = q.len; d.sample = q.sample; d.cluster = cluster;
+      d.flags = (target ? 1u : 0u) | (amb ? 2u : 0u);
       d.start = q.start; d.end = q.end; d.offset = q.offset; d.strand = q.strand;
       d.rec_off = 0; d.pos_off = 0; d.wrec_off = 0; d.pwide_off = 0;
       out[i] = d;
       SeqLite l;
-      l.word_off = (uint32_t)(base_off >> 5); l.len = q.len; l.sample_flags = q.sample; l.amb_word_off = 0;
+      l.word_off = (uint32_t)(base_off >> 5); l.len = q.len;
+      l.sample_flags = q.sample | (amb ? 0x80000000u : 0u);
+      l.amb_word_off = (uint32_t)(amb_off >> 5);
       lite[i] = l;
       const uint32_t nwin = q.len >= (uint32_t)k ? q.len - (uint32_t)k + 1u : 0u;
       bases = q.len; windows = nwin; posw = target ? nwin : 0u;

@@ -4,15 +4,26 @@
 namespace pf {
 // ---- planning helpers that run on the device (tile lists are pure functions of the
 //      per-cluster record ranges; generating them there saves host loops and H2D) -------
+__device__ __forceinline__ uint2 cluster_range(const ClusterDev& cd, int width /* 0 narrow, 1 wide, 2 256-bit */) {
+  return width == 2 ? make_uint2(cd.xrec_start, cd.xrec_end)
+                    : width ? make_uint2(cd.wrec_start, cd.wrec_end) : make_uint2(cd.rec_start, cd.rec_end);
+}
+// tiles of every cluster's record range of one width; scan_inplace turns them into tile bases
+__global__ void plan_tile_counts(const ClusterDev* __restrict__ clusters, uint32_t n_clusters, uint32_t tile_size,
+                                 int width, uint32_t* __restrict__ out) {
+  const uint32_t c = blockIdx.x * blockDim.x + threadIdx.x;
+  if (c >= n_clusters) return;
+  const uint2 r = cluster_range(clusters[c], width);
+  out[c] = (r.y - r.x + tile_size - 1) / tile_size;
+}
 __global__ void plan_expand_tiles(const ClusterDev* __restrict__ clusters, uint32_t n_clusters,
                                   const uint32_t* __restrict__ tile_base, uint32_t tile_size,
                                   int width /* record range: 0 narrow, 1 wide, 2 256-bit */,
                                   TileDev* __restrict__ tiles) {
   const uint32_t c = blockIdx.x;
   if (c >= n_clusters) return;
-  const ClusterDev& cd = clusters[c];
-  const uint32_t lo = width == 2 ? cd.xrec_start : width ? cd.wrec_start : cd.rec_start;
-  const uint32_t hi = width == 2 ? cd.xrec_end : width ? cd.wrec_end : cd.rec_end;
+  const uint2 r = cluster_range(clusters[c], width);
+  const uint32_t lo = r.x, hi = r.y;
   const uint32_t first = tile_base[c];
   const uint32_t n = (hi - lo + tile_size - 1) / tile_size;
   for (uint32_t i = threadIdx.x; i < n; i += blockDim.x) {
@@ -29,6 +40,73 @@ __global__ void plan_seq_rec_off(const SeqDev* __restrict__ seqs, uint32_t n_seq
   const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n_seqs) out[i] = seqs[i].rec_off;
   else if (i == n_seqs) out[i] = total;
+}
+// Record offsets (plan_records): every sequence's count of each field, exclusive scans of them
+// (scan_inplace, one per field; stride n + 1, the total lands behind each field), then the
+// offsets into SeqDev and the per-cluster record ranges.  Two-word k-mers (k > 32): every window
+// is a record of the 128-bit pipeline; the windows of a sequence with N/IUPAC symbols are ALSO
+// records of the 256-bit pipeline, whose offsets take the place of the narrow ones.
+enum : uint32_t { kOffRec, kOffWrec, kOffPos, kOffPwide, kOffWide, kOffPxwide, kOffFields };
+__global__ void plan_rec_counts(const SeqDev* __restrict__ seqs, uint32_t n, int k, uint32_t mult, bool long_k,
+                                uint32_t* __restrict__ cnt) {
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const SeqDev d = seqs[i];
+  const bool target = d.flags & 1u, amb = d.flags & 2u;
+  const uint32_t nwin = d.len >= (uint32_t)k ? d.len - (uint32_t)k + 1u : 0u, recs = nwin * mult;
+  const size_t st = (size_t)n + 1;
+  cnt[kOffRec * st + i] = !long_k || amb ? recs : 0u;          // narrow, or 256-bit at k > 32
+  cnt[kOffWrec * st + i] = amb || long_k ? recs : 0u;
+  cnt[kOffPos * st + i] = target ? nwin : 0u;
+  cnt[kOffPwide * st + i] = (amb || long_k) && target ? nwin : 0u;
+  cnt[kOffWide * st + i] = amb ? 1u : 0u;                      // -> index in the list of ambiguous sequences
+  cnt[kOffPxwide * st + i] = long_k && amb && target ? nwin : 0u;
+}
+__global__ void plan_rec_offsets(SeqDev* __restrict__ seqs, uint32_t n, bool long_k, const uint32_t* __restrict__ off,
+                                 uint32_t* __restrict__ wide_seqs, uint32_t* __restrict__ xpos_slot) {
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const size_t st = (size_t)n + 1;
+  SeqDev& d = seqs[i];
+  d.rec_off = off[kOffRec * st + i];
+  d.wrec_off = off[kOffWrec * st + i];
+  d.pos_off = off[kOffPos * st + i];
+  d.pwide_off = off[kOffPwide * st + i];
+  if (d.flags & 2u) {
+    const uint32_t w = off[kOffWide * st + i];
+    wide_seqs[w] = i;
+    if (long_k) xpos_slot[w] = off[kOffPxwide * st + i];   // first positional 256-bit slot
+  }
+}
+// one thread per cluster: its record range of every width (a cluster without sequences: empty, at
+// the start of the next one), the segment starts of the sort and the largest segment per width
+__global__ void plan_cluster_records(const SeqDev* __restrict__ seqs, uint32_t n, uint32_t n_clusters, bool long_k,
+                                     const uint32_t* __restrict__ off, ClusterDev* __restrict__ clusters,
+                                     uint32_t* __restrict__ seg_n, uint32_t* __restrict__ seg_w,
+                                     uint32_t* __restrict__ seg_x, PlanTotals* __restrict__ tot) {
+  const uint32_t c = blockIdx.x * blockDim.x + threadIdx.x;
+  if (c >= n_clusters) return;
+  auto lower = [&](uint32_t v) {              // first sequence with cluster >= v
+    uint32_t lo = 0, hi = n;
+    while (lo < hi) {
+      const uint32_t mid = (lo + hi) >> 1;
+      if (seqs[mid].cluster < v) lo = mid + 1; else hi = mid;
+    }
+    return lo;
+  };
+  const uint32_t s0 = lower(c), s1 = lower(c + 1);
+  const size_t st = (size_t)n + 1;
+  const uint32_t r0 = off[kOffRec * st + s0], r1 = off[kOffRec * st + s1];
+  const uint32_t w0 = off[kOffWrec * st + s0], w1 = off[kOffWrec * st + s1];
+  const uint32_t n0 = long_k ? 0u : r0, n1 = long_k ? 0u : r1, x0 = long_k ? r0 : 0u, x1 = long_k ? r1 : 0u;
+  ClusterDev& cd = clusters[c];
+  cd.rec_start = n0; cd.rec_end = n1;
+  cd.wrec_start = w0; cd.wrec_end = w1;
+  cd.xrec_start = x0; cd.xrec_end = x1;
+  seg_n[c] = n0; seg_w[c] = w0; seg_x[c] = x0;
+  if (n1 > n0) atomicMax(&tot->max_seg[0], n1 - n0);
+  if (w1 > w0) atomicMax(&tot->max_seg[1], w1 - w0);
+  if (x1 > x0) atomicMax(&tot->max_seg[2], x1 - x0);
 }
 // Counter read-back without a copy engine: the D2H engine may be busy with the previous
 // batch's rows, and a 64-byte memcpy queued behind them would stall the pipeline's host side.
@@ -113,8 +191,7 @@ struct WidthState {       // per key width (narrow u64 / wide Key128 / Key256)
   DevBuf keys[2], vals[2];
   DevBuf tiles, seg_start, seg_hist, lookback, cursors;
   DevBuf ltiles, tile_first_run;     // partition mode: 2048-record tiles of the local reduce
-  PinBuf h_tiles, h_seg_start, h_ltiles;       // h_tiles / h_ltiles now hold per-cluster tile bases
-  DevBuf d_tile_base, d_ltile_base;
+  DevBuf d_tile_base, d_ltile_base;  // [n_clusters + 1] first sort / local-reduce tile of every cluster
   uint32_t n_tiles = 0, n_ltiles = 0, max_seg = 0;
   uint32_t n_records = 0;
   uint32_t n_runs = 0;
@@ -136,9 +213,10 @@ struct BatchState {
   uint32_t n_seqs = 0, n_clusters = 0, n_wide_seqs = 0;
   uint64_t n_words = 0, n_amb_words = 0, n_bases = 0;
   uint32_t n_pos = 0, n_pos_wide = 0, n_pos_xwide = 0;
-  PinBuf h_seqs, h_clusters, h_wide_seqs;
-  PinBuf h_xpos_slot;            // k > 32: first positional 256-bit slot of every listed ambiguous sequence
-  DevBuf d_bases, d_amb, d_ambbits, d_seqs, d_clusters, d_wide_seqs, d_presence, d_xpos_slot;
+  PinBuf h_clusters;
+  DevBuf d_bases, d_amb, d_ambbits, d_seqs, d_clusters, d_presence;
+  DevBuf d_wide_seqs;            // sequences with N/IUPAC symbols
+  DevBuf d_xpos_slot;            // k > 32: first positional 256-bit slot of every listed ambiguous sequence
   WidthState nar, wid;
   WidthState xwd;                // k > 32: the windows holding N/IUPAC symbols, Key256 records
   // rows (narrow first, then wide, then 256-bit)
@@ -147,8 +225,7 @@ struct BatchState {
   DevBuf d_pos_kmer, d_pos_seq, d_pos_cstart, d_pos_gstart, d_pos_flags, d_pos_wide, d_pos_xwide;
   DevBuf d_pos_bits;             // compact positional form: used_strand bit plane, indexed like d_bases
   DevBuf d_seq_rec_off, d_tile_first_seq;
-  PinBuf h_seq_rec_off, h_tile_first_seq;
-  std::vector<std::pair<uint32_t, uint32_t>> nar_ranges;   // narrow record range of every cluster
+  uint32_t local_tile = 0;       // records per tile of the local reduce (4096 direct / 2048 general)
   uint32_t n_items = 0;          // (cluster, block) work items of the batch (block aggregation)
   DevBuf d_seq_lite, d_cblk, d_item_base, d_item_cluster, d_plan_total, d_bsum_slot, d_slice_seq, d_item_desc;
   PinBuf h_plan;
@@ -161,23 +238,21 @@ struct BatchState {
   // the slot's result arrays have left the device
   cudaEvent_t ev_up_done = nullptr, ev_exec_end = nullptr, ev_out_done = nullptr;
   PinBuf h_done;                 // pinned mirror of the batch's new k-mer pattern count (K4)
-  // device-side planning ("lite" upload, plan_from_raw): the caller's descriptors as uploaded, the
-  // totals the kernel computed, and what a later fall-back to the record engine needs to re-plan
-  // the batch on the host
-  bool lite = false;
-  DevBuf d_raw, d_lite_tot;
-  PinBuf h_raw, h_lite_tot;
-  std::vector<pf_cluster_desc> lite_clusters;
-  std::vector<uint32_t> lite_presence;
-  const pf_seq_desc* lite_src = nullptr;     // caller's descriptors of the sub-range (valid during the call)
-  uint32_t lite_c0 = 0;                      // rebasing of the sub-range (cluster index, first base)
-  uint64_t lite_b0 = 0;
+  // planning (upload_async): the caller's descriptors as uploaded, the totals and offsets the
+  // planning kernels computed, and whether the slot has a block plan / record offsets and tiles
+  DevBuf d_raw, d_plan_tot, d_rec_off;
+  PinBuf h_raw, h_plan_tot;
+  bool blocks_planned = false, records_planned = false;
+  // the caller's sub-batch and its rebasing (cluster index, first base, first symbol), for
+  // describe_bad_seq; valid while the pf_upload / pf_submit call runs
+  pf_batch src{};
+  uint32_t src_c0 = 0;
+  uint64_t src_b0 = 0, src_a0 = 0;
 };
 
 
-// Host worker threads that stay alive with the context: the per-sequence planning of an upload
-// runs on them (a std::thread per chunk and phase cost more than the planning of a sub-batch),
-// and one of them enqueues the uploads of the pipelined submit.
+// Host worker threads that stay alive with the context: the pinned staging copy of a pageable
+// descriptor array runs on them (a std::thread per chunk cost more than the copy of a sub-batch).
 class WorkerPool {
  public:
   ~WorkerPool() {
@@ -301,7 +376,7 @@ struct pf_ctx : BatchState {
   uint32_t W = 0, Wk = 0;
   std::unordered_map<uint32_t, std::pair<uint32_t, uint32_t>> maf_cache;
   std::mutex maf_mu;       // the upload helper thread of the pipelined submit shares the cache
-  WorkerPool pool;         // planning threads
+  WorkerPool pool;         // staging-copy threads
   AsyncWorker uploader;    // enqueues the uploads of the pipelined submit
   AsyncWorker grower;      // maps more memory behind a pattern pool before it is needed
 
@@ -317,7 +392,6 @@ struct pf_ctx : BatchState {
   bool partition = true;   // mode 0: few radix passes + shared-memory hash grouping (k3_local)
   bool use_direct = true;  // S <= 1024: bitsets for every distinct key in shared memory
   bool runs_from_hist = false;   // one pass: prefix-runs are the digit buckets of the histogram
-  uint32_t local_tile = 0;       // records per tile of the local reduce (4096 direct / 2048 general)
   bool fused = false;            // K1 fused into the histogram and the first pass (no record write in K1)
   DevBuf d_digests;
   int extra_bits = 0;      // sort bits added after a table overflow (sticky)
@@ -376,7 +450,6 @@ struct pf_ctx : BatchState {
   uint32_t pipe_min_seqs = 200000;   // batches with fewer sequences are not split
   uint32_t pipe_target_seqs = 262144;   // sequences per sub-batch
   uint32_t pipe_first_seqs = 98304;     // ... of the first one (its upload is not hidden)
-  bool lite_ok = true;           // device-side planning of uploads (PF_LITE=0 disables; off after a record fall-back)
   XRunState* xrun = nullptr;     // created by the first pf_exchange_run
   AssocState assoc;
 };

@@ -768,7 +768,6 @@ extern "C" int pf_execute(pf_ctx* ctx) {
         } else {
           blk = false;
           if (++ctx->block_fallbacks >= 2) ctx->block_mode = false;
-          TRY(replan_full(ctx));            // (a device-planned upload has no record offsets yet)
           TRY(ensure_records());
         }
         continue;
@@ -811,6 +810,9 @@ extern "C" int pf_execute(pf_ctx* ctx) {
       break;
     }
     // ---- K1 + K2 -------------------------------------------------------------
+    // (a slot uploaded for the block engine has no record offsets yet: after a fall-back, or when
+    //  block_mode went off while it was uploaded ahead)
+    if (!ctx->records_planned) TRY(plan_records_now(ctx, *ctx, st));
     ctx->fused = part && ctx->use_direct && N.passes <= 2 && !(ctx->prm.debug_flags & 1u);
     TRY(launch_k1(ctx));
     STAGE("k1_extract");
@@ -876,8 +878,10 @@ extern "C" int pf_execute(pf_ctx* ctx) {
         TRY(dev_ensure(ctx, N.seg_hist, std::max<size_t>(1, (size_t)ctx->n_clusters * N.passes * kRadix) * 4));
       } else if (ctx->use_direct) {
         ctx->use_direct = false;
-        TRY(plan_local_tiles(ctx, *ctx, st));
+        TRY(local_tiles_count(ctx, *ctx, st));
+        mirror_counters<<<1, 32, 0, st>>>(ctx->h_plan_tot.as<uint32_t>(), ctx->d_plan_tot.as<uint32_t>(), 32);
         CU(cudaStreamSynchronize(st));
+        TRY(local_tiles_finish(ctx, *ctx, st));
       } else {
         return fail(ctx, PF_ERR_INTERNAL, "local table overflow at 64 sorted bits");
       }

@@ -7,7 +7,7 @@
 
 // Threads a host-side entry point uses when its caller passes n_threads = 0: every core, or
 // PF_HOST_THREADS when that is set (several ranks of one box share the host's cores; the CLI
-// under torchrun sets it to cores / ranks, like the planning threads of pf_upload read it).
+// under torchrun sets it to cores / ranks, as the staging-copy threads of pf_upload read it).
 inline uint32_t pf_host_threads() {
   static const uint32_t n = []() {
     const char* e = getenv("PF_HOST_THREADS");

@@ -200,7 +200,6 @@ extern "C" int pf_create(pf_ctx** out, int device, const pf_params* p) {
     cudaFuncSetAttribute(kA_block_aggregate<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBlkMaxSmem);
     cudaFuncSetAttribute(kA_block_aggregate<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBlkMaxSmem);
   }
-  if (const char* e = getenv("PF_LITE")) ctx->lite_ok = atoi(e) != 0;
   ctx->row_ratio = std::min(1.0 / 48, 16.0 / (double)std::max<uint32_t>(1u, p->n_samples));
   const int k3_smem = (int)(8 * ctx->W * sizeof(uint32_t));
   if (k3_smem > 48 * 1024) {
@@ -235,17 +234,16 @@ extern "C" void pf_destroy(pf_ctx* ctx) {
                       &bs->d_row_pattern, &bs->d_cl_pattern, &bs->d_pos_kmer, &bs->d_pos_seq, &bs->d_pos_cstart,
                       &bs->d_pos_gstart, &bs->d_pos_flags, &bs->d_pos_wide, &bs->d_pos_bits, &bs->d_seq_rec_off,
                       &bs->d_tile_first_seq, &bs->d_seq_lite, &bs->d_cblk, &bs->d_item_base, &bs->d_item_cluster,
-                      &bs->d_plan_total, &bs->d_bsum_slot, &bs->d_slice_seq, &bs->d_item_desc, &bs->d_raw, &bs->d_lite_tot})
+                      &bs->d_plan_total, &bs->d_bsum_slot, &bs->d_slice_seq, &bs->d_item_desc, &bs->d_raw, &bs->d_plan_tot,
+                      &bs->d_rec_off})
       fd(*b);
     for (WidthState* w : {&bs->nar, &bs->wid, &bs->xwd}) {
       for (DevBuf* b : {&w->keys[0], &w->keys[1], &w->vals[0], &w->vals[1], &w->tiles, &w->seg_start,
                         &w->seg_hist, &w->lookback, &w->cursors, &w->ltiles, &w->tile_first_run,
                         &w->d_tile_base, &w->d_ltile_base})
         fd(*b);
-      fp(w->h_tiles); fp(w->h_seg_start); fp(w->h_ltiles);
     }
-    for (PinBuf* b : {&bs->h_seqs, &bs->h_clusters, &bs->h_wide_seqs, &bs->h_xpos_slot, &bs->h_seq_rec_off, &bs->h_tile_first_seq,
-                      &bs->h_plan, &bs->h_done, &bs->h_raw, &bs->h_lite_tot})
+    for (PinBuf* b : {&bs->h_clusters, &bs->h_plan, &bs->h_done, &bs->h_raw, &bs->h_plan_tot})
       fp(*b);
   }
   for (DevBuf* b : {&ctx->d_counters, &ctx->d_bsum, &ctx->d_cand, &ctx->d_row_cand, &ctx->d_cand_pattern, &ctx->d_rep, &ctx->d_slot_of, &ctx->d_winner,

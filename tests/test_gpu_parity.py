@@ -418,16 +418,15 @@ def test_synthetic_device_batch_matches_oracle():
     assert st["unique_kmers"] == want["n_unique"]
 
 
-@pytest.mark.parametrize("lite", ["1", "0"])
-def test_malformed_batches_are_refused_with_the_same_message(lite, monkeypatch):
-    """Descriptor validation runs on the device for the block engine (plan_from_raw) and on the
-    host otherwise (PF_LITE=0): both must refuse a malformed batch, naming the first bad sequence
-    with the same message, and leave the context usable."""
+@pytest.mark.parametrize("engine", ["block", "records"])
+def test_malformed_batches_are_refused_with_the_same_message(engine):
+    """Descriptor validation runs on the device (plan_from_raw), whether the context plans for the
+    block engine or plans record offsets at upload (debug_flags=2): a malformed batch is refused
+    with one message naming the first bad sequence, and the context stays usable."""
     from panfeed_b200 import capi
-    monkeypatch.setenv("PF_LITE", lite)
     S, C, L, k = 40, 3, 200, 31
     good = capi.synth_batch(0, 5, S, C, total_clusters=C, gene_len=L)
-    ctx = capi.Context(k, S, maf=0.01)
+    ctx = capi.Context(k, S, maf=0.01, debug_flags=ENGINES[engine]["debug_flags"])
     try:
         cases = []
         bad = capi.HostBatch(good.packed, good.seqs.copy(), good.clusters, good.presence.copy())
@@ -448,15 +447,58 @@ def test_malformed_batches_are_refused_with_the_same_message(lite, monkeypatch):
         j = int(np.nonzero(bad.seqs["cluster"] == 1)[0][3])       # a sequence inside cluster 1 claims cluster 0
         bad.seqs["cluster"][j] = 0
         cases.append((bad, f"seq {j}: clusters must be non-decreasing"))
+        # sequence 9 flagged as holding N/IUPAC symbols, against a 4-bit plane that covers it
+        n_sym = int(good.seqs["len"][9] + 63) // 64 * 64
+        for amb_off, amb_words, msg in ((16, n_sym // 16, "seq 9: amb_off must be a multiple of 32"),
+                                        (0, 1, "seq 9: symbols run past the 4-bit plane"),
+                                        (0, 0, "seq 9 is ambiguous but amb_codes is NULL")):
+            seqs = good.seqs.copy()
+            seqs["flags"][9] |= 2
+            seqs["amb_off"][9] = amb_off
+            amb = np.zeros(amb_words, np.uint64) if amb_words else None
+            cases.append((capi.HostBatch(good.packed, seqs, good.clusters, good.presence, amb), msg))
         for hb, msg in cases:
             with pytest.raises(capi.PfError) as e:
                 ctx.submit(hb)
-            assert msg in str(e.value), (msg, str(e.value))
+            assert str(e.value).split(": ", 1)[1] == msg, (msg, str(e.value))
         ctx.submit(good)
         r = ctx.collect()
         assert len(r["row_cluster"]) > 0
     finally:
         ctx.close()
+
+
+def _related_cluster(rng, S, L, name):
+    """Every sample carries one copy of one of three close founders: a position block holds a
+    few dozen distinct k-mers."""
+    comp = str.maketrans("ACGT", "TGCA")
+    anc = rng.choice(list("ACGT"), L)
+    founders = []
+    for _ in range(3):
+        f = anc.copy()
+        m = rng.random(L) < 0.02
+        f[m] = rng.choice(list("ACGT"), int(m.sum()))
+        founders.append("".join(f))
+    cluster = {}
+    for i in range(S):
+        q = founders[int(rng.integers(3))]
+        cluster[f"g{i:04d}"] = [ref_port.CutSeq(q, q.translate(comp), f"g{i:04d}_f", "c", 1, L, 1, 0)]
+    return (cluster, name, np.ones(S, dtype=int))
+
+
+def test_pipelined_submit_with_two_consecutive_fallbacks(monkeypatch):
+    """Sub-batches 1 and 2 fall back from the block engine to the records; the second fall-back
+    turns the block engine off for the context while sub-batch 3 has already been uploaded with a
+    block plan only.  That sub-batch must still run through the record engine, exactly."""
+    monkeypatch.setenv("PF_PIPELINE_SEQS", "1024")       # one 700-sequence cluster per sub-batch
+    rng = np.random.default_rng(24)
+    S, k = 700, 31
+    items = ([_related_cluster(rng, S, 200, "r0")]
+             + [_unrelated_cluster(rng, S, 80, f"u{i}") for i in range(2)]
+             + [_related_cluster(rng, S, 200, f"r{i}") for i in range(1, 4)])
+    out, want = _compare_with_oracle(items, set(), S, k, True, False, False, 0.0,
+                                     batch_clusters=len(items))
+    assert out["stats"]["sub_batches"] >= 4
 
 
 @pytest.mark.parametrize("canon", [True, False])

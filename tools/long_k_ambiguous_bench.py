@@ -5,9 +5,10 @@ through the 256-bit records).  One resident batch per step: pipelined submits ar
 (PF_PIPELINE_SEQS=0; batches with N/IUPAC symbols are never pipelined), so all variants take the
 same path.  400 clusters are 157,106 sequences, 1.9e8 windows.
 
-Reports the resident time per step from the library's CUDA events (pf_stats.ms_total) and the
-per-stage times, variants alternated --repeats times after a warm-up, the card's name and power
-limit read in the same run; then compares sampled clusters of the 10 % variant with the C oracle
+Reports the resident time per step from the library's CUDA events (pf_stats.ms_total), the
+per-stage times and a host wall clock around submit + collect (upload and planning included),
+variants alternated --repeats times after a warm-up, the card's name and power limit read in the
+same run; then compares sampled clusters of the 10 % variant with the C oracle
 (at maf 0, where the rows of the one-sample N windows survive).
 
     python tools/long_k_ambiguous_bench.py [--clusters 400] [--steps 5] [--repeats 3] [--out FILE]
@@ -90,10 +91,12 @@ def timed(ctx, hb, steps):
     rows = []
     for _ in range(steps):
         ctx.reset_patterns()
+        t0 = time.perf_counter()
         ctx.submit(hb)
         r = ctx.collect(copy=False)
+        wall_ms = (time.perf_counter() - t0) * 1e3          # host side included: upload, planning, D2H
         st = ctx.stats()
-        rows.append({s: float(st[s]) for s in STAGES} |
+        rows.append({s: float(st[s]) for s in STAGES} | {"wall_ms": wall_ms} |
                     {"rows": int(len(r["row_cluster"]) + len(r["wide_row_cluster"]) + len(r["xwide_row_cluster"])),
                      "xwide_rows": int(len(r["xwide_row_cluster"]))})
     return rows
@@ -196,6 +199,8 @@ def main():
             "ms_total_median_per_repeat": per_rep,
             "ms_total_median": float(np.median([x["ms_total"] for rr in reps for x in rr])),
             "stages_median": {s: float(np.median([x[s] for rr in reps for x in rr])) for s in STAGES},
+            "wall_ms_median": float(np.median([x["wall_ms"] for rr in reps for x in rr])),
+            "wall_ms_median_per_repeat": [float(np.median([x["wall_ms"] for x in rr])) for rr in reps],
             "rows": reps[0][0]["rows"], "xwide_rows": reps[0][0]["xwide_rows"]}
     acgt = out["results"]["acgt"]["ms_total_median"]
     for v in ("amb1", "amb10"):
